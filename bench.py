@@ -14,6 +14,7 @@ with the position list and the fetched vector still materialised, as the operato
 drives all N GPUs (host/query_shim.c), wall clock, every count and sum read back by the host.
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            engine arm
+  python bench.py ... --dump-outputs DIR                          + what the last timed step computed
   python bench.py --impl reference ...                           reference CPU arm
 N > 1 is launched by torchrun (one rank per GPU); total work is fixed (strong scaling).
 """
@@ -42,6 +43,7 @@ NOMINAL_GBS = 8000.0                # the ~8 TB/s per-GPU figure north_star quot
 # the e2e leg drives the table as 2 columns of 2 B rows (a reference column holds < 2^31 rows:
 # positions are int, src/query.c:94-95), each row-range sharded over the N GPUs by the shim
 E2E_PARTS, E2E_PART_ROWS = 2, 2_000_000_000
+DUMP_SAMPLE = 1 << 18                # list entries per shard that --dump-outputs keeps
 METRIC = "rows/sec for select+fetch+sum"
 UNIT = "rows/s"
 
@@ -358,6 +360,8 @@ def run_engine(args):
     peak, peak_src = measured_peak()
     hits_local = [int(r[2].to_host(1, np.int64)[0]) for r in res]
     par = chain_parity(eng, my_shards, res, shard_rows, lo, hi)     # before anything reuses `res`
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, my_shards, res, (g_sum, g_cnt, g_min, g_max), rank)
     mask_ms, fused_ms = [], []
     if timed_marks:
         for k in range(len(marked_steps)):
@@ -583,6 +587,28 @@ def chain_parity(eng, my_shards, res, shard_rows, lo, hi, window=1 << 22):
     return {"ok": ok, "detail": f"{len(my_shards)} shards x first {window} rows vs {kind}: {checked} tuples"}
 
 
+def dump_outputs(out_dir, my_shards, res, agg, rank):
+    """What the timed chain handed its caller in its last step, as float64 .npy files (exact: every
+    value is an integer below 2^53).  Per shard: `shard<s>_hits` (the length of the position list)
+    and `shard<s>_positions` / `shard<s>_values`, the entries of the position list and of the
+    fetched vector at DUMP_SAMPLE indices drawn with a seed fixed per shard (the whole lists when
+    they are shorter).  Rank 0 adds `aggregate`: [sum >> 32, sum & 0xffffffff, count, min, max]."""
+    os.makedirs(out_dir, exist_ok=True)
+    for i, s_ in enumerate(my_shards):
+        pos, val, cnt = res[i]
+        h = int(cnt.to_host(1, np.int64)[0])
+        idx = np.arange(h)
+        if h > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(SEED + s_).choice(h, DUMP_SAMPLE, replace=False))
+        np.save(os.path.join(out_dir, f"shard{s_}_hits.npy"), np.array([h], np.float64))
+        np.save(os.path.join(out_dir, f"shard{s_}_positions.npy"), pos.to_host(h)[idx].astype(np.float64))
+        np.save(os.path.join(out_dir, f"shard{s_}_values.npy"), val.to_host(h)[idx].astype(np.float64))
+    if rank == 0:
+        g_sum, g_cnt, g_min, g_max = agg
+        np.save(os.path.join(out_dir, "aggregate.npy"),
+                np.array([g_sum >> 32, g_sum & 0xFFFFFFFF, g_cnt, g_min, g_max], np.float64))
+
+
 def measure_e2e(args, eng, cols, shard_rows, lo, hi, world, dist, rank, expect):
     """The same chain through the reference-facing operator API -- the C host drop-in
     (host/query_shim.c -> libadb_query.so) called exactly as src/server.c:137-290 calls
@@ -679,7 +705,7 @@ def measure_e2e(args, eng, cols, shard_rows, lo, hi, world, dist, rank, expect):
                                                C.POINTER(C.c_size_t), C.POINTER(C.c_double)]
     sel_arr = (C.POINTER(q.Column) * len(hcols))(*[C.pointer(a) for a, _ in hcols])
     fet_arr = (C.POINTER(q.Column) * len(hcols))(*[C.pointer(b) for _, b in hcols])
-    steps = max(3, min(args.steps, 20))
+    steps = args.steps
     l0 = lib.adb_launch_count_all()
     tot_py, hits_py = step()                    # the Python spelling of the same chain, once
     c_sum, c_hits, c_sec = C.c_long(0), C.c_size_t(0), C.c_double(0.0)
@@ -1284,7 +1310,12 @@ def main():
                     help="debug (N = 1): run the last shard through the exchange-carrying chain kernel")
     ap.add_argument("--ops", action="store_true",
                     help="also time shared scan / index / join at the BASELINE config sizes")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="engine arm: after the timed steps, write what the chain computed in the last one "
+                         "to DIR as .npy files (a seeded sample of every shard's lists; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "engine" else args.warmup
     quiet_stdout()
     if args.impl == "reference":

@@ -4,6 +4,8 @@
 logic, C-ABI symbol checks.  `-m gpu` are the parity tests proper: they call the CUDA
 engine through its C-ABI and compare against the oracle.
 """
+import hashlib
+import json
 import os
 import sys
 
@@ -62,6 +64,97 @@ class PinnedOracle:
         return both
 
 
+REFERENCE_ANSWERS = os.path.join(ROOT, "tests", "golden", "reference_answers.json")
+
+
+def digest(x) -> str:
+    """128-bit digest of a call's arguments or answer: arrays by dtype, shape and bytes; ints,
+    floats (nan included), bools, None, bytes and tuples / lists of those by value."""
+    h = hashlib.sha256()
+
+    def feed(v):
+        if isinstance(v, np.ndarray):
+            a = np.ascontiguousarray(v)
+            h.update(b"a%s%s:" % (a.dtype.str.encode(), repr(a.shape).encode()))
+            h.update(a.tobytes())
+        elif isinstance(v, (tuple, list)):
+            h.update(b"(%d" % len(v))
+            for e in v:
+                feed(e)
+            h.update(b")")
+        elif v is None:
+            h.update(b"n")
+        elif isinstance(v, (bool, np.bool_)):
+            h.update(b"b%d" % bool(v))
+        elif isinstance(v, (int, np.integer)):
+            h.update(b"i%d" % int(v))
+        elif isinstance(v, (float, np.floating)):
+            h.update(b"f" + float(v).hex().encode())
+        elif isinstance(v, bytes):
+            h.update(b"y%d:" % len(v) + v)
+        elif isinstance(v, str):
+            feed(v.encode())
+        else:
+            raise TypeError(f"cannot digest {type(v).__name__}")
+    feed(x)
+    return h.hexdigest()[:32]
+
+
+class RecordedReference:
+    """The reference operators (oracle/_ref) as recorded in tests/golden/reference_answers.json:
+    for every call the tests make on them, a digest of the arguments maps to a digest of the
+    reference's answer.  Where oracle/_ref is not built, a call is answered by the restatement,
+    and that answer must have the recorded reference answer's digest -- so a test that compares
+    with the reference still does, bit for bit, on the inputs it was recorded with.
+
+    ADB_RECORD_REFERENCE=<file> records instead: the answers of oracle/_ref when it is built,
+    else of the restatement, are merged into <file> at the end of the session (the restatement's
+    answers were recorded at a commit where they equalled oracle/_ref's on every one of these
+    calls).  Copy the file over tests/golden/reference_answers.json to keep it."""
+
+    def __init__(self, impl, opt: str, answers: dict, recording: bool):
+        self._impl, self._opt, self._answers, self._recording = impl, opt, answers, recording
+
+    def __getattr__(self, name):
+        fn = getattr(self._impl, name)
+
+        def call(*a, **kw):
+            out = fn(*a, **kw)
+            key, got = digest((self._opt, name, a, sorted(kw.items()))), digest(out)
+            if self._recording:
+                assert self._answers.setdefault(key, got) == got, f"two answers recorded for one {name} call"
+            else:
+                want = self._answers.get(key)
+                assert want is not None, (f"no recorded reference answer for this {name} call: record one "
+                                          "with ADB_RECORD_REFERENCE where oracle/_ref is built")
+                assert got == want, f"the restatement's {name} differs from the reference's recorded answer"
+            return out
+        return call
+
+
+@pytest.fixture(scope="session")
+def _reference_answers():
+    record = os.environ.get("ADB_RECORD_REFERENCE")
+    answers = {}
+    if os.path.exists(record or REFERENCE_ANSWERS):
+        with open(record or REFERENCE_ANSWERS) as f:
+            answers = json.load(f)
+    yield answers, bool(record)
+    if record:
+        with open(record, "w") as f:
+            json.dump(dict(sorted(answers.items())), f, indent=0)
+            f.write("\n")
+
+
+def _reference(opt, answers):
+    from oracle import oracle
+    answers, recording = answers
+    r = oracle.reference(opt)
+    if r is not None and not recording:
+        return r
+    return RecordedReference(r or oracle.port(), opt, answers, recording)
+
+
 @pytest.fixture(scope="session")
 def port():
     from oracle import oracle
@@ -69,21 +162,13 @@ def port():
 
 
 @pytest.fixture(scope="session")
-def ref():
-    from oracle import oracle
-    r = oracle.reference("O2")
-    if r is None:
-        pytest.skip("oracle/_ref not built (reference sources absent)")
-    return r
+def ref(_reference_answers):
+    return _reference("O2", _reference_answers)
 
 
 @pytest.fixture(scope="session")
-def ref_o0():
-    from oracle import oracle
-    r = oracle.reference("O0")
-    if r is None:
-        pytest.skip("oracle/_ref not built (reference sources absent)")
-    return r
+def ref_o0(_reference_answers):
+    return _reference("O0", _reference_answers)
 
 
 @pytest.fixture

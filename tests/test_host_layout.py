@@ -4,9 +4,8 @@ export the whole operator API.  CPU-only."""
 import ctypes as C
 import os
 import subprocess
+import sys
 import tempfile
-
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF_INC = "/root/reference/src/include"
@@ -51,11 +50,15 @@ def test_stand_in_types_have_the_expected_layout():
     assert out["Column.data"] == "64" and out["Column.row_count"] == "80" and out["Column.index"] == "96"
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_INC), reason="reference headers absent on this host")
 def test_stand_in_types_match_the_reference_headers():
+    """tests/golden/reference_layout.txt is the probe's output compiled against the reference's
+    own headers (recorded from the stand-ins at a commit where the two outputs were equal); where
+    the reference headers are present the probe is compiled against them as well."""
     mine = _run_probe([])
-    theirs = _run_probe(["-DADB_WITH_REFERENCE_HEADERS", "-I" + REF_INC])
-    assert mine == theirs
+    with open(os.path.join(ROOT, "tests", "golden", "reference_layout.txt")) as f:
+        assert mine == f.read()
+    if os.path.isdir(REF_INC):
+        assert mine == _run_probe(["-DADB_WITH_REFERENCE_HEADERS", "-I" + REF_INC])
 
 
 def test_ctypes_view_matches_the_header():
@@ -82,18 +85,24 @@ def test_operator_library_exports_the_whole_api():
     assert declared <= set(q.OPERATORS) | set(q.HOOKS), declared - set(q.OPERATORS) - set(q.HOOKS)
 
 
+NO_DEVICE_PROBE = r'''
+import ctypes as C
+import numpy as np
+import query_api as q
+api = q.Api()
+col = api.column(np.arange(10, dtype=np.int32))
+st = q.Status(99, None)
+lo = C.c_int(1)
+assert not api.lib.select_column(C.byref(col), C.byref(lo), None, C.byref(st))
+assert st.code == q.ERROR and b"no CPU fallback" in api.lib.adb_host_last_error()
+'''
+
+
 def test_operators_fail_loudly_without_a_device():
-    try:
-        import torch
-        if torch.cuda.is_available():
-            pytest.skip("GPU present")
-    except ImportError:
-        pass
-    import numpy as np
+    """In a process that sees no CUDA device (none visible on a GPU host either)."""
+    import analytical_database_b200 as adb
     import query_api as q
-    api = q.Api()
-    col = api.column(np.arange(10, dtype=np.int32))
-    st = q.Status(99, None)
-    lo = C.c_int(1)
-    assert not api.lib.select_column(C.byref(col), C.byref(lo), None, C.byref(st))
-    assert st.code == q.ERROR and b"no CPU fallback" in api.lib.adb_host_last_error()
+    if not os.path.exists(q.LIB):
+        adb.build_native()
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    subprocess.run([sys.executable, "-c", NO_DEVICE_PROBE], cwd=os.path.join(ROOT, "tests"), env=env, check=True)
