@@ -415,12 +415,6 @@ int launch_select_mask(const SelectArgs &a, bool with_total, cudaStream_t s);
 int launch_select_expand(const SelectArgs &a, cudaStream_t s);
 int launch_select_expand_fetch_agg(const SelectArgs &a, cudaStream_t s);     // a.out == a.val_out == NULL: aggregate only
 int launch_scan_gather_agg(const SelectArgs &a, cudaStream_t s);
-// sliced, overlapped form of mask + expand_fetch_agg (select_scan.cu); agg_scratch must hold
-// slices * ceil(chunks_per_slice / 8) partials, agg_ticket `slices` zeroed counters;
-// returns -1 when the geometry does not fit (caller uses the unsliced chain)
-int launch_chain_sliced(const SelectArgs &a, uint32_t slices, uint32_t chunks_per_slice, adb_agg *slice_parts,
-                        cudaStream_t main_s, cudaStream_t side_s, cudaEvent_t *mask_done, uint32_t *slices_used);
-constexpr int kChainMaxSlices = 16;
 size_t select_mask_words(uint32_t n, int sm_count);
 constexpr uint32_t kMaxSelectChunks = 1u << 16;
 
@@ -626,19 +620,14 @@ int launch_hj_expand(const uint2 *gc_by_j, const unsigned long long *warp_base, 
 
 // The join sharded over several contexts (SURVEY.md 8e): the build side is hash-partitioned
 // over the owners (adb_peer_exchange_pairs' routing hash), every owner builds the tables of its
-// share, and every context probes ITS probe rows -- in their original order -- against the
-// owner of each key over NVLink peer memory.  Output pairs then come out probe-major per
-// context, and the contexts' outputs concatenated in shard order are the reference's list.
+// share, and every context's probe rows -- in their original order -- are answered by the owner
+// of each key (the routed probe above).  Output pairs then come out probe-major per context, and
+// the contexts' outputs concatenated in shard order are the reference's list.  The expansion
+// reads a multi-row group's build positions from its owner over NVLink peer memory.
 struct JoinOwners {
-    const unsigned long long *toff[kMaxPeers];
-    const uint4 *table[kMaxPeers];
     const int32_t *bpos[kMaxPeers];                  // build positions sorted by hash (multi-row groups)
-    uint32_t part_bits[kMaxPeers];
     uint32_t route_bits;                             // owner = (key * 0x85EBCA6B) >> (32 - route_bits)
 };
-int launch_hj_probe_sharded(const uint32_t *pkeys, uint32_t n_probe, const HjProbeGeom &pg, const JoinOwners &owners,
-                            uint2 *gc_by_j, unsigned long long *warp_sums, unsigned long long *total,
-                            cudaStream_t s);
 int launch_hj_expand_sharded(const uint2 *gc_by_j, const unsigned long long *warp_base, const HjProbeGeom &pg,
                              uint32_t n_probe, const uint32_t *pkeys, const JoinOwners &owners,
                              const int32_t *probe_pos, int32_t *out_build, int32_t *out_probe, cudaStream_t s);

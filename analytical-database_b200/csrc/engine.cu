@@ -34,7 +34,11 @@ struct Engine {
     uint32_t *sel_mask = nullptr;
     size_t sel_mask_words = 0;
     uint32_t *sel_counts = nullptr;
-    // aggregate fold state
+    // aggregate fold state: one partial per CTA, and two self-re-arming tickets -- [0] for every
+    // grid-wide aggregate fold (one arrival per CTA), [1] for the count phase's fused total
+    // (mask_kernel<true>, one arrival per warp-chunk).  The fused count must not share a counter
+    // with the fold: each finds its last arrival by comparing the ticket it drew with its own
+    // number of arrivals, which only holds while no other kernel draws from the same counter.
     adb_agg *agg_scratch = nullptr;
     unsigned int *agg_ticket = nullptr;
     int64_t *idx_bounds = nullptr;      // {first, count} of the last index select
@@ -79,8 +83,9 @@ struct Engine {
         int32_t *build_pos_sorted = nullptr;   // all three live in the arena
         const int32_t *probe_pos = nullptr;
         bool swapped = false;
-        // sharded form (adb_join_build / adb_join_probe_sharded): this context's tables, read by
-        // every context's probe; the probe keys and the owner table for the expansion
+        // sharded form (adb_join_build ... adb_join_finish_routed): this context's tables, probed
+        // here for the keys every context routes to it; the probe keys and the owner table for the
+        // expansion
         bool built = false, sharded = false;
         uint32_t part_bits = 1;
         const unsigned long long *toff = nullptr;
@@ -97,10 +102,6 @@ struct Engine {
     // join tables: one open-addressing table per build partition, 16-byte slots (grow-only)
     void *hj_table = nullptr;
     unsigned long long hj_table_slots = 0;
-    // sharded join: local copies of the other contexts' partition -> slot-range tables (a probe
-    // then costs ONE remote read, the slot, instead of two dependent ones)
-    unsigned long long *toff_replica = nullptr;
-    size_t toff_replica_words = 0;
     // routed probe, owner side: the keys other contexts sent here and the answers (grow-only)
     uint32_t *rt32_pos = nullptr, *rt32_rows = nullptr, *rt32_val = nullptr;   // routed fetch (arena)
     uint32_t rt32_n = 0;
@@ -158,12 +159,6 @@ struct Engine {
     int64_t launches = 0;
     int32_t chain_mark_base = -1;       // adb_chain_marks(): slots for the next chain call
     bool peer_local = false;            // mailboxes mapped by peer access inside one process (no IPC handles)
-    // sliced chain (launch_chain_sliced): a higher-priority side stream for the expansions
-    cudaStream_t side = nullptr;
-    cudaEvent_t slice_ev[adb::kChainMaxSlices] = {};
-    cudaEvent_t side_done = nullptr;
-    adb_agg *slice_parts = nullptr;
-    int chain_slices = 0, chain_cps_div = 2;        // ADB_CHAIN_SLICES (0 = by size), ADB_CHAIN_CPS_DIV
     // Front cache of adb_alloc / adb_free.  Result buffers of one query shape come and go in
     // the same few sizes; cudaMallocAsync / cudaFreeAsync cost 5-10 us each (r02h: 14 + 2 x 18 us
     // per select -> fetch -> sum chain on 8 GPUs), a hit here is host bookkeeping.  Blocks keep
@@ -549,19 +544,9 @@ adb_status adb_init(int device_ordinal) {
             cudaGetLastError();                 // readbacks fall back to cudaMemcpyAsync
         }
     }
-    CU(cudaMalloc(&g.agg_scratch, sizeof(adb_agg) * adb::kAggMaxBlocks * adb::kChainMaxSlices));
-    CU(cudaMalloc(&g.agg_ticket, sizeof(unsigned int) * (adb::kChainMaxSlices + 1)));
-    CU(cudaMemset(g.agg_ticket, 0, sizeof(unsigned int) * (adb::kChainMaxSlices + 1)));
-    {
-        int lo_prio = 0, hi_prio = 0;
-        CU(cudaDeviceGetStreamPriorityRange(&lo_prio, &hi_prio));
-        CU(cudaStreamCreateWithPriority(&g.side, cudaStreamNonBlocking, hi_prio));
-        for (cudaEvent_t &e : g.slice_ev) CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        CU(cudaEventCreateWithFlags(&g.side_done, cudaEventDisableTiming));
-        CU(cudaMalloc(&g.slice_parts, sizeof(adb_agg) * adb::kChainMaxSlices));
-        if (const char *e = getenv("ADB_CHAIN_SLICES")) g.chain_slices = atoi(e);
-        if (const char *e = getenv("ADB_CHAIN_CPS_DIV")) g.chain_cps_div = atoi(e) > 0 ? atoi(e) : 1;
-    }
+    CU(cudaMalloc(&g.agg_scratch, sizeof(adb_agg) * adb::kAggMaxBlocks));
+    CU(cudaMalloc(&g.agg_ticket, sizeof(unsigned int) * 2));
+    CU(cudaMemset(g.agg_ticket, 0, sizeof(unsigned int) * 2));
     // every kernel of the engine is loaded here, per device: see preload_* (adb_common.cuh)
     adb::preload_csv_load(); adb::preload_format_text(); adb::preload_gather_agg(); adb::preload_hash_join();
     adb::preload_index_lookup(); adb::preload_peer_agg(); adb::preload_peer_exchange(); adb::preload_radix();
@@ -613,7 +598,6 @@ static adb_status shutdown_current() {
     cudaFree(g.sc_sums);
     cudaFree(g.arena);
     cudaFree(g.hj_table);
-    cudaFree(g.toff_replica);
     cudaFree(g.rt_recv_keys);
     cudaFree(g.rt_recv_res);
     cudaFree(g.fmt.block_len);
@@ -628,14 +612,10 @@ static adb_status shutdown_current() {
     cudaFree(g.csv.total);
     cudaFree(g.agg_scratch);
     cudaFree(g.agg_ticket);
-    cudaFree(g.slice_parts);
     for (int k = 0; k < Engine::kBlobSlots; ++k) {
         if (g.blob[k]) cudaFreeHost(g.blob[k]);
         if (g.blob_ev[k]) cudaEventDestroy(g.blob_ev[k]);
     }
-    if (g.side) { cudaStreamSynchronize(g.side); cudaStreamDestroy(g.side); }
-    for (cudaEvent_t &e : g.slice_ev) if (e) cudaEventDestroy(e);
-    if (g.side_done) cudaEventDestroy(g.side_done);
     if (g.mbox) cudaFreeHost(g.mbox);
     peer_close();
     for (int l = 0; l < g.stage_lanes; ++l) {
@@ -855,17 +835,6 @@ adb_status adb_mark_elapsed(int32_t from_slot, int32_t to_slot, float *ms) {
     return ADB_OK;
 }
 
-// slices: row slices per adb_chain_select_fetch_agg call (0 = by size: 4 from 2^26 rows, else 1);
-// cps_div: every slice's grid fills 1/cps_div of the machine (the rest is the other kernel's)
-adb_status adb_chain_config(int32_t slices, int32_t cps_div) {
-    NEED_UP();
-    if (slices < 0 || slices > adb::kChainMaxSlices || cps_div < 1 || cps_div > 8)
-        return fail(ADB_ERR_INVALID, "adb_chain_config: slices in [0, %d], cps_div in [1, 8]", adb::kChainMaxSlices);
-    g.chain_slices = slices;
-    g.chain_cps_div = cps_div;
-    return ADB_OK;
-}
-
 adb_status adb_chain_marks(int32_t base_slot) {
     NEED_UP();
     if (base_slot >= 0 && base_slot + 2 >= ADB_MAX_MARKS)
@@ -955,7 +924,7 @@ adb_status adb_select_count_base(const int32_t *d_col, int64_t n, const int32_t 
     // the host wants the count: the kernel that totals it also hands it over (no publish launch)
     const bool fused_pub = h_count && g.mbox && a.n > 0;
     if (fused_pub) { a.pub = g.mbox_dev; a.pub_seq = ++g.mbox_seq; }
-    a.mask_ticket = g.agg_ticket + adb::kChainMaxSlices;       // (a spare, zeroed counter next to the slices')
+    a.mask_ticket = g.agg_ticket + 1;
     if (adb_status s = after_launch("select_count", adb::launch_select_mask(a, true, g.stream))) return s;
     const unsigned long long seq = a.pub_seq;
     a.pub = nullptr; a.pub_seq = 0; a.mask_ticket = nullptr;
@@ -1492,28 +1461,6 @@ static adb_status chain_impl(const int32_t *d_sel_col, const int32_t *d_fetch_co
     // aggregates fused in (positions and values are still materialised)
     const int32_t mb = g.chain_mark_base;
     g.chain_mark_base = -1;
-    // Large shards: cut into row slices so that the predicate pass of slice k+1 overlaps the
-    // expansion + gather + aggregate of slice k (launch_chain_sliced).  Not when per-kernel
-    // marks were asked for (they need the two kernels back to back on one stream) and not for
-    // the exchange-carrying form.
-    // (r02: measured on 500 M-row shards, 0.415 ms sliced 4 x 1/2 against 0.418 ms plain -- the
-    // gather alone already moves 3.7 TB/s of 64-byte sectors, there is little idle bandwidth to
-    // fill; profiles/r02_chain_slices.md.  Kept selectable, off by default.)
-    uint32_t slices = g.chain_slices > 0 ? (uint32_t)g.chain_slices : 1u;
-    if (slices > (uint32_t)adb::kChainMaxSlices) slices = adb::kChainMaxSlices;
-    if (slices > 1 && mb < 0 && !px) {
-        const uint32_t wave = (uint32_t)g.sm_count * 8u * 8u;
-        uint32_t cps = wave / (uint32_t)g.chain_cps_div;
-        if (cps * slices > adb::kMaxSelectChunks) cps = adb::kMaxSelectChunks / slices;
-        uint32_t used = 0;
-        const int l_ = adb::launch_chain_sliced(a, slices, cps, g.slice_parts, g.stream, g.side, g.slice_ev, &used);
-        if (l_ > 0) {
-            int c_ = adb::launch_agg_combine(g.slice_parts, (int32_t)used, d_agg, g.side);
-            CU(cudaEventRecord(g.side_done, g.side));
-            CU(cudaStreamWaitEvent(g.stream, g.side_done, 0));
-            return after_launch("chain (sliced)", l_ + c_);
-        }
-    }
     if (mb >= 0) adb_mark(mb);
     int k_ = adb::launch_select_mask(a, false, g.stream);
     if (mb >= 0) adb_mark(mb + 1);
@@ -2288,9 +2235,9 @@ static adb_status join_count(const int32_t *bv, const int32_t *bp, int64_t nb64,
 
 // ---- the join sharded over the contexts of one process (SURVEY.md 8e) ----------------------------
 // Every context calls adb_join_build on its share of the build side (what adb_peer_exchange_pairs
-// delivered), the host waits for all of them, then every context calls adb_join_probe_sharded
-// with ITS probe rows and adb_join_emit_sharded.  The probe rows keep their original order, so
-// the contexts' outputs concatenated in shard order are the reference's probe-major list.
+// delivered), the host waits for all of them, then every context's probe rows go through the
+// routed probe below and adb_join_emit.  The probe rows keep their original order, so the
+// contexts' outputs concatenated in shard order are the reference's probe-major list.
 adb_status adb_join_build(const int32_t *d_v, const int32_t *d_p, int64_t n, int64_t probe_rows_hint) {
     NEED_UP();
     join_release();
@@ -2308,74 +2255,14 @@ adb_status adb_join_build(const int32_t *d_v, const int32_t *d_p, int64_t n, int
     return ADB_OK;
 }
 
-adb_status adb_join_probe_sharded(int32_t world, const int32_t *d_pv, const int32_t *d_pp, int64_t np64,
-                                  int32_t swapped, int64_t *h_matches) {
-    NEED_UP();
-    auto &j = g.join;
-    if (!j.built) return fail(ADB_ERR_INVALID, "adb_join_probe_sharded: no preceding adb_join_build on this context");
-    if (world < 1 || world > ADB_MAX_PEERS || (world & (world - 1)))
-        return fail(ADB_ERR_INVALID, "adb_join_probe_sharded: world %d must be a power of two <= %d", world, ADB_MAX_PEERS);
-    if (adb_status s = check_len(np64, "adb_join_probe_sharded")) return s;
-    if ((uint32_t)np64 > j.n_probe) return fail(ADB_ERR_INVALID, "adb_join_probe_sharded: more probe rows than adb_join_build reserved for");
-    if (np64 > 0 && (!d_pv || !d_pp)) return fail(ADB_ERR_INVALID, "adb_join_probe_sharded: NULL device pointer");
-    const uint32_t np = (uint32_t)np64;
-    adb::JoinOwners o{};
-    size_t replica_used = 0;
-    for (int r = 0; r < world; ++r) {
-        const Engine &E = g_ctx[r];
-        if (!E.up || !E.join.built) return fail(ADB_ERR_INVALID, "adb_join_probe_sharded: context %d has built no tables", r);
-        o.toff[r] = E.join.toff;
-        const size_t words = ((size_t)1 << E.join.part_bits) + 1;
-        if (&E != &g && np64 > 0 && replica_used + words <= g.toff_replica_words) {
-            // a local copy of the owner's (small) partition table: the probe's only remote read is the slot
-            unsigned long long *mine = g.toff_replica + replica_used;
-            if (E.device == g.device) CU(cudaMemcpyAsync(mine, E.join.toff, words * 8, cudaMemcpyDeviceToDevice, g.stream));
-            else CU(cudaMemcpyPeerAsync(mine, g.device, E.join.toff, E.device, words * 8, g.stream));
-            o.toff[r] = mine;
-            replica_used += words;
-        }
-        o.table[r] = static_cast<const uint4 *>(E.hj_table);
-        o.bpos[r] = E.join.build_pos_sorted;
-        o.part_bits[r] = E.join.part_bits;
-    }
-    while ((1 << o.route_bits) < world) ++o.route_bits;
-    j.owners = o;
-    j.sharded = true;
-    j.swapped = swapped != 0;
-    j.n_probe = np;
-    j.probe_pos = d_pp;
-    j.probe_keys = reinterpret_cast<const uint32_t *>(d_pv);
-    j.matches = 0;
-    if (np == 0) {
-        j.ready = true;
-        if (h_matches) *h_matches = 0;
-        return ADB_OK;
-    }
-    int launches = 0;
-    unsigned long long *tot = ARENA_TAKE(unsigned long long, 2);
-    j.pg = adb::hj_probe_geom(np, g.sm_count);
-    j.gc_by_j = ARENA_TAKE(uint2, np);
-    j.warp_base = ARENA_TAKE(unsigned long long, j.pg.warps);
-    StageTrace tr;
-    launches += adb::launch_hj_probe_sharded(j.probe_keys, np, j.pg, o, j.gc_by_j, j.warp_base, tot, g.stream);
-    if (adb_status s = read_back(&j.matches, tot, sizeof(int64_t))) return s;
-    tr.lap("probe (peer table reads) + piece offsets");
-    if (adb_status s = after_launch("join_probe_sharded", launches)) return s;
-    if (j.matches >= (int64_t)1 << 31)
-        return fail(ADB_ERR_INVALID, "join produces %lld pairs on one context; the result must stay below 2^31",
-                    (long long)j.matches);
-    j.ready = true;
-    if (h_matches) *h_matches = j.matches;
-    return ADB_OK;
-}
-
-// ---- the sharded join's ROUTED probe -------------------------------------------------------------
-// adb_join_probe_sharded reads every remote key's slot over NVLink: 16 useful bytes per 32-byte
-// response, 8.8 G reads/s per GPU -- 1.2 ms for the 11 M remote rows of an 8-GPU 100 M-row probe
-// (profiles/r02_join_sharded.md).  Routed instead: the keys travel to their owners in bulk
-// (4 bytes per row), the owner probes them against its own tables, the 8-byte answers travel
-// back in bulk, and the rows' home puts them back in row order (the same gather as the one-GPU
-// partitioned probe; cells = owners).  Steps, each on every context with a host barrier between:
+// ---- the sharded join's probe: keys routed to their owners ---------------------------------------
+// The keys travel to their owners in bulk (4 bytes per row), the owner probes them against its own
+// tables, the 8-byte answers travel back in bulk, and the rows' home puts them back in row order
+// (the same gather as the one-GPU partitioned probe; cells = owners).  Probing in place and reading
+// each remote key's slot over NVLink instead costs one 32-byte response per 16 useful bytes, 8.8 G
+// reads/s per GPU: 1.2 ms for the 11 M remote rows of an 8-GPU 100 M-row probe, and the whole
+// 100 M x 100 M join on 8 GPUs took 2.71 ms that way against 2.08 ms routed
+// (profiles/r02_join_sharded.md).  Steps, each on every context with a host barrier between:
 //   1. adb_join_route_probe     stable partition of my probe keys by owner; per-owner counts
 //   2. adb_join_recv_buffers + adb_copy_from_ctx per source + adb_join_probe_received
 //   3. adb_copy_from_ctx per owner into *d_answers + adb_join_finish_routed, then adb_join_emit
@@ -2521,10 +2408,7 @@ adb_status adb_join_finish_routed(int32_t world, const int32_t *d_pv, const int3
     for (int r = 0; r < world; ++r) {
         const Engine &E = g_ctx[r];
         if (!E.up || !E.join.built) return fail(ADB_ERR_INVALID, "adb_join_finish_routed: context %d has built no tables", r);
-        o.toff[r] = E.join.toff;
-        o.table[r] = static_cast<const uint4 *>(E.hj_table);
         o.bpos[r] = E.join.build_pos_sorted;
-        o.part_bits[r] = E.join.part_bits;
     }
     while ((1 << o.route_bits) < world) ++o.route_bits;
     j.owners = o;
@@ -2641,17 +2525,6 @@ adb_status adb_peer_exchange_reserve(int64_t send_pairs, int64_t build_pairs, in
                                      arena_round((size_t)(num_parts + 1) * 8) + join_partition_scratch(np) +
                                      join_owner_scratch(np) + kJoinSmallScratch))
         return s;
-    {
-        const size_t words = (size_t)ADB_MAX_PEERS * ((size_t)num_parts + 1);
-        if (words > g.toff_replica_words) {
-            CU(cudaStreamSynchronize(g.stream));
-            if (g.toff_replica) CU(cudaFree(g.toff_replica));
-            g.toff_replica = nullptr;
-            g.toff_replica_words = 0;
-            CU(cudaMalloc(&g.toff_replica, words * sizeof(unsigned long long)));
-            g.toff_replica_words = words;
-        }
-    }
     // tables: <= 2.5 slots per build row (power-of-two capacity at <= 80 % load) + 16 per partition
     const unsigned long long slots = (unsigned long long)nb * 5 / 2 + 16ull * num_parts + 4096;
     if (slots > g.hj_table_slots) {

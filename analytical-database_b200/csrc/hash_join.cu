@@ -22,9 +22,6 @@
 //      position to out2[off[j] ..]; long groups (skewed keys) are spread over a warp.
 // Partitions too large for the shared-memory table (heavy skew) build directly in their
 // global slots.
-#include <cstdlib>
-#include <cstring>
-
 #include "adb_common.cuh"
 
 namespace adb {
@@ -189,33 +186,33 @@ __device__ __forceinline__ uint32_t hj_mix(uint32_t tag) {
     return (uint32_t)(((unsigned long long)tag * 0x9E3779B97F4A7C15ull) >> 29);
 }
 
-// One CTA per partition.  Partitions whose slot range is at most HJ_SLOTS (<= 3276 build rows)
+// One CTA per partition.  Partitions whose slot range is at most HJ_BUILD_SLOTS (<= 1638 build rows)
 // build in shared memory in ONE phase -- every build row claims / finds its key's slot and
 // adds 1 to the size, the group leader (first row of the run of equal keys) adds its offset
 // in the same atomic -- and stream the finished table out.  Larger partitions (heavy skew)
 // run the same steps directly on their global slots.
 // CTA shape (r02za: 256 threads around a 4096-slot table = 32 KB kept 7 CTAs per SM resident
 // and the kernel, a string of dependent round trips per partition, ran at 2.9 TB/s): partitions
-// average <= 1024 rows, i.e. <= 2048 slots, so the default is 128 threads around 2048 slots
+// average <= 1024 rows, i.e. <= 2048 slots, so the CTA is 128 threads around 2048 slots
 // (16 KB, 14 CTAs per SM); the few larger partitions take the global-memory path.
-template <int THREADS, uint32_t SLOTS>
-__global__ void __launch_bounds__(THREADS)
+constexpr int HJ_BUILD_THREADS = 128;
+constexpr uint32_t HJ_BUILD_SLOTS = 2048;                // shared-memory table slots
+__global__ void __launch_bounds__(HJ_BUILD_THREADS)
 hj_table_build_kernel(const uint32_t *__restrict__ bkeys /* sorted by hash */,
                       const int32_t *__restrict__ bpos /* build positions in the same order */,
                       const uint32_t *__restrict__ off1, const unsigned long long *__restrict__ toff,
                       uint32_t part_bits, uint4 *__restrict__ table) {
-    constexpr uint32_t HJ_THREADS = THREADS, HJ_SLOTS = SLOTS;    // shared-memory table slots
-    __shared__ uint32_t s_tag[HJ_SLOTS];
-    __shared__ uint32_t s_gc[HJ_SLOTS];                 // {group start within the partition : 16, size : 16}
+    __shared__ uint32_t s_tag[HJ_BUILD_SLOTS];
+    __shared__ uint32_t s_gc[HJ_BUILD_SLOTS];           // {group start within the partition : 16, size : 16}
     const uint32_t p = blockIdx.x;
     const uint32_t b0 = off1[p], b1 = off1[p + 1];
     if (b1 == b0) return;                               // capacity 0: nothing to write
     const unsigned long long t0 = toff[p], cap64 = toff[p + 1] - t0;
-    if (cap64 <= HJ_SLOTS) {
+    if (cap64 <= HJ_BUILD_SLOTS) {
         const uint32_t cap = (uint32_t)cap64, mask = cap - 1;
-        for (uint32_t s = threadIdx.x; s < cap; s += HJ_THREADS) { s_tag[s] = 0u; s_gc[s] = 0u; }
+        for (uint32_t s = threadIdx.x; s < cap; s += HJ_BUILD_THREADS) { s_tag[s] = 0u; s_gc[s] = 0u; }
         __syncthreads();
-        for (uint32_t i = b0 + threadIdx.x; i < b1; i += HJ_THREADS) {
+        for (uint32_t i = b0 + threadIdx.x; i < b1; i += HJ_BUILD_THREADS) {
             const uint32_t k = bkeys[i];
             const bool leader = i == b0 || bkeys[i - 1] != k;
             const uint32_t tag = hj_tag(k, part_bits);
@@ -229,7 +226,7 @@ hj_table_build_kernel(const uint32_t *__restrict__ bkeys /* sorted by hash */,
         }
         __syncthreads();
         uint4 *__restrict__ out = table + t0;
-        for (uint32_t s = threadIdx.x; s < cap; s += HJ_THREADS) {
+        for (uint32_t s = threadIdx.x; s < cap; s += HJ_BUILD_THREADS) {
             const uint32_t w = s_gc[s], c = w & 0xFFFFu, gs = b0 + (w >> 16);
             const uint2 v = c ? hj_slot_value(gs, c, bpos) : make_uint2(0u, 0u);
             out[s] = make_uint4(s_tag[s], v.x, v.y, 0u);
@@ -238,10 +235,10 @@ hj_table_build_kernel(const uint32_t *__restrict__ bkeys /* sorted by hash */,
     }
     uint32_t *T = reinterpret_cast<uint32_t *>(table + t0);          // 4 words per slot
     const unsigned long long mask = cap64 - 1;
-    for (unsigned long long s = threadIdx.x; s < cap64; s += HJ_THREADS)
+    for (unsigned long long s = threadIdx.x; s < cap64; s += HJ_BUILD_THREADS)
         reinterpret_cast<uint4 *>(T)[s] = make_uint4(0u, 0u, 0u, 0u);
     __syncthreads();
-    for (uint32_t i = b0 + threadIdx.x; i < b1; i += HJ_THREADS) {
+    for (uint32_t i = b0 + threadIdx.x; i < b1; i += HJ_BUILD_THREADS) {
         const uint32_t k = bkeys[i];
         const bool leader = i == b0 || bkeys[i - 1] != k;
         const uint32_t tag = hj_tag(k, part_bits);
@@ -255,7 +252,7 @@ hj_table_build_kernel(const uint32_t *__restrict__ bkeys /* sorted by hash */,
         if (leader) T[4 * s + 1] = i;                    // only the leader writes this word
     }
     __syncthreads();
-    for (unsigned long long s = threadIdx.x; s < cap64; s += HJ_THREADS) {
+    for (unsigned long long s = threadIdx.x; s < cap64; s += HJ_BUILD_THREADS) {
         const uint32_t c = T[4 * s + 2];
         if (c == 1u || c == 2u) {
             const uint2 v = hj_slot_value(T[4 * s + 1], c, bpos);
@@ -677,62 +674,19 @@ hj_expand_kernel(const uint2 *__restrict__ gc_by_j, const unsigned long long *__
                    probe_pos, out_build, out_probe);
 }
 
-// ---- the same two kernels when the tables live on several contexts ------------------------------
+// ---- the expansion when the tables live on several contexts -------------------------------------
 // The owner table travels as a kernel parameter and is copied to shared memory once per CTA.
 struct HjOwnersShared {
-    const unsigned long long *toff[kMaxPeers];
-    const uint4 *table[kMaxPeers];
     const int32_t *bpos[kMaxPeers];
-    uint32_t part_bits[kMaxPeers];
 };
 __device__ __forceinline__ void hj_load_owners(const JoinOwners &o, HjOwnersShared &s) {
     if (threadIdx.x == 0)
 #pragma unroll
-        for (int k = 0; k < kMaxPeers; ++k) {
-            s.toff[k] = o.toff[k];
-            s.table[k] = o.table[k];
-            s.bpos[k] = o.bpos[k];
-            s.part_bits[k] = o.part_bits[k];
-        }
+        for (int k = 0; k < kMaxPeers; ++k) s.bpos[k] = o.bpos[k];
     __syncthreads();
 }
 __device__ __forceinline__ uint32_t hj_owner(uint32_t key, uint32_t route_bits) {
     return route_bits ? (key * 0x85EBCA6Bu) >> (32 - route_bits) : 0u;
-}
-
-__global__ void __launch_bounds__(HJ_THREADS)
-hj_probe_sharded_kernel(const uint32_t *__restrict__ pkeys, uint32_t n_probe, uint32_t rows_per_warp,
-                        const JoinOwners owners, uint2 *__restrict__ gc_by_j,
-                        unsigned long long *__restrict__ warp_sums) {
-    __shared__ HjOwnersShared so;
-    hj_load_owners(owners, so);
-    uint32_t j0, j1;
-    hj_warp_range(rows_per_warp, n_probe, &j0, &j1);
-    unsigned long long acc = 0;
-    for (uint32_t j = j0 + (threadIdx.x & 31); j < j1; j += kWarp) {
-        const uint32_t k = (uint32_t)ld_stream(reinterpret_cast<const int32_t *>(pkeys) + j);
-        const uint32_t w = hj_owner(k, owners.route_bits);
-        const uint32_t part_bits = so.part_bits[w];
-        const unsigned long long *__restrict__ toff = so.toff[w];
-        const uint32_t p = hj_pid(k, part_bits);
-        const unsigned long long t0 = toff[p], cap = toff[p + 1] - t0;      // (peer loads when w is remote)
-        uint2 r = make_uint2(0u, 0u);
-        if (cap) {
-            const uint4 *__restrict__ table = so.table[w];
-            const uint32_t tag = hj_tag(k, part_bits);
-            const unsigned long long mask = cap - 1;
-            unsigned long long s = hj_mix(tag) & mask;
-            while (true) {
-                const uint4 sl = ld_gather(table + t0 + s);
-                if (sl.x == tag) { r = make_uint2(sl.y, sl.z); break; }
-                if (sl.x == 0u) break;
-                s = (s + 1) & mask;
-            }
-        }
-        gc_by_j[j] = r;
-        acc += hj_matches(r.y);
-    }
-    hj_warp_sum_out(acc, warp_sums);
 }
 
 struct HjOwnerLists {
@@ -776,10 +730,7 @@ int launch_hj_geometry(const uint32_t *off1, uint32_t num_parts, unsigned long l
 int launch_hj_table_build(const uint32_t *bkeys, const int32_t *bpos, const uint32_t *off1,
                           const unsigned long long *toff, uint32_t num_parts, uint32_t part_bits,
                           uint4 *table, cudaStream_t s) {
-    static int wide = -1;                                  // ADB_HJ_TABLE_CTA=wide: the 256 x 4096 form
-    if (wide < 0) { const char *e = getenv("ADB_HJ_TABLE_CTA"); wide = e && !strcmp(e, "wide"); }
-    if (wide) hj_table_build_kernel<256, 4096><<<num_parts, 256, 0, s>>>(bkeys, bpos, off1, toff, part_bits, table);
-    else hj_table_build_kernel<128, 2048><<<num_parts, 128, 0, s>>>(bkeys, bpos, off1, toff, part_bits, table);
+    hj_table_build_kernel<<<num_parts, HJ_BUILD_THREADS, 0, s>>>(bkeys, bpos, off1, toff, part_bits, table);
     return 1;
 }
 
@@ -886,16 +837,6 @@ int launch_hj_expand(const uint2 *gc_by_j, const unsigned long long *warp_base, 
     return 1;
 }
 
-int launch_hj_probe_sharded(const uint32_t *pkeys, uint32_t n_probe, const HjProbeGeom &pg, const JoinOwners &owners,
-                            uint2 *gc_by_j, unsigned long long *warp_sums, unsigned long long *total,
-                            cudaStream_t s) {
-    if (n_probe == 0) return 0;
-    hj_probe_sharded_kernel<<<pg.blocks, HJ_THREADS, 0, s>>>(pkeys, n_probe, pg.rows_per_warp, owners, gc_by_j,
-                                                             warp_sums);
-    hj_sums_scan_kernel<<<1, 1024, 0, s>>>(warp_sums, pg.warps, total);
-    return 2;
-}
-
 int launch_hj_expand_sharded(const uint2 *gc_by_j, const unsigned long long *warp_base, const HjProbeGeom &pg,
                              uint32_t n_probe, const uint32_t *pkeys, const JoinOwners &owners,
                              const int32_t *probe_pos, int32_t *out_build, int32_t *out_probe, cudaStream_t s) {
@@ -908,7 +849,6 @@ int launch_hj_expand_sharded(const uint2 *gc_by_j, const unsigned long long *war
 // Load this file's kernels now (CUDA loads them lazily, on first launch): a first launch that
 // has to load code while another context's kernel spin-waits for this one can stall behind it.
 void preload_hash_join() {
-    preload_one(reinterpret_cast<const void *>(&hj_probe_sharded_kernel));
     preload_one(reinterpret_cast<const void *>(&hj_expand_sharded_kernel));
     preload_one(reinterpret_cast<const void *>(&hj_expand_kernel));
     preload_one(reinterpret_cast<const void *>(&hj_geometry_local_kernel));
@@ -920,8 +860,7 @@ void preload_hash_join() {
     preload_one(reinterpret_cast<const void *>(&hj_unpartition_routed_kernel));
     preload_one(reinterpret_cast<const void *>(&rows_unpartition32_kernel));
     preload_one(reinterpret_cast<const void *>(&hj_sums_local_kernel));
-    { auto *fp = &hj_table_build_kernel<128, 2048>; preload_one(reinterpret_cast<const void *>(fp)); }
-    { auto *fp = &hj_table_build_kernel<256, 4096>; preload_one(reinterpret_cast<const void *>(fp)); }
+    preload_one(reinterpret_cast<const void *>(&hj_table_build_kernel));
     preload_one(reinterpret_cast<const void *>(&hj_bounds_kernel));
 }
 

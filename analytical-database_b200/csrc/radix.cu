@@ -181,18 +181,16 @@ __global__ void rx_bucket_base_kernel(const uint32_t *__restrict__ totals_all, u
 // holds the offset of this rank's piece inside every destination buffer.  The run-contiguous
 // write-out is what makes the remote stores full 128-byte transactions.
 constexpr int RX_TILE = (int)kRadixTile;                 // rows per tile = CTA threads x keys per thread
-constexpr int RX_T_A = RX_TILE / 16 < 256 ? 256 : RX_TILE / 16 > 512 ? 512 : RX_TILE / 16;   // the default shape (16 keys per thread at 4096 rows)
-constexpr int RX_T_B = 2 * RX_T_A;                       // ADB_RX_THREADS=<this>: half the keys per thread
-constexpr int RX_DEFAULT_THREADS = RX_T_A;
-// CTA shape: T threads of 4096 / T keys each.  256 x 16: 64 registers, 56 KB -> 4 CTAs = 32 warps
-// per SM; 512 x 8: 40 registers, 60 KB -> 3 CTAs = 48 warps per SM (ADB_RX_THREADS picks; r02zc:
-// 13.8 vs 12.0 ms per 500 M pairs).  Other tile sizes (-DADB_RADIX_TILE, r02zn): 2048 rows x 8 keys
-// per thread 17.3 ms (runs of 8 rows, twice the histogram), 8192 rows x 512 threads 12.7 ms.
-template <int T>
+constexpr int RX_ST = RX_TILE / 16 < 256 ? 256 : RX_TILE / 16 > 512 ? 512 : RX_TILE / 16;   // scatter CTA threads (16 keys each at 4096 rows)
+constexpr int RX_KPT = RX_TILE / RX_ST, RX_SWARPS = RX_ST / kWarp;
+// CTA shape: 256 threads x 16 keys: 64 registers, 56 KB -> 4 CTAs = 32 warps per SM.  512 x 8 was
+// measured and dropped: 40 registers, 60 KB -> 3 CTAs = 48 warps per SM, but 13.8 vs 12.0 ms per
+// 500 M pairs (r02zc).  Other tile sizes (-DADB_RADIX_TILE, r02zn): 2048 rows x 8 keys per thread
+// 17.3 ms (runs of 8 rows, twice the histogram), 8192 rows x 512 threads 12.7 ms.
 struct RxShared {
     uint2 kv[RX_TILE];                                   // tile-sorted {key, payload}
     uint32_t pay_in[RX_TILE];                            // the tile's payloads in row order (cp.async)
-    uint16_t wcnt[T / kWarp][RX_BUCKETS];                // per-warp digit counts -> first slot of (warp, digit)
+    uint16_t wcnt[RX_SWARPS][RX_BUCKETS];                // per-warp digit counts -> first slot of (warp, digit)
     uint32_t gofs[RX_BUCKETS];                           // global address = gofs[d] + tile slot
     uint32_t ws[RX_BUCKETS / kWarp];
     uint32_t *peer[kMaxPeers];
@@ -206,13 +204,12 @@ __device__ __forceinline__ void cp_async_16(void *smem, const void *gmem) {
 }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;" ::: "memory"); }
 
-template <int T, int HASH, int BITS, bool REMOTE, bool FULL>
-__device__ __forceinline__ void rx_scatter_tile(RxShared<T> &sh, const uint32_t *__restrict__ keys,
+template <int HASH, int BITS, bool REMOTE, bool FULL>
+__device__ __forceinline__ void rx_scatter_tile(RxShared &sh, const uint32_t *__restrict__ keys,
                                                 const uint32_t *__restrict__ pay, uint32_t tile, uint32_t end,
                                                 const RadixPass &p, uint32_t my_off, uint32_t *__restrict__ keys_out,
                                                 uint32_t *__restrict__ pay_out, unsigned long long key_off,
                                                 unsigned long long pay_off) {
-    constexpr int RX_KPT = RX_TILE / T, RX_THREADS = T, RX_WARPS = T / kWarp;
     const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const RxDigit<HASH> digit(p);
     const uint32_t lt = (1u << lane) - 1u;
@@ -223,7 +220,7 @@ __device__ __forceinline__ void rx_scatter_tile(RxShared<T> &sh, const uint32_t 
         if (FULL && (reinterpret_cast<uintptr_t>(pay) & 15) == 0) {
 #pragma unroll
             for (int i = 0; i < RX_KPT / 4; ++i) {
-                const uint32_t q = (i * RX_THREADS + threadIdx.x) * 4;
+                const uint32_t q = (i * RX_ST + threadIdx.x) * 4;
                 cp_async_16(&sh.pay_in[q], pay + tile + q);
             }
         } else {
@@ -279,11 +276,11 @@ __device__ __forceinline__ void rx_scatter_tile(RxShared<T> &sh, const uint32_t 
     // 2. digit `threadIdx.x` (the first 256 threads): exclusive prefix over the warps, then over
     //    the digits
     {
-        const bool digit_thread = T == RX_BUCKETS || threadIdx.x < RX_BUCKETS;
-        uint32_t c[RX_WARPS], tot = 0;
+        const bool digit_thread = RX_ST == RX_BUCKETS || threadIdx.x < RX_BUCKETS;
+        uint32_t c[RX_SWARPS], tot = 0;
         if (digit_thread) {
 #pragma unroll
-            for (int w = 0; w < RX_WARPS; ++w) { c[w] = sh.wcnt[w][threadIdx.x]; tot += c[w]; }
+            for (int w = 0; w < RX_SWARPS; ++w) { c[w] = sh.wcnt[w][threadIdx.x]; tot += c[w]; }
         }
         const uint32_t incl = warp_incl_scan(tot, lane);
         if (digit_thread && lane == 31) sh.ws[warp] = incl;
@@ -296,7 +293,7 @@ __device__ __forceinline__ void rx_scatter_tile(RxShared<T> &sh, const uint32_t 
             sh.gofs[threadIdx.x] = my_off - tbase;          // modular: slot >= tbase for this digit
             uint32_t run = tbase;
 #pragma unroll
-            for (int w = 0; w < RX_WARPS; ++w) { sh.wcnt[w][threadIdx.x] = (uint16_t)run; run += c[w]; }
+            for (int w = 0; w < RX_SWARPS; ++w) { sh.wcnt[w][threadIdx.x] = (uint16_t)run; run += c[w]; }
         }
     }
     if (pay) cp_async_wait_all();
@@ -314,7 +311,7 @@ __device__ __forceinline__ void rx_scatter_tile(RxShared<T> &sh, const uint32_t 
     // 4. write out, run by run
     const uint32_t count = FULL ? (uint32_t)RX_TILE : end - tile;
 #pragma unroll 4
-    for (uint32_t slot = threadIdx.x; slot < count; slot += RX_THREADS) {
+    for (uint32_t slot = threadIdx.x; slot < count; slot += RX_ST) {
         const uint2 kv = sh.kv[slot];
         const uint32_t d = digit(kv.x);
         const uint32_t dst = sh.gofs[d] + slot;
@@ -329,8 +326,8 @@ __device__ __forceinline__ void rx_scatter_tile(RxShared<T> &sh, const uint32_t 
     }
 }
 
-template <int T, int HASH, int BITS, bool REMOTE>
-__global__ void __launch_bounds__(T, (RX_TILE / T >= 16 ? 1024 : 1536) / T)
+template <int HASH, int BITS, bool REMOTE>
+__global__ void __launch_bounds__(RX_ST, (RX_KPT >= 16 ? 1024 : 1536) / RX_ST)
 rx_scatter_kernel(const uint32_t *__restrict__ keys, const uint32_t *__restrict__ pay, uint32_t n,
                   RadixPass p, uint32_t seg_tiles, const uint32_t *__restrict__ hist,
                   const uint32_t *__restrict__ base,
@@ -338,7 +335,7 @@ rx_scatter_kernel(const uint32_t *__restrict__ keys, const uint32_t *__restrict_
                   uint32_t *const *__restrict__ peer_base, unsigned long long key_off,
                   unsigned long long pay_off, const uint32_t *__restrict__ abort_flag) {
     extern __shared__ __align__(16) unsigned char rx_smem[];
-    RxShared<T> &sh = *reinterpret_cast<RxShared<T> *>(rx_smem);
+    RxShared &sh = *reinterpret_cast<RxShared *>(rx_smem);
     if (REMOTE) {
         if (*abort_flag) return;                            // a receive region would overflow
         if (threadIdx.x < (1u << p.bits)) sh.peer[threadIdx.x] = peer_base[threadIdx.x];
@@ -346,14 +343,14 @@ rx_scatter_kernel(const uint32_t *__restrict__ keys, const uint32_t *__restrict_
     // next free global slot of digit `threadIdx.x` for this tile
     const uint32_t seg = blockIdx.x / seg_tiles, t = blockIdx.x - seg * seg_tiles;
     uint32_t my_off = 0;
-    if (T == RX_BUCKETS || threadIdx.x < RX_BUCKETS)
+    if (RX_ST == RX_BUCKETS || threadIdx.x < RX_BUCKETS)
         my_off = base[seg * RX_BUCKETS + threadIdx.x] +
                  hist[((size_t)seg * RX_BUCKETS + threadIdx.x) * seg_tiles + t];
     const uint32_t tile = blockIdx.x * RX_TILE;
     if (tile + RX_TILE <= n)
-        rx_scatter_tile<T, HASH, BITS, REMOTE, true>(sh, keys, pay, tile, n, p, my_off, keys_out, pay_out, key_off, pay_off);
+        rx_scatter_tile<HASH, BITS, REMOTE, true>(sh, keys, pay, tile, n, p, my_off, keys_out, pay_out, key_off, pay_off);
     else
-        rx_scatter_tile<T, HASH, BITS, REMOTE, false>(sh, keys, pay, tile, n, p, my_off, keys_out, pay_out, key_off, pay_off);
+        rx_scatter_tile<HASH, BITS, REMOTE, false>(sh, keys, pay, tile, n, p, my_off, keys_out, pay_out, key_off, pay_off);
 }
 
 // One CTA per 4096-row tile, launched in row order: the CTAs resident at any moment work on
@@ -369,46 +366,32 @@ RadixGeom radix_geom(uint32_t n, int sm_count) {
     return g;
 }
 
-template <int T>
-static void rx_set_attributes_shape() {
-    auto allow = [](auto *kernel) {
-        cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RxShared<T>));
-    };
-    allow(&rx_scatter_kernel<T, 0, 8, false>);
-    allow(&rx_scatter_kernel<T, 1, 8, false>);
-    allow(&rx_scatter_kernel<T, 0, 0, false>);
-    allow(&rx_scatter_kernel<T, 1, 0, false>);
-    allow(&rx_scatter_kernel<T, 2, 0, false>);
-    allow(&rx_scatter_kernel<T, 2, 0, true>);
-    allow(&rx_scatter_kernel<T, 3, 0, false>);
-}
 // function attributes are per device: once per device the engine launches on
 static void rx_set_attributes() {
     static bool done[64] = {};
     int dev = 0;
     cudaGetDevice(&dev);
     if (done[dev & 63]) return;
-    rx_set_attributes_shape<RX_T_A>();
-    rx_set_attributes_shape<RX_T_B>();
+    auto allow = [](auto *kernel) {
+        cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RxShared));
+    };
+    allow(&rx_scatter_kernel<0, 8, false>);
+    allow(&rx_scatter_kernel<1, 8, false>);
+    allow(&rx_scatter_kernel<0, 0, false>);
+    allow(&rx_scatter_kernel<1, 0, false>);
+    allow(&rx_scatter_kernel<2, 0, false>);
+    allow(&rx_scatter_kernel<2, 0, true>);
+    allow(&rx_scatter_kernel<3, 0, false>);
     done[dev & 63] = true;
 }
-static int rx_threads() {
-    static int t = 0;
-    if (!t) {
-        const char *e = getenv("ADB_RX_THREADS");
-        t = e && atoi(e) == RX_T_B ? RX_T_B : RX_DEFAULT_THREADS;
-    }
-    return t;
-}
 
-template <int T>
 static void rx_launch_scatter(uint32_t ctas, const uint32_t *keys_in, const uint32_t *pay_in, uint32_t n, RadixPass p,
                               uint32_t seg_tiles, const uint32_t *hist, const uint32_t *base, uint32_t *keys_out,
                               uint32_t *pay_out, cudaStream_t s) {
-    const size_t sm = sizeof(RxShared<T>);
+    const size_t sm = sizeof(RxShared);
 #define RX_LAUNCH(H, B)                                                                                      \
-    rx_scatter_kernel<T, H, B, false><<<ctas, T, sm, s>>>(keys_in, pay_in, n, p, seg_tiles, hist, base, keys_out, \
-                                                          pay_out, nullptr, 0, 0, nullptr)
+    rx_scatter_kernel<H, B, false><<<ctas, RX_ST, sm, s>>>(keys_in, pay_in, n, p, seg_tiles, hist, base, keys_out, \
+                                                           pay_out, nullptr, 0, 0, nullptr)
     if (p.hash == 0 && p.bits == 8) RX_LAUNCH(0, 8);
     else if (p.hash == 1 && p.bits == 8) RX_LAUNCH(1, 8);
     else if (p.hash == 0) RX_LAUNCH(0, 0);
@@ -461,10 +444,7 @@ int launch_radix_pass_segmented(const uint32_t *keys_in, const uint32_t *pay_in,
     else
         rx_row_scan_kernel<<<segs * RX_BUCKETS, 1024, 0, s>>>(hist, seg_tiles, g.ctas, totals);
     rx_bucket_base_kernel<<<segs, RX_BUCKETS, 0, s>>>(totals, base, seg_tiles * RX_TILE);
-    if (rx_threads() == RX_T_B)
-        rx_launch_scatter<RX_T_B>(g.ctas, keys_in, pay_in, n, p, seg_tiles, hist, base, keys_out, pay_out, s);
-    else
-        rx_launch_scatter<RX_T_A>(g.ctas, keys_in, pay_in, n, p, seg_tiles, hist, base, keys_out, pay_out, s);
+    rx_launch_scatter(g.ctas, keys_in, pay_in, n, p, seg_tiles, hist, base, keys_out, pay_out, s);
     return 4;
 }
 
@@ -494,12 +474,8 @@ int launch_radix_scatter_remote(const uint32_t *keys_in, const uint32_t *pay_in,
     if (p.hash != 2) return -1;                              // the routing hash is the only remote user
     rx_set_attributes();
     const RadixGeom g = radix_geom(n, sm_count);
-    if (rx_threads() == RX_T_B)
-        rx_scatter_kernel<RX_T_B, 2, 0, true><<<g.ctas, RX_T_B, sizeof(RxShared<RX_T_B>), s>>>(
-            keys_in, pay_in, n, p, g.ctas, hist, base, nullptr, nullptr, peer_base, key_off, pay_off, abort_flag);
-    else
-        rx_scatter_kernel<RX_T_A, 2, 0, true><<<g.ctas, RX_T_A, sizeof(RxShared<RX_T_A>), s>>>(
-            keys_in, pay_in, n, p, g.ctas, hist, base, nullptr, nullptr, peer_base, key_off, pay_off, abort_flag);
+    rx_scatter_kernel<2, 0, true><<<g.ctas, RX_ST, sizeof(RxShared), s>>>(
+        keys_in, pay_in, n, p, g.ctas, hist, base, nullptr, nullptr, peer_base, key_off, pay_off, abort_flag);
     return 1;
 }
 
@@ -588,16 +564,13 @@ void preload_radix() {
     preload_one(reinterpret_cast<const void *>(&rx_row_scan_kernel));
     preload_one(reinterpret_cast<const void *>(&rx_row_scan_warp_kernel));
     preload_one(reinterpret_cast<const void *>(&rx_bucket_base_kernel));
-#define RX_PRELOAD(T)                                                                                        \
-    { auto *fp = &rx_scatter_kernel<T, 0, 8, false>; preload_one(reinterpret_cast<const void *>(fp)); }         \
-    { auto *fp = &rx_scatter_kernel<T, 1, 8, false>; preload_one(reinterpret_cast<const void *>(fp)); }         \
-    { auto *fp = &rx_scatter_kernel<T, 0, 0, false>; preload_one(reinterpret_cast<const void *>(fp)); }         \
-    { auto *fp = &rx_scatter_kernel<T, 1, 0, false>; preload_one(reinterpret_cast<const void *>(fp)); }         \
-    { auto *fp = &rx_scatter_kernel<T, 2, 0, false>; preload_one(reinterpret_cast<const void *>(fp)); }         \
-    { auto *fp = &rx_scatter_kernel<T, 2, 0, true>; preload_one(reinterpret_cast<const void *>(fp)); }          \
-    { auto *fp = &rx_scatter_kernel<T, 3, 0, false>; preload_one(reinterpret_cast<const void *>(fp)); }
-    if (rx_threads() == RX_T_B) { RX_PRELOAD(RX_T_B) } else { RX_PRELOAD(RX_T_A) }
-#undef RX_PRELOAD
+    { auto *fp = &rx_scatter_kernel<0, 8, false>; preload_one(reinterpret_cast<const void *>(fp)); }
+    { auto *fp = &rx_scatter_kernel<1, 8, false>; preload_one(reinterpret_cast<const void *>(fp)); }
+    { auto *fp = &rx_scatter_kernel<0, 0, false>; preload_one(reinterpret_cast<const void *>(fp)); }
+    { auto *fp = &rx_scatter_kernel<1, 0, false>; preload_one(reinterpret_cast<const void *>(fp)); }
+    { auto *fp = &rx_scatter_kernel<2, 0, false>; preload_one(reinterpret_cast<const void *>(fp)); }
+    { auto *fp = &rx_scatter_kernel<2, 0, true>; preload_one(reinterpret_cast<const void *>(fp)); }
+    { auto *fp = &rx_scatter_kernel<3, 0, false>; preload_one(reinterpret_cast<const void *>(fp)); }
     preload_one(reinterpret_cast<const void *>(&sc_chunk_scan_kernel));
     preload_one(reinterpret_cast<const void *>(&sc_chunk_sum_kernel));
     rx_set_attributes();

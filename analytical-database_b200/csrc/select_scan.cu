@@ -101,9 +101,9 @@ template <bool TOTAL>
 __global__ void __launch_bounds__(SEL_THREADS)
 mask_kernel(const int32_t *__restrict__ val, const int64_t *__restrict__ d_n, uint32_t n_host,
             Range rg, uint32_t chunk_rows, uint32_t num_chunks, uint32_t *__restrict__ mask,
-            uint32_t *__restrict__ counts, bool stable_val, uint32_t chunk_offset, MaskTotal tot) {
+            uint32_t *__restrict__ counts, bool stable_val, MaskTotal tot) {
     const uint32_t lane = threadIdx.x & 31;
-    const uint32_t chunk = chunk_offset + blockIdx.x * SEL_WARPS + (threadIdx.x >> 5);
+    const uint32_t chunk = blockIdx.x * SEL_WARPS + (threadIdx.x >> 5);
     pdl_launch_dependents();
     if (chunk >= num_chunks) return;
     // Anything but a base column may be the output of the kernel this one was launched behind
@@ -210,14 +210,14 @@ __global__ void __launch_bounds__(SEL_THREADS)
 expand_kernel(const uint32_t *__restrict__ mask, const uint32_t *__restrict__ counts,
               uint32_t chunk_rows, uint32_t num_chunks, const int32_t *__restrict__ pos_in,
               int32_t base_pos, int32_t *__restrict__ out, int64_t *__restrict__ d_count,
-              const typename ChainOf<EXCH>::type chx, uint32_t chunk_offset, uint32_t chunk_end) {
+              const typename ChainOf<EXCH>::type chx) {
     const ChainArgs &ch = chain_of(chx);
     pdl_launch_dependents();
     pdl_wait();                                              // bitmap + counts come from mask_kernel
     __shared__ uint32_t s_red[SEL_WARPS];
     __shared__ int32_t s_stage[SEL_WARPS][kWarp * 32 * EXP_WORDS / 4];   // 1024 positions per warp
     const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const uint32_t first_chunk = chunk_offset + blockIdx.x * SEL_WARPS;
+    const uint32_t first_chunk = blockIdx.x * SEL_WARPS;
     const int32_t *__restrict__ fcol = ch.fetch_col;
     int32_t *__restrict__ vout = ch.val_out;
     AggAcc acc{0, INT32_MAX, INT32_MIN};
@@ -233,13 +233,13 @@ expand_kernel(const uint32_t *__restrict__ mask, const uint32_t *__restrict__ co
     for (int w = 0; w < SEL_WARPS; ++w) base += s_red[w];
     uint32_t my_count = 0;
     for (uint32_t w = 0; w < SEL_WARPS; ++w) {
-        const uint32_t c = first_chunk + w < chunk_end ? counts[first_chunk + w] : 0u;
+        const uint32_t c = first_chunk + w < num_chunks ? counts[first_chunk + w] : 0u;
         if (w < warp) base += c;
         if (w == warp) my_count = c;
     }
     const uint32_t chunk = first_chunk + warp;
     if (chunk == num_chunks - 1 && lane == 0) *d_count = (int64_t)base + my_count;
-    const bool active = chunk < chunk_end && my_count != 0;
+    const bool active = chunk < num_chunks && my_count != 0;
     if (!FETCH && !active) return;
 
     if (active) {
@@ -345,7 +345,7 @@ expand_kernel(const uint32_t *__restrict__ mask, const uint32_t *__restrict__ co
         }
     }
     if (FETCH) {
-        const bool last = agg_grid_fold<SEL_THREADS>(acc, lane == 0 && chunk < chunk_end ? (int64_t)my_count : 0,
+        const bool last = agg_grid_fold<SEL_THREADS>(acc, lane == 0 && chunk < num_chunks ? (int64_t)my_count : 0,
                                                      ch.agg_out, ch.agg_scratch, ch.agg_ticket);
         // multi-GPU: the CTA that completed this shard's aggregate folds the rank's partials and
         // exchanges them with every peer over NVLink (agg_out is one of px.parts: publish it first)
@@ -509,10 +509,10 @@ scan_gather_agg_kernel(const int32_t *__restrict__ val, const int32_t *__restric
 struct SelectGeom {
     uint32_t chunk_rows, num_chunks, grid;
 };
-static SelectGeom select_geom(uint32_t n, int sm_count, uint32_t max_chunks = 0) {
+static SelectGeom select_geom(uint32_t n, int sm_count) {
     SelectGeom g{};
     const uint32_t wtiles = (n + SEL_WTILE - 1) / SEL_WTILE;
-    if (max_chunks == 0) max_chunks = (uint32_t)sm_count * 8u * SEL_WARPS;      // 8 CTAs per SM resident
+    const uint32_t max_chunks = (uint32_t)sm_count * 8u * SEL_WARPS;             // 8 CTAs per SM resident
     uint32_t tiles_per_chunk = (wtiles + max_chunks - 1) / max_chunks;
     if (tiles_per_chunk == 0) tiles_per_chunk = 1;
     g.chunk_rows = tiles_per_chunk * SEL_WTILE;
@@ -523,9 +523,7 @@ static SelectGeom select_geom(uint32_t n, int sm_count, uint32_t max_chunks = 0)
 
 size_t select_mask_words(uint32_t n, int sm_count) {
     const SelectGeom g = select_geom(n, sm_count);
-    // room for the finer geometry of the sliced chain as well (up to kMaxSelectChunks chunks,
-    // each padded to a whole warp-tile)
-    return (size_t)g.num_chunks * (g.chunk_rows / 32) + (size_t)kMaxSelectChunks * (SEL_WTILE / 32);
+    return (size_t)g.num_chunks * (g.chunk_rows / 32);
 }
 
 // One CTA folds the per-chunk hit counts into the select's total (count phase of the
@@ -555,12 +553,12 @@ int launch_select_mask(const SelectArgs &a, bool with_total, cudaStream_t s) {
     const SelectGeom g = select_geom(a.n, a.sm_count);
     if (with_total && a.mask_ticket) {
         launch_pdl(mask_kernel<true>, g.grid, SEL_THREADS, 0, s, a.val, a.d_n, a.n, a.range, g.chunk_rows,
-                   g.num_chunks, a.mask, a.counts, a.stable_val, 0u,
+                   g.num_chunks, a.mask, a.counts, a.stable_val,
                    MaskTotal{a.d_count, a.mask_ticket, a.pub, a.pub_seq});
         return 1;
     }
     launch_pdl(mask_kernel<false>, g.grid, SEL_THREADS, 0, s, a.val, a.d_n, a.n, a.range, g.chunk_rows,
-               g.num_chunks, a.mask, a.counts, a.stable_val, 0u, MaskTotal{});
+               g.num_chunks, a.mask, a.counts, a.stable_val, MaskTotal{});
     if (!with_total) return 1;
     count_total_kernel<<<1, 1024, 0, s>>>(a.counts, g.num_chunks, a.d_count, a.pub, a.pub_seq);
     return 2;
@@ -571,12 +569,10 @@ int launch_select_expand(const SelectArgs &a, cudaStream_t s) {
     const SelectGeom g = select_geom(a.n, a.sm_count);
     if (a.pos_in)
         expand_kernel<true, false><<<g.grid, SEL_THREADS, 0, s>>>(
-            a.mask, a.counts, g.chunk_rows, g.num_chunks, a.pos_in, a.base_pos, a.out, a.d_count,
-            ChainArgs{}, 0u, g.num_chunks);
+            a.mask, a.counts, g.chunk_rows, g.num_chunks, a.pos_in, a.base_pos, a.out, a.d_count, ChainArgs{});
     else
         expand_kernel<false, false><<<g.grid, SEL_THREADS, 0, s>>>(
-            a.mask, a.counts, g.chunk_rows, g.num_chunks, nullptr, a.base_pos, a.out, a.d_count,
-            ChainArgs{}, 0u, g.num_chunks);
+            a.mask, a.counts, g.chunk_rows, g.num_chunks, nullptr, a.base_pos, a.out, a.d_count, ChainArgs{});
     return 1;
 }
 
@@ -597,50 +593,11 @@ int launch_select_expand_fetch_agg(const SelectArgs &a, cudaStream_t s) {
     }
     if (a.px.world)
         launch_pdl(expand_kernel<false, true, true>, g.grid, SEL_THREADS, 0, s, a.mask, a.counts, g.chunk_rows,
-                   g.num_chunks, (const int32_t *)nullptr, a.base_pos, a.out, a.d_count, ChainArgsX{c, a.px}, 0u,
-                   g.num_chunks);
+                   g.num_chunks, (const int32_t *)nullptr, a.base_pos, a.out, a.d_count, ChainArgsX{c, a.px});
     else
         launch_pdl(expand_kernel<false, true, false>, g.grid, SEL_THREADS, 0, s, a.mask, a.counts, g.chunk_rows,
-                   g.num_chunks, (const int32_t *)nullptr, a.base_pos, a.out, a.d_count, c, 0u, g.num_chunks);
+                   g.num_chunks, (const int32_t *)nullptr, a.base_pos, a.out, a.d_count, c);
     return 1;
-}
-
-// ---- the sliced chain: the shard is cut into `slices` row slices; the predicate pass of slice
-// k+1 (main stream) runs WHILE slice k is expanded, gathered and aggregated (side stream, higher
-// priority): the gather runs at the DRAM random-access rate and leaves half the bandwidth idle
-// when it runs alone (profiles/r01zi_chain_ncu_summary.md), the scan fills it.  Every slice is
-// `chunks_per_slice` warp-chunks of one common size, numbered through the whole shard, so the
-// expansion's prefix over "all chunks before mine" and the bitmap layout are those of the
-// unsliced chain.  Slice k's aggregate goes to slice_parts[k]; the caller folds them.
-int launch_chain_sliced(const SelectArgs &a, uint32_t slices, uint32_t chunks_per_slice, adb_agg *slice_parts,
-                        cudaStream_t main_s, cudaStream_t side_s, cudaEvent_t *mask_done /* [slices] */,
-                        uint32_t *slices_used) {
-    *slices_used = 0;
-    if (a.n == 0) return -1;
-    const SelectGeom g = select_geom(a.n, a.sm_count, slices * chunks_per_slice);
-    const uint32_t cps = (g.num_chunks + slices - 1) / slices;
-    const uint32_t grid_cap = (cps + SEL_WARPS - 1) / SEL_WARPS;
-    if ((int)grid_cap > kAggMaxBlocks || g.num_chunks > kMaxSelectChunks) return -1;
-    int launched = 0;
-    for (uint32_t k = 0; k < slices; ++k) {
-        const uint32_t c0 = k * cps;
-        if (c0 >= g.num_chunks) break;
-        const uint32_t c1 = c0 + cps < g.num_chunks ? c0 + cps : g.num_chunks;
-        const uint32_t grid = (c1 - c0 + SEL_WARPS - 1) / SEL_WARPS;
-        // mask: chunks [c0, c1) (the kernel's own bound is num_chunks; a CTA's spare warps past
-        // c1 would redo the next slice's first chunks, so the bound passed is c1)
-        launch_pdl(mask_kernel<false>, grid, SEL_THREADS, 0, main_s, a.val, a.d_n, a.n, a.range, g.chunk_rows, c1,
-                   a.mask, a.counts, a.stable_val, c0, MaskTotal{});
-        cudaEventRecord(mask_done[k], main_s);
-        cudaStreamWaitEvent(side_s, mask_done[k], 0);
-        const ChainArgs c{a.fetch_col, a.val_out, slice_parts + k, a.agg_scratch + (size_t)k * grid_cap, a.agg_ticket + k};
-        expand_kernel<false, true, false><<<grid, SEL_THREADS, 0, side_s>>>(
-            a.mask, a.counts, g.chunk_rows, g.num_chunks, (const int32_t *)nullptr, a.base_pos, a.out, a.d_count, c,
-            c0, c1);
-        launched += 2;
-        ++*slices_used;
-    }
-    return launched;
 }
 
 // the chain with neither handle materialised: one kernel, 4N + 4H bytes

@@ -182,13 +182,11 @@ class Engine:
         "adb_narrow_u64_to_i32": (C.c_int32, [C.c_void_p, C.c_int64, _I32P]),
         "adb_widen_i32_to_u64": (C.c_int32, [_I32P, C.c_int64, C.c_void_p]),
         "adb_iota_i32": (C.c_int32, [_I32P, C.c_int64, C.c_int32]),
-        "adb_chain_config": (C.c_int32, [C.c_int32, C.c_int32]),
         "adb_update_rows": (C.c_int32, [_I32P, C.c_int64, _I32P, C.c_int64, C.c_int32, C.c_int32]),
         "adb_delete_rows_plan": (C.c_int32, [C.c_int64, _I32P, C.c_int64, C.c_int32, _I64P]),
         "adb_delete_rows_apply": (C.c_int32, [_I32P, _I32P]),
         "adb_join_build": (C.c_int32, [_I32P, _I32P, C.c_int64, C.c_int64]),
         "adb_peer_exchange_reserve": (C.c_int32, [C.c_int64, C.c_int64, C.c_int64]),
-        "adb_join_probe_sharded": (C.c_int32, [C.c_int32, _I32P, _I32P, C.c_int64, C.c_int32, _I64P]),
         "adb_copy_from_ctx_ready": (C.c_int32, [C.c_void_p, C.c_int32, C.c_void_p, C.c_size_t]),
         "adb_route_rows": (C.c_int32, [C.c_int32, C.c_int64, _I32P, C.c_int64, _I64P, C.POINTER(_I32P),
                                        C.POINTER(C.c_void_p)]),

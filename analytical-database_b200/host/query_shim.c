@@ -2489,9 +2489,9 @@ Result *sub(Result *column_one, Result *column_two, Status *ret_status) {
  * operands are brought to context 0 over peer copies and joined there. */
 /* G = 2, 4, 8, 16: the join itself is sharded.  The build side is hash-partitioned over the GPUs
  * through peer memory (adb_peer_exchange_pairs), every GPU builds the tables of its keys, and
- * every GPU probes ITS slice of the probe side, in its original order, reading a key's table
- * from its owner over NVLink.  The slices' outputs concatenated in shard order are the
- * reference's probe-major list, so nothing is gathered and nothing re-sorted. */
+ * every GPU's slice of the probe side, in its original order, is routed to the keys' owners,
+ * probed there, and the answers come home in bulk.  The slices' outputs concatenated in shard
+ * order are the reference's probe-major list, so nothing is gathered and nothing re-sorted. */
 typedef struct JoinJob {
     ShardErr err;
     Staged *bv, *bp, *pv, *pp;
@@ -2505,21 +2505,6 @@ typedef struct JoinJob {
     void *answers_owner[MAXG];                      /* GPU o's answers, in the order it received the keys */
 } JoinJob;
 
-/* ADB_JOIN_SHARDED_PROBE=peer: every GPU probes its rows in place and reads a remote key's slot
- * over NVLink (adb_join_probe_sharded) instead of routing the keys to their owners. */
-static int join_probe_routed(void) {
-    const char *e = getenv("ADB_JOIN_SHARDED_PROBE");
-    return !(e && !strcmp(e, "peer"));
-}
-static void join_finish_shard(int g, JoinJob *a, int64_t m) {
-    void *x = NULL, *y = NULL;
-    SCK(adb_alloc(&x, 4 * (size_t)m));
-    a->o1.d[g] = x;
-    SCK(adb_alloc(&y, 4 * (size_t)m));
-    a->o2.d[g] = y;
-    a->o1.n[g] = a->o2.n[g] = (size_t)m;
-    SCK(adb_join_emit(x, y));
-}
 static void join_shard(int g, void *arg) {
     JoinJob *a = arg;
     if (a->phase == -1) {
@@ -2542,18 +2527,12 @@ static void join_shard(int g, void *arg) {
         SCK(adb_join_build(rv, rp, rn, (int64_t)a->pv->n[g]));
         return;
     }
-    if (a->phase == 1) {                            /* probe in place, remote slots over NVLink */
-        int64_t m = 0;
-        SCK(adb_join_probe_sharded(S.G, a->pv->d[g], a->pp->d[g], (int64_t)a->pv->n[g], a->swapped, &m));
-        join_finish_shard(g, a, m);
-        return;
-    }
-    if (a->phase == 2) {                            /* routed probe, 3a: my keys grouped by owner */
+    if (a->phase == 1) {                            /* routed probe, 3a: my keys grouped by owner */
         SCK(adb_join_route_probe(S.G, a->pv->d[g], (int64_t)a->pv->n[g], a->sent[g], &a->routed_keys[g],
                                  &a->answers_home[g]));
         return;
     }
-    if (a->phase == 3) {                            /* 3b: I own what the others sent me */
+    if (a->phase == 2) {                            /* 3b: I own what the others sent me */
         int64_t n_recv = 0;
         for (int s = 0; s < S.G; ++s) n_recv += a->sent[s][g];
         int32_t *keys = NULL;
@@ -2572,7 +2551,7 @@ static void join_shard(int g, void *arg) {
         SCK(adb_join_probe_received(n_recv));
         return;
     }
-    /* phase 4, 3c: the owners' answers come home, back to row order, expand */
+    /* phase 3, 3c: the owners' answers come home, back to row order, expand */
     for (int k = 0; k < S.G; ++k) {
         const int o = (g + k) % S.G;
         int64_t at = 0, from = 0;                   /* my piece inside owner o's received list */
@@ -2585,7 +2564,13 @@ static void join_shard(int g, void *arg) {
     }
     int64_t m = 0;
     SCK(adb_join_finish_routed(S.G, a->pv->d[g], a->pp->d[g], (int64_t)a->pv->n[g], a->swapped, &m));
-    join_finish_shard(g, a, m);
+    void *x = NULL, *y = NULL;
+    SCK(adb_alloc(&x, 4 * (size_t)m));
+    a->o1.d[g] = x;
+    SCK(adb_alloc(&y, 4 * (size_t)m));
+    a->o2.d[g] = y;
+    a->o1.n[g] = a->o2.n[g] = (size_t)m;
+    SCK(adb_join_emit(x, y));
 }
 
 static int ensure_join_exchange(size_t cap) {
@@ -2640,13 +2625,7 @@ static Result **join_sharded(Result *v1, Result *p1, Result *v2, Result *p2, int
             goto fail;
         }
     }
-    if (join_probe_routed()) {
-        for (job.phase = 2; job.phase <= 4; ++job.phase) {
-            run_shards(join_shard, &job);
-            if (shard_errs(&job.err)) goto fail;
-        }
-    } else {
-        job.phase = 1;
+    for (job.phase = 1; job.phase <= 3; ++job.phase) {
         run_shards(join_shard, &job);
         if (shard_errs(&job.err)) goto fail;
     }

@@ -307,12 +307,6 @@ ADB_API adb_status adb_chain_select_fetch_agg(const int32_t *d_sel_col, const in
 ADB_API adb_status adb_chain_select_agg(const int32_t *d_sel_col, const int32_t *d_fetch_col, int64_t n,
                                 const int32_t *lo, const int32_t *hi, int64_t *d_count, adb_agg *d_agg,
                                 adb_agg *h_agg);
-/* How adb_chain_select_fetch_agg cuts a shard into row slices whose predicate pass (slice k+1)
- * overlaps the expansion + gather + aggregate of slice k on a second, higher-priority stream:
- * slices = 0 or 1 is the plain two-kernel chain (the default: measured, slicing gains nothing);
- * cps_div: each slice's grids fill 1/cps_div of the resident CTA slots.  Results are identical
- * for every setting (the chunks are numbered through the whole shard). */
-ADB_API adb_status adb_chain_config(int32_t slices, int32_t cps_div);
 
 /* ---- batched shared scan -- replaces shared_select + select_task, src/query.c:450-583
  * One pass over d_col evaluates q_count (<= ADB_MAX_BATCH, the dispatcher's chunk,
@@ -435,42 +429,38 @@ ADB_API adb_status adb_nested_loop_join_count(const int32_t *d_v1, const int32_t
                                               int64_t *h_matches);
 ADB_API adb_status adb_join_emit(int32_t *d_out1, int32_t *d_out2);
 /* The join sharded over the contexts of ONE process (SURVEY.md 8e "hash join: hash-partition both
- * (key, pos) lists by key to G GPUs"), keeping the reference's output order:
+ * (key, pos) lists by key to G GPUs"), keeping the reference's output order.  world = number of
+ * contexts, a power of two >= 2; swapped as in adb_nested_loop_join_count.  Every step on every
+ * context, a host barrier after each:
  *   1. every context routes its slice of the BUILD side to the keys' owners
  *      (adb_peer_exchange_pairs, side 0: pieces land in source-rank order = insertion order);
  *   2. every context calls adb_join_build on what it received (sort on the hash + one table per
  *      partition, as steps 1-3 of adb_hash_join_count); probe_rows_hint = the probe rows this
  *      context will bring (scratch is reserved for them).  Synchronises;
- *   3. once EVERY context has built, each calls adb_join_probe_sharded with its own slice of the
- *      PROBE side, in its original order: a key's table is read from its owner over NVLink peer
- *      memory; *h_matches = this context's pair count;
+ *   3. each context's slice of the PROBE side, in its original order, is answered by the keys'
+ *      owners: the keys travel to them in bulk and the answers come back in bulk (reading every
+ *      remote slot over NVLink instead costs one 32-byte response per 16-byte slot, ~9 G reads/s
+ *      per GPU):
+ *      3a. adb_join_route_probe: stable partition of this context's probe keys by owner;
+ *          h_counts[r] = keys bound for context r (they sit at offset sum(h_counts[0..r)) of
+ *          *d_routed_keys, in row order); *d_answers = where context r's answers belong, at the
+ *          same offsets, 8 bytes per key;
+ *      3b. adb_join_recv_buffers(n_recv) + one adb_copy_from_ctx[_ready] per source context
+ *          (pieces in source-context order) + adb_join_probe_received(n_recv): the answers land in
+ *          *d_answers of adb_join_recv_buffers, in the order of the received keys.  Synchronises;
+ *      3c. one adb_copy_from_ctx[_ready] per owner into 3a's *d_answers + adb_join_finish_routed:
+ *          *h_matches = this context's pair count.
+ *      (3a and 3b end synchronised, so with a host barrier after each the _ready copies are safe.)
  *   4. adb_join_emit writes this context's pairs (multi-row groups read the owner's sorted build
  *      positions over peer memory).  Synchronises.
- * The contexts' outputs concatenated in context order are the reference's probe-major list.
- * world = number of contexts, a power of two; swapped as in adb_nested_loop_join_count. */
+ * Each context's pairs are probe-major over its own probe rows, so the contexts' outputs
+ * concatenated in context order are the reference's probe-major list. */
 /* Sizes every scratch buffer steps 1-3 will need on this context (exchange of send_pairs pairs,
  * build over up to build_pairs received pairs, probe_rows probe rows) BEFORE the collective
  * starts: device memory management may wait for the device to go idle, which must not happen
  * while a context sharing the device spin-waits for this one.  Every context, then a barrier. */
 ADB_API adb_status adb_peer_exchange_reserve(int64_t send_pairs, int64_t build_pairs, int64_t probe_rows);
 ADB_API adb_status adb_join_build(const int32_t *d_v, const int32_t *d_p, int64_t n, int64_t probe_rows_hint);
-ADB_API adb_status adb_join_probe_sharded(int32_t world, const int32_t *d_pv, const int32_t *d_pp, int64_t np,
-                                          int32_t swapped, int64_t *h_matches);
-
-/* Step 3 with the probe keys ROUTED to their owners instead of every remote slot being read over
- * NVLink (one 32-byte response per 16-byte slot, ~9 G reads/s per GPU): keys out in bulk, answers
- * back in bulk, the rows' home restores row order.  On every context, a host barrier after each:
- *   3a. adb_join_route_probe: stable partition of this context's probe keys by owner;
- *       h_counts[r] = keys bound for context r (they sit at offset sum(h_counts[0..r)) of
- *       *d_routed_keys, in row order); *d_answers = where context r's answers belong, at the same
- *       offsets, 8 bytes per key;
- *   3b. adb_join_recv_buffers(n_recv) + one adb_copy_from_ctx[_ready] per source context (pieces
- *       in source-context order) + adb_join_probe_received(n_recv): the answers land in
- *       *d_answers of adb_join_recv_buffers, in the order of the received keys.  Synchronises;
- *   3c. one adb_copy_from_ctx[_ready] per owner into 3a's *d_answers + adb_join_finish_routed
- *       (what adb_join_probe_sharded returns), then adb_join_emit.
- * (3a and 3b end synchronised, so with a host barrier after each the _ready copies are safe.)
- * Output order and content are those of adb_join_probe_sharded. */
 ADB_API adb_status adb_join_route_probe(int32_t world, const int32_t *d_pv, int64_t np, int64_t *h_counts,
                                         const int32_t **d_routed_keys, void **d_answers);
 ADB_API adb_status adb_join_recv_buffers(int64_t n_recv, int32_t **d_keys, void **d_answers);

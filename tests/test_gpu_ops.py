@@ -138,16 +138,12 @@ def test_add_sub_wrap(eng, port, rng, n):
     assert np.array_equal(eng.ewise(da, db, n, True).to_host(n), port.sub(a, b))
 
 
-@pytest.mark.parametrize("slices,cps_div", [(1, 2), (2, 1), (3, 2), (7, 4), (16, 2)],
-                         ids=["plain", "2slices", "3slices", "7slices", "16slices"])
 @pytest.mark.parametrize("n", [0, 1, 513, 4097, 1_000_003])
-def test_chain_matches_oracle_and_reference(eng, port, rng, n, slices, cps_div):
+def test_chain_matches_oracle_and_reference(eng, port, rng, n):
     """s=select(col1,lo,hi); f=fetch(col2,s); a=sum(f)/min/max/avg -- the north-star chain
-    (predicate pass + expansion with the gather and the aggregates fused in), plain and cut into
-    row slices whose predicate pass overlaps the previous slice's expansion (adb_chain_config):
-    every setting must give the same positions, values and aggregates."""
+    (predicate pass + expansion with the gather and the aggregates fused in): the same positions,
+    values and aggregates as the oracle and the reference."""
     import ctypes as C
-    eng._ck(eng.lib.adb_chain_config(slices, cps_div))
     from oracle import oracle
     ref = oracle.reference("O2")
     sel = rng.integers(-n // 2 - 1, n // 2 + 1, n).astype(np.int32)
@@ -179,7 +175,6 @@ def test_chain_matches_oracle_and_reference(eng, port, rng, n, slices, cps_div):
         if h:
             assert agg.min == port.min(exp_val) and agg.max == port.max(exp_val)
             assert agg.avg == port.avg(exp_val)
-    eng._ck(eng.lib.adb_chain_config(0, 2))
 
 
 @pytest.mark.parametrize("n", [0, 1, 513, 4097, 1_000_003])

@@ -790,14 +790,12 @@ def test_long_print_across_shards(api, rng):
     api.drop(s), api.drop(f)
 
 
-@pytest.mark.parametrize("sharded_probe", ["routed", "routed-partitioned", "peer"])
+@pytest.mark.parametrize("sharded_probe", ["routed", "routed-partitioned"])
 def test_join_of_sharded_operands(api, cpu, rng, monkeypatch, sharded_probe):
     """With several GPUs the probe keys are routed to their owners and the answers gathered back
-    into row order (default; the owner probes what it received directly or, for a table far
-    beyond L2, slice by slice: ADB_JOIN_PROBE=partitioned forces that at any size), or every GPU
-    probes in place and reads remote slots over peer memory (ADB_JOIN_SHARDED_PROBE=peer): same
-    pairs, same order."""
-    monkeypatch.setenv("ADB_JOIN_SHARDED_PROBE", sharded_probe.split("-")[0])
+    into row order; the owner probes what it received directly or, for a table far beyond L2,
+    slice by slice (ADB_JOIN_PROBE=partitioned forces that at any size): same pairs, same order
+    as the reference."""
     if sharded_probe.endswith("partitioned"):
         monkeypatch.setenv("ADB_JOIN_PROBE", "partitioned")
     n1, n2 = 70_000, 50_000
