@@ -7,6 +7,7 @@
 #include <atomic>
 #include <chrono>
 #include <thread>
+#include <tuple>
 #include <cstdarg>
 #include <vector>
 #include <cstdio>
@@ -21,6 +22,13 @@ namespace {
 
 thread_local std::string g_err;
 
+// A device allocation the engine owns: grown by grow(), freed by release(); reads as a T *.
+template <class T> struct DevBuf {
+    T *p = nullptr;
+    size_t cap = 0;                     // bytes
+    operator T *() const { return p; }
+};
+
 struct Engine {
     bool up = false;
     int32_t ctx_index = 0;
@@ -31,17 +39,15 @@ struct Engine {
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     cudaEvent_t marks[ADB_MAX_MARKS] = {};
     // select scratch: selection bitmap (grown on demand) + per-chunk counts
-    uint32_t *sel_mask = nullptr;
-    size_t sel_mask_words = 0;
-    uint32_t *sel_counts = nullptr;
+    DevBuf<uint32_t> sel_mask, sel_counts;
     // aggregate fold state: one partial per CTA, and two self-re-arming tickets -- [0] for every
     // grid-wide aggregate fold (one arrival per CTA), [1] for the count phase's fused total
     // (mask_kernel<true>, one arrival per warp-chunk).  The fused count must not share a counter
     // with the fold: each finds its last arrival by comparing the ticket it drew with its own
     // number of arrivals, which only holds while no other kernel draws from the same counter.
-    adb_agg *agg_scratch = nullptr;
-    unsigned int *agg_ticket = nullptr;
-    int64_t *idx_bounds = nullptr;      // {first, count} of the last index select
+    DevBuf<adb_agg> agg_scratch;
+    DevBuf<unsigned int> agg_ticket;
+    DevBuf<int64_t> idx_bounds;         // {first, count} of the last index select
     int64_t idx_pending_n = -1;         // >= 0 between adb_select_index_count and _emit
     adb::SelectArgs sel_pending{};      // valid between adb_select_*_count and adb_select_emit
     bool sel_ready = false;
@@ -50,23 +56,20 @@ struct Engine {
     unsigned long long *mbox = nullptr;  // kMboxWords payload words, then the flag word
     unsigned long long *mbox_dev = nullptr;
     unsigned long long mbox_seq = 0;
-    int64_t *scratch_count = nullptr;   // device int64 for callers that pass no d_count
+    DevBuf<int64_t> scratch_count;      // device int64 for callers that pass no d_count
     // batched shared scan state (count phase -> emit phase)
-    unsigned char *ss_plan_mem = nullptr;   // bounds | cov_off | cov_q
-    uint32_t *ss_hits = nullptr;            // per-chunk hit lists, chunk_rows entries each
-    size_t ss_hits_rows = 0;
-    uint32_t *ss_chunk_hits = nullptr;
-    uint32_t *ss_counts = nullptr;
-    int64_t *ss_totals = nullptr;
-    int32_t **ss_outs = nullptr;
+    DevBuf<unsigned char> ss_plan_mem;  // bounds | cov_off | cov_q
+    DevBuf<uint32_t> ss_hits;           // per-chunk hit lists, chunk_rows entries each
+    DevBuf<uint32_t> ss_chunk_hits, ss_counts;
+    DevBuf<int64_t> ss_totals;
+    DevBuf<int32_t *> ss_outs;
     adb::SharedScanPlan ss_plan{};
     adb::SharedScanGeom ss_geom{};
     bool ss_ready = false;
     int32_t ss_base_pos = 0;            // added to every emitted row (shard base)
     // radix / join scratch
-    uint32_t *rx_hist = nullptr, *rx_totals = nullptr, *rx_base = nullptr;
-    size_t rx_hist_elems = 0;
-    unsigned long long *sc_sums = nullptr;
+    DevBuf<uint32_t> rx_hist, rx_totals, rx_base;
+    DevBuf<unsigned long long> sc_sums;
     struct JoinState {
         bool ready = false;
         uint32_t n_probe = 0, n_build = 0;
@@ -94,20 +97,18 @@ struct Engine {
     } join;
     // grow-only scratch arena for the sort / join temporaries: cudaMallocAsync of many
     // differently sized multi-hundred-MB blocks made the pool re-map memory on every join
-    unsigned char *arena = nullptr;
-    size_t arena_cap = 0, arena_used = 0;
+    DevBuf<unsigned char> arena;
+    size_t arena_used = 0;
     // delete plan (adb_delete_rows_plan -> _apply): flags and prefix in the arena
     uint32_t *del_dead = nullptr, *del_before = nullptr;
     int64_t del_rows = -1;
     // join tables: one open-addressing table per build partition, 16-byte slots (grow-only)
-    void *hj_table = nullptr;
-    unsigned long long hj_table_slots = 0;
+    DevBuf<uint4> hj_table;
     // routed probe, owner side: the keys other contexts sent here and the answers (grow-only)
     uint32_t *rt32_pos = nullptr, *rt32_rows = nullptr, *rt32_val = nullptr;   // routed fetch (arena)
     uint32_t rt32_n = 0;
-    uint32_t *rt_recv_keys = nullptr;
-    uint2 *rt_recv_res = nullptr;
-    size_t rt_recv_cap = 0;
+    DevBuf<uint32_t> rt_recv_keys;
+    DevBuf<uint2> rt_recv_res;
     // bulk CSV load state (adb_csv_index -> adb_csv_parse); scratch is grow-only
     struct CsvState {
         const unsigned char *text = nullptr;
@@ -115,24 +116,20 @@ struct Engine {
         unsigned long long newlines = 0, rows = 0;
         uint32_t skip = 0;
         bool ready = false;
-        uint32_t *block_counts = nullptr, *block_base = nullptr;
-        size_t blocks_cap = 0;
-        unsigned long long *line_end = nullptr;
-        size_t lines_cap = 0;
-        unsigned char *n_fields = nullptr;
-        size_t fields_cap = 0;
-        int32_t **col_table = nullptr;          // 256 device pointers
-        uint32_t *flags = nullptr;
-        int64_t *total = nullptr;
+        DevBuf<uint32_t> block_counts, block_base;
+        DevBuf<unsigned long long> line_end;
+        DevBuf<unsigned char> n_fields;
+        DevBuf<int32_t *> col_table;        // 256 device pointers
+        DevBuf<uint32_t> flags;
+        DevBuf<int64_t> total;
     } csv;
     // print formatting state (adb_format_i32_count -> _emit)
     struct FmtState {
         const int32_t *val = nullptr;
         int64_t n = 0, bytes = 0;
         bool ready = false;
-        uint32_t *block_len = nullptr, *block_off = nullptr;
-        size_t cap_len = 0, cap_off = 0;
-        int64_t *total = nullptr;
+        DevBuf<uint32_t> block_len, block_off;
+        DevBuf<int64_t> total;
     } fmt;
     // pinned staging lanes for large pageable copies (staged_copy)
     struct StageLane { void *buf[2] = {nullptr, nullptr}; cudaEvent_t ev[2] = {nullptr, nullptr}; cudaStream_t st = nullptr; };
@@ -140,22 +137,22 @@ struct Engine {
     int stage_lanes = 0;
     cudaEvent_t stage_ready = nullptr;
     // aggregate exchange over peer memory (adb_peer_*): own mailbox + the peers' mappings
-    adb::PeerRecord *peer_box = nullptr;
+    DevBuf<adb::PeerRecord> peer_box;
     adb::PeerBoxes peer_boxes{};
-    adb::PeerBoxes *peer_boxes_dev = nullptr;     // the same table in device memory (kernels index it)
+    DevBuf<adb::PeerBoxes> peer_boxes_dev;  // the same table in device memory (kernels index it)
     int32_t peer_world = 0, peer_rank = -1;
     bool peer_connected = false;
     uint32_t peer_epoch = 0;
     // pair exchange of the sharded join (adb_peer_join_*): my receive buffer (2 sides x
     // {values, positions} x jx_cap ints), the peers' mapped buffers, a device table of them
-    int32_t *jx_recv = nullptr;
+    DevBuf<int32_t> jx_recv;
     unsigned long long jx_cap = 0;
     uint32_t *jx_peer_host[ADB_MAX_PEERS] = {};
-    uint32_t **jx_peer_dev = nullptr;
+    DevBuf<uint32_t *> jx_peer_dev;
     bool jx_connected = false;
     uint32_t jx_epoch = 0;
-    uint32_t *jx_status = nullptr;          // device: 0 ok, 1 overflow, 2 timeout
-    int64_t *jx_total = nullptr;            // device: pairs this rank receives
+    DevBuf<uint32_t> jx_status;         // device: 0 ok, 1 overflow, 2 timeout
+    DevBuf<int64_t> jx_total;           // device: pairs this rank receives
     int64_t launches = 0;
     int32_t chain_mark_base = -1;       // adb_chain_marks(): slots for the next chain call
     bool peer_local = false;            // mailboxes mapped by peer access inside one process (no IPC handles)
@@ -179,6 +176,16 @@ struct Engine {
     cudaEvent_t blob_ev[kBlobSlots] = {};
     int blob_next = 0;
 };
+
+// Every device buffer a context owns outside its peer connection (peer_close frees those):
+// shutting the context down, or an adb_init that failed half way, releases exactly these.
+auto context_bufs(Engine &E) {
+    return std::tie(E.sel_mask, E.sel_counts, E.agg_scratch, E.agg_ticket, E.idx_bounds, E.scratch_count,
+                    E.ss_plan_mem, E.ss_hits, E.ss_chunk_hits, E.ss_counts, E.ss_totals, E.ss_outs, E.rx_hist,
+                    E.rx_totals, E.rx_base, E.sc_sums, E.arena, E.hj_table, E.rt_recv_keys, E.rt_recv_res,
+                    E.csv.block_counts, E.csv.block_base, E.csv.line_end, E.csv.n_fields, E.csv.col_table,
+                    E.csv.flags, E.csv.total, E.fmt.block_len, E.fmt.block_off, E.fmt.total);
+}
 
 // One context per GPU of the box (several may share a device: a 1-GPU box then runs the
 // multi-shard host path unchanged).  Every entry point works on the calling THREAD's current
@@ -312,55 +319,85 @@ adb_status check_len(int64_t n, const char *what) {
     return ADB_OK;
 }
 
-// The bitmap scratch only ever grows; a select over the largest shard (2^31 rows) needs 256 MB.
-adb_status ensure_select_scratch(uint32_t n) {
-    const size_t need = adb::select_mask_words(n, g.sm_count);
-    if (need <= g.sel_mask_words) return ADB_OK;
-    if (g.sel_mask) {
-        CU(cudaStreamSynchronize(g.stream));
-        CU(cudaFree(g.sel_mask));
-        g.sel_mask = nullptr;
-        g.sel_mask_words = 0;
+// ---- engine-owned device memory --------------------------------------------------------------
+// give every cached block back to the pool (before shutdown, or when the device runs short)
+void cache_flush(Engine &E) {
+    for (int i = 0; i < E.cache_n; ++i) cudaFreeAsync(E.cache[i].p, E.stream);
+    E.cache_n = 0;
+    E.cache_bytes = 0;
+    cudaGetLastError();
+}
+
+// Out of device memory: clear the error, flush the front cache and wait until its blocks are free.
+void cache_drop(Engine &E) {
+    cudaGetLastError();
+    cache_flush(E);
+    cudaStreamSynchronize(E.stream);
+}
+
+template <class T> cudaError_t release(DevBuf<T> &b) {
+    const cudaError_t e = b.p ? cudaFree(b.p) : cudaSuccess;
+    b = DevBuf<T>{};
+    return e;
+}
+
+// cudaMalloc of `bytes` into the empty buffer `b`.  Out of memory, the front cache goes back to
+// the pool and the pool hands its idle blocks back to the device (its release threshold keeps
+// them otherwise, adb_init), then the allocation is tried once more.
+template <class T> adb_status dev_alloc(DevBuf<T> &b, size_t bytes, const char *what) {
+    cudaError_t e = cudaMalloc(&b.p, bytes);
+    if (e == cudaErrorMemoryAllocation) {
+        cache_drop(g);
+        cudaMemPool_t pool;
+        if (cudaDeviceGetDefaultMemPool(&pool, g.device) == cudaSuccess) cudaMemPoolTrimTo(pool, 0);
+        cudaGetLastError();
+        e = cudaMalloc(&b.p, bytes);
     }
-    const size_t words = need + need / 8 + 4096;
-    cudaError_t e = cudaMalloc(&g.sel_mask, words * sizeof(uint32_t));
     if (e != cudaSuccess) {
         cudaGetLastError();
-        return fail(ADB_ERR_NOMEM, "select bitmap scratch: %s", cudaGetErrorString(e));
+        b = DevBuf<T>{};
+        return fail(e == cudaErrorMemoryAllocation ? ADB_ERR_NOMEM : ADB_ERR_CUDA, "%s (%zu bytes): %s", what, bytes,
+                    cudaGetErrorString(e));
     }
-    g.sel_mask_words = words;
+    b.cap = bytes;
     return ADB_OK;
+}
+
+// Grow-only scratch: nothing happens while `need` bytes fit; otherwise the old block is freed
+// once the stream is done with it and the new one has room for need + need / 8 + 1 MiB.  The
+// routed probe picks its form by the arena's capacity, so this slack is part of its behaviour.
+template <class T> adb_status grow(DevBuf<T> &b, size_t need, const char *what) {
+    if (need <= b.cap) return ADB_OK;
+    if (b.p) {
+        CU(cudaStreamSynchronize(g.stream));
+        CU(release(b));
+    }
+    return dev_alloc(b, need + need / 8 + (1 << 20), what);
 }
 
 void jx_close() {
     for (int r = 0; r < g.peer_world; ++r)
         if (r != g.peer_rank && g.jx_peer_host[r] && !g.peer_local) cudaIpcCloseMemHandle(g.jx_peer_host[r]);
-    if (g.jx_recv) cudaFree(g.jx_recv);
-    if (g.jx_peer_dev) cudaFree(g.jx_peer_dev);
-    if (g.jx_status) cudaFree(g.jx_status);
-    if (g.jx_total) cudaFree(g.jx_total);
+    release(g.jx_recv);
+    release(g.jx_peer_dev);
+    release(g.jx_status);
+    release(g.jx_total);
     cudaGetLastError();
-    g.jx_recv = nullptr;
     g.jx_cap = 0;
     for (auto &p : g.jx_peer_host) p = nullptr;
-    g.jx_peer_dev = nullptr;
     g.jx_connected = false;
     // jx_epoch is NOT reset: the epoch words live in the aggregate mailbox, which outlives the
     // receive regions -- a new connection that started over at epoch 1 would take the previous
     // connection's count rows for its own (only peer_close, which frees the mailbox, resets it)
-    g.jx_status = nullptr;
-    g.jx_total = nullptr;
 }
 
 void peer_close() {
     jx_close();
     for (int r = 0; r < g.peer_world; ++r)
         if (r != g.peer_rank && g.peer_boxes.box[r] && !g.peer_local) cudaIpcCloseMemHandle(g.peer_boxes.box[r]);
-    if (g.peer_box) cudaFree(g.peer_box);
-    if (g.peer_boxes_dev) cudaFree(g.peer_boxes_dev);
-    g.peer_boxes_dev = nullptr;
+    release(g.peer_box);
+    release(g.peer_boxes_dev);
     cudaGetLastError();
-    g.peer_box = nullptr;
     g.peer_boxes = adb::PeerBoxes{};
     g.peer_world = 0;
     g.peer_rank = -1;
@@ -490,8 +527,16 @@ adb_status adb_ctx_init(int32_t ctx, int device_ordinal) {
     return adb_init(device_ordinal);
 }
 
+static adb_status init_current(int device_ordinal);
+static void teardown_current();
 adb_status adb_init(int device_ordinal) {
     if (g.up) return ADB_OK;
+    const adb_status s = init_current(device_ordinal);
+    if (s != ADB_OK) teardown_current();        // nothing stays allocated: a later adb_init starts afresh
+    return s;
+}
+
+static adb_status init_current(int device_ordinal) {
     // (takes effect when this is the first CUDA call of the process; otherwise the preload_*
     // calls below do the same for the engine's own kernels)
     setenv("CUDA_MODULE_LOADING", "EAGER", 0);
@@ -516,9 +561,9 @@ adb_status adb_init(int device_ordinal) {
     CU(cudaDeviceGetDefaultMemPool(&pool, device_ordinal));
     uint64_t keep = UINT64_MAX;
     CU(cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &keep));
-    CU(cudaMalloc(&g.sel_counts, sizeof(uint32_t) * adb::kMaxSelectChunks));
-    CU(cudaMalloc(&g.idx_bounds, 2 * sizeof(int64_t)));
-    CU(cudaMalloc(&g.scratch_count, sizeof(int64_t)));
+    if (adb_status s = dev_alloc(g.sel_counts, sizeof(uint32_t) * adb::kMaxSelectChunks, "select chunk counts")) return s;
+    if (adb_status s = dev_alloc(g.idx_bounds, 2 * sizeof(int64_t), "index select bounds")) return s;
+    if (adb_status s = dev_alloc(g.scratch_count, sizeof(int64_t), "select count")) return s;
     // Gathers over sparse position lists touch one 32-byte sector per hit; ask L2 not to
     // widen those misses (r01b: 570 MB of DRAM reads for 180 MB of requested sectors).
     // A hint only -- streaming kernels request whole lines anyway.  ADB_L2_FETCH overrides.
@@ -544,9 +589,9 @@ adb_status adb_init(int device_ordinal) {
             cudaGetLastError();                 // readbacks fall back to cudaMemcpyAsync
         }
     }
-    CU(cudaMalloc(&g.agg_scratch, sizeof(adb_agg) * adb::kAggMaxBlocks));
-    CU(cudaMalloc(&g.agg_ticket, sizeof(unsigned int) * 2));
-    CU(cudaMemset(g.agg_ticket, 0, sizeof(unsigned int) * 2));
+    if (adb_status s = dev_alloc(g.agg_scratch, sizeof(adb_agg) * adb::kAggMaxBlocks, "aggregate partials")) return s;
+    if (adb_status s = dev_alloc(g.agg_ticket, sizeof(unsigned int) * 2, "aggregate tickets")) return s;
+    CU(cudaMemset(g.agg_ticket.p, 0, sizeof(unsigned int) * 2));
     // every kernel of the engine is loaded here, per device: see preload_* (adb_common.cuh)
     adb::preload_csv_load(); adb::preload_format_text(); adb::preload_gather_agg(); adb::preload_hash_join();
     adb::preload_index_lookup(); adb::preload_peer_agg(); adb::preload_peer_exchange(); adb::preload_radix();
@@ -562,56 +607,28 @@ adb_status adb_init(int device_ordinal) {
     return ADB_OK;
 }
 
-static adb_status shutdown_current();
-static void cache_flush(Engine &E);
 // Shuts down every context of the process (the hook is called once, from shutdown_server()).
 adb_status adb_shutdown(void) {
     const int keep = g_cur;
     // first quiesce every stream: a context's kernels may still touch a peer's mailbox
     for (int c = 0; c < ADB_MAX_CONTEXTS; ++c)
         if (g_ctx[c].up) { cudaSetDevice(g_ctx[c].device); cudaStreamSynchronize(g_ctx[c].stream); }
-    for (int c = 0; c < ADB_MAX_CONTEXTS; ++c) { g_cur = c; shutdown_current(); }
+    for (int c = 0; c < ADB_MAX_CONTEXTS; ++c) {
+        g_cur = c;
+        if (g.up) teardown_current();
+    }
     g_cur = keep;
     return ADB_OK;
 }
 
-static adb_status shutdown_current() {
-    if (!g.up) return ADB_OK;
-    cudaSetDevice(g.device);
+// Frees everything the current context holds; also a context that adb_init left half built.
+static void teardown_current() {
+    if (g.device >= 0) cudaSetDevice(g.device);
     cache_flush(g);
     delete g.live;
     g.live = nullptr;
     cudaStreamSynchronize(g.stream);
-    cudaFree(g.sel_mask);
-    cudaFree(g.sel_counts);
-    cudaFree(g.idx_bounds);
-    cudaFree(g.scratch_count);
-    cudaFree(g.ss_plan_mem);
-    cudaFree(g.ss_hits);
-    cudaFree(g.ss_chunk_hits);
-    cudaFree(g.ss_counts);
-    cudaFree(g.ss_totals);
-    cudaFree(g.ss_outs);
-    cudaFree(g.rx_hist);
-    cudaFree(g.rx_totals);
-    cudaFree(g.rx_base);
-    cudaFree(g.sc_sums);
-    cudaFree(g.arena);
-    cudaFree(g.hj_table);
-    cudaFree(g.rt_recv_keys);
-    cudaFree(g.rt_recv_res);
-    cudaFree(g.fmt.block_len);
-    cudaFree(g.fmt.block_off);
-    cudaFree(g.fmt.total);
-    cudaFree(g.csv.block_counts);
-    cudaFree(g.csv.block_base);
-    cudaFree(g.csv.line_end);
-    cudaFree(g.csv.n_fields);
-    cudaFree(g.csv.col_table);
-    cudaFree(g.csv.flags);
-    cudaFree(g.csv.total);
-    cudaFree(g.agg_scratch);
-    cudaFree(g.agg_ticket);
+    std::apply([](auto &...b) { (release(b), ...); }, context_bufs(g));
     for (int k = 0; k < Engine::kBlobSlots; ++k) {
         if (g.blob[k]) cudaFreeHost(g.blob[k]);
         if (g.blob_ev[k]) cudaEventDestroy(g.blob_ev[k]);
@@ -623,13 +640,13 @@ static adb_status shutdown_current() {
         cudaStreamDestroy(g.stage[l].st);
     }
     if (g.stage_ready) cudaEventDestroy(g.stage_ready);
-    cudaEventDestroy(g.ev0);
-    cudaEventDestroy(g.ev1);
+    if (g.ev0) cudaEventDestroy(g.ev0);
+    if (g.ev1) cudaEventDestroy(g.ev1);
     for (cudaEvent_t &m : g.marks)
         if (m) cudaEventDestroy(m);
     if (g.own_stream) cudaStreamDestroy(g.stream);
+    cudaGetLastError();
     g = Engine{};
-    return ADB_OK;
 }
 
 void *adb_stream(void) { return g.stream; }
@@ -662,14 +679,6 @@ static void *cache_take(Engine &E, size_t cls) {
         }
     return nullptr;
 }
-// give every cached block back to the pool (before shutdown, or when the device runs short)
-static void cache_flush(Engine &E) {
-    for (int i = 0; i < E.cache_n; ++i) cudaFreeAsync(E.cache[i].p, E.stream);
-    E.cache_n = 0;
-    E.cache_bytes = 0;
-    cudaGetLastError();
-}
-
 adb_status adb_alloc(void **d_ptr, size_t bytes) {
     NEED_UP();
     if (!d_ptr) return fail(ADB_ERR_INVALID, "adb_alloc: NULL out pointer");
@@ -681,9 +690,7 @@ adb_status adb_alloc(void **d_ptr, size_t bytes) {
     }
     cudaError_t e = cudaMallocAsync(d_ptr, cls, g.stream);
     if (e == cudaErrorMemoryAllocation && g.cache_n) {          // short of memory: drop the cache, once more
-        cudaGetLastError();
-        cache_flush(g);
-        cudaStreamSynchronize(g.stream);
+        cache_drop(g);
         e = cudaMallocAsync(d_ptr, cls, g.stream);
     }
     if (e == cudaErrorMemoryAllocation) {
@@ -866,7 +873,9 @@ static adb_status select_prepare(const char *what, const int32_t *d_val, const i
     a->stable_val = stable_val;
     fold_range(lo, hi, &a->range);
     a->d_count = d_count ? d_count : g.scratch_count;
-    if (adb_status s = ensure_select_scratch(a->n)) return s;
+    // the bitmap only ever grows; a select over the largest shard (2^31 rows) needs 256 MB
+    if (adb_status s = grow(g.sel_mask, sizeof(uint32_t) * adb::select_mask_words(a->n, g.sm_count), "select bitmap"))
+        return s;
     a->mask = g.sel_mask; a->counts = g.sel_counts; a->sm_count = g.sm_count;
     return ADB_OK;
 }
@@ -1083,18 +1092,59 @@ adb_status adb_agg_combine(const adb_agg *d_parts, int32_t k, adb_agg *d_out, ad
 }
 
 // ---- aggregate exchange over NVLink peer memory ------------------------------------------
+// The peer setup shared by the IPC path (adb_peer_create / _connect, adb_peer_join_create /
+// _connect) and the one-process path (adb_peer_connect_local, adb_peer_join_connect_local).
+// The mailbox and the receive region may be exported through IPC, so they are plain cudaMalloc
+// blocks of exactly their size.
+
+// Closes the current connection and gives this context a fresh mailbox, zeroed (epoch 0 =
+// nothing arrived yet) and idle before anyone maps it.
+static adb_status peer_mailbox_create() {
+    CU(cudaStreamSynchronize(g.stream));
+    peer_close();
+    if (adb_status s = dev_alloc(g.peer_box, adb::kPeerBoxBytes, "peer mailbox")) return s;
+    CU(cudaMemset(g.peer_box.p, 0, adb::kPeerBoxBytes));
+    CU(cudaDeviceSynchronize());
+    return ADB_OK;
+}
+
+// g.peer_boxes (every rank's mailbox, as this context sees it) -> the device table kernels index.
+static adb_status peer_boxes_upload() {
+    if (adb_status s = grow(g.peer_boxes_dev, sizeof(adb::PeerBoxes), "peer mailbox table")) return s;
+    CU(cudaMemcpy(g.peer_boxes_dev.p, &g.peer_boxes, sizeof(adb::PeerBoxes), cudaMemcpyHostToDevice));
+    g.peer_connected = true;
+    g.peer_epoch = 0;
+    return ADB_OK;
+}
+
+// Closes the current receive region and makes this context's: 2 sides x {values, positions} x
+// `cap` ints, with the table of the peers' regions, the exchange status and the received total.
+static adb_status jx_region_create(unsigned long long cap) {
+    CU(cudaStreamSynchronize(g.stream));
+    jx_close();
+    if (adb_status s = dev_alloc(g.jx_recv, cap * 4 * sizeof(int32_t), "join receive buffer")) return s;
+    if (adb_status s = grow(g.jx_peer_dev, sizeof(uint32_t *) * ADB_MAX_PEERS, "join receive-buffer table")) return s;
+    if (adb_status s = grow(g.jx_status, 4 * sizeof(uint32_t), "join exchange status")) return s;
+    if (adb_status s = grow(g.jx_total, 2 * sizeof(int64_t), "join exchange total")) return s;
+    g.jx_cap = cap;
+    return ADB_OK;
+}
+
+// g.jx_peer_host (every rank's receive region, as this context sees it) -> the device table.
+static adb_status jx_table_upload() {
+    CU(cudaMemcpy(g.jx_peer_dev.p, g.jx_peer_host, sizeof(uint32_t *) * ADB_MAX_PEERS, cudaMemcpyHostToDevice));
+    g.jx_connected = true;
+    return ADB_OK;
+}
+
 adb_status adb_peer_create(int32_t world, int32_t rank, unsigned char *handle_out) {
     NEED_UP();
     static_assert(sizeof(cudaIpcMemHandle_t) == ADB_PEER_HANDLE_BYTES, "handle size");
     if (world < 1 || world > ADB_MAX_PEERS || rank < 0 || rank >= world || !handle_out)
         return fail(ADB_ERR_INVALID, "adb_peer_create: world %d (max %d), rank %d", world, ADB_MAX_PEERS, rank);
-    CU(cudaStreamSynchronize(g.stream));
-    peer_close();
-    CU(cudaMalloc(&g.peer_box, adb::kPeerBoxBytes));
-    CU(cudaMemset(g.peer_box, 0, adb::kPeerBoxBytes));          // epoch 0 = nothing arrived yet
-    CU(cudaDeviceSynchronize());
+    if (adb_status s = peer_mailbox_create()) return s;
     cudaIpcMemHandle_t h;
-    CU(cudaIpcGetMemHandle(&h, g.peer_box));
+    CU(cudaIpcGetMemHandle(&h, g.peer_box.p));
     memcpy(handle_out, &h, sizeof h);
     g.peer_world = world;
     g.peer_rank = rank;
@@ -1104,7 +1154,7 @@ adb_status adb_peer_create(int32_t world, int32_t rank, unsigned char *handle_ou
 
 adb_status adb_peer_connect(const unsigned char *handles) {
     NEED_UP();
-    if (!g.peer_box || !handles) return fail(ADB_ERR_INVALID, "adb_peer_connect: adb_peer_create first");
+    if (!g.peer_box.p || !handles) return fail(ADB_ERR_INVALID, "adb_peer_connect: adb_peer_create first");
     for (int r = 0; r < g.peer_world; ++r) {
         if (r == g.peer_rank) continue;
         cudaIpcMemHandle_t h;
@@ -1118,11 +1168,7 @@ adb_status adb_peer_connect(const unsigned char *handles) {
         }
         g.peer_boxes.box[r] = static_cast<adb::PeerRecord *>(p);
     }
-    CU(cudaMalloc(&g.peer_boxes_dev, sizeof(adb::PeerBoxes)));
-    CU(cudaMemcpy(g.peer_boxes_dev, &g.peer_boxes, sizeof(adb::PeerBoxes), cudaMemcpyHostToDevice));
-    g.peer_connected = true;
-    g.peer_epoch = 0;
-    return ADB_OK;
+    return peer_boxes_upload();
 }
 
 adb_status adb_agg_combine_allreduce(const adb_agg *d_parts, int32_t k, adb_agg *d_out, adb_agg *h_out) {
@@ -1149,26 +1195,19 @@ adb_status adb_peer_join_create(int64_t cap_pairs, unsigned char *handle_out) {
     if (!g.peer_connected) return fail(ADB_ERR_INVALID, "adb_peer_join_create: adb_peer_connect first");
     if (cap_pairs < 1 || cap_pairs >= ((int64_t)1 << 31) || !handle_out)
         return fail(ADB_ERR_INVALID, "adb_peer_join_create: capacity %lld outside [1, 2^31)", (long long)cap_pairs);
-    CU(cudaStreamSynchronize(g.stream));
-    jx_close();
     const unsigned long long cap = ((unsigned long long)cap_pairs + 63) & ~63ull;     // regions stay 256-byte aligned
-    cudaError_t e = cudaMalloc(&g.jx_recv, cap * 4 * sizeof(int32_t));
-    if (e != cudaSuccess) { cudaGetLastError(); return fail(ADB_ERR_NOMEM, "join receive buffer (%llu pairs x 4 regions): %s", cap, cudaGetErrorString(e)); }
-    CU(cudaMalloc(&g.jx_peer_dev, sizeof(uint32_t *) * ADB_MAX_PEERS));
-    CU(cudaMalloc(&g.jx_status, 4 * sizeof(uint32_t)));
-    CU(cudaMalloc(&g.jx_total, 2 * sizeof(int64_t)));
+    if (adb_status s = jx_region_create(cap)) return s;
     CU(cudaDeviceSynchronize());
     cudaIpcMemHandle_t h;
-    CU(cudaIpcGetMemHandle(&h, g.jx_recv));
+    CU(cudaIpcGetMemHandle(&h, g.jx_recv.p));
     memcpy(handle_out, &h, sizeof h);
-    g.jx_cap = cap;
-    g.jx_peer_host[g.peer_rank] = reinterpret_cast<uint32_t *>(g.jx_recv);
+    g.jx_peer_host[g.peer_rank] = reinterpret_cast<uint32_t *>(g.jx_recv.p);
     return ADB_OK;
 }
 
 adb_status adb_peer_join_connect(const unsigned char *handles) {
     NEED_UP();
-    if (!g.jx_recv || !handles) return fail(ADB_ERR_INVALID, "adb_peer_join_connect: adb_peer_join_create first");
+    if (!g.jx_recv.p || !handles) return fail(ADB_ERR_INVALID, "adb_peer_join_connect: adb_peer_join_create first");
     for (int r = 0; r < g.peer_world; ++r) {
         if (r == g.peer_rank) continue;
         cudaIpcMemHandle_t h;
@@ -1181,9 +1220,7 @@ adb_status adb_peer_join_connect(const unsigned char *handles) {
         }
         g.jx_peer_host[r] = static_cast<uint32_t *>(p);
     }
-    CU(cudaMemcpy(g.jx_peer_dev, g.jx_peer_host, sizeof(uint32_t *) * ADB_MAX_PEERS, cudaMemcpyHostToDevice));
-    g.jx_connected = true;
-    return ADB_OK;
+    return jx_table_upload();
 }
 
 adb_status adb_peer_exchange_pairs(int32_t side, const int32_t *d_val, const int32_t *d_pos, int64_t n,
@@ -1285,12 +1322,7 @@ adb_status adb_peer_connect_local(int32_t world) {
         g_cur = r;
         auto one = [&]() -> adb_status {
             CU(cudaSetDevice(g.device));
-            CU(cudaStreamSynchronize(g.stream));
-            peer_close();
-            CU(cudaMalloc(&g.peer_box, adb::kPeerBoxBytes));
-            CU(cudaMemset(g.peer_box, 0, adb::kPeerBoxBytes));
-            CU(cudaDeviceSynchronize());
-            return ADB_OK;
+            return peer_mailbox_create();
         };
         rc = one();
     }
@@ -1302,11 +1334,7 @@ adb_status adb_peer_connect_local(int32_t world) {
             g.peer_world = world;
             g.peer_rank = r;
             g.peer_local = true;
-            CU(cudaMalloc(&g.peer_boxes_dev, sizeof(adb::PeerBoxes)));
-            CU(cudaMemcpy(g.peer_boxes_dev, &g.peer_boxes, sizeof(adb::PeerBoxes), cudaMemcpyHostToDevice));
-            g.peer_connected = true;
-            g.peer_epoch = 0;
-            return ADB_OK;
+            return peer_boxes_upload();
         };
         rc = one();
     }
@@ -1327,15 +1355,7 @@ adb_status adb_peer_join_connect_local(int64_t cap_pairs) {
         g_cur = r;
         auto one = [&]() -> adb_status {
             CU(cudaSetDevice(g.device));
-            CU(cudaStreamSynchronize(g.stream));
-            jx_close();
-            cudaError_t e = cudaMalloc(&g.jx_recv, cap * 4 * sizeof(int32_t));
-            if (e != cudaSuccess) { cudaGetLastError(); return fail(ADB_ERR_NOMEM, "join receive buffer (%llu pairs x 4 regions): %s", cap, cudaGetErrorString(e)); }
-            CU(cudaMalloc(&g.jx_peer_dev, sizeof(uint32_t *) * ADB_MAX_PEERS));
-            CU(cudaMalloc(&g.jx_status, 4 * sizeof(uint32_t)));
-            CU(cudaMalloc(&g.jx_total, 2 * sizeof(int64_t)));
-            g.jx_cap = cap;
-            return ADB_OK;
+            return jx_region_create(cap);
         };
         rc = one();
     }
@@ -1343,10 +1363,8 @@ adb_status adb_peer_join_connect_local(int64_t cap_pairs) {
         g_cur = r;
         auto one = [&]() -> adb_status {
             CU(cudaSetDevice(g.device));
-            for (int q = 0; q < world; ++q) g.jx_peer_host[q] = reinterpret_cast<uint32_t *>(g_ctx[q].jx_recv);
-            CU(cudaMemcpy(g.jx_peer_dev, g.jx_peer_host, sizeof(uint32_t *) * ADB_MAX_PEERS, cudaMemcpyHostToDevice));
-            g.jx_connected = true;
-            return ADB_OK;
+            for (int q = 0; q < world; ++q) g.jx_peer_host[q] = reinterpret_cast<uint32_t *>(g_ctx[q].jx_recv.p);
+            return jx_table_upload();
         };
         rc = one();
     }
@@ -1693,19 +1711,17 @@ static adb_status shared_select_count_impl(const int32_t *d_col, int64_t n, cons
         return fail(ADB_ERR_INVALID, "adb_shared_select_count: q_count %d outside [1, %d] (server.c:366-371 chunks "
                     "batches to 150)", q_count, ADB_MAX_BATCH);
     if (!lows || !highs || (n > 0 && !d_col)) return fail(ADB_ERR_INVALID, "adb_shared_select_count: NULL pointer");
-    if (!g.ss_plan_mem) {
-        CU(cudaMalloc(&g.ss_plan_mem, kSsPlanBytes));
-        CU(cudaMalloc(&g.ss_counts, sizeof(uint32_t) * ADB_MAX_BATCH * kSsMaxChunks));
-        CU(cudaMalloc(&g.ss_totals, sizeof(int64_t) * ADB_MAX_BATCH));
-        CU(cudaMalloc(&g.ss_outs, sizeof(int32_t *) * ADB_MAX_BATCH));
-        CU(cudaMalloc(&g.ss_chunk_hits, sizeof(uint32_t) * kSsMaxChunks));
-    }
+    if (adb_status s = grow(g.ss_plan_mem, kSsPlanBytes, "shared scan plan")) return s;
+    if (adb_status s = grow(g.ss_counts, sizeof(uint32_t) * ADB_MAX_BATCH * kSsMaxChunks, "shared scan counts")) return s;
+    if (adb_status s = grow(g.ss_totals, sizeof(int64_t) * ADB_MAX_BATCH, "shared scan totals")) return s;
+    if (adb_status s = grow(g.ss_outs, sizeof(int32_t *) * ADB_MAX_BATCH, "shared scan outputs")) return s;
+    if (adb_status s = grow(g.ss_chunk_hits, sizeof(uint32_t) * kSsMaxChunks, "shared scan chunk hits")) return s;
     SsHostPlan hp;
     ss_build_plan(lows, highs, q_count, &hp);
     // one packed upload, staged through a pinned slot (the host vector goes out of scope below)
     if (adb_status s = upload_blob(g.ss_plan_mem, hp.bytes.data(), hp.bytes.size())) return s;
     const uint32_t m = hp.m, lut_shift = hp.lut_shift, bit_shift = hp.bit_shift, span = hp.span, deepest = hp.deepest;
-    g.ss_plan = adb::SharedScanPlan{reinterpret_cast<const int32_t *>(g.ss_plan_mem),
+    g.ss_plan = adb::SharedScanPlan{reinterpret_cast<const int32_t *>(g.ss_plan_mem.p),
                                     reinterpret_cast<const uint16_t *>(g.ss_plan_mem + kSsBoundsBytes),
                                     g.ss_plan_mem + kSsCovOff, m, (uint32_t)q_count,
                                     reinterpret_cast<const uint16_t *>(g.ss_plan_mem + kSsLutOff),
@@ -1728,12 +1744,7 @@ static adb_status shared_select_count_impl(const int32_t *d_col, int64_t n, cons
         g.ss_plan.pair_depth = deepest;
         rows *= deepest;
     }
-    if (rows > g.ss_hits_rows) {
-        if (g.ss_hits) { CU(cudaStreamSynchronize(g.stream)); CU(cudaFree(g.ss_hits)); g.ss_hits = nullptr; g.ss_hits_rows = 0; }
-        cudaError_t e = cudaMalloc(&g.ss_hits, (rows + rows / 8 + 4096) * sizeof(uint32_t));
-        if (e != cudaSuccess) { cudaGetLastError(); return fail(ADB_ERR_NOMEM, "shared scan hit-list scratch: %s", cudaGetErrorString(e)); }
-        g.ss_hits_rows = rows + rows / 8 + 4096;
-    }
+    if (adb_status s = grow(g.ss_hits, rows * sizeof(uint32_t), "shared scan hit lists")) return s;
     const int k_ = adb::launch_shared_classify(d_col, (uint32_t)n, g.ss_plan, g.ss_geom, g.ss_hits,
                                                g.ss_chunk_hits, g.ss_counts, g.ss_totals, g.stream);
     if (adb_status s = after_launch("shared_classify", k_)) return s;
@@ -1789,23 +1800,14 @@ adb_status adb_shared_select(const int32_t *d_col, int64_t n, const int32_t *low
 
 // ---- radix sort / partition helpers ---------------------------------------------------------
 static adb_status ensure_radix_scratch(uint32_t n) {
-    if (!g.rx_totals) {
-        CU(cudaMalloc(&g.rx_totals, sizeof(uint32_t) * 256 * 256));     // <= 256 segments (segmented pass)
-        CU(cudaMalloc(&g.rx_base, sizeof(uint32_t) * 256 * 256));
-        CU(cudaMalloc(&g.sc_sums, sizeof(unsigned long long) * (size_t)(g.sm_count * 2 + 8)));
-    }
+    // <= 256 segments (segmented pass)
+    if (adb_status s = grow(g.rx_totals, sizeof(uint32_t) * 256 * 256, "radix totals")) return s;
+    if (adb_status s = grow(g.rx_base, sizeof(uint32_t) * 256 * 256, "radix bases")) return s;
+    if (adb_status s = grow(g.sc_sums, sizeof(unsigned long long) * (size_t)(g.sm_count * 2 + 8), "scan chunk sums"))
+        return s;
     // [segment][bucket][tiles per segment]: <= 256 segments, the last one padded
-    const size_t need = 256 * ((size_t)adb::radix_geom(n, g.sm_count).ctas + 256);
-    if (need <= g.rx_hist_elems) return ADB_OK;
-    CU(cudaStreamSynchronize(g.stream));
-    if (g.rx_hist) CU(cudaFree(g.rx_hist));
-    g.rx_hist = nullptr;
-    g.rx_hist_elems = 0;
-    const size_t want = need + need / 4 + 256 * 64;
-    cudaError_t e = cudaMalloc(&g.rx_hist, want * sizeof(uint32_t));
-    if (e != cudaSuccess) { cudaGetLastError(); return fail(ADB_ERR_NOMEM, "radix histogram: %s", cudaGetErrorString(e)); }
-    g.rx_hist_elems = want;
-    return ADB_OK;
+    return grow(g.rx_hist, sizeof(uint32_t) * 256 * ((size_t)adb::radix_geom(n, g.sm_count).ctas + 256),
+                "radix histogram");
 }
 
 // ---- scratch arena ------------------------------------------------------------------------------
@@ -1817,19 +1819,7 @@ static adb_status arena_reserve(size_t bytes) {
     g.join = Engine::JoinState{};
     g.del_rows = -1;
     g.arena_used = 0;
-    if (bytes <= g.arena_cap) return ADB_OK;
-    CU(cudaStreamSynchronize(g.stream));
-    if (g.arena) CU(cudaFree(g.arena));
-    g.arena = nullptr;
-    g.arena_cap = 0;
-    const size_t want = bytes + bytes / 8 + (1 << 20);
-    cudaError_t e = cudaMalloc(&g.arena, want);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        return fail(ADB_ERR_NOMEM, "sort/join scratch of %zu bytes: %s", want, cudaGetErrorString(e));
-    }
-    g.arena_cap = want;
-    return ADB_OK;
+    return grow(g.arena, bytes, "sort/join scratch");
 }
 static void *arena_take_bytes(size_t bytes) {
     void *p = g.arena + g.arena_used;
@@ -1933,29 +1923,14 @@ adb_status adb_route_pairs(const int32_t *d_val, const int32_t *d_pos, int64_t n
 }
 
 // ---- bulk CSV load ---------------------------------------------------------------------------------
-static adb_status csv_grow_bytes(void **p, size_t *cap, size_t need, size_t elem) {
-    if (need <= *cap) return ADB_OK;
-    if (*p) { CU(cudaStreamSynchronize(g.stream)); CU(cudaFree(*p)); }
-    *p = nullptr;
-    *cap = 0;
-    const size_t want = need + need / 8 + 1024;
-    cudaError_t e = cudaMalloc(p, want * elem);
-    if (e != cudaSuccess) { cudaGetLastError(); return fail(ADB_ERR_NOMEM, "csv scratch (%zu elements): %s", want, cudaGetErrorString(e)); }
-    *cap = want;
-    return ADB_OK;
-}
-#define csv_grow(pp, cap, need) csv_grow_bytes(reinterpret_cast<void **>(pp), cap, need, sizeof(**(pp)))
-
 adb_status adb_csv_index(const char *d_text, size_t bytes, int32_t skip_lines, int64_t *h_rows) {
     NEED_UP();
     auto &c = g.csv;
     c.ready = false;
     if (skip_lines < 0 || !h_rows || (bytes && !d_text)) return fail(ADB_ERR_INVALID, "adb_csv_index: bad arguments");
-    if (!c.col_table) {
-        CU(cudaMalloc(&c.col_table, 256 * sizeof(int32_t *)));
-        CU(cudaMalloc(&c.flags, 4 * sizeof(uint32_t)));
-        CU(cudaMalloc(&c.total, 2 * sizeof(int64_t)));
-    }
+    if (adb_status s = grow(c.col_table, 256 * sizeof(int32_t *), "csv column table")) return s;
+    if (adb_status s = grow(c.flags, 4 * sizeof(uint32_t), "csv flags")) return s;
+    if (adb_status s = grow(c.total, 2 * sizeof(int64_t), "csv line count")) return s;
     c.text = reinterpret_cast<const unsigned char *>(d_text);
     c.bytes = bytes;
     c.skip = (uint32_t)skip_lines;
@@ -1964,9 +1939,8 @@ adb_status adb_csv_index(const char *d_text, size_t bytes, int32_t skip_lines, i
     if (bytes == 0) { *h_rows = 0; c.ready = true; return ADB_OK; }
     if (reinterpret_cast<uintptr_t>(d_text) & 15u) return fail(ADB_ERR_INVALID, "adb_csv_index: text must be 16-byte aligned (adb_alloc is)");
     const uint32_t blocks = adb::csv_blocks(bytes);
-    size_t cap2 = c.blocks_cap;
-    if (adb_status s = csv_grow(&c.block_counts, &c.blocks_cap, blocks)) return s;
-    if (adb_status s = csv_grow(&c.block_base, &cap2, blocks)) return s;
+    if (adb_status s = grow(c.block_counts, sizeof(uint32_t) * blocks, "csv block counts")) return s;
+    if (adb_status s = grow(c.block_base, sizeof(uint32_t) * blocks, "csv block bases")) return s;
     if (adb_status s = ensure_radix_scratch(1)) return s;            // the scan's chunk sums live there
     int k_ = adb::launch_csv_count(c.text, bytes, c.block_counts, g.stream);
     k_ += adb::launch_exclusive_scan(c.block_counts, 1, c.block_base, blocks, g.sc_sums, c.total, g.sm_count, g.stream);
@@ -1976,7 +1950,7 @@ adb_status adb_csv_index(const char *d_text, size_t bytes, int32_t skip_lines, i
     CU(cudaMemcpyAsync(&last, c.text + bytes - 1, 1, cudaMemcpyDeviceToHost, g.stream));
     CU(cudaStreamSynchronize(g.stream));
     if (newlines >= (int64_t)1 << 32) return fail(ADB_ERR_INVALID, "adb_csv_index: %lld lines in one call; split the text at a line boundary", (long long)newlines);
-    if (adb_status s = csv_grow(&c.line_end, &c.lines_cap, (size_t)newlines + 1)) return s;
+    if (adb_status s = grow(c.line_end, sizeof(unsigned long long) * ((size_t)newlines + 1), "csv line ends")) return s;
     k_ += adb::launch_csv_index(c.text, bytes, c.block_base, c.line_end, g.stream);
     if (adb_status s = after_launch("csv_index", k_)) return s;
     const unsigned long long lines = (unsigned long long)newlines + (last != '\n' ? 1 : 0);
@@ -1997,7 +1971,7 @@ adb_status adb_csv_parse(int32_t n_cols, int32_t *const *d_cols) {
     if (c.rows == 0) return ADB_OK;
     for (int32_t i = 0; i < n_cols; ++i)
         if (!d_cols[i]) return fail(ADB_ERR_INVALID, "adb_csv_parse: column %d is NULL", i);
-    if (adb_status s = csv_grow(&c.n_fields, &c.fields_cap, (size_t)c.rows)) return s;
+    if (adb_status s = grow(c.n_fields, (size_t)c.rows, "csv field counts")) return s;
     if (adb_status s = upload_blob(c.col_table, d_cols, sizeof(int32_t *) * n_cols)) return s;
     CU(cudaMemsetAsync(c.flags, 0, 4 * sizeof(uint32_t), g.stream));
     int k_ = adb::launch_csv_parse(c.text, c.bytes, c.line_end, c.newlines, c.skip, c.rows, (uint32_t)n_cols,
@@ -2027,10 +2001,10 @@ adb_status adb_format_i32_count(const int32_t *d_val, int64_t n, int64_t *h_byte
     f.n = n;
     f.bytes = 0;
     if (n == 0) { *h_bytes = 0; f.ready = true; return ADB_OK; }
-    if (!f.total) CU(cudaMalloc(&f.total, 2 * sizeof(int64_t)));
+    if (adb_status s = grow(f.total, 2 * sizeof(int64_t), "print byte count")) return s;
     const uint32_t blocks = adb::fmt_blocks(n);
-    if (adb_status s = csv_grow(&f.block_len, &f.cap_len, blocks)) return s;
-    if (adb_status s = csv_grow(&f.block_off, &f.cap_off, blocks)) return s;
+    if (adb_status s = grow(f.block_len, sizeof(uint32_t) * blocks, "print block lengths")) return s;
+    if (adb_status s = grow(f.block_off, sizeof(uint32_t) * blocks, "print block offsets")) return s;
     if (adb_status s = ensure_radix_scratch(1)) return s;
     int k_ = adb::launch_fmt_len(d_val, n, f.block_len, g.stream);
     k_ += adb::launch_exclusive_scan(f.block_len, 1, f.block_off, blocks, g.sc_sums, f.total, g.sm_count, g.stream);
@@ -2148,19 +2122,11 @@ static adb_status join_build(const int32_t *bv, const int32_t *bp, uint32_t nb, 
                                          g.stream);
     unsigned long long slots = 0;
     if (adb_status s = read_back(&slots, toff + num_parts, sizeof slots)) return s;
-    if (slots > g.hj_table_slots) {
-        if (g.hj_table) CU(cudaFree(g.hj_table));
-        g.hj_table = nullptr;
-        g.hj_table_slots = 0;
-        const unsigned long long want = slots + slots / 8 + 4096;
-        cudaError_t e = cudaMalloc(&g.hj_table, want * 16);
-        if (e != cudaSuccess) { cudaGetLastError(); return fail(ADB_ERR_NOMEM, "join tables (%llu slots): %s", want, cudaGetErrorString(e)); }
-        g.hj_table_slots = want;
-    }
+    if (adb_status s = grow(g.hj_table, slots * 16, "join tables")) return s;
     tr.lap("partition boundaries");
     // 3. one table per partition
     *launches += adb::launch_hj_table_build(bk, j.build_pos_sorted, off1, toff, num_parts, part_bits,
-                                            static_cast<uint4 *>(g.hj_table), g.stream);
+                                            g.hj_table, g.stream);
     tr.lap("per-partition tables");
     return ADB_OK;
 }
@@ -2212,11 +2178,11 @@ static adb_status join_count(const int32_t *bv, const int32_t *bp, int64_t nb64,
         // (the pass' scanned histogram stays in g.rx_hist: where each 4096-row tile's entries
         // sit inside the cells)
         launches += adb::launch_hj_probe_partitioned(pk, rows, g.rx_base, g.rx_hist, segs, seg_tiles, np, j.pg,
-                                                     j.toff, j.part_bits, static_cast<const uint4 *>(g.hj_table),
+                                                     j.toff, j.part_bits, g.hj_table,
                                                      res, j.gc_by_j, j.warp_base, chunk_sums, tot, g.stream);
     } else {
         launches += adb::launch_hj_probe(reinterpret_cast<const uint32_t *>(pv), np, j.pg, j.toff, j.part_bits,
-                                         static_cast<const uint4 *>(g.hj_table), j.gc_by_j, j.warp_base, tot,
+                                         g.hj_table, j.gc_by_j, j.warp_base, tot,
                                          g.stream);
     }
     if (adb_status s = read_back(&j.matches, tot, sizeof(int64_t))) return s;
@@ -2290,7 +2256,7 @@ adb_status adb_join_route_probe(int32_t world, const int32_t *d_pv, int64_t np64
     j.rt_keys = ARENA_TAKE(uint32_t, np);
     j.rt_rows = ARENA_TAKE(uint32_t, np);
     j.rt_res = ARENA_TAKE(uint2, np);
-    if (g.arena_used > g.arena_cap) return fail(ADB_ERR_NOMEM, "adb_join_route_probe: scratch arena too small");
+    if (g.arena_used > g.arena.cap) return fail(ADB_ERR_NOMEM, "adb_join_route_probe: scratch arena too small");
     const int k_ = adb::launch_radix_pass_segmented(reinterpret_cast<const uint32_t *>(d_pv), nullptr, j.rt_keys,
                                                     j.rt_rows, np, adb::RadixPass{32 - bits, bits, 2}, 0, g.rx_hist,
                                                     g.rx_totals, g.rx_base, g.sm_count, g.stream);
@@ -2308,26 +2274,10 @@ adb_status adb_join_recv_buffers(int64_t n_recv, int32_t **d_keys, void **d_answ
     NEED_UP();
     if (adb_status s = check_len(n_recv, "adb_join_recv_buffers")) return s;
     if (!d_keys || !d_answers) return fail(ADB_ERR_INVALID, "adb_join_recv_buffers: NULL pointer");
-    if ((size_t)n_recv > g.rt_recv_cap) {
-        CU(cudaStreamSynchronize(g.stream));
-        if (g.rt_recv_keys) CU(cudaFree(g.rt_recv_keys));
-        if (g.rt_recv_res) CU(cudaFree(g.rt_recv_res));
-        g.rt_recv_keys = nullptr;
-        g.rt_recv_res = nullptr;
-        g.rt_recv_cap = 0;
-        const size_t want = (size_t)n_recv + (size_t)n_recv / 8 + 4096;
-        cudaError_t e = cudaMalloc(&g.rt_recv_keys, want * 4);
-        if (e == cudaSuccess) e = cudaMalloc(&g.rt_recv_res, want * 8);
-        if (e != cudaSuccess) {
-            cudaGetLastError();
-            if (g.rt_recv_keys) cudaFree(g.rt_recv_keys);
-            g.rt_recv_keys = nullptr;
-            return fail(ADB_ERR_NOMEM, "routed probe: %zu received keys: %s", want, cudaGetErrorString(e));
-        }
-        g.rt_recv_cap = want;
-    }
-    *d_keys = reinterpret_cast<int32_t *>(g.rt_recv_keys);
-    *d_answers = g.rt_recv_res;
+    if (adb_status s = grow(g.rt_recv_keys, (size_t)n_recv * 4, "routed probe: received keys")) return s;
+    if (adb_status s = grow(g.rt_recv_res, (size_t)n_recv * 8, "routed probe: answers")) return s;
+    *d_keys = reinterpret_cast<int32_t *>(g.rt_recv_keys.p);
+    *d_answers = g.rt_recv_res.p;
     return ADB_OK;
 }
 
@@ -2336,7 +2286,8 @@ adb_status adb_join_probe_received(int64_t n_recv) {
     auto &j = g.join;
     if (!j.built) return fail(ADB_ERR_INVALID, "adb_join_probe_received: no tables on this context");
     if (adb_status s = check_len(n_recv, "adb_join_probe_received")) return s;
-    if ((size_t)n_recv > g.rt_recv_cap) return fail(ADB_ERR_INVALID, "adb_join_probe_received: more keys than adb_join_recv_buffers made room for");
+    if ((size_t)n_recv * 4 > g.rt_recv_keys.cap || (size_t)n_recv * 8 > g.rt_recv_res.cap)
+        return fail(ADB_ERR_INVALID, "adb_join_probe_received: more keys than adb_join_recv_buffers made room for");
     if (n_recv == 0) return ADB_OK;
     const uint32_t n = (uint32_t)n_recv;
     StageTrace tr;
@@ -2364,7 +2315,7 @@ adb_status adb_join_probe_received(int64_t n_recv) {
         // (what adb_join_finish_routed still takes for this context's own probe rows stays free)
         const size_t finish = arena_round((size_t)j.rt_rows_n * 8) + arena_round(((size_t)j.rt_rows_n / 512 + 8) * 8) +
                               (1 << 20);
-        if (g.arena_used + need + finish <= g.arena_cap) {
+        if (g.arena_used + need + finish <= g.arena.cap) {
             uint32_t *pk = ARENA_TAKE(uint32_t, n), *rows = ARENA_TAKE(uint32_t, n);
             uint2 *res = ARENA_TAKE(uint2, n);
             uint32_t *hist = ARENA_TAKE(uint32_t, hist_elems);
@@ -2375,7 +2326,7 @@ adb_status adb_join_probe_received(int64_t n_recv) {
             k_ += adb::launch_radix_pass_segmented(g.rt_recv_keys, nullptr, pk, rows, n, adb::RadixPass{24, 8, 1},
                                                    want_tiles, hist, totals, base, g.sm_count, g.stream);
             k_ += adb::launch_hj_probe_partitioned(pk, rows, base, hist, segs, seg_tiles, n, pg, j.toff, j.part_bits,
-                                                   static_cast<const uint4 *>(g.hj_table), res, g.rt_recv_res, sums,
+                                                   g.hj_table, res, g.rt_recv_res, sums,
                                                    chunk_sums, tot, g.stream);
         } else {
             partitioned = false;
@@ -2384,8 +2335,8 @@ adb_status adb_join_probe_received(int64_t n_recv) {
     if (!partitioned) {
         const adb::HjProbeGeom pg = adb::hj_probe_geom(n, g.sm_count);
         unsigned long long *sums = ARENA_TAKE(unsigned long long, pg.warps);
-        if (g.arena_used > g.arena_cap) return fail(ADB_ERR_NOMEM, "adb_join_probe_received: scratch arena too small");
-        k_ += adb::launch_hj_probe_plain(g.rt_recv_keys, n, j.toff, j.part_bits, static_cast<const uint4 *>(g.hj_table),
+        if (g.arena_used > g.arena.cap) return fail(ADB_ERR_NOMEM, "adb_join_probe_received: scratch arena too small");
+        k_ += adb::launch_hj_probe_plain(g.rt_recv_keys, n, j.toff, j.part_bits, g.hj_table,
                                          g.rt_recv_res, sums, g.sm_count, g.stream);
     }
     if (adb_status s = after_launch("join_probe_received", k_)) return s;
@@ -2429,7 +2380,7 @@ adb_status adb_join_finish_routed(int32_t world, const int32_t *d_pv, const int3
     j.gc_by_j = ARENA_TAKE(uint2, np);
     j.warp_base = ARENA_TAKE(unsigned long long, j.pg.warps);
     unsigned long long *chunk_sums = ARENA_TAKE(unsigned long long, j.pg.warps / 1024 + 2);
-    if (g.arena_used > g.arena_cap) return fail(ADB_ERR_NOMEM, "adb_join_finish_routed: scratch arena too small");
+    if (g.arena_used > g.arena.cap) return fail(ADB_ERR_NOMEM, "adb_join_finish_routed: scratch arena too small");
     StageTrace tr;
     int launches = adb::launch_hj_unpartition_routed(j.rt_rows, j.rt_res, g.rx_base, g.rx_hist, np, (uint32_t)world,
                                                      j.pg, j.gc_by_j, j.warp_base, chunk_sums, tot, g.stream);
@@ -2527,16 +2478,7 @@ adb_status adb_peer_exchange_reserve(int64_t send_pairs, int64_t build_pairs, in
         return s;
     // tables: <= 2.5 slots per build row (power-of-two capacity at <= 80 % load) + 16 per partition
     const unsigned long long slots = (unsigned long long)nb * 5 / 2 + 16ull * num_parts + 4096;
-    if (slots > g.hj_table_slots) {
-        CU(cudaStreamSynchronize(g.stream));
-        if (g.hj_table) CU(cudaFree(g.hj_table));
-        g.hj_table = nullptr;
-        g.hj_table_slots = 0;
-        cudaError_t e = cudaMalloc(&g.hj_table, slots * 16);
-        if (e != cudaSuccess) { cudaGetLastError(); return fail(ADB_ERR_NOMEM, "join tables (%llu slots): %s", slots, cudaGetErrorString(e)); }
-        g.hj_table_slots = slots;
-    }
-    return ADB_OK;
+    return grow(g.hj_table, slots * 16, "join tables");
 }
 
 adb_status adb_hash_join_count(const int32_t *d_v1, const int32_t *d_p1, int64_t n1,
@@ -2584,7 +2526,7 @@ struct adb_index {
     const int32_t *values;
     const int32_t *positions;
     int64_t n;
-    int32_t *tree_mem;
+    DevBuf<int32_t> tree_mem;
     adb::BTreeView tree;
     bool slice = false;
 };
@@ -2595,7 +2537,7 @@ adb_status adb_index_create(const int32_t *d_values, const int32_t *d_positions,
     if (adb_status s = check_len(n, "adb_index_create")) return s;
     if (!out || (n > 0 && (!d_values || !d_positions)))
         return fail(ADB_ERR_INVALID, "adb_index_create: NULL pointer");
-    adb_index *ix = new adb_index{d_values, d_positions, n, nullptr, adb::BTreeView{}, false};
+    adb_index *ix = new adb_index{d_values, d_positions, n, DevBuf<int32_t>{}, adb::BTreeView{}, false};
     if (with_btree && n > 32) {
         int64_t lens[adb::kBTreeMaxDepth], total = 0;
         int depth = 0;
@@ -2604,11 +2546,9 @@ adb_status adb_index_create(const int32_t *d_values, const int32_t *d_positions,
             total += len;
             if (len <= 32 || depth == adb::kBTreeMaxDepth) break;
         }
-        cudaError_t e = cudaMalloc(&ix->tree_mem, total * sizeof(int32_t));
-        if (e != cudaSuccess) {
-            cudaGetLastError();
+        if (adb_status s = dev_alloc(ix->tree_mem, total * sizeof(int32_t), "adb_index_create: B+-tree")) {
             delete ix;
-            return fail(ADB_ERR_NOMEM, "adb_index_create: %s", cudaGetErrorString(e));
+            return s;
         }
         int32_t *p = ix->tree_mem;
         const int32_t *below = d_values;
@@ -2623,7 +2563,7 @@ adb_status adb_index_create(const int32_t *d_values, const int32_t *d_positions,
             p += lens[l];
         }
         ix->tree.depth = depth;
-        if (adb_status s = after_launch("btree_level", launches)) { cudaFree(ix->tree_mem); delete ix; return s; }
+        if (adb_status s = after_launch("btree_level", launches)) { release(ix->tree_mem); delete ix; return s; }
     }
     *out = ix;
     return ADB_OK;
@@ -2643,7 +2583,7 @@ adb_status adb_index_destroy(adb_index *ix) {
     NEED_UP();
     if (!ix) return ADB_OK;
     CU(cudaStreamSynchronize(g.stream));
-    if (ix->tree_mem) cudaFree(ix->tree_mem);
+    release(ix->tree_mem);
     delete ix;
     return ADB_OK;
 }
