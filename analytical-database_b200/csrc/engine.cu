@@ -29,6 +29,14 @@ template <class T> struct DevBuf {
     operator T *() const { return p; }
 };
 
+// Home side of a routed exchange (adb_engine.h), in the arena: this context's items grouped by
+// owner, their row numbers, and where the owners' answers are collected
+struct RouteState {
+    uint32_t *items = nullptr, *rows = nullptr;
+    void *answers = nullptr;
+    uint32_t n = 0;
+};
+
 struct Engine {
     bool up = false;
     int32_t ctx_index = 0;
@@ -77,11 +85,7 @@ struct Engine {
         uint2 *gc_by_j = nullptr;           // {group start, match count} per probe row
         unsigned long long *warp_base = nullptr;   // first output slot of every probing warp (pg.warps)
         adb::HjProbeGeom pg{};
-        // routed probe (adb_join_route_probe): this context's probe keys / row numbers by owner,
-        // and where the owners' answers are collected (arena)
-        uint32_t *rt_keys = nullptr, *rt_rows = nullptr;
-        uint2 *rt_res = nullptr;
-        uint32_t rt_rows_n = 0;
+        RouteState route;                   // routed probe (adb_join_route_probe), 8-byte answers
         bool routed = false;
         int32_t *build_pos_sorted = nullptr;   // all three live in the arena
         const int32_t *probe_pos = nullptr;
@@ -104,9 +108,9 @@ struct Engine {
     int64_t del_rows = -1;
     // join tables: one open-addressing table per build partition, 16-byte slots (grow-only)
     DevBuf<uint4> hj_table;
-    // routed probe, owner side: the keys other contexts sent here and the answers (grow-only)
-    uint32_t *rt32_pos = nullptr, *rt32_rows = nullptr, *rt32_val = nullptr;   // routed fetch (arena)
-    uint32_t rt32_n = 0;
+    // routed fetch (adb_route_rows), 4-byte answers: apart from the join's, which it may run beside
+    RouteState fetch_route;
+    // routed exchange, owner side: the items other contexts sent here and the answers (grow-only)
     DevBuf<uint32_t> rt_recv_keys;
     DevBuf<uint2> rt_recv_res;
     // bulk CSV load state (adb_csv_index -> adb_csv_parse); scratch is grow-only
@@ -1373,28 +1377,33 @@ adb_status adb_peer_join_connect_local(int64_t cap_pairs) {
     return rc;
 }
 
-// Copy between contexts (peer DMA when the devices differ), ordered on the CURRENT context's
-// stream after everything already enqueued on the source context's stream.
-adb_status adb_copy_from_ctx(void *d_dst, int32_t src_ctx, const void *d_src, size_t bytes) {
+// The current context's stream waits for everything enqueued so far on context `other`'s stream
+// (`what` names the caller in errors).
+static adb_status ctx_wait(int32_t other, const char *what) {
     NEED_UP();
-    if (src_ctx < 0 || src_ctx >= ADB_MAX_CONTEXTS || !g_ctx[src_ctx].up)
-        return fail(ADB_ERR_INVALID, "adb_copy_from_ctx: context %d is not initialised", src_ctx);
-    if (bytes == 0) return ADB_OK;
-    if (!d_dst || !d_src) return fail(ADB_ERR_INVALID, "adb_copy_from_ctx: NULL pointer");
-    Engine &src = g_ctx[src_ctx];
-    if (&src != &g) {
-        // the source bytes are produced on the source context's stream
-        cudaEvent_t ev;
-        CU(cudaSetDevice(src.device));
-        CU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-        CU(cudaEventRecord(ev, src.stream));
-        CU(cudaSetDevice(g.device));
-        CU(cudaStreamWaitEvent(g.stream, ev, 0));
-        CU(cudaEventDestroy(ev));                  // released once the wait has consumed it
-    }
-    if (src.device == g.device) CU(cudaMemcpyAsync(d_dst, d_src, bytes, cudaMemcpyDeviceToDevice, g.stream));
-    else CU(cudaMemcpyPeerAsync(d_dst, g.device, d_src, src.device, bytes, g.stream));
+    if (other < 0 || other >= ADB_MAX_CONTEXTS || !g_ctx[other].up)
+        return fail(ADB_ERR_INVALID, "%s: context %d is not initialised", what, other);
+    Engine &o = g_ctx[other];
+    if (&o == &g) return ADB_OK;
+    cudaEvent_t ev;
+    CU(cudaSetDevice(o.device));
+    CU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
+    CU(cudaEventRecord(ev, o.stream));
+    CU(cudaSetDevice(g.device));
+    CU(cudaStreamWaitEvent(g.stream, ev, 0));
+    CU(cudaEventDestroy(ev));                      // released once the wait has consumed it
     return ADB_OK;
+}
+
+adb_status adb_ctx_wait(int32_t other_ctx) { return ctx_wait(other_ctx, "adb_ctx_wait"); }
+
+// Copy between contexts (peer DMA when the devices differ), ordered on the CURRENT context's
+// stream after everything already enqueued on the source context's stream: the wait, then the
+// _ready copy.
+adb_status adb_copy_from_ctx(void *d_dst, int32_t src_ctx, const void *d_src, size_t bytes) {
+    if (bytes)
+        if (adb_status s = ctx_wait(src_ctx, "adb_copy_from_ctx")) return s;
+    return adb_copy_from_ctx_ready(d_dst, src_ctx, d_src, bytes);
 }
 
 // The same copy when the caller KNOWS the source bytes are complete (the source context has
@@ -1409,23 +1418,6 @@ adb_status adb_copy_from_ctx_ready(void *d_dst, int32_t src_ctx, const void *d_s
     const Engine &src = g_ctx[src_ctx];
     if (src.device == g.device) CU(cudaMemcpyAsync(d_dst, d_src, bytes, cudaMemcpyDeviceToDevice, g.stream));
     else CU(cudaMemcpyPeerAsync(d_dst, g.device, d_src, src.device, bytes, g.stream));
-    return ADB_OK;
-}
-
-// The current context's stream waits for everything enqueued so far on `other_ctx`'s stream.
-adb_status adb_ctx_wait(int32_t other_ctx) {
-    NEED_UP();
-    if (other_ctx < 0 || other_ctx >= ADB_MAX_CONTEXTS || !g_ctx[other_ctx].up)
-        return fail(ADB_ERR_INVALID, "adb_ctx_wait: context %d is not initialised", other_ctx);
-    Engine &o = g_ctx[other_ctx];
-    if (&o == &g) return ADB_OK;
-    cudaEvent_t ev;
-    CU(cudaSetDevice(o.device));
-    CU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-    CU(cudaEventRecord(ev, o.stream));
-    CU(cudaSetDevice(g.device));
-    CU(cudaStreamWaitEvent(g.stream, ev, 0));
-    CU(cudaEventDestroy(ev));
     return ADB_OK;
 }
 
@@ -2061,14 +2053,13 @@ struct StageTrace {
 // leaves {build_pos_sorted, toff, part_bits} in g.join and the tables in g.hj_table.  The arena
 // is reserved for the build AND for `np` probe rows' worth of {group, count} + offsets.
 // Probe rows partitioned for L2 locality (hash_join.cu, P1-P3) when the tables will not fit L2
-// by a wide margin: ~21 bytes of table per build row against 126 MB.  ADB_JOIN_PROBE=direct /
+// by a wide margin (`by_size`: each caller's own size rule).  ADB_JOIN_PROBE=direct /
 // partitioned overrides (tests run both forms on the same inputs).
-static bool join_probe_partitioned(uint32_t nb, uint32_t np) {
-    if (const char *e = getenv("ADB_JOIN_PROBE")) {
-        if (!strcmp(e, "direct")) return false;
-        if (!strcmp(e, "partitioned")) return np > 0;
-    }
-    return nb >= (6u << 20) && np >= (4u << 20);
+static bool join_probe_partitioned(bool by_size) {
+    const char *e = getenv("ADB_JOIN_PROBE");
+    if (e && !strcmp(e, "direct")) return false;
+    if (e && !strcmp(e, "partitioned")) return true;
+    return by_size;
 }
 // the routed probe's owner side probing ~np received keys slice by slice: the same buffers once
 // more and the segmented pass' own histogram, totals and bases
@@ -2083,19 +2074,29 @@ static size_t join_owner_scratch(uint32_t np) {
            2 * arena_round((size_t)256 * 256 * 4) + 8192;
 }
 
-static adb_status join_build(const int32_t *bv, const int32_t *bp, uint32_t nb, uint32_t np, int *launches,
-                             StageTrace &tr, bool part_scratch = false, bool owner_scratch = false) {
+static uint32_t join_part_bits(uint32_t nb) {
     uint32_t part_bits = 1;                    // >= 1: the table's key tag needs one spare bit
     // (up to 2^20 partitions: a 500 M-row build side still gets ~500-row partitions that fit the
     // shared-memory table, instead of 2^16 oversized ones built slot by slot in global memory)
     while (part_bits < 20 && (nb >> part_bits) > 1024) ++part_bits;
+    return part_bits;
+}
+
+// The arena join_build reserves for nb build rows and np probe rows.  The sharded join's owner
+// picks its probe form from what is left of it (adb_join_probe_received), so
+// adb_peer_exchange_reserve must reserve exactly this.
+static size_t join_arena_bytes(uint32_t nb, uint32_t np, bool part_scratch, bool owner_scratch) {
+    const uint32_t num_parts = 1u << join_part_bits(nb);
+    return radix_scratch_bytes(nb, 4) + arena_round((size_t)np * 8) + arena_round((size_t)(num_parts + 1) * 4) +
+           arena_round((size_t)(num_parts + 1) * 8) + (part_scratch ? join_partition_scratch(np) : 0) +
+           (owner_scratch ? join_owner_scratch(np) : 0) + kJoinSmallScratch;
+}
+
+static adb_status join_build(const int32_t *bv, const int32_t *bp, uint32_t nb, uint32_t np, int *launches,
+                             StageTrace &tr, bool part_scratch = false, bool owner_scratch = false) {
+    const uint32_t part_bits = join_part_bits(nb);
     const uint32_t num_parts = 1u << part_bits;
-    const size_t pbytes = (size_t)(num_parts + 1) * 4;
-    if (adb_status s = arena_reserve(radix_scratch_bytes(nb, 4) + arena_round((size_t)np * 8) +
-                                     arena_round(pbytes) + arena_round((size_t)(num_parts + 1) * 8) +
-                                     (part_scratch ? join_partition_scratch(np) : 0) +
-                                     (owner_scratch ? join_owner_scratch(np) : 0) + kJoinSmallScratch))
-        return s;
+    if (adb_status s = arena_reserve(join_arena_bytes(nb, np, part_scratch, owner_scratch))) return s;
     auto &j = g.join;
     j.part_bits = part_bits;
     j.n_build = nb;
@@ -2148,7 +2149,8 @@ static adb_status join_count(const int32_t *bv, const int32_t *bp, int64_t nb64,
     }
     int launches = 0;
     StageTrace tr;
-    const bool partitioned = join_probe_partitioned(nb, np);
+    // ~21 bytes of table per build row against 126 MB of L2
+    const bool partitioned = join_probe_partitioned(nb >= (6u << 20) && np >= (4u << 20));
     if (partitioned)
         if (adb_status s = ensure_radix_scratch(np > nb ? np : nb)) return s;
     if (adb_status s = join_build(bv, bp, nb, np, &launches, tr, partitioned)) return s;
@@ -2221,17 +2223,51 @@ adb_status adb_join_build(const int32_t *d_v, const int32_t *d_p, int64_t n, int
     return ADB_OK;
 }
 
-// ---- the sharded join's probe: keys routed to their owners ---------------------------------------
-// The keys travel to their owners in bulk (4 bytes per row), the owner probes them against its own
-// tables, the 8-byte answers travel back in bulk, and the rows' home puts them back in row order
-// (the same gather as the one-GPU partitioned probe; cells = owners).  Probing in place and reading
+// ---- routed exchange (adb_engine.h): the sharded join's probe and the routed fetch ---------------
+// Step 1 on the home side: one stable pass (`pass` picks the owner's digit) groups this context's n
+// items by owner into the arena, with their row numbers and room for answer_bytes of answer each;
+// h_counts[o] = items bound for owner o.  The arena is reserved here for this exchange alone when
+// `reserve` (a join waiting for its emit phase is dropped), else the one adb_join_build reserved
+// is used.  The pass' scanned histogram stays in g.rx_hist / g.rx_base for step 3.
+static adb_status route_partition(const char *what, int32_t world, const int32_t *d_in, int64_t n64,
+                                  adb::RadixPass pass, size_t answer_bytes, bool reserve, RouteState &rt,
+                                  int64_t *h_counts, const int32_t **d_routed, void **d_answers) {
+    if (adb_status s = check_len(n64, what)) return s;
+    if (!h_counts || !d_routed || !d_answers || (n64 > 0 && !d_in)) return fail(ADB_ERR_INVALID, "%s: NULL pointer", what);
+    for (int r = 0; r < world; ++r) h_counts[r] = 0;
+    *d_routed = nullptr;
+    *d_answers = nullptr;
+    const uint32_t n = (uint32_t)n64;
+    rt.n = n;
+    if (n == 0) return ADB_OK;
+    if (adb_status s = ensure_radix_scratch(n)) return s;
+    if (reserve)
+        if (adb_status s = arena_reserve(2 * arena_round((size_t)n * 4) + arena_round((size_t)n * answer_bytes) + 4096))
+            return s;
+    rt.items = ARENA_TAKE(uint32_t, n);
+    rt.rows = ARENA_TAKE(uint32_t, n);
+    rt.answers = arena_take_bytes((size_t)n * answer_bytes);
+    if (g.arena_used > g.arena.cap) return fail(ADB_ERR_NOMEM, "%s: scratch arena too small", what);
+    const int k_ = adb::launch_radix_pass_segmented(reinterpret_cast<const uint32_t *>(d_in), nullptr, rt.items,
+                                                    rt.rows, n, pass, 0, g.rx_hist, g.rx_totals, g.rx_base,
+                                                    g.sm_count, g.stream);
+    if (adb_status s = after_launch(what, k_)) return s;
+    uint32_t totals[ADB_MAX_PEERS];
+    CU(cudaMemcpyAsync(totals, g.rx_totals, sizeof(uint32_t) * world, cudaMemcpyDeviceToHost, g.stream));
+    CU(cudaStreamSynchronize(g.stream));
+    for (int r = 0; r < world; ++r) h_counts[r] = totals[r];
+    *d_routed = reinterpret_cast<const int32_t *>(rt.items);
+    *d_answers = rt.answers;
+    return ADB_OK;
+}
+
+// The sharded join's probe routes the keys by the top bits of the routing hash; the owner probes
+// them against its own tables and the rows' home puts the 8-byte answers back in row order (the
+// same gather as the one-GPU partitioned probe; cells = owners).  Probing in place and reading
 // each remote key's slot over NVLink instead costs one 32-byte response per 16 useful bytes, 8.8 G
 // reads/s per GPU: 1.2 ms for the 11 M remote rows of an 8-GPU 100 M-row probe, and the whole
 // 100 M x 100 M join on 8 GPUs took 2.71 ms that way against 2.08 ms routed
-// (profiles/r02_join_sharded.md).  Steps, each on every context with a host barrier between:
-//   1. adb_join_route_probe     stable partition of my probe keys by owner; per-owner counts
-//   2. adb_join_recv_buffers + adb_copy_from_ctx per source + adb_join_probe_received
-//   3. adb_copy_from_ctx per owner into *d_answers + adb_join_finish_routed, then adb_join_emit
+// (profiles/r02_join_sharded.md).
 adb_status adb_join_route_probe(int32_t world, const int32_t *d_pv, int64_t np64, int64_t *h_counts,
                                 const int32_t **d_routed_keys, void **d_answers) {
     NEED_UP();
@@ -2239,34 +2275,13 @@ adb_status adb_join_route_probe(int32_t world, const int32_t *d_pv, int64_t np64
     if (!j.built) return fail(ADB_ERR_INVALID, "adb_join_route_probe: no preceding adb_join_build on this context");
     if (world < 2 || world > ADB_MAX_PEERS || (world & (world - 1)))
         return fail(ADB_ERR_INVALID, "adb_join_route_probe: world %d must be a power of two in [2, %d]", world, ADB_MAX_PEERS);
-    if (adb_status s = check_len(np64, "adb_join_route_probe")) return s;
-    if ((uint32_t)np64 > j.n_probe) return fail(ADB_ERR_INVALID, "adb_join_route_probe: more probe rows than adb_join_build reserved for");
-    if (!h_counts || !d_routed_keys || !d_answers || (np64 > 0 && !d_pv))
-        return fail(ADB_ERR_INVALID, "adb_join_route_probe: NULL pointer");
-    for (int r = 0; r < world; ++r) h_counts[r] = 0;
-    *d_routed_keys = nullptr;
-    *d_answers = nullptr;
-    const uint32_t np = (uint32_t)np64;
-    j.rt_rows_n = np;
-    j.routed = true;
-    if (np == 0) return ADB_OK;
-    if (adb_status s = ensure_radix_scratch(np)) return s;
+    if (np64 > (int64_t)j.n_probe) return fail(ADB_ERR_INVALID, "adb_join_route_probe: more probe rows than adb_join_build reserved for");
     int bits = 0;
     while ((1 << bits) < world) ++bits;
-    j.rt_keys = ARENA_TAKE(uint32_t, np);
-    j.rt_rows = ARENA_TAKE(uint32_t, np);
-    j.rt_res = ARENA_TAKE(uint2, np);
-    if (g.arena_used > g.arena.cap) return fail(ADB_ERR_NOMEM, "adb_join_route_probe: scratch arena too small");
-    const int k_ = adb::launch_radix_pass_segmented(reinterpret_cast<const uint32_t *>(d_pv), nullptr, j.rt_keys,
-                                                    j.rt_rows, np, adb::RadixPass{32 - bits, bits, 2}, 0, g.rx_hist,
-                                                    g.rx_totals, g.rx_base, g.sm_count, g.stream);
-    if (adb_status s = after_launch("join_route_probe", k_)) return s;
-    uint32_t totals[ADB_MAX_PEERS];
-    CU(cudaMemcpyAsync(totals, g.rx_totals, sizeof(uint32_t) * world, cudaMemcpyDeviceToHost, g.stream));
-    CU(cudaStreamSynchronize(g.stream));
-    for (int r = 0; r < world; ++r) h_counts[r] = totals[r];
-    *d_routed_keys = reinterpret_cast<const int32_t *>(j.rt_keys);
-    *d_answers = j.rt_res;
+    if (adb_status s = route_partition("adb_join_route_probe", world, d_pv, np64, adb::RadixPass{32 - bits, bits, 2},
+                                       sizeof(uint2), false, j.route, h_counts, d_routed_keys, d_answers))
+        return s;
+    j.routed = true;
     return ADB_OK;
 }
 
@@ -2297,11 +2312,7 @@ adb_status adb_join_probe_received(int64_t n_recv) {
     // keys arrived in.  The pass needs a histogram of its own: g.rx_hist / g.rx_base still hold
     // this context's ROUTING pass, which adb_join_finish_routed reads.  No room in the arena (a
     // skewed key set sent most of the probe side here): the direct probe.
-    bool partitioned = n >= (4u << 20) && j.n_build >= (24u << 20);
-    if (const char *e = getenv("ADB_JOIN_PROBE")) {
-        if (!strcmp(e, "direct")) partitioned = false;
-        if (!strcmp(e, "partitioned")) partitioned = true;
-    }
+    bool partitioned = join_probe_partitioned(n >= (4u << 20) && j.n_build >= (24u << 20));
     if (partitioned) {
         const uint32_t tiles = (n + adb::kRadixTile - 1) / adb::kRadixTile;
         const uint32_t want_tiles = (tiles + 255) / 256;
@@ -2313,7 +2324,7 @@ adb_status adb_join_probe_received(int64_t n_recv) {
                             arena_round(hist_elems * 4) + 2 * arena_round((size_t)segs * 256 * 4) +
                             arena_round((size_t)pg.warps * 8) + arena_round(((size_t)pg.warps / 1024 + 2) * 8) + 4096;
         // (what adb_join_finish_routed still takes for this context's own probe rows stays free)
-        const size_t finish = arena_round((size_t)j.rt_rows_n * 8) + arena_round(((size_t)j.rt_rows_n / 512 + 8) * 8) +
+        const size_t finish = arena_round((size_t)j.route.n * 8) + arena_round(((size_t)j.route.n / 512 + 8) * 8) +
                               (1 << 20);
         if (g.arena_used + need + finish <= g.arena.cap) {
             uint32_t *pk = ARENA_TAKE(uint32_t, n), *rows = ARENA_TAKE(uint32_t, n);
@@ -2352,7 +2363,7 @@ adb_status adb_join_finish_routed(int32_t world, const int32_t *d_pv, const int3
     if (!j.built || !j.routed) return fail(ADB_ERR_INVALID, "adb_join_finish_routed: no preceding adb_join_route_probe");
     if (world < 2 || world > ADB_MAX_PEERS || (world & (world - 1)))
         return fail(ADB_ERR_INVALID, "adb_join_finish_routed: world %d must be a power of two in [2, %d]", world, ADB_MAX_PEERS);
-    if ((uint32_t)np64 != j.rt_rows_n) return fail(ADB_ERR_INVALID, "adb_join_finish_routed: row count differs from adb_join_route_probe");
+    if ((uint32_t)np64 != j.route.n) return fail(ADB_ERR_INVALID, "adb_join_finish_routed: row count differs from adb_join_route_probe");
     if (np64 > 0 && (!d_pv || !d_pp)) return fail(ADB_ERR_INVALID, "adb_join_finish_routed: NULL device pointer");
     const uint32_t np = (uint32_t)np64;
     adb::JoinOwners o{};
@@ -2382,8 +2393,9 @@ adb_status adb_join_finish_routed(int32_t world, const int32_t *d_pv, const int3
     unsigned long long *chunk_sums = ARENA_TAKE(unsigned long long, j.pg.warps / 1024 + 2);
     if (g.arena_used > g.arena.cap) return fail(ADB_ERR_NOMEM, "adb_join_finish_routed: scratch arena too small");
     StageTrace tr;
-    int launches = adb::launch_hj_unpartition_routed(j.rt_rows, j.rt_res, g.rx_base, g.rx_hist, np, (uint32_t)world,
-                                                     j.pg, j.gc_by_j, j.warp_base, chunk_sums, tot, g.stream);
+    int launches = adb::launch_hj_unpartition_routed(j.route.rows, static_cast<const uint2 *>(j.route.answers),
+                                                     g.rx_base, g.rx_hist, np, (uint32_t)world, j.pg, j.gc_by_j,
+                                                     j.warp_base, chunk_sums, tot, g.stream);
     if (adb_status s = read_back(&j.matches, tot, sizeof(int64_t))) return s;
     tr.lap("answers back to row order + piece offsets");
     if (adb_status s = after_launch("join_finish_routed", launches)) return s;
@@ -2398,59 +2410,34 @@ adb_status adb_join_finish_routed(int32_t world, const int32_t *d_pv, const int3
 // ---- routed fetch over a position list that is not aligned with the column's shards ---------------
 // adb_fetch_sharded reads every remote row over NVLink, 4 useful bytes per 32-byte response
 // (~12 G rows/s per GPU: an index-ordered 10 % select + fetch over 500 M rows took 3.6 ms on two
-// GPUs against 1.2 ms on one).  Routed, like the join's probe: the positions travel to the GPUs
-// that hold the rows, those gather locally (adb_fetch with the shard's base), the values travel
-// back in bulk and the list's home puts them in list order.  Steps, a host barrier after each:
-//   1. adb_route_rows           stable partition of my positions by shard (= owner)
-//   2. adb_join_recv_buffers + adb_copy_from_ctx_ready per source + adb_fetch(..., shard base, ...)
-//      into the answers buffer + adb_sync
-//   3. adb_copy_from_ctx_ready per owner into *d_answers + adb_route_finish32
-// Scratch is the sort / join arena: a join waiting for its emit phase is dropped.
+// GPUs against 1.2 ms on one).  Routed instead: the positions go to the GPUs that hold the rows
+// (the digit is the shard, position / shard_rows), those gather locally (adb_fetch with the
+// shard's base) and the list's home puts the 4-byte values back in list order.  It reserves the
+// sort / join arena afresh: a join waiting for its emit phase is dropped.
 adb_status adb_route_rows(int32_t world, int64_t shard_rows, const int32_t *d_pos, int64_t n64, int64_t *h_counts,
                           const int32_t **d_routed_pos, void **d_answers) {
     NEED_UP();
     if (world < 2 || world > ADB_MAX_PEERS) return fail(ADB_ERR_INVALID, "adb_route_rows: world %d must be in [2, %d]", world, ADB_MAX_PEERS);
     if (shard_rows < 1 || shard_rows > 0x7FFFFFFF) return fail(ADB_ERR_INVALID, "adb_route_rows: bad shard size");
-    if (adb_status s = check_len(n64, "adb_route_rows")) return s;
-    if (!h_counts || !d_routed_pos || !d_answers || (n64 > 0 && !d_pos))
-        return fail(ADB_ERR_INVALID, "adb_route_rows: NULL pointer");
-    for (int r = 0; r < world; ++r) h_counts[r] = 0;
-    *d_routed_pos = nullptr;
-    *d_answers = nullptr;
-    const uint32_t n = (uint32_t)n64;
-    g.rt32_n = n;
-    if (n == 0) return ADB_OK;
-    if (adb_status s = ensure_radix_scratch(n)) return s;
-    if (adb_status s = arena_reserve(3 * arena_round((size_t)n * 4) + 4096)) return s;
-    g.rt32_pos = ARENA_TAKE(uint32_t, n);
-    g.rt32_rows = ARENA_TAKE(uint32_t, n);
-    g.rt32_val = ARENA_TAKE(uint32_t, n);
     int bits = 1;
     while ((1 << bits) < world) ++bits;
     adb::RadixPass pass{0, bits, 3};
     pass.div = (uint32_t)shard_rows;
-    const int k_ = adb::launch_radix_pass_segmented(reinterpret_cast<const uint32_t *>(d_pos), nullptr, g.rt32_pos,
-                                                    g.rt32_rows, n, pass, 0, g.rx_hist, g.rx_totals, g.rx_base,
-                                                    g.sm_count, g.stream);
-    if (adb_status s = after_launch("route_rows", k_)) return s;
-    uint32_t totals[ADB_MAX_PEERS];
-    CU(cudaMemcpyAsync(totals, g.rx_totals, sizeof(uint32_t) * world, cudaMemcpyDeviceToHost, g.stream));
-    CU(cudaStreamSynchronize(g.stream));
-    for (int r = 0; r < world; ++r) h_counts[r] = totals[r];
-    *d_routed_pos = reinterpret_cast<const int32_t *>(g.rt32_pos);
-    *d_answers = g.rt32_val;
-    return ADB_OK;
+    return route_partition("adb_route_rows", world, d_pos, n64, pass, sizeof(uint32_t), true, g.fetch_route, h_counts,
+                           d_routed_pos, d_answers);
 }
 
 adb_status adb_route_finish32(int32_t world, int32_t *d_out, int64_t n64) {
     NEED_UP();
+    RouteState &rt = g.fetch_route;
     if (world < 2 || world > ADB_MAX_PEERS) return fail(ADB_ERR_INVALID, "adb_route_finish32: world %d must be in [2, %d]", world, ADB_MAX_PEERS);
-    if ((uint32_t)n64 != g.rt32_n) return fail(ADB_ERR_INVALID, "adb_route_finish32: row count differs from adb_route_rows");
+    if ((uint32_t)n64 != rt.n) return fail(ADB_ERR_INVALID, "adb_route_finish32: row count differs from adb_route_rows");
     if (n64 == 0) return ADB_OK;
     if (!d_out) return fail(ADB_ERR_INVALID, "adb_route_finish32: NULL output");
-    const int k_ = adb::launch_rows_unpartition32(g.rt32_rows, g.rt32_val, g.rx_base, g.rx_hist, g.rt32_n,
-                                                  (uint32_t)world, reinterpret_cast<uint32_t *>(d_out), g.stream);
-    g.rt32_n = 0;
+    const int k_ = adb::launch_rows_unpartition32(rt.rows, static_cast<const uint32_t *>(rt.answers), g.rx_base,
+                                                  g.rx_hist, rt.n, (uint32_t)world, reinterpret_cast<uint32_t *>(d_out),
+                                                  g.stream);
+    rt.n = 0;
     return after_launch("route_finish32", k_);
 }
 
@@ -2468,14 +2455,8 @@ adb_status adb_peer_exchange_reserve(int64_t send_pairs, int64_t build_pairs, in
     if ((uint32_t)probe_rows > big) big = (uint32_t)probe_rows;            // the routed probe's partition pass
     if (adb_status s = ensure_radix_scratch(big ? big : 1)) return s;
     const uint32_t nb = (uint32_t)build_pairs, np = (uint32_t)probe_rows;
-    uint32_t part_bits = 1;
-    while (part_bits < 20 && (nb >> part_bits) > 1024) ++part_bits;
-    const uint32_t num_parts = 1u << part_bits;
-    if (adb_status s = arena_reserve(radix_scratch_bytes(nb, 4) + arena_round((size_t)np * 8) +
-                                     arena_round((size_t)(num_parts + 1) * 4) +
-                                     arena_round((size_t)(num_parts + 1) * 8) + join_partition_scratch(np) +
-                                     join_owner_scratch(np) + kJoinSmallScratch))
-        return s;
+    if (adb_status s = arena_reserve(join_arena_bytes(nb, np, true, true))) return s;
+    const uint32_t num_parts = 1u << join_part_bits(nb);
     // tables: <= 2.5 slots per build row (power-of-two capacity at <= 80 % load) + 16 per partition
     const unsigned long long slots = (unsigned long long)nb * 5 / 2 + 16ull * num_parts + 4096;
     return grow(g.hj_table, slots * 16, "join tables");

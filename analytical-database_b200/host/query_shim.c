@@ -328,6 +328,57 @@ static int shard_errs(const ShardErr *e) {
         }                                           \
     } while (0)
 
+/* ---- routed exchange (adb_engine.h), phases 1-3 of a job with a host barrier after each.  Phases 1
+ * and 2 end synchronised, so the pulls are _ready copies. */
+typedef struct Route {
+    int64_t sent[MAXG][MAXG];                       /* sent[g][o] = items of GPU g owned by GPU o */
+    const int32_t *items[MAXG];                     /* GPU g's items grouped by owner */
+    void *answers_home[MAXG];                       /* where GPU g collects the owners' answers */
+    void *answers_owner[MAXG];                      /* GPU o's answers, in the order it received the items */
+} Route;
+
+static int run_routed(shard_fn fn, void *arg, int *phase, const ShardErr *err) {
+    for (*phase = 1; *phase <= 3; ++*phase) {
+        run_shards(fn, arg);
+        if (shard_errs(err)) return -1;
+    }
+    return 0;
+}
+
+/* Owner g: room for what every GPU sent it, its pieces pulled in in source order.  The pulls start
+ * at g's own piece and go round, so that at any moment every GPU reads from a different source
+ * (r02zj: all eight starting at GPU 0 queued up behind one another on its port). */
+static adb_status route_pull(int g, Route *r, int32_t **items, int64_t *n_recv) {
+    *n_recv = 0;
+    for (int s = 0; s < S.G; ++s) *n_recv += r->sent[s][g];
+    adb_status st = adb_join_recv_buffers(*n_recv, items, &r->answers_owner[g]);
+    for (int k = 0; k < S.G && st == ADB_OK; ++k) {
+        const int s = (g + k) % S.G;
+        int64_t at = 0, from = 0;
+        for (int t = 0; t < s; ++t) at += r->sent[t][g];
+        for (int o = 0; o < g; ++o) from += r->sent[s][o];
+        if (r->sent[s][g])
+            st = adb_copy_from_ctx_ready(*items + at, s, r->items[s] + from, 4 * (size_t)r->sent[s][g]);
+    }
+    return st;
+}
+
+/* Home g: its answers (elem_bytes each) from every owner, in the same rotated order. */
+static adb_status route_return(int g, const Route *r, size_t elem_bytes) {
+    adb_status st = ADB_OK;
+    for (int k = 0; k < S.G && st == ADB_OK; ++k) {
+        const int o = (g + k) % S.G;
+        int64_t at = 0, from = 0;                   /* g's piece inside owner o's received list */
+        for (int t = 0; t < o; ++t) at += r->sent[g][t];
+        for (int s = 0; s < g; ++s) from += r->sent[s][o];
+        if (r->sent[g][o])
+            st = adb_copy_from_ctx_ready((char *)r->answers_home[g] + elem_bytes * (size_t)at, o,
+                                         (const char *)r->answers_owner[o] + elem_bytes * (size_t)from,
+                                         elem_bytes * (size_t)r->sent[g][o]);
+    }
+    return st;
+}
+
 /* Main-thread engine calls on another context (cheap bookkeeping: allocations, frees). */
 static void on_ctx(int g) {
     if (S.G > 1) adb_ctx_select(g);
@@ -2115,11 +2166,8 @@ typedef struct FetchJob {
     DevColumn *c;
     Staged *p;
     Shards out;
-    /* routed form (phases 1-3): sent[g][o] = positions of GPU g's list that name rows of GPU o */
     int phase;
-    int64_t sent[MAXG][MAXG];
-    const int32_t *routed_pos[MAXG];
-    void *answers_home[MAXG], *answers_owner[MAXG];
+    Route route;                                    /* routed form (phases 1-3): items = positions */
 } FetchJob;
 /* A position list that is not aligned with the column's shards (index order, a join's output):
  * above this many positions they are routed to the GPUs that hold the rows and the values come
@@ -2143,35 +2191,18 @@ static void fetch_shard(int g, void *arg) {
     FetchJob *a = arg;
     DevColumn *c = a->c;
     const size_t n = a->p->n[g];
-    if (a->phase == 2) {                            /* owner: pull my pieces, gather them from my shard */
-        int64_t n_recv = 0;
-        for (int s = 0; s < S.G; ++s) n_recv += a->sent[s][g];
+    Route *r = &a->route;
+    if (a->phase == 2) {                            /* owner: gather my pieces from my shard */
         int32_t *pos = NULL;
-        SCK(adb_join_recv_buffers(n_recv, &pos, &a->answers_owner[g]));
-        for (int k = 0; k < S.G; ++k) {
-            const int s = (g + k) % S.G;
-            int64_t at = 0, from = 0;
-            for (int t = 0; t < s; ++t) at += a->sent[t][g];
-            for (int o = 0; o < g; ++o) from += a->sent[s][o];
-            if (a->sent[s][g])
-                SCK(adb_copy_from_ctx_ready(pos + at, s, a->routed_pos[s] + from, 4 * (size_t)a->sent[s][g]));
-        }
+        int64_t n_recv = 0;
+        SCK(route_pull(g, r, &pos, &n_recv));
         if (n_recv)
-            SCK(adb_fetch(c->d_data[g], pos, n_recv, NULL, shard_base(g, c->shard_rows), a->answers_owner[g]));
+            SCK(adb_fetch(c->d_data[g], pos, n_recv, NULL, shard_base(g, c->shard_rows), r->answers_owner[g]));
         SCK(adb_sync());
         return;
     }
     if (a->phase == 3) {                            /* home: the values back into list order */
-        for (int k = 0; k < S.G; ++k) {
-            const int o = (g + k) % S.G;
-            int64_t at = 0, from = 0;
-            for (int t = 0; t < o; ++t) at += a->sent[g][t];
-            for (int s = 0; s < g; ++s) from += a->sent[s][o];
-            if (a->sent[g][o])
-                SCK(adb_copy_from_ctx_ready((char *)a->answers_home[g] + 4 * (size_t)at, o,
-                                            (const char *)a->answers_owner[o] + 4 * (size_t)from,
-                                            4 * (size_t)a->sent[g][o]));
-        }
+        SCK(route_return(g, r, 4));
         SCK(adb_route_finish32(S.G, a->out.d[g], (int64_t)n));
         return;
     }
@@ -2180,8 +2211,8 @@ static void fetch_shard(int g, void *arg) {
     a->out.d[g] = out;
     a->out.n[g] = n;
     if (a->phase == 1) {                            /* home: my positions grouped by the shard they name */
-        SCK(adb_route_rows(S.G, (int64_t)c->shard_rows, a->p->d[g], (int64_t)n, a->sent[g], &a->routed_pos[g],
-                           &a->answers_home[g]));
+        SCK(adb_route_rows(S.G, (int64_t)c->shard_rows, a->p->d[g], (int64_t)n, r->sent[g], &r->items[g],
+                           &r->answers_home[g]));
         return;
     }
     if (!n) return;
@@ -2246,10 +2277,7 @@ static Result *fetch_column_impl(Column *column, Result *position_result, Status
     job.p = &p;
     if (S.G > 1 && !(p.aligned && p.aligned == c->shard_rows) && p.total >= fetch_route_min() &&
         c->shard_rows > 0) {
-        for (job.phase = 1; job.phase <= 3; ++job.phase) {
-            run_shards(fetch_shard, &job);
-            if (shard_errs(&job.err)) goto fail;
-        }
+        if (run_routed(fetch_shard, &job, &job.phase, &job.err)) goto fail;
     } else {
         run_shards(fetch_shard, &job);
         if (shard_errs(&job.err)) goto fail;
@@ -2498,11 +2526,7 @@ typedef struct JoinJob {
     int swapped, phase, overflow;
     size_t cap;                                     /* pairs a GPU can receive */
     Shards o1, o2;
-    /* routed probe (phases 1-3): sent[g][o] = probe keys of GPU g owned by GPU o */
-    int64_t sent[MAXG][MAXG];
-    const int32_t *routed_keys[MAXG];               /* GPU g's keys grouped by owner */
-    void *answers_home[MAXG];                       /* where GPU g collects the owners' answers */
-    void *answers_owner[MAXG];                      /* GPU o's answers, in the order it received the keys */
+    Route route;                                    /* routed probe (phases 1-3): items = probe keys */
 } JoinJob;
 
 static void join_shard(int g, void *arg) {
@@ -2527,41 +2551,21 @@ static void join_shard(int g, void *arg) {
         SCK(adb_join_build(rv, rp, rn, (int64_t)a->pv->n[g]));
         return;
     }
+    Route *r = &a->route;
     if (a->phase == 1) {                            /* routed probe, 3a: my keys grouped by owner */
-        SCK(adb_join_route_probe(S.G, a->pv->d[g], (int64_t)a->pv->n[g], a->sent[g], &a->routed_keys[g],
-                                 &a->answers_home[g]));
+        SCK(adb_join_route_probe(S.G, a->pv->d[g], (int64_t)a->pv->n[g], r->sent[g], &r->items[g],
+                                 &r->answers_home[g]));
         return;
     }
     if (a->phase == 2) {                            /* 3b: I own what the others sent me */
-        int64_t n_recv = 0;
-        for (int s = 0; s < S.G; ++s) n_recv += a->sent[s][g];
         int32_t *keys = NULL;
-        SCK(adb_join_recv_buffers(n_recv, &keys, &a->answers_owner[g]));
-        /* pieces land in source order; the pulls start at my own piece and go round, so that at
-         * any moment every GPU reads from a different source (r02zj: all eight starting at GPU 0
-         * queued up behind one another on its port) */
-        for (int k = 0; k < S.G; ++k) {
-            const int s = (g + k) % S.G;
-            int64_t at = 0, from = 0;
-            for (int t = 0; t < s; ++t) at += a->sent[t][g];
-            for (int o = 0; o < g; ++o) from += a->sent[s][o];
-            if (a->sent[s][g])                      /* 3a ended synchronised, a host barrier since */
-                SCK(adb_copy_from_ctx_ready(keys + at, s, a->routed_keys[s] + from, 4 * (size_t)a->sent[s][g]));
-        }
+        int64_t n_recv = 0;
+        SCK(route_pull(g, r, &keys, &n_recv));
         SCK(adb_join_probe_received(n_recv));
         return;
     }
     /* phase 3, 3c: the owners' answers come home, back to row order, expand */
-    for (int k = 0; k < S.G; ++k) {
-        const int o = (g + k) % S.G;
-        int64_t at = 0, from = 0;                   /* my piece inside owner o's received list */
-        for (int t = 0; t < o; ++t) at += a->sent[g][t];
-        for (int s = 0; s < g; ++s) from += a->sent[s][o];
-        if (a->sent[g][o])                          /* 3b ended synchronised, a host barrier since */
-            SCK(adb_copy_from_ctx_ready((char *)a->answers_home[g] + 8 * (size_t)at, o,
-                                        (const char *)a->answers_owner[o] + 8 * (size_t)from,
-                                        8 * (size_t)a->sent[g][o]));
-    }
+    SCK(route_return(g, r, 8));
     int64_t m = 0;
     SCK(adb_join_finish_routed(S.G, a->pv->d[g], a->pp->d[g], (int64_t)a->pv->n[g], a->swapped, &m));
     void *x = NULL, *y = NULL;
@@ -2625,10 +2629,7 @@ static Result **join_sharded(Result *v1, Result *p1, Result *v2, Result *p2, int
             goto fail;
         }
     }
-    for (job.phase = 1; job.phase <= 3; ++job.phase) {
-        run_shards(join_shard, &job);
-        if (shard_errs(&job.err)) goto fail;
-    }
+    if (run_routed(join_shard, &job, &job.phase, &job.err)) goto fail;
     unstage(&a); unstage(&b); unstage(&c); unstage(&d);
     results = malloc(2 * sizeof *results);
     if (!results) {

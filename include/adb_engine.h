@@ -428,6 +428,21 @@ ADB_API adb_status adb_nested_loop_join_count(const int32_t *d_v1, const int32_t
                                               const int32_t *d_v2, const int32_t *d_p2, int64_t n2,
                                               int64_t *h_matches);
 ADB_API adb_status adb_join_emit(int32_t *d_out1, int32_t *d_out2);
+/* ---- routed exchange (several contexts of one process) --------------------------------------
+ * Items travel in bulk to the context that owns them, the owner answers them, and the answers
+ * travel back in bulk to their home, which puts them in the items' original order.  The sharded
+ * join's probe and the routed fetch below take it; every step on every context, a host barrier
+ * after each:
+ *   1. partition (adb_join_route_probe / adb_route_rows): a stable partition of this context's
+ *      items by owner.  h_counts[o] = items bound for context o; they sit at offset
+ *      sum(h_counts[0..o)) of *d_routed_keys / *d_routed_pos, in row order.  *d_answers = where
+ *      context o's answers belong, at the same offsets.  Synchronises;
+ *   2. owner: adb_join_recv_buffers(n_recv) + one adb_copy_from_ctx[_ready] per source context
+ *      (pieces in source-context order), then the owner's own work writes one answer per received
+ *      item, in the order received, into *d_answers of adb_join_recv_buffers.  Synchronises;
+ *   3. home: one adb_copy_from_ctx[_ready] per owner into step 1's *d_answers, then the finish
+ *      call (adb_join_finish_routed / adb_route_finish32) puts the answers back in row order.
+ * Steps 1 and 2 end synchronised, so with a host barrier after each the _ready copies are safe. */
 /* The join sharded over the contexts of ONE process (SURVEY.md 8e "hash join: hash-partition both
  * (key, pos) lists by key to G GPUs"), keeping the reference's output order.  world = number of
  * contexts, a power of two >= 2; swapped as in adb_nested_loop_join_count.  Every step on every
@@ -438,19 +453,11 @@ ADB_API adb_status adb_join_emit(int32_t *d_out1, int32_t *d_out2);
  *      partition, as steps 1-3 of adb_hash_join_count); probe_rows_hint = the probe rows this
  *      context will bring (scratch is reserved for them).  Synchronises;
  *   3. each context's slice of the PROBE side, in its original order, is answered by the keys'
- *      owners: the keys travel to them in bulk and the answers come back in bulk (reading every
- *      remote slot over NVLink instead costs one 32-byte response per 16-byte slot, ~9 G reads/s
- *      per GPU):
- *      3a. adb_join_route_probe: stable partition of this context's probe keys by owner;
- *          h_counts[r] = keys bound for context r (they sit at offset sum(h_counts[0..r)) of
- *          *d_routed_keys, in row order); *d_answers = where context r's answers belong, at the
- *          same offsets, 8 bytes per key;
- *      3b. adb_join_recv_buffers(n_recv) + one adb_copy_from_ctx[_ready] per source context
- *          (pieces in source-context order) + adb_join_probe_received(n_recv): the answers land in
- *          *d_answers of adb_join_recv_buffers, in the order of the received keys.  Synchronises;
- *      3c. one adb_copy_from_ctx[_ready] per owner into 3a's *d_answers + adb_join_finish_routed:
- *          *h_matches = this context's pair count.
- *      (3a and 3b end synchronised, so with a host barrier after each the _ready copies are safe.)
+ *      owners through the routed exchange above, 8 bytes per answer (reading every remote slot
+ *      over NVLink instead costs one 32-byte response per 16-byte slot, ~9 G reads/s per GPU):
+ *      3a. partition: adb_join_route_probe, the owner taken from the keys' routing hash;
+ *      3b. owner: adb_join_probe_received(n_recv) probes what it received;
+ *      3c. home: adb_join_finish_routed sets *h_matches = this context's pair count.
  *   4. adb_join_emit writes this context's pairs (multi-row groups read the owner's sorted build
  *      positions over peer memory).  Synchronises.
  * Each context's pairs are probe-major over its own probe rows, so the contexts' outputs
@@ -469,14 +476,12 @@ ADB_API adb_status adb_join_finish_routed(int32_t world, const int32_t *d_pv, co
                                           int32_t swapped, int64_t *h_matches);
 
 /* ---- routed fetch (several contexts, a position list that is not aligned with the shards) ----
- * Instead of adb_fetch_sharded's one NVLink read per remote row: (1) adb_route_rows groups this
- * context's positions by the shard that holds the row (shard = position / shard_rows, at most
- * world - 1); h_counts / *d_routed_pos / *d_answers as for adb_join_route_probe, 4-byte answers;
- * (2) every owner pulls its pieces (adb_join_recv_buffers + adb_copy_from_ctx_ready), gathers
- * them with adb_fetch(column shard, received positions, n, NULL, shard base, answers) and
- * synchronises; (3) the list's home pulls the answers into *d_answers and adb_route_finish32
- * writes d_out[i] = value of position i.  A host barrier after each step.  Uses the sort / join
- * scratch arena (a join waiting for its emit phase is dropped). */
+ * Instead of adb_fetch_sharded's one NVLink read per remote row, the routed exchange above with
+ * 4-byte answers: (1) partition: adb_route_rows, the owner being the shard that holds the row
+ * (shard = position / shard_rows, at most world - 1); (2) owner: adb_fetch(column shard, received
+ * positions, n, NULL, shard base, answers) + adb_sync; (3) home: adb_route_finish32 writes
+ * d_out[i] = value of position i.  Uses the sort / join scratch arena (a join waiting for its emit
+ * phase is dropped). */
 ADB_API adb_status adb_route_rows(int32_t world, int64_t shard_rows, const int32_t *d_pos, int64_t n,
                                   int64_t *h_counts, const int32_t **d_routed_pos, void **d_answers);
 ADB_API adb_status adb_route_finish32(int32_t world, int32_t *d_out, int64_t n);
