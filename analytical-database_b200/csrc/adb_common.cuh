@@ -559,8 +559,15 @@ int launch_csv_parse(const unsigned char *text, size_t bytes, const unsigned lon
                      unsigned long long n_newlines, uint32_t skip_lines, unsigned long long rows,
                      uint32_t n_cols, int32_t *const *cols, unsigned char *n_fields, uint32_t *flags,
                      cudaStream_t s);
-int launch_csv_fixup(unsigned long long rows, uint32_t n_cols, int32_t *const *cols,
-                     const unsigned char *n_fields, cudaStream_t s);
+// forward fill of short rows: per-tile records of the last row with each field, scanned over
+// the tiles (summary: the piece's last value of every column, then whether it exists)
+uint32_t csv_tiles(unsigned long long rows);
+int launch_csv_tile_scan(unsigned long long rows, uint32_t n_cols, int32_t *const *cols,
+                         const unsigned char *n_fields, int32_t *tile_last, int32_t *summary, cudaStream_t s);
+int launch_csv_last_row(unsigned long long rows, uint32_t n_cols, int32_t *const *cols, int32_t *summary,
+                        cudaStream_t s);
+int launch_csv_fill(unsigned long long rows, uint32_t n_cols, int32_t *const *cols, const unsigned char *n_fields,
+                    const int32_t *tile_prev, const int32_t *carry, cudaStream_t s);
 
 // Result text for print (format_text.cu).
 uint32_t fmt_blocks(int64_t n);

@@ -113,19 +113,22 @@ struct Engine {
     // routed exchange, owner side: the items other contexts sent here and the answers (grow-only)
     DevBuf<uint32_t> rt_recv_keys;
     DevBuf<uint2> rt_recv_res;
-    // bulk CSV load state (adb_csv_index -> adb_csv_parse); scratch is grow-only
+    // bulk CSV load state (adb_csv_index -> adb_csv_parse[_piece] -> adb_csv_fill); scratch is grow-only
     struct CsvState {
         const unsigned char *text = nullptr;
         size_t bytes = 0;
         unsigned long long newlines = 0, rows = 0;
-        uint32_t skip = 0;
+        uint32_t skip = 0, n_cols = 0;
         bool ready = false;
+        bool fill_ready = false;            // a piece was parsed and has short rows: adb_csv_fill may run
         DevBuf<uint32_t> block_counts, block_base;
         DevBuf<unsigned long long> line_end;
         DevBuf<unsigned char> n_fields;
         DevBuf<int32_t *> col_table;        // 256 device pointers
         DevBuf<uint32_t> flags;
         DevBuf<int64_t> total;
+        DevBuf<int32_t> tile_last;          // per tile and column: last row with the field (scanned)
+        DevBuf<int32_t> piece;              // [0, 256) last values, [256, 512) have-flags, [512, 768) carry
     } csv;
     // print formatting state (adb_format_i32_count -> _emit)
     struct FmtState {
@@ -188,7 +191,7 @@ auto context_bufs(Engine &E) {
                     E.ss_plan_mem, E.ss_hits, E.ss_chunk_hits, E.ss_counts, E.ss_totals, E.ss_outs, E.rx_hist,
                     E.rx_totals, E.rx_base, E.sc_sums, E.arena, E.hj_table, E.rt_recv_keys, E.rt_recv_res,
                     E.csv.block_counts, E.csv.block_base, E.csv.line_end, E.csv.n_fields, E.csv.col_table,
-                    E.csv.flags, E.csv.total, E.fmt.block_len, E.fmt.block_off, E.fmt.total);
+                    E.csv.flags, E.csv.total, E.csv.tile_last, E.csv.piece, E.fmt.block_len, E.fmt.block_off, E.fmt.total);
 }
 
 // One context per GPU of the box (several may share a device: a 1-GPU box then runs the
@@ -1919,6 +1922,7 @@ adb_status adb_csv_index(const char *d_text, size_t bytes, int32_t skip_lines, i
     NEED_UP();
     auto &c = g.csv;
     c.ready = false;
+    c.fill_ready = false;
     if (skip_lines < 0 || !h_rows || (bytes && !d_text)) return fail(ADB_ERR_INVALID, "adb_csv_index: bad arguments");
     if (adb_status s = grow(c.col_table, 256 * sizeof(int32_t *), "csv column table")) return s;
     if (adb_status s = grow(c.flags, 4 * sizeof(uint32_t), "csv flags")) return s;
@@ -1954,16 +1958,22 @@ adb_status adb_csv_index(const char *d_text, size_t bytes, int32_t skip_lines, i
     return ADB_OK;
 }
 
-adb_status adb_csv_parse(int32_t n_cols, int32_t *const *d_cols) {
-    NEED_UP();
+// Parse the indexed rows into d_cols; *h_short = some row had fewer than n_cols fields.  With
+// `summary`, also the piece's last value of every column (c.piece); when a row was short, the
+// tile records the fill needs are left in c.tile_last.
+static adb_status csv_parse_rows(const char *what, int32_t n_cols, int32_t *const *d_cols, bool summary,
+                                 bool *h_short) {
     auto &c = g.csv;
-    if (!c.ready) return fail(ADB_ERR_INVALID, "adb_csv_parse: no preceding adb_csv_index");
+    *h_short = false;
+    if (!c.ready) return fail(ADB_ERR_INVALID, "%s: no preceding adb_csv_index", what);
     c.ready = false;
-    if (n_cols < 1 || n_cols > 254 || !d_cols) return fail(ADB_ERR_INVALID, "adb_csv_parse: n_cols %d outside [1, 254]", n_cols);
-    if (c.rows == 0) return ADB_OK;
+    c.fill_ready = false;
+    if (n_cols < 1 || n_cols > 254 || !d_cols) return fail(ADB_ERR_INVALID, "%s: n_cols %d outside [1, 254]", what, n_cols);
+    if (c.rows == 0 && !summary) return ADB_OK;
     for (int32_t i = 0; i < n_cols; ++i)
-        if (!d_cols[i]) return fail(ADB_ERR_INVALID, "adb_csv_parse: column %d is NULL", i);
-    if (adb_status s = grow(c.n_fields, (size_t)c.rows, "csv field counts")) return s;
+        if (!d_cols[i] && c.rows) return fail(ADB_ERR_INVALID, "%s: column %d is NULL", what, i);
+    if (adb_status s = grow(c.n_fields, (size_t)c.rows + 1, "csv field counts")) return s;
+    if (adb_status s = grow(c.piece, 3 * 256 * sizeof(int32_t), "csv piece summary")) return s;
     if (adb_status s = upload_blob(c.col_table, d_cols, sizeof(int32_t *) * n_cols)) return s;
     CU(cudaMemsetAsync(c.flags, 0, 4 * sizeof(uint32_t), g.stream));
     int k_ = adb::launch_csv_parse(c.text, c.bytes, c.line_end, c.newlines, c.skip, c.rows, (uint32_t)n_cols,
@@ -1973,13 +1983,65 @@ adb_status adb_csv_parse(int32_t n_cols, int32_t *const *d_cols) {
     CU(cudaStreamSynchronize(g.stream));
     if (adb_status s = after_launch("csv_parse", k_)) return s;
     if (flags[1])
-        return fail(ADB_ERR_INVALID, "adb_csv_parse: a line is longer than 1023 bytes (fgets would split it, "
-                    "src/db_manager.c:23,306)");
-    if (flags[0]) {
-        k_ = adb::launch_csv_fixup(c.rows, (uint32_t)n_cols, c.col_table, c.n_fields, g.stream);
-        if (adb_status s = after_launch("csv_fixup", k_)) return s;
+        return fail(ADB_ERR_INVALID, "%s: a line is longer than 1023 bytes (fgets would split it, "
+                    "src/db_manager.c:23,306)", what);
+    c.n_cols = (uint32_t)n_cols;
+    *h_short = flags[0] != 0;
+    if (*h_short) {
+        const uint32_t tiles = adb::csv_tiles(c.rows);
+        if (adb_status s = grow(c.tile_last, sizeof(int32_t) * (size_t)tiles * n_cols, "csv fill tiles")) return s;
+        k_ = adb::launch_csv_tile_scan(c.rows, (uint32_t)n_cols, c.col_table, c.n_fields, c.tile_last, c.piece,
+                                       g.stream);
+        if (adb_status s = after_launch("csv_tile_scan", k_)) return s;
+        c.fill_ready = true;
+    } else if (summary) {
+        k_ = adb::launch_csv_last_row(c.rows, (uint32_t)n_cols, c.col_table, c.piece, g.stream);
+        if (adb_status s = after_launch("csv_last_row", k_)) return s;
     }
     return ADB_OK;
+}
+
+static adb_status csv_fill(const int32_t *h_carry) {
+    auto &c = g.csv;
+    if (!c.fill_ready) return ADB_OK;                                 // no short row: nothing to fill
+    c.fill_ready = false;
+    if (h_carry) {
+        if (adb_status s = upload_blob(c.piece + 512, h_carry, sizeof(int32_t) * c.n_cols)) return s;
+    } else {
+        CU(cudaMemsetAsync(c.piece + 512, 0, sizeof(int32_t) * c.n_cols, g.stream));
+    }
+    const int k_ = adb::launch_csv_fill(c.rows, c.n_cols, c.col_table, c.n_fields, c.tile_last, c.piece + 512, g.stream);
+    return after_launch("csv_fill", k_);
+}
+
+adb_status adb_csv_parse(int32_t n_cols, int32_t *const *d_cols) {
+    NEED_UP();
+    bool short_rows = false;
+    if (adb_status s = csv_parse_rows("adb_csv_parse", n_cols, d_cols, false, &short_rows)) return s;
+    return csv_fill(nullptr);                                          // a missing field of the first rows is 0
+}
+
+adb_status adb_csv_parse_piece(int32_t n_cols, int32_t *const *d_cols, int32_t *h_last, int32_t *h_has,
+                               int32_t *h_short) {
+    NEED_UP();
+    if (!h_last || !h_has || !h_short) return fail(ADB_ERR_INVALID, "adb_csv_parse_piece: NULL output");
+    bool short_rows = false;
+    if (adb_status s = csv_parse_rows("adb_csv_parse_piece", n_cols, d_cols, true, &short_rows)) return s;
+    auto &c = g.csv;
+    int32_t sum[512];
+    CU(cudaMemcpyAsync(sum, c.piece, sizeof sum, cudaMemcpyDeviceToHost, g.stream));
+    CU(cudaStreamSynchronize(g.stream));
+    for (int32_t i = 0; i < n_cols; ++i) {
+        h_last[i] = sum[i];
+        h_has[i] = sum[256 + i];
+    }
+    *h_short = short_rows;
+    return ADB_OK;
+}
+
+adb_status adb_csv_fill(const int32_t *h_carry) {
+    NEED_UP();
+    return csv_fill(h_carry);
 }
 
 // ---- result text ------------------------------------------------------------------------------------

@@ -137,6 +137,8 @@ class Engine:
         "adb_format_i32_emit": (C.c_int32, [C.c_void_p]),
         "adb_csv_index": (C.c_int32, [C.c_void_p, C.c_size_t, C.c_int32, _I64P]),
         "adb_csv_parse": (C.c_int32, [C.c_int32, C.POINTER(C.c_void_p)]),
+        "adb_csv_parse_piece": (C.c_int32, [C.c_int32, C.POINTER(C.c_void_p), _I32P, _I32P, _I32P]),
+        "adb_csv_fill": (C.c_int32, [_I32P]),
         "adb_peer_create": (C.c_int32, [C.c_int32, C.c_int32, C.c_char_p]),
         "adb_peer_connect": (C.c_int32, [C.c_char_p]),
         "adb_agg_combine_allreduce": (C.c_int32, [C.POINTER(_AggStruct), C.c_int32, C.POINTER(_AggStruct), C.POINTER(_AggStruct)]),

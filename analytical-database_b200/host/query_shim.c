@@ -68,6 +68,7 @@
 #include <string.h>
 
 #include "adb_engine.h"
+#include "adb_load_api.h"
 #include "adb_query_api.h"
 
 #define MAXG ADB_MAX_PEERS
@@ -175,10 +176,12 @@ static void op_ok(Status *st) {
  * adb_host_shutdown / adb_host_profile_dump ------------------------------------------------- */
 #include <time.h>
 enum { PF_SELECT, PF_SELECT_JOB, PF_FETCH, PF_FETCH_JOB, PF_AGG, PF_AGG_JOB, PF_NEWRESULT, PF_RELEASE,
-       PF_FREE_JOB, PF_COUNT };
+       PF_FREE_JOB, PF_LOAD_UPLOAD, PF_LOAD_PARSE, PF_LOAD_FILL, PF_LOAD_RECUT, PF_LOAD_AGG, PF_LOAD_DOWNLOAD,
+       PF_COUNT };
 static const char *const pf_names[PF_COUNT] = {"select_column", "  its shard job", "fetch_column", "  its shard job",
                                                "aggregate", "  its shard job", "new_dev_result", "payload release",
-                                               "  free job"};
+                                               "  free job", "load: upload", "load: index+parse", "load: fill",
+                                               "load: re-cut", "load: aggregate", "load: download"};
 static struct { int on; double t[PF_COUNT]; long n[PF_COUNT]; } PF;
 static inline double pf_now(void) {
     struct timespec ts;
@@ -738,9 +741,11 @@ static void result_buffers_free(DevResult *r) {
     r->slab = NULL;
 }
 
+static void load_release(void);
 void adb_host_shutdown(void) {
     if (!S.up) return;
     adb_host_profile_dump();
+    load_release();
     lock();
     if (P.active) lazy_done(&P);
     while (nR) lazy_done(&R[nR - 1]);
@@ -1801,6 +1806,287 @@ done:
     if (out) adb_free(out);
     if (gathered) adb_free(gathered);
     unstage(&p);
+    return rc;
+}
+
+/* ---- bulk load (SURVEY.md 8f rank 1): CSV text -> row-sharded device columns ---------------------
+ * What load_db's ingest loop does (src/db_manager.c:304-318), with every GPU parsing a piece of the
+ * file that came over its own host link.  Two phases, because the catalog grows its mmap'd columns
+ * between them:
+ *   count  the text after `skip_lines` lines is cut into G pieces: piece g > 0 starts right after
+ *          the first '\n' at or after byte g*len/G (pieces may be empty; no line spans two).  Every
+ *          GPU uploads, indexes and parses its piece (adb_csv_parse_piece); the host resolves the
+ *          carry chain (a missing field takes the value of the nearest earlier row of the FILE that
+ *          had it); pieces with short rows are filled; then the pieces are re-cut into shards of
+ *          shard_rows_for(rows) rows and every shard's min / max is taken.
+ *   emit   every GPU downloads its shard into Column.data + old_rows + g*S; min / max are folded as
+ *          insert_row folds them (db_manager.c:193-194) and row_count is set.  Into an empty table
+ *          the shards become the columns' device copies, so the next operator uploads nothing. */
+typedef struct Load {
+    int pending, n_cols;
+    size_t rows, shard_rows;                        /* rows of the text; S of the new shards */
+    int32_t **d[MAXG];                              /* d[g][c]: shard g of column c (context g) */
+    int mn[256], mx[256];                           /* the new rows' min / max per column */
+} Load;
+static Load L;
+
+typedef struct LoadJob {
+    ShardErr err;
+    int step, n_cols;
+    const char *text;
+    size_t begin[MAXG + 1];                         /* piece g = text[begin[g], begin[g+1]) */
+    void *d_text[MAXG];
+    int32_t **piece[MAXG];                          /* piece[g][c], rows[g] ints */
+    size_t rows[MAXG];
+    int32_t last[MAXG][256], has[MAXG][256], carry[MAXG][256];
+    int32_t shorts[MAXG];
+    adb_agg agg[MAXG][256];
+} LoadJob;
+
+static void load_shard(int g, void *arg) {
+    LoadJob *a = arg;
+    const size_t bytes = a->begin[g + 1] - a->begin[g];
+    switch (a->step) {
+    case 0: {                                       /* this GPU's piece over its own link */
+        void *p = NULL;
+        SCK(adb_alloc(&p, bytes ? bytes : 16));
+        a->d_text[g] = p;
+        if (bytes) SCK(adb_upload(p, a->text + a->begin[g], bytes));
+        break;
+    }
+    case 1: {                                       /* index + parse, without the fill */
+        int64_t rows = 0;
+        SCK(adb_csv_index(a->d_text[g], bytes, 0, &rows));
+        a->rows[g] = (size_t)rows;
+        for (int c = 0; c < a->n_cols; ++c) {
+            void *p = NULL;
+            SCK(adb_alloc(&p, 4 * (rows ? (size_t)rows : 1)));
+            a->piece[g][c] = p;
+        }
+        SCK(adb_csv_parse_piece(a->n_cols, a->piece[g], a->last[g], a->has[g], &a->shorts[g]));
+        SCK(adb_free(a->d_text[g]));
+        a->d_text[g] = NULL;
+        break;
+    }
+    case 2:                                         /* enqueued only: the re-cut's copies wait for it */
+        if (a->shorts[g]) SCK(adb_csv_fill(a->carry[g]));
+        break;
+    case 3: {                                       /* min / max of the new shards */
+        const size_t n = shard_len(L.rows, L.shard_rows, g);
+        for (int c = 0; c < a->n_cols && n; ++c)
+            SCK(adb_aggregate(L.d[g][c], (int64_t)n, NULL, S.d_part[g], &a->agg[g][c]));
+        break;
+    }
+    }
+}
+
+/* the pending load's shard buffers (NULL: none) */
+static void load_release(void) {
+    for (int g = 0; g < MAXG; ++g) {
+        if (!L.d[g]) continue;
+        for (int c = 0; c < L.n_cols; ++c) free_on(g, L.d[g][c]);
+        free(L.d[g]);
+        L.d[g] = NULL;
+    }
+    L.pending = 0;
+}
+
+static void load_job_free(LoadJob *job) {
+    for (int g = 0; g < S.G; ++g) {
+        free_on(g, job->d_text[g]);
+        if (!job->piece[g]) continue;
+        for (int c = 0; c < job->n_cols; ++c) free_on(g, job->piece[g][c]);
+        free(job->piece[g]);
+    }
+    free(job);
+}
+
+static int load_step(LoadJob *job, int step, int pf) {
+    PF_BEGIN(load);
+    job->step = step;
+    run_shards(load_shard, job);
+    if (PF.on) {
+        PF.t[pf] += pf_now() - pf_t0_load;
+        ++PF.n[pf];
+    }
+    return shard_errs(&job->err);
+}
+
+int adb_host_load_csv_count(const char *text, size_t bytes, int skip_lines, int n_cols, size_t *rows) {
+    t_err[0] = '\0';
+    if (ensure_up()) return -1;
+    load_release();                                 /* a second count drops a pending one */
+    if (!rows || (bytes && !text) || skip_lines < 0 || n_cols < 1 || n_cols > 254) {
+        set_err("adb_host_load_csv_count: bad arguments (n_cols %d outside [1, 254]?)", n_cols);
+        return -1;
+    }
+    size_t off = 0;                                 /* the header lines load_db consumes (db_manager.c:263) */
+    for (int k = 0; k < skip_lines && off < bytes; ++k) {
+        const char *nl = memchr(text + off, '\n', bytes - off);
+        off = nl ? (size_t)(nl - text) + 1 : bytes;
+    }
+    LoadJob *job = calloc(1, sizeof *job);
+    if (!job) {
+        set_err("out of host memory");
+        return -1;
+    }
+    job->text = text;
+    job->n_cols = n_cols;
+    const size_t len = bytes - off;
+    job->begin[0] = off;
+    for (int g = 1; g < S.G; ++g) {
+        const size_t at = off + (size_t)((unsigned __int128)g * len / (unsigned)S.G);
+        const char *nl = at < bytes ? memchr(text + at, '\n', bytes - at) : NULL;
+        job->begin[g] = nl ? (size_t)(nl - text) + 1 : bytes;
+    }
+    job->begin[S.G] = bytes;
+    for (int g = 0; g < S.G; ++g)
+        if (!(job->piece[g] = calloc((size_t)n_cols, sizeof(int32_t *)))) {
+            set_err("out of host memory");
+            load_job_free(job);
+            return -1;
+        }
+    if (load_step(job, 0, PF_LOAD_UPLOAD) || load_step(job, 1, PF_LOAD_PARSE)) {
+        load_job_free(job);
+        return -1;
+    }
+    size_t total = 0;
+    for (int g = 0; g < S.G; ++g) total += job->rows[g];
+    if (total >= ((size_t)1 << 31)) {
+        set_err("adb_host_load_csv_count: %zu rows: positions are int (src/query.c:94-95)", total);
+        load_job_free(job);
+        return -1;
+    }
+    /* the carry chain: what the reference's row[] holds when piece g starts */
+    for (int g = 1; g < S.G; ++g)
+        for (int c = 0; c < n_cols; ++c)
+            job->carry[g][c] = job->has[g - 1][c] ? job->last[g - 1][c] : job->carry[g - 1][c];
+    if (load_step(job, 2, PF_LOAD_FILL)) {
+        load_job_free(job);
+        return -1;
+    }
+    /* every fill is enqueued: the re-cut's copies (adb_copy_from_ctx) wait for them */
+    PF_BEGIN(recut);
+    L.n_cols = n_cols;
+    L.rows = total;
+    L.shard_rows = shard_rows_for(total);
+    size_t want[MAXG];
+    for (int g = 0; g < S.G; ++g) {
+        want[g] = shard_len(total, L.shard_rows, g);
+        if (!(L.d[g] = calloc((size_t)n_cols, sizeof(int32_t *)))) {
+            set_err("out of host memory");
+            goto fail;
+        }
+    }
+    for (int c = 0; c < n_cols; ++c) {
+        int32_t *src[MAXG], *dst[MAXG] = {0};
+        for (int g = 0; g < S.G; ++g) src[g] = job->piece[g][c];
+        const int rc = recut(src, job->rows, want, dst);
+        for (int g = 0; g < S.G; ++g) L.d[g][c] = dst[g];
+        if (rc) goto fail;
+        for (int g = 0; g < S.G; ++g) {            /* recut waited for its copies */
+            free_on(g, job->piece[g][c]);
+            job->piece[g][c] = NULL;
+        }
+    }
+    if (PF.on) {
+        PF.t[PF_LOAD_RECUT] += pf_now() - pf_t0_recut;
+        ++PF.n[PF_LOAD_RECUT];
+    }
+    if (load_step(job, 3, PF_LOAD_AGG)) goto fail;
+    for (int c = 0; c < n_cols; ++c) {
+        L.mn[c] = INT_MAX;
+        L.mx[c] = INT_MIN;
+        for (int g = 0; g < S.G; ++g) {
+            if (!shard_len(total, L.shard_rows, g)) continue;
+            if (job->agg[g][c].min < L.mn[c]) L.mn[c] = job->agg[g][c].min;
+            if (job->agg[g][c].max > L.mx[c]) L.mx[c] = job->agg[g][c].max;
+        }
+    }
+    load_job_free(job);
+    L.pending = 1;
+    *rows = total;
+    return 0;
+fail:
+    load_release();
+    load_job_free(job);
+    return -1;
+}
+
+typedef struct EmitJob {
+    ShardErr err;
+    Column **cols;
+    size_t old_rows;
+} EmitJob;
+static void load_emit_shard(int g, void *arg) {
+    EmitJob *a = arg;
+    const size_t n = shard_len(L.rows, L.shard_rows, g);
+    for (int c = 0; c < L.n_cols && n; ++c)
+        SCK(adb_download(a->cols[c]->data + a->old_rows + (size_t)g * L.shard_rows, L.d[g][c], 4 * n));
+}
+
+int adb_host_load_csv_emit(Column **cols, int n_cols) {
+    t_err[0] = '\0';
+    if (ensure_up()) return -1;
+    if (!L.pending) {
+        set_err("adb_host_load_csv_emit: no pending adb_host_load_csv_count");
+        return -1;
+    }
+    int rc = -1;
+    const size_t old = cols && n_cols > 0 && cols[0] ? cols[0]->row_count : 0;
+    if (!cols || n_cols != L.n_cols) {
+        set_err("adb_host_load_csv_emit: %d columns, the count parsed %d", n_cols, L.n_cols);
+        goto done;
+    }
+    for (int c = 0; c < n_cols; ++c)
+        if (!cols[c] || !cols[c]->data || cols[c]->row_count != old) {
+            set_err("adb_host_load_csv_emit: the table's columns must be host-backed and equally long");
+            goto done;
+        }
+    if (old + L.rows >= ((size_t)1 << 31)) {
+        set_err("adb_host_load_csv_emit: %zu + %zu rows: positions are int (src/query.c:94-95)", old, L.rows);
+        goto done;
+    }
+    for (int c = 0; c < n_cols; ++c) {              /* handles and indexes of the old rows go first */
+        DevColumn *dc = dev_column_slot(cols[c]);
+        if (!dc) goto done;
+        dev_column_drop(dc);
+    }
+    PF_BEGIN(download);
+    EmitJob job;
+    memset(&job, 0, sizeof job);
+    job.cols = cols;
+    job.old_rows = old;
+    run_shards(load_emit_shard, &job);
+    if (PF.on) {
+        PF.t[PF_LOAD_DOWNLOAD] += pf_now() - pf_t0_download;
+        ++PF.n[PF_LOAD_DOWNLOAD];
+    }
+    if (shard_errs(&job.err)) goto done;
+    for (int c = 0; c < n_cols; ++c) {
+        Column *col = cols[c];
+        if (L.rows && L.mn[c] < col->min) col->min = L.mn[c];
+        if (L.rows && L.mx[c] > col->max) col->max = L.mx[c];
+        col->row_count = old + L.rows;
+        if (old || !L.rows) continue;               /* an append: the next operator uploads the whole column */
+        DevColumn *dc = dev_column_slot(col);
+        if (dc->uploaded_from != col->data || dc->uploaded_bytes != 4 * L.rows) {
+            column_unregister(dc);
+            dc->uploaded_from = col->data;
+            dc->uploaded_bytes = 4 * L.rows;
+        }
+        ++dc->uploads;
+        for (int g = 0; g < S.G; ++g) {
+            dc->d_data[g] = L.d[g][c];
+            L.d[g][c] = NULL;                       /* the column owns them now (adopted = 0) */
+        }
+        dc->host_data = col->data;
+        dc->rows = L.rows;
+        dc->shard_rows = L.shard_rows;
+    }
+    rc = 0;
+done:
+    load_release();
     return rc;
 }
 

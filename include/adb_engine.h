@@ -209,13 +209,29 @@ ADB_API adb_status adb_agg_import(const int64_t *d_sum_count, const int32_t *d_m
  *                   values are bit-identical to atoi's (glibc: (int) strtol): leading
  *                   whitespace, sign, digits to the first non-digit, saturation at
  *                   LONG_MAX/LONG_MIN then truncation.  Fields beyond n_cols are ignored; a
- *                   missing field repeats the previous row's value as the reference's
- *                   reused row[] does (0 in the first row, where the reference reads
- *                   uninitialised stack).  A line longer than 1023 bytes (fgets would split
- *                   it, db_manager.c:23) is ADB_ERR_INVALID.  n_cols <= 254.
- * d_cols is a HOST array of n_cols device pointers. */
+ *                   missing field repeats the value of the nearest earlier row that had the
+ *                   field, as the reference's reused row[] does (0 if no earlier row had it,
+ *                   where the reference reads uninitialised stack).  A line longer than 1023
+ *                   bytes (fgets would split it, db_manager.c:23) is ADB_ERR_INVALID.
+ *                   n_cols <= 254.  It is adb_csv_parse_piece + adb_csv_fill with a zero carry.
+ * d_cols is a HOST array of n_cols device pointers.
+ *
+ * A file cut into pieces at line boundaries (one per GPU): the first rows of a piece may inherit
+ * a value from an earlier piece, so the parse and the fill are split:
+ *   adb_csv_parse_piece  after adb_csv_index: adb_csv_parse without the fill.  For every column
+ *                        c < n_cols, h_has[c] = some row of the piece has field c, h_last[c] = its
+ *                        value in the last such row (0 if none); *h_short = some row had fewer
+ *                        than n_cols fields.  Synchronises.
+ *   adb_csv_fill         fills the missing fields of that piece: the nearest earlier row of the
+ *                        piece that has the field, else h_carry[c] (n_cols ints; NULL = zeros).
+ *                        Enqueued on the stream, not waited for; nothing to do without a short
+ *                        row.  Linear in rows plus missing cells.
+ * The carry into piece g is piece g-1's h_last[c] where h_has[c], else the carry into g-1. */
 ADB_API adb_status adb_csv_index(const char *d_text, size_t bytes, int32_t skip_lines, int64_t *h_rows);
 ADB_API adb_status adb_csv_parse(int32_t n_cols, int32_t *const *d_cols);
+ADB_API adb_status adb_csv_parse_piece(int32_t n_cols, int32_t *const *d_cols, int32_t *h_last, int32_t *h_has,
+                                       int32_t *h_short);
+ADB_API adb_status adb_csv_fill(const int32_t *h_carry);
 
 /* ---- result text: the INT branch of print, src/query.c:262-269 ("%d" per tuple, "\n"
  * between tuples, nothing after the last); SURVEY.md 8f rank 2.  Two-phase like the
