@@ -100,13 +100,21 @@ typedef struct Slab {
     long refs;
 } Slab;
 
+/* One list as G device buffers: d[g] holds n[g] entries on context g, the list is their
+ * concatenation in context order.  An operator's output, an operator's input and a registered
+ * result are all one of these; list_release() frees what the list owns. */
+typedef struct ShardList {
+    int32_t *d[MAXG];
+    size_t n[MAXG];
+    size_t total;               /* sum of n[]: stage() and new_dev_result() set it */
+    size_t aligned;             /* S > 0: shard g's entries are positions inside rows [g*S, (g+1)*S) */
+    Slab *slab;                 /* the buffers are views into this slab, which owns them */
+    int borrowed;               /* the buffers are a registered result's: this view owns nothing */
+} ShardList;
+
 typedef struct DevResult {
     void *payload;              /* key: the host block handed out as Result.payload */
-    int32_t *d_ptr[MAXG];
-    size_t tuples[MAXG];
-    size_t total;
-    size_t aligned;             /* S > 0: shard g's entries are positions inside rows [g*S, (g+1)*S) */
-    Slab *slab;                 /* NULL: the buffers are this result's own */
+    ShardList list;
 } DevResult;
 
 #define SLOT_EMPTY ((void *)0)
@@ -728,17 +736,22 @@ static void column_unregister(DevColumn *c) {
     c->uploaded_bytes = 0;
 }
 
-static void result_buffers_free(DevResult *r) {
-    if (r->slab) {
-        if (--r->slab->refs == 0) {
-            for (int g = 0; g < S.G; ++g) free_on(g, r->slab->base[g]);
-            free(r->slab);
-        }
-    } else {
-        free_shards(r->d_ptr);
+/* give back `refs` references to a slab; the last one frees it */
+static void slab_drop(Slab *slab, long refs) {
+    slab->refs -= refs;
+    if (slab->refs == 0) {
+        for (int g = 0; g < S.G; ++g) free_on(g, slab->base[g]);
+        free(slab);
     }
-    memset(r->d_ptr, 0, sizeof r->d_ptr);
-    r->slab = NULL;
+}
+
+/* release what the list owns (stream-ordered: safe right after the last launch that reads it) */
+static void list_release(ShardList *l) {
+    if (!l->borrowed) {
+        if (l->slab) slab_drop(l->slab, 1);
+        else free_shards(l->d);
+    }
+    memset(l, 0, sizeof *l);
 }
 
 static void load_release(void);
@@ -754,7 +767,7 @@ void adb_host_shutdown(void) {
     capR = 0;
     for (size_t i = 0; i < S.nslots; ++i)
         if (S.slots[i].payload != SLOT_EMPTY && S.slots[i].payload != SLOT_TOMB)
-            result_buffers_free(&S.slots[i]);
+            list_release(&S.slots[i].list);
     DevResult *old = S.slots;
     S.slots = NULL;
     S.nslots = S.nused = 0;
@@ -1272,12 +1285,12 @@ static int registry_grow(void) {
 }
 
 /* Detach the device buffers registered under `payload` (if any); returns 1 and fills *out. */
-static int registry_take(const void *payload, DevResult *out) {
+static int registry_take(const void *payload, ShardList *out) {
     int found = 0;
     lock();
     DevResult *r = registry_find(payload);
     if (r) {
-        *out = *r;
+        *out = r->list;
         memset(r, 0, sizeof *r);
         r->payload = SLOT_TOMB;
         --S.nlive;
@@ -1298,8 +1311,8 @@ void adb_host_payload_freed(void *payload) {
     if (!known) return;
     PF_BEGIN(PF_RELEASE);
     const int keep = pending_payload_gone(payload);
-    DevResult dead;
-    if (registry_take(payload, &dead) && !keep) result_buffers_free(&dead);
+    ShardList dead;
+    if (registry_take(payload, &dead) && !keep) list_release(&dead);
     PF_END(PF_RELEASE);
 }
 
@@ -1320,83 +1333,61 @@ void adb_host_results_drop(Result **results, int n) {
     }
 }
 
-/* What new_dev_result wraps: G device buffers (this call takes ownership). */
-typedef struct Shards {
-    int32_t *d[MAXG];
-    size_t n[MAXG];
-    size_t aligned;
-    Slab *slab;
-} Shards;
-
-static void shards_free(Shards *s) {
-    if (s->slab) return;                            /* the slab's owner frees it */
-    free_shards(s->d);
-    memset(s->d, 0, sizeof s->d);
-}
-
-static int download_shards(void *dst, int32_t *const d[], const size_t n[]) {
+static int download_shards(void *dst, const ShardList *l) {
     size_t off = 0;
     int rc = 0;
     for (int g = 0; g < S.G; ++g) {
-        if (!n[g]) continue;
+        if (!l->n[g]) continue;
         on_ctx(g);
-        if (adb_download((char *)dst + 4 * off, d[g], 4 * n[g]) != ADB_OK) {
+        if (adb_download((char *)dst + 4 * off, l->d[g], 4 * l->n[g]) != ADB_OK) {
             set_err("adb_download: %s", adb_last_error());
             rc = -1;
             break;
         }
-        off += n[g];
+        off += l->n[g];
     }
     on_ctx(0);
     return rc;
 }
 
-/* Wrap G device buffers as a Result the plumbing can own. */
-static Result *new_dev_result_impl(Shards *sh);
-static Result *new_dev_result(Shards *sh) {
+/* Register a list as a Result the plumbing can own; the result takes its buffers over and *l
+ * still describes them afterwards (with total set).  On failure an owned list is released; a
+ * slab view is not -- shared_select gives the slab's references back itself. */
+static Result *new_dev_result_impl(ShardList *l);
+static Result *new_dev_result(ShardList *l) {
     PF_BEGIN(PF_NEWRESULT);
-    Result *r = new_dev_result_impl(sh);
+    Result *r = new_dev_result_impl(l);
     PF_END(PF_NEWRESULT);
     return r;
 }
-static Result *new_dev_result_impl(Shards *sh) {
-    size_t tuples = 0;
-    for (int g = 0; g < S.G; ++g) tuples += sh->n[g];
+static Result *new_dev_result_impl(ShardList *l) {
+    l->total = 0;
+    for (int g = 0; g < S.G; ++g) l->total += l->n[g];
+    const size_t tuples = l->total;
     Result *r = malloc(sizeof *r);
     size_t bytes = 4 * tuples < 16 ? 16 : 4 * tuples;
     void *payload = malloc(bytes);
     if (!r || !payload) {
-        free(r);
-        free(payload);
-        shards_free(sh);
         set_err("out of host memory for a %zu-tuple result", tuples);
-        return NULL;
+        goto fail;
     }
-    if (S.mirror && tuples && download_shards(payload, sh->d, sh->n)) {
-        free(r);
-        free(payload);
-        shards_free(sh);
-        return NULL;
-    }
+    if (S.mirror && tuples && download_shards(payload, l)) goto fail;
     /* malloc returned an address we still hold buffers for: that payload was freed by the
      * plumbing without telling us -- reclaim its HBM now.  No engine call is made with the
      * registry lock held (with the free() interposer other threads' frees wait on it). */
     const int keep_dead = pending_payload_gone(payload);    /* an unwritten fetch may keep the dead select's buffers */
-    DevResult dead;
+    ShardList dead;
     int have_dead = 0;
     lock();
     DevResult *e = registry_find(payload);
     if (e) {
-        dead = *e;
+        dead = e->list;
         have_dead = 1;
     } else {
         if (4 * (S.nused + 1) > 3 * S.nslots && registry_grow()) {
             unlock();
-            free(r);
-            free(payload);
-            shards_free(sh);
             set_err("out of host memory");
-            return NULL;
+            goto fail;
         }
         size_t j = slot_of(payload, S.nslots);
         while (S.slots[j].payload != SLOT_EMPTY && S.slots[j].payload != SLOT_TOMB)
@@ -1405,22 +1396,20 @@ static Result *new_dev_result_impl(Shards *sh) {
         e = &S.slots[j];
         ++S.nlive;
     }
-    memset(e, 0, sizeof *e);
     e->payload = payload;
-    for (int g = 0; g < S.G; ++g) {
-        e->d_ptr[g] = sh->d[g];
-        e->tuples[g] = sh->n[g];
-    }
-    e->total = tuples;
-    e->aligned = sh->aligned;
-    e->slab = sh->slab;
+    e->list = *l;
     unlock();
-    if (have_dead && !keep_dead) result_buffers_free(&dead);
+    if (have_dead && !keep_dead) list_release(&dead);
     payload_stamp(payload);
     r->num_tuples = tuples;
     r->data_type = INT;
     r->payload = payload;
     return r;
+fail:
+    free(r);
+    free(payload);
+    if (!l->slab) list_release(l);
+    return NULL;
 }
 
 static void drop_result(Result *r) {
@@ -1430,21 +1419,67 @@ static void drop_result(Result *r) {
     free(r);
 }
 
-/* An operator input: the device buffers behind a Result.  A Result whose payload is not in
- * the registry is an ordinary host array (built by a test or by foreign code); it is staged
- * into temporary device buffers that the caller releases with unstage().  `like` (optional):
- * the split the operand must have -- a device result cut differently is re-cut with peer
- * copies, a host array is uploaded that way. */
-typedef struct Staged {
-    int32_t *d[MAXG];
-    size_t n[MAXG];
-    size_t total, aligned;
-    int temp;
-} Staged;
+/* Hand an operator's list out as its Result and set the Status. */
+static Result *hand_out(ShardList *l, Status *st, const char *what) {
+    Result *r = new_dev_result(l);
+    if (!r) return op_fail(st, what);
+    op_ok(st);
+    return r;
+}
 
-static void unstage(Staged *s) {
-    if (s->temp) free_shards(s->d);                 /* stream-ordered: safe right after the launch */
-    memset(s, 0, sizeof *s);
+/* The same for the two lists of a join (results[0], results[1]); on failure both are released. */
+static Result **hand_out_pair(ShardList *l1, ShardList *l2, Status *st, const char *what) {
+    Result **results = malloc(2 * sizeof *results);
+    if (!results) {
+        set_err("out of host memory");
+        list_release(l1);
+        list_release(l2);
+        return op_fail(st, what);
+    }
+    results[0] = new_dev_result(l1);
+    if (!results[0]) {
+        list_release(l2);
+        goto fail;
+    }
+    results[1] = new_dev_result(l2);
+    if (!results[1]) {
+        drop_result(results[0]);
+        goto fail;
+    }
+    op_ok(st);
+    return results;
+fail:
+    free(results);
+    return op_fail(st, what);
+}
+
+/* The device buffers registered under r's payload, as a borrowed view cut to r->num_tuples.
+ * Returns 1 and fills *v; 0 when the payload is no device result (a scalar or a host array
+ * built by a test or by foreign code); -1 (t_err set) when the result cannot be read. */
+static int result_view(const Result *r, ShardList *v) {
+    if (resolve_payload(r->payload)) return -1; /* about to be read: write it if it is unwritten */
+    lock();
+    DevResult *e = registry_find(r->payload);
+    if (e) *v = e->list;
+    unlock();
+    if (!e) return 0;
+    if (!payload_is_ours(r->payload)) {
+        /* the address was recycled: the registered device buffers belong to a dead handle */
+        adb_host_payload_freed(r->payload);
+        return 0;
+    }
+    if (v->total < r->num_tuples) {
+        set_err("result claims %zu tuples but its device buffers hold %zu", r->num_tuples, v->total);
+        return -1;
+    }
+    size_t left = r->num_tuples;                /* a caller shortened the list: drop the tail */
+    for (int g = 0; g < S.G; ++g) {
+        v->n[g] = v->n[g] < left ? v->n[g] : left;
+        left -= v->n[g];
+    }
+    v->total = r->num_tuples;
+    v->borrowed = 1;
+    return 1;
 }
 
 static int same_split(const size_t a[], const size_t b[]) {
@@ -1496,7 +1531,11 @@ static int recut(int32_t *const src[], const size_t have[], const size_t want[],
     return rc;
 }
 
-static int stage(const Result *r, const size_t *like, Staged *out) {
+/* An operator input: the device buffers behind a Result, released with list_release().  A
+ * device result is borrowed; a host array (built by a test or by foreign code) is uploaded into
+ * buffers the list owns.  `like` (optional): the split the operand must have -- a device result
+ * cut differently is re-cut with peer copies, a host array is uploaded that way. */
+static int stage(const Result *r, const size_t *like, ShardList *out) {
     memset(out, 0, sizeof *out);
     if (!r) {
         set_err("NULL result operand");
@@ -1506,44 +1545,18 @@ static int stage(const Result *r, const size_t *like, Staged *out) {
         set_err("result of %zu tuples exceeds the int position domain (src/query.c:40-43)", r->num_tuples);
         return -1;
     }
-    if (resolve_payload(r->payload)) return -1; /* an operand is about to be read: write it if unwritten */
-    lock();
-    DevResult *e = registry_find(r->payload);
-    DevResult dv;
-    if (e) dv = *e;
-    unlock();
-    if (e && r->payload && !payload_is_ours(r->payload)) {
-        /* the address was recycled: the registered device buffers belong to a dead handle */
-        adb_host_payload_freed(r->payload);
-        e = NULL;
-    }
+    ShardList v;
+    const int found = result_view(r, &v);
+    if (found < 0) return -1;
     out->total = r->num_tuples;
-    if (e) {
-        if (dv.total < r->num_tuples) {
-            set_err("result claims %zu tuples but its device buffers hold %zu", r->num_tuples, dv.total);
-            return -1;
-        }
-        size_t have[MAXG];
-        memcpy(have, dv.tuples, sizeof have);
-        if (dv.total > r->num_tuples) {         /* a caller shortened the list: drop the tail */
-            size_t left = r->num_tuples;
-            for (int g = 0; g < S.G; ++g) {
-                have[g] = have[g] < left ? have[g] : left;
-                left -= have[g];
-            }
-        }
-        if (!like || same_split(have, like)) {
-            for (int g = 0; g < S.G; ++g) {
-                out->d[g] = dv.d_ptr[g];
-                out->n[g] = have[g];
-            }
-            out->aligned = dv.aligned;
+    if (found) {
+        if (!like || same_split(v.n, like)) {
+            *out = v;
             return 0;
         }
-        out->temp = 1;
         memcpy(out->n, like, sizeof(size_t) * (size_t)S.G);
-        if (recut(dv.d_ptr, have, like, out->d)) {
-            unstage(out);
+        if (recut(v.d, v.n, like, out->d)) {
+            list_release(out);
             return -1;
         }
         return 0;
@@ -1553,7 +1566,6 @@ static int stage(const Result *r, const size_t *like, Staged *out) {
         return -1;
     }
     /* host array: upload, cut like the partner or evenly */
-    out->temp = 1;
     const size_t per = (r->num_tuples + (size_t)S.G - 1) / (size_t)S.G;
     size_t off = 0;
     int rc = 0;
@@ -1573,61 +1585,47 @@ static int stage(const Result *r, const size_t *like, Staged *out) {
         off += n;
     }
     on_ctx(0);
-    if (rc) unstage(out);
+    if (rc) list_release(out);
     return rc;
 }
 
 int adb_host_result_to_host(const Result *result, void *dst) {
     if (!result) return -1;
     if (result->num_tuples == 0) return 0;
-    if (resolve_payload(result->payload)) return -1;
-    lock();
-    DevResult *e = registry_find(result->payload);
-    DevResult dv;
-    if (e) dv = *e;
-    unlock();
-    if (e && result->data_type == INT && !payload_is_ours(result->payload)) {
-        adb_host_payload_freed(result->payload);        /* recycled address: see payload_stamp */
-        e = NULL;
-    }
-    if (!e) {                               /* scalar or foreign host payload */
-        size_t w = result->data_type == INT || result->data_type == FLOAT ? 4 : 8;
-        memcpy(dst, result->payload, w * result->num_tuples);
-        return 0;
-    }
-    size_t have[MAXG], left = result->num_tuples;
-    for (int g = 0; g < S.G; ++g) {
-        have[g] = dv.tuples[g] < left ? dv.tuples[g] : left;
-        left -= have[g];
-    }
-    return download_shards(dst, dv.d_ptr, have);
+    ShardList v;
+    const int found = result_view(result, &v);
+    if (found) return found < 0 ? -1 : download_shards(dst, &v);
+    /* scalar or foreign host payload */
+    size_t w = result->data_type == INT || result->data_type == FLOAT ? 4 : 8;
+    memcpy(dst, result->payload, w * result->num_tuples);
+    return 0;
 }
 
 /* allocate n[g] ints on every context (each context's thread allocates its own) */
 typedef struct AllocJob {
     ShardErr err;
-    Shards *sh;
+    ShardList *l;
 } AllocJob;
 static void alloc_shard(int g, void *arg) {
     AllocJob *a = arg;
     void *p = NULL;
-    if (a->sh->d[g]) return;                        /* served from the cache already */
-    SCK(adb_alloc(&p, 4 * a->sh->n[g]));
-    a->sh->d[g] = p;
+    if (a->l->d[g]) return;                         /* served from the cache already */
+    SCK(adb_alloc(&p, 4 * a->l->n[g]));
+    a->l->d[g] = p;
 }
-static int alloc_shards(Shards *sh) {
+static int alloc_shards(ShardList *l) {
     AllocJob job;
     memset(&job, 0, sizeof job);
-    job.sh = sh;
+    job.l = l;
     int missing = 0;
     for (int g = 0; g < S.G; ++g) {
         void *p = NULL;
-        sh->d[g] = adb_alloc_cached_on(g, &p, 4 * sh->n[g]) ? p : NULL;
-        missing |= sh->d[g] == NULL;
+        l->d[g] = adb_alloc_cached_on(g, &p, 4 * l->n[g]) ? p : NULL;
+        missing |= l->d[g] == NULL;
     }
     if (missing) run_shards(alloc_shard, &job);
     if (shard_errs(&job.err)) {
-        shards_free(sh);
+        list_release(l);
         return -1;
     }
     return 0;
@@ -1688,7 +1686,7 @@ int adb_host_relational_update(Column **cols, int n_cols, int which, Result *pos
         return -1;
     }
     Column *column = cols[which];
-    Staged p;
+    ShardList p;
     memset(&p, 0, sizeof p);
     int32_t *all[MAXG] = {0};
     int rc = -1;
@@ -1736,7 +1734,7 @@ int adb_host_relational_update(Column **cols, int n_cols, int which, Result *pos
     if (column->has_index) rc = rebuild_index(cols, n_cols, which);
 done:
     for (int g = 0; g < S.G; ++g) free_on(g, all[g]);
-    unstage(&p);
+    list_release(&p);
     return rc;
 }
 
@@ -1757,7 +1755,7 @@ int adb_host_relational_delete(Column **cols, int n_cols, Result *positions) {
             set_err("relational_delete: the table's columns must be host-backed and equally long");
             return -1;
         }
-    Staged p;
+    ShardList p;
     memset(&p, 0, sizeof p);
     size_t all0[MAXG] = {0};
     all0[0] = positions->num_tuples;
@@ -1805,7 +1803,7 @@ int adb_host_relational_delete(Column **cols, int n_cols, Result *positions) {
 done:
     if (out) adb_free(out);
     if (gathered) adb_free(gathered);
-    unstage(&p);
+    list_release(&p);
     return rc;
 }
 
@@ -2105,7 +2103,7 @@ typedef struct SelectJob {
     DevColumn *c;
     int *low, *high;
     int use_btree, defer;
-    Shards out;
+    ShardList out;
     uint64_t generation[MAXG];
 } SelectJob;
 
@@ -2149,18 +2147,18 @@ static Result *select_index_path(Column *column, DevColumn *c, int *low, int *hi
             q2.use_btree = job.use_btree;
             run_shards(select_index_shard, &q2);
             if (shard_errs(&q2.err)) {
-                shards_free(&q2.out);
+                list_release(&q2.out);
                 goto fail;
             }
             int first = -1;
             for (int g = 0; g < S.G; ++g)
                 if (q2.out.n[g] && first < 0) first = g;
             if (first >= 0) {                       /* keep the first tuple only */
-                shards_free(&job.out);
+                list_release(&job.out);
                 job.out = q2.out;
                 for (int g = 0; g < S.G; ++g) job.out.n[g] = g == first ? 1 : 0;
             } else {
-                shards_free(&q2.out);
+                list_release(&q2.out);
             }
         }
     }
@@ -2176,26 +2174,21 @@ static Result *select_index_path(Column *column, DevColumn *c, int *low, int *hi
             if (job.out.n[g] > most) most = job.out.n[g];
         }
         if (total >= S.rebalance_min && most > 2 * (total / (size_t)S.G)) {
-            Shards even;
+            ShardList even;
             memset(&even, 0, sizeof even);
             const size_t per = (total + (size_t)S.G - 1) / (size_t)S.G;
             for (int g = 0; g < S.G; ++g) even.n[g] = shard_len(total, per, g);
             if (recut(job.out.d, job.out.n, even.n, even.d)) {
-                shards_free(&even);
+                list_release(&even);
                 goto fail;
             }
-            shards_free(&job.out);
+            list_release(&job.out);
             job.out = even;
         }
     }
-    {
-        Result *r = new_dev_result(&job.out);
-        if (!r) return op_fail(st, "select_column");
-        op_ok(st);
-        return r;
-    }
+    return hand_out(&job.out, st, "select_column");
 fail:
-    shards_free(&job.out);
+    list_release(&job.out);
     return op_fail(st, "select_column");
 }
 
@@ -2241,43 +2234,36 @@ static Result *select_column_impl(Column *column, int *low, int *high, Status *r
     PF_END(PF_SELECT_JOB);
     if (shard_errs(&job.err)) goto fail;
     job.out.aligned = c->shard_rows;
-    {
-        size_t total = 0;
-        for (int g = 0; g < S.G; ++g) total += job.out.n[g];
-        Shards keep = job.out;
-        Result *r = new_dev_result(&job.out);
-        if (!r) return op_fail(ret_status, "select_column");
-        if (job.defer && total > 0) {               /* positions are written by whoever needs them first */
-            memset(&P, 0, sizeof P);
-            P.sel_payload = r->payload;
-            for (int g = 0; g < S.G; ++g) {
-                P.sel_d[g] = keep.d[g];
-                P.h[g] = keep.n[g];
-                P.d_col[g] = c->d_data[g];
-                P.rows[g] = shard_len(c->rows, c->shard_rows, g);
-                P.generation[g] = job.generation[g];
-            }
-            P.shard_rows = c->shard_rows;
-            P.has_lo = low != NULL;
-            P.has_hi = high != NULL;
-            P.lo = low ? *low : 0;
-            P.hi = high ? *high : 0;
-            P.active = 1;
+    Result *r = hand_out(&job.out, ret_status, "select_column");
+    if (r && job.defer && job.out.total > 0) {      /* positions are written by whoever needs them first */
+        memset(&P, 0, sizeof P);
+        P.sel_payload = r->payload;
+        for (int g = 0; g < S.G; ++g) {
+            P.sel_d[g] = job.out.d[g];
+            P.h[g] = job.out.n[g];
+            P.d_col[g] = c->d_data[g];
+            P.rows[g] = shard_len(c->rows, c->shard_rows, g);
+            P.generation[g] = job.generation[g];
         }
-        op_ok(ret_status);
-        return r;
+        P.shard_rows = c->shard_rows;
+        P.has_lo = low != NULL;
+        P.has_hi = high != NULL;
+        P.lo = low ? *low : 0;
+        P.hi = high ? *high : 0;
+        P.active = 1;
     }
+    return r;
 fail:
-    shards_free(&job.out);
+    list_release(&job.out);
     return op_fail(ret_status, "select_column");
 }
 
 /* src/query.c:38-86: predicate over a fetched value vector, emits the paired positions. */
 typedef struct PairsJob {
     ShardErr err;
-    Staged *v, *p;
+    ShardList *v, *p;
     int *low, *high;
-    Shards out;
+    ShardList out;
 } PairsJob;
 static void select_pairs_shard(int g, void *arg) {
     PairsJob *a = arg;
@@ -2293,7 +2279,7 @@ static void select_pairs_shard(int g, void *arg) {
 Result *select_result(Result *column, Result *position, int *low_pointer, int *high_pointer,
                       Status *ret_status) {
     t_err[0] = '\0';
-    Staged v, p;
+    ShardList v, p;
     memset(&v, 0, sizeof v);
     memset(&p, 0, sizeof p);
     PairsJob job;
@@ -2318,18 +2304,13 @@ Result *select_result(Result *column, Result *position, int *low_pointer, int *h
     run_shards(select_pairs_shard, &job);
     if (shard_errs(&job.err)) goto fail;
     job.out.aligned = p.aligned;
-    unstage(&v);
-    unstage(&p);
-    {
-        Result *r = new_dev_result(&job.out);
-        if (!r) return op_fail(ret_status, "select_result");
-        op_ok(ret_status);
-        return r;
-    }
+    list_release(&v);
+    list_release(&p);
+    return hand_out(&job.out, ret_status, "select_result");
 fail:
-    shards_free(&job.out);
-    unstage(&v);
-    unstage(&p);
+    list_release(&job.out);
+    list_release(&v);
+    list_release(&p);
     return op_fail(ret_status, "select_result");
 }
 
@@ -2407,22 +2388,17 @@ Result **shared_select(SelectOperator *operators, int query_count, Column *colum
     for (int g = 0; g < S.G; ++g) slab->base[g] = job->slab[g];
     slab->refs = query_count;
     for (int q = 0; q < query_count; ++q) {
-        Shards sh;
-        memset(&sh, 0, sizeof sh);
+        ShardList view;
+        memset(&view, 0, sizeof view);
         for (int g = 0; g < S.G; ++g) {
-            sh.d[g] = job->slab[g] + job->off[g][q];
-            sh.n[g] = (size_t)job->counts[g][q];
+            view.d[g] = job->slab[g] + job->off[g][q];
+            view.n[g] = (size_t)job->counts[g][q];
         }
-        sh.aligned = c->shard_rows;
-        sh.slab = slab;
-        results[q] = new_dev_result(&sh);
+        view.aligned = c->shard_rows;
+        view.slab = slab;
+        results[q] = new_dev_result(&view);
         if (!results[q]) {
-            /* the views not handed out yet give their references back */
-            slab->refs -= query_count - q;
-            if (slab->refs == 0) {
-                for (int g = 0; g < S.G; ++g) free_on(g, slab->base[g]);
-                free(slab);
-            }
+            slab_drop(slab, query_count - q);       /* the views not handed out yet give their references back */
             slab = NULL;
             goto fail;
         }
@@ -2450,8 +2426,8 @@ fail:
 typedef struct FetchJob {
     ShardErr err;
     DevColumn *c;
-    Staged *p;
-    Shards out;
+    ShardList *p;
+    ShardList out;
     int phase;
     Route route;                                    /* routed form (phases 1-3): items = positions */
 } FetchJob;
@@ -2518,7 +2494,7 @@ Result *fetch_column(Column *column, Result *position_result, Status *ret_status
 }
 static Result *fetch_column_impl(Column *column, Result *position_result, Status *ret_status) {
     t_err[0] = '\0';
-    Staged p;
+    ShardList p;
     memset(&p, 0, sizeof p);
     FetchJob job;
     memset(&job, 0, sizeof job);
@@ -2536,20 +2512,19 @@ static Result *fetch_column_impl(Column *column, Result *position_result, Status
             if (shard_len(c->rows, c->shard_rows, g) < P.rows[g]) fits = 0;
         }
         if (fits && position_result->num_tuples == total) {
-            Shards sh;
-            memset(&sh, 0, sizeof sh);
-            memcpy(sh.n, P.h, sizeof sh.n);
+            ShardList vals;
+            memset(&vals, 0, sizeof vals);
+            memcpy(vals.n, P.h, sizeof vals.n);
             PF_BEGIN(PF_FETCH_JOB);
-            const int arc = alloc_shards(&sh);
+            const int arc = alloc_shards(&vals);
             PF_END(PF_FETCH_JOB);
             if (arc) goto fail;
-            Shards keep = sh;
-            Result *r = new_dev_result(&sh);
+            Result *r = new_dev_result(&vals);
             if (!r) return op_fail(ret_status, "fetch_column");
             if (P.active) {                         /* (new_dev_result may have flushed) */
                 P.fetch_payload = r->payload;
                 for (int g = 0; g < S.G; ++g) {
-                    P.fetch_d[g] = keep.d[g];
+                    P.fetch_d[g] = vals.d[g];
                     P.d_fetch_col[g] = c->d_data[g];
                 }
                 op_ok(ret_status);
@@ -2569,16 +2544,11 @@ static Result *fetch_column_impl(Column *column, Result *position_result, Status
         if (shard_errs(&job.err)) goto fail;
     }
     job.out.aligned = p.aligned;                    /* values pair with their positions shard by shard */
-    unstage(&p);
-    {
-        Result *r = new_dev_result(&job.out);
-        if (!r) return op_fail(ret_status, "fetch_column");
-        op_ok(ret_status);
-        return r;
-    }
+    list_release(&p);
+    return hand_out(&job.out, ret_status, "fetch_column");
 fail:
-    shards_free(&job.out);
-    unstage(&p);
+    list_release(&job.out);
+    list_release(&p);
     return op_fail(ret_status, "fetch_column");
 }
 
@@ -2632,7 +2602,7 @@ static int aggregate_result(const Result *r, adb_agg *h) {
     return rc;
 }
 static int aggregate_result_impl(const Result *r, adb_agg *h) {
-    Staged v;
+    ShardList v;
     memset(&v, 0, sizeof v);
     if (ensure_up()) return -1;
     /* aggregate of the unwritten fetch of the newest select: the hit rows are gathered and
@@ -2658,7 +2628,7 @@ static int aggregate_result_impl(const Result *r, adb_agg *h) {
     }
     if (stage(r, NULL, &v)) return -1;
     int rc = aggregate_shards(v.d, v.n, h);
-    unstage(&v);
+    list_release(&v);
     return rc;
 }
 
@@ -2737,9 +2707,9 @@ Result *max(Result *column, Status *ret_status) {
  * length (it would read out of bounds) -- here a shorter column_two is an ERROR. */
 typedef struct EwiseJob {
     ShardErr err;
-    Staged *a, *b;
+    ShardList *a, *b;
     int subtract;
-    Shards out;
+    ShardList out;
 } EwiseJob;
 static void ewise_shard(int g, void *arg) {
     EwiseJob *a = arg;
@@ -2753,7 +2723,7 @@ static void ewise_shard(int g, void *arg) {
 static Result *ewise(Result *one, Result *two, int subtract, Status *st) {
     t_err[0] = '\0';
     const char *what = subtract ? "sub" : "add";
-    Staged a, b;
+    ShardList a, b;
     memset(&a, 0, sizeof a);
     memset(&b, 0, sizeof b);
     EwiseJob job;
@@ -2774,18 +2744,13 @@ static Result *ewise(Result *one, Result *two, int subtract, Status *st) {
     run_shards(ewise_shard, &job);
     if (shard_errs(&job.err)) goto fail;
     job.out.aligned = a.aligned;
-    unstage(&a);
-    unstage(&b);
-    {
-        Result *r = new_dev_result(&job.out);
-        if (!r) return op_fail(st, what);
-        op_ok(st);
-        return r;
-    }
+    list_release(&a);
+    list_release(&b);
+    return hand_out(&job.out, st, what);
 fail:
-    shards_free(&job.out);
-    unstage(&a);
-    unstage(&b);
+    list_release(&job.out);
+    list_release(&a);
+    list_release(&b);
     return op_fail(st, what);
 }
 Result *add(Result *column_one, Result *column_two, Status *ret_status) {
@@ -2808,10 +2773,10 @@ Result *sub(Result *column_one, Result *column_two, Status *ret_status) {
  * order are the reference's probe-major list, so nothing is gathered and nothing re-sorted. */
 typedef struct JoinJob {
     ShardErr err;
-    Staged *bv, *bp, *pv, *pp;
+    ShardList *bv, *bp, *pv, *pp;
     int swapped, phase, overflow;
     size_t cap;                                     /* pairs a GPU can receive */
-    Shards o1, o2;
+    ShardList o1, o2;
     Route route;                                    /* routed probe (phases 1-3): items = probe keys */
 } JoinJob;
 
@@ -2879,11 +2844,10 @@ static int ensure_join_exchange(size_t cap) {
 
 static Result **join_sharded(Result *v1, Result *p1, Result *v2, Result *p2, int nested, Status *st) {
     const char *what = nested ? "nested_loop_join" : "hash_join";
-    Staged a, b, c, d;
+    ShardList a, b, c, d;
     memset(&a, 0, sizeof a); memset(&b, 0, sizeof b); memset(&c, 0, sizeof c); memset(&d, 0, sizeof d);
     JoinJob job;
     memset(&job, 0, sizeof job);
-    Result **results = NULL;
     {
         Result h1 = *p1, h2 = *p2;
         h1.num_tuples = v1->num_tuples;
@@ -2916,33 +2880,12 @@ static Result **join_sharded(Result *v1, Result *p1, Result *v2, Result *p2, int
         }
     }
     if (run_routed(join_shard, &job, &job.phase, &job.err)) goto fail;
-    unstage(&a); unstage(&b); unstage(&c); unstage(&d);
-    results = malloc(2 * sizeof *results);
-    if (!results) {
-        set_err("out of host memory");
-        goto fail;
-    }
-    results[0] = new_dev_result(&job.o1);
-    if (!results[0]) {
-        shards_free(&job.o2);
-        memset(&job.o1, 0, sizeof job.o1);
-        memset(&job.o2, 0, sizeof job.o2);
-        goto fail;
-    }
-    results[1] = new_dev_result(&job.o2);
-    if (!results[1]) {
-        drop_result(results[0]);
-        memset(&job.o1, 0, sizeof job.o1);
-        memset(&job.o2, 0, sizeof job.o2);
-        goto fail;
-    }
-    op_ok(st);
-    return results;
+    list_release(&a); list_release(&b); list_release(&c); list_release(&d);
+    return hand_out_pair(&job.o1, &job.o2, st, what);
 fail:
-    shards_free(&job.o1);
-    shards_free(&job.o2);
-    unstage(&a); unstage(&b); unstage(&c); unstage(&d);
-    free(results);
+    list_release(&job.o1);
+    list_release(&job.o2);
+    list_release(&a); list_release(&b); list_release(&c); list_release(&d);
     return op_fail(st, what);
 }
 
@@ -2953,10 +2896,9 @@ static Result **join(Result *v1, Result *p1, Result *v2, Result *p2, int nested,
     if (S.G > 1 && (S.G & (S.G - 1)) == 0 && v1 && p1 && v2 && p2 && v1->num_tuples && v2->num_tuples &&
         p1->num_tuples >= v1->num_tuples && p2->num_tuples >= v2->num_tuples)
         return join_sharded(v1, p1, v2, p2, nested, st);
-    Staged a, b, c, d;
+    ShardList a, b, c, d, o1, o2;
     memset(&a, 0, sizeof a); memset(&b, 0, sizeof b); memset(&c, 0, sizeof c); memset(&d, 0, sizeof d);
-    int32_t *o1 = NULL, *o2 = NULL;
-    Result **results = NULL;
+    memset(&o1, 0, sizeof o1); memset(&o2, 0, sizeof o2);
     int64_t m = 0;
     size_t all1[MAXG] = {0}, all2[MAXG] = {0};
     if (ensure_up() || !v1 || !p1 || !v2 || !p2) goto fail;
@@ -2979,59 +2921,34 @@ static Result **join(Result *v1, Result *p1, Result *v2, Result *p2, int nested,
     }
     {
         void *x = NULL, *y = NULL;
-        if (adb_alloc(&x, 4 * (size_t)m) != ADB_OK || adb_alloc(&y, 4 * (size_t)m) != ADB_OK) {
+        const int ok = adb_alloc(&x, 4 * (size_t)m) == ADB_OK && adb_alloc(&y, 4 * (size_t)m) == ADB_OK;
+        o1.d[0] = x;
+        o2.d[0] = y;
+        if (!ok) {
             set_err("adb_alloc: %s", adb_last_error());
-            if (x) adb_free(x);
             goto fail;
         }
-        o1 = x;
-        o2 = y;
+        o1.n[0] = o2.n[0] = (size_t)m;
     }
-    if (adb_join_emit(o1, o2) != ADB_OK) {
+    if (adb_join_emit(o1.d[0], o2.d[0]) != ADB_OK) {
         set_err("adb_join_emit: %s", adb_last_error());
         goto fail;
     }
-    unstage(&a); unstage(&b); unstage(&c); unstage(&d);
-    results = malloc(2 * sizeof *results);
-    if (!results) {
-        set_err("out of host memory");
-        goto fail;
+    list_release(&a); list_release(&b); list_release(&c); list_release(&d);
+    for (int g = 1; g < S.G; ++g) {                 /* the other contexts hold empty pieces */
+        void *x = NULL, *y = NULL;
+        on_ctx(g);
+        adb_alloc(&x, 0);
+        adb_alloc(&y, 0);
+        o1.d[g] = x;
+        o2.d[g] = y;
     }
-    {
-        Shards s1, s2;
-        memset(&s1, 0, sizeof s1);
-        memset(&s2, 0, sizeof s2);
-        s1.n[0] = s2.n[0] = (size_t)m;
-        s1.d[0] = o1;
-        s2.d[0] = o2;
-        for (int g = 1; g < S.G; ++g) {             /* the other contexts hold empty pieces */
-            void *x = NULL, *y = NULL;
-            on_ctx(g);
-            adb_alloc(&x, 0);
-            adb_alloc(&y, 0);
-            s1.d[g] = x;
-            s2.d[g] = y;
-        }
-        on_ctx(0);
-        o1 = o2 = NULL;
-        results[0] = new_dev_result(&s1);
-        if (!results[0]) {
-            shards_free(&s2);
-            goto fail;
-        }
-        results[1] = new_dev_result(&s2);
-        if (!results[1]) {
-            drop_result(results[0]);
-            goto fail;
-        }
-    }
-    op_ok(st);
-    return results;
+    on_ctx(0);
+    return hand_out_pair(&o1, &o2, st, what);
 fail:
-    if (o1) adb_free(o1);
-    if (o2) adb_free(o2);
-    unstage(&a); unstage(&b); unstage(&c); unstage(&d);
-    free(results);
+    list_release(&o1);
+    list_release(&o2);
+    list_release(&a); list_release(&b); list_release(&c); list_release(&d);
     return op_fail(st, what);
 }
 Result **nested_loop_join(Result *column_one, Result *position_one, Result *column_two,
@@ -3106,8 +3023,6 @@ char *print(Result **results, int result_num, Status *ret_status) {
     t_err[0] = '\0';
     Text t = {0};
     void *host = NULL;
-    for (int i = 0; i < result_num; ++i)
-        if (results[i] && resolve_payload(results[i]->payload)) return op_fail(ret_status, "print");
     if (text_room(&t, 16)) goto oom;
     t.s[0] = '\0';
     for (int i = 0; i < result_num; ++i) {
@@ -3121,26 +3036,19 @@ char *print(Result **results, int result_num, Status *ret_status) {
         if (r->data_type == INT && n >= PRINT_ON_DEVICE_MIN) {
             /* a long device-resident INT result is formatted where it lives; the text, not
              * the integers, crosses PCIe and no sprintf runs (SURVEY.md 8f rank 2) */
-            lock();
-            DevResult *e = registry_find(r->payload);
-            DevResult dv;
-            if (e) dv = *e;
-            unlock();
-            if (e && dv.total >= n) {
-                size_t have[MAXG], left = n;
-                for (int g = 0; g < S.G; ++g) {
-                    have[g] = dv.tuples[g] < left ? dv.tuples[g] : left;
-                    left -= have[g];
-                }
+            ShardList v;
+            const int found = result_view(r, &v);
+            if (found < 0) goto dev_fail;
+            if (found) {
                 FormatJob job;
                 memset(&job, 0, sizeof job);
-                job.d = dv.d_ptr;
-                job.n = have;
+                job.d = v.d;
+                job.n = v.n;
                 run_shards(format_shard, &job);
                 size_t bytes = 0;
                 int pieces = 0;
                 for (int g = 0; g < S.G; ++g)
-                    if (have[g]) { bytes += (size_t)job.bytes[g]; ++pieces; }
+                    if (v.n[g]) { bytes += (size_t)job.bytes[g]; ++pieces; }
                 bytes += pieces ? (size_t)pieces - 1 : 0;            /* '\n' between the shards' texts */
                 int bad = shard_errs(&job.err);
                 if (!bad && text_room(&t, bytes)) bad = 2;
@@ -3148,7 +3056,7 @@ char *print(Result **results, int result_num, Status *ret_status) {
                     size_t off = t.len;
                     int seen = 0;
                     for (int g = 0; g < S.G; ++g) {
-                        if (!have[g]) continue;
+                        if (!v.n[g]) continue;
                         if (seen++) t.s[off++] = '\n';
                         job.dst[g] = t.s + off;
                         off += (size_t)job.bytes[g];

@@ -212,6 +212,18 @@ def test_error_behaviour(api, rng):
     lo = C.c_int(1)
     assert not api.lib.select_column(C.byref(flagged), C.byref(lo), C.byref(lo), C.byref(st))
     assert st.code == ERROR and b"ColumnIndex" in api.lib.adb_host_last_error()
+    # a Result that claims more tuples than its device buffers hold is refused by every reader
+    s = api.select_column(col, 10, 20)
+    api.tuples(s)                                                      # written, registered
+    s.contents.num_tuples += 1
+    out = np.empty(s.contents.num_tuples, np.int32)
+    assert api.lib.adb_host_result_to_host(s, out.ctypes.data_as(C.c_void_p)) == -1
+    st = Status(99, None)
+    assert not api.lib.print((type(s) * 1)(s), 1, C.byref(st)) and st.code == ERROR
+    st = Status(99, None)
+    assert not api.lib.fetch_column(C.byref(col), s, C.byref(st)) and st.code == ERROR
+    s.contents.num_tuples -= 1
+    api.drop(s)
 
 
 def test_column_reupload_after_insert(api, cpu):
@@ -574,6 +586,7 @@ def test_recycled_payload_address_is_not_mistaken_for_a_device_result(api, rng):
         foreign = np.ctypeslib.as_array(C.cast(p, C.POINTER(C.c_int)), shape=(m,))
         foreign[:] = np.arange(m, dtype=np.int32)[::-1] % n
         r = Result(m, INT, p)
+        assert api.print(C.pointer(r)) == "\n".join(map(str, foreign.tolist()))
         f = api.fetch_column(col, C.pointer(r))
         assert np.array_equal(api.tuples(f), data[foreign])
         got = np.empty(m, np.int32)
