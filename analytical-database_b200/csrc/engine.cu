@@ -37,6 +37,17 @@ struct RouteState {
     uint32_t n = 0;
 };
 
+// Arena buffers the layout functions fill: radix_run's keys and payload, twice; a join build's
+// partition bounds, table offsets, geometry scan chunk sums and sort; a probe's (probe_layout).
+struct RadixBufs { uint32_t *k[2], *v[2]; };
+struct JoinBuildBufs { uint32_t *off1; unsigned long long *toff, *chunk_sums; RadixBufs radix; };
+struct ProbeBufs {
+    adb::HjProbeGeom pg{};
+    unsigned long long *tot = nullptr, *warp_base = nullptr, *chunk_sums = nullptr;
+    uint2 *gc_by_j = nullptr, *res = nullptr;
+    uint32_t *pk = nullptr, *rows = nullptr, *hist = nullptr, *totals = nullptr, *base = nullptr;
+};
+
 struct Engine {
     bool up = false;
     int32_t ctx_index = 0;
@@ -82,12 +93,10 @@ struct Engine {
         bool ready = false;
         uint32_t n_probe = 0, n_build = 0;
         int64_t matches = 0;
-        uint2 *gc_by_j = nullptr;           // {group start, match count} per probe row
-        unsigned long long *warp_base = nullptr;   // first output slot of every probing warp (pg.warps)
-        adb::HjProbeGeom pg{};
+        ProbeBufs probe;                    // what the expansion reads: gc_by_j, warp_base, pg
         RouteState route;                   // routed probe (adb_join_route_probe), 8-byte answers
         bool routed = false;
-        int32_t *build_pos_sorted = nullptr;   // all three live in the arena
+        int32_t *build_pos_sorted = nullptr;
         const int32_t *probe_pos = nullptr;
         bool swapped = false;
         // sharded form (adb_join_build ... adb_join_finish_routed): this context's tables, probed
@@ -95,7 +104,7 @@ struct Engine {
         // expansion
         bool built = false, sharded = false;
         uint32_t part_bits = 1;
-        const unsigned long long *toff = nullptr;
+        JoinBuildBufs build;                // in the arena, like probe and build_pos_sorted
         const uint32_t *probe_keys = nullptr;
         adb::JoinOwners owners{};
     } join;
@@ -380,6 +389,42 @@ template <class T> adb_status grow(DevBuf<T> &b, size_t need, const char *what) 
         CU(release(b));
     }
     return dev_alloc(b, need + need / 8 + (1 << 20), what);
+}
+
+// ---- scratch arena ------------------------------------------------------------------------------
+// A bump allocation over the arena in 256-byte steps; dry (no base, no capacity) it only sums its
+// takes, so an arena user's layout function run dry is what that user reserves.  Past cap: NULL.
+struct Carve {
+    unsigned char *base = nullptr;
+    size_t cap = SIZE_MAX, used = 0;
+    template <class T> T *take(size_t count) {
+        const size_t at = used;
+        used += (count * sizeof(T) + 255) & ~(size_t)255;
+        return base && used <= cap ? reinterpret_cast<T *>(base + at) : nullptr;
+    }
+};
+
+// Make room for `bytes` of temporaries and start a fresh bump allocation.  Whatever lived in
+// the arena before (a join waiting for its emit phase) is gone.
+adb_status arena_reserve(size_t bytes) {
+    g.join = Engine::JoinState{};
+    g.del_rows = -1;
+    g.arena_used = 0;
+    return grow(g.arena, bytes, "sort/join scratch");
+}
+// Take what `layout` carves from where the arena's bump allocation stands; with `reserve`, the
+// arena is first reserved afresh for exactly that (the layout's dry run).  An overrun fails as `what`.
+template <class Layout> adb_status arena_take(Layout &&layout, const char *what, bool reserve = false) {
+    if (reserve) {
+        Carve dry;
+        layout(dry);
+        if (adb_status s = arena_reserve(dry.used)) return s;
+    }
+    Carve c{g.arena.p, g.arena.cap, g.arena_used};
+    layout(c);
+    if (c.used > c.cap) return fail(ADB_ERR_NOMEM, "%s: scratch arena too small", what);
+    g.arena_used = c.used;
+    return ADB_OK;
 }
 
 void jx_close() {
@@ -1805,54 +1850,23 @@ static adb_status ensure_radix_scratch(uint32_t n) {
                 "radix histogram");
 }
 
-// ---- scratch arena ------------------------------------------------------------------------------
-static size_t arena_round(size_t bytes) { return (bytes + 255) & ~(size_t)255; }
-
-// Make room for `bytes` of temporaries and start a fresh bump allocation.  Whatever lived in
-// the arena before (a join waiting for its emit phase) is gone.
-static adb_status arena_reserve(size_t bytes) {
-    g.join = Engine::JoinState{};
-    g.del_rows = -1;
-    g.arena_used = 0;
-    return grow(g.arena, bytes, "sort/join scratch");
-}
-static void *arena_take_bytes(size_t bytes) {
-    void *p = g.arena + g.arena_used;
-    g.arena_used += arena_round(bytes);
-    return p;
-}
-#define ARENA_TAKE(T, count) static_cast<T *>(arena_take_bytes((size_t)(count) * sizeof(T)))
-static size_t radix_scratch_bytes(uint32_t n, int npass) {
-    const size_t one = arena_round((size_t)(n ? n : 1) * 4);
-    return npass == 0 ? one : (npass > 1 ? 4 : 2) * one;
+static RadixBufs radix_layout(Carve &c, uint32_t n) {
+    const size_t m = n ? n : 1;
+    return {{c.take<uint32_t>(m), c.take<uint32_t>(m)}, {c.take<uint32_t>(m), c.take<uint32_t>(m)}};
 }
 
-// Runs `npass` stable passes over (keys, payload); payload starts as pay0, or the row index.  Buffers
-// come from the arena (reserve radix_scratch_bytes first).  The last pass writes to
-// (final_k, final_v) when given.  With npass == 0 the keys are copied and the payload is
-// left NULL (meaning identity).
-static adb_status radix_run(const uint32_t *keys_in, uint32_t n, const adb::RadixPass *passes,
-                            int npass, uint32_t *final_k, uint32_t *final_v, uint32_t **keys_out,
+// Runs `npass` stable passes over (keys, payload) through the buffers `b`; payload starts as pay0,
+// or the row index.  The last pass writes to (final_k, final_v) when given.
+static adb_status radix_run(const uint32_t *keys_in, uint32_t n, const adb::RadixPass *passes, int npass,
+                            const RadixBufs &b, uint32_t *final_k, uint32_t *final_v, uint32_t **keys_out,
                             uint32_t **pay_out, int *launches, const uint32_t *pay0 = nullptr) {
     *keys_out = nullptr;
     *pay_out = nullptr;
     if (adb_status s = ensure_radix_scratch(n)) return s;
-    const size_t cnt = n ? n : 1;
-    if (npass == 0) {
-        uint32_t *k0 = final_k ? final_k : ARENA_TAKE(uint32_t, cnt);
-        if (n) CU(cudaMemcpyAsync(k0, keys_in, (size_t)n * 4, cudaMemcpyDeviceToDevice, g.stream));
-        *keys_out = k0;
-        return ADB_OK;
-    }
-    uint32_t *k[2] = {nullptr, nullptr}, *v[2] = {nullptr, nullptr};
-    for (int i = 0; i < (npass > 1 ? 2 : 1); ++i) {
-        k[i] = ARENA_TAKE(uint32_t, cnt);
-        v[i] = ARENA_TAKE(uint32_t, cnt);
-    }
     const uint32_t *src_k = keys_in, *src_v = pay0;       // pay0 == NULL: payload = row index
     int cur = 0;
     for (int p = 0; p < npass; ++p) {
-        uint32_t *dk = k[cur], *dv = v[cur];
+        uint32_t *dk = b.k[cur], *dv = b.v[cur];
         if (p == npass - 1 && final_k && final_v) { dk = final_k; dv = final_v; }
         *launches += adb::launch_radix_pass(src_k, src_v, dk, dv, n, passes[p], g.rx_hist,
                                             g.rx_totals, g.rx_base, g.sm_count, g.stream);
@@ -1872,10 +1886,11 @@ adb_status adb_index_sort(const int32_t *d_col, int64_t n, int32_t *d_values_out
     if (n == 0) return ADB_OK;
     if (!d_col || !d_values_out || !d_positions_out) return fail(ADB_ERR_INVALID, "adb_index_sort: NULL pointer");
     const adb::RadixPass passes[4] = {{0, 8, 0}, {8, 8, 0}, {16, 8, 0}, {24, 8, 0}};
-    if (adb_status s = arena_reserve(radix_scratch_bytes((uint32_t)n, 4))) return s;
+    RadixBufs b;
+    if (adb_status s = arena_take([&](Carve &c) { b = radix_layout(c, (uint32_t)n); }, "adb_index_sort", true)) return s;
     uint32_t *k = nullptr, *v = nullptr;
     int launches = 0;
-    if (adb_status s = radix_run(reinterpret_cast<const uint32_t *>(d_col), (uint32_t)n, passes, 4,
+    if (adb_status s = radix_run(reinterpret_cast<const uint32_t *>(d_col), (uint32_t)n, passes, 4, b,
                                  reinterpret_cast<uint32_t *>(d_values_out),
                                  reinterpret_cast<uint32_t *>(d_positions_out), &k, &v, &launches)) return s;
     return after_launch("index_sort", launches);
@@ -2089,9 +2104,6 @@ adb_status adb_format_i32_emit(char *d_text) {
 
 // ---- hash join ------------------------------------------------------------------------------------
 static void join_release() { g.join = Engine::JoinState{}; }      // its buffers are arena memory
-// per-warp match counts of the probe (<= 8 warps x 8 CTAs x SMs), the geometry's chunk sums
-// (<= 2^20 partitions / 1024) and a few totals
-static constexpr size_t kJoinSmallScratch = 512 * 1024;
 
 // ADB_TRACE=1: synchronise after every stage of a join and print its wall-clock time.
 struct StageTrace {
@@ -2112,8 +2124,7 @@ struct StageTrace {
 // probe = the side walked in row order.  Output pair k is (build position, probe position).
 //
 // join_build: steps 1-3 (sort on the hash, partition boundaries, one table per partition);
-// leaves {build_pos_sorted, toff, part_bits} in g.join and the tables in g.hj_table.  The arena
-// is reserved for the build AND for `np` probe rows' worth of {group, count} + offsets.
+// leaves {build_pos_sorted, part_bits} in g.join and the tables in g.hj_table.
 // Probe rows partitioned for L2 locality (hash_join.cu, P1-P3) when the tables will not fit L2
 // by a wide margin (`by_size`: each caller's own size rule).  ADB_JOIN_PROBE=direct /
 // partitioned overrides (tests run both forms on the same inputs).
@@ -2122,18 +2133,6 @@ static bool join_probe_partitioned(bool by_size) {
     if (e && !strcmp(e, "direct")) return false;
     if (e && !strcmp(e, "partitioned")) return true;
     return by_size;
-}
-// the routed probe's owner side probing ~np received keys slice by slice: the same buffers once
-// more and the segmented pass' own histogram, totals and bases
-static size_t join_owner_scratch(uint32_t np);
-static size_t join_partition_scratch(uint32_t np) {      // keys + row numbers + results in partition order,
-    return 2 * arena_round((size_t)np * 4) + arena_round((size_t)np * 8) +      // 8 piece sums per 4096 rows
-           arena_round(((size_t)np / adb::kRadixTile + 2) * 8 * 8) + 4096;
-}
-
-static size_t join_owner_scratch(uint32_t np) {
-    return join_partition_scratch(np) + arena_round(((size_t)np / adb::kRadixTile + 512) * 256 * 4) +
-           2 * arena_round((size_t)256 * 256 * 4) + 8192;
 }
 
 static uint32_t join_part_bits(uint32_t nb) {
@@ -2144,29 +2143,80 @@ static uint32_t join_part_bits(uint32_t nb) {
     return part_bits;
 }
 
-// The arena join_build reserves for nb build rows and np probe rows.  The sharded join's owner
-// picks its probe form from what is left of it (adb_join_probe_received), so
-// adb_peer_exchange_reserve must reserve exactly this.
-static size_t join_arena_bytes(uint32_t nb, uint32_t np, bool part_scratch, bool owner_scratch) {
+static JoinBuildBufs join_build_layout(Carve &c, uint32_t nb) {
     const uint32_t num_parts = 1u << join_part_bits(nb);
-    return radix_scratch_bytes(nb, 4) + arena_round((size_t)np * 8) + arena_round((size_t)(num_parts + 1) * 4) +
-           arena_round((size_t)(num_parts + 1) * 8) + (part_scratch ? join_partition_scratch(np) : 0) +
-           (owner_scratch ? join_owner_scratch(np) : 0) + kJoinSmallScratch;
+    return {c.take<uint32_t>(num_parts + 1), c.take<unsigned long long>(num_parts + 1),
+            c.take<unsigned long long>(num_parts / 1024 + 2), radix_layout(c, nb)};
 }
 
-static adb_status join_build(const int32_t *bv, const int32_t *bp, uint32_t nb, uint32_t np, int *launches,
-                             StageTrace &tr, bool part_scratch = false, bool owner_scratch = false) {
+// The partitioned probe's (P1-P3) windows: <= 256 of whole 4096-row tiles.
+static uint32_t probe_window_tiles(uint32_t n) { return ((n + adb::kRadixTile - 1) / adb::kRadixTile + 255) / 256; }
+
+// A probe of n keys by the one-GPU join, by adb_join_finish_routed (partitioned geometry; the rows
+// come back probed) or by the owner of received keys (answers straight into g.rt_recv_res).
+// warp_base: per-warp match counts, scanned into every warp's first output slot.
+enum ProbeUser { kJoinProbe, kFinishProbe, kOwnerProbe };
+static ProbeBufs probe_layout(Carve &c, uint32_t n, bool partitioned, ProbeUser who) {
+    ProbeBufs b;
+    b.pg = partitioned ? adb::hj_probe_geom_partitioned(n) : adb::hj_probe_geom(n, g.sm_count);
+    b.tot = c.take<unsigned long long>(2);
+    if (who != kOwnerProbe) b.gc_by_j = c.take<uint2>(n);
+    b.warp_base = c.take<unsigned long long>(b.pg.warps);
+    if (!partitioned) return b;
+    b.chunk_sums = c.take<unsigned long long>(b.pg.warps / 1024 + 2);
+    if (who == kFinishProbe) return b;
+    b.pk = c.take<uint32_t>(n);
+    b.rows = c.take<uint32_t>(n);
+    b.res = c.take<uint2>(n);
+    if (who == kJoinProbe) return b;
+    // the owner's own: g.rx_hist / g.rx_base still hold the routing pass adb_join_finish_routed reads
+    const uint32_t segs = adb::radix_segments(n, probe_window_tiles(n));
+    b.hist = c.take<uint32_t>(adb::radix_hist_elems(n, probe_window_tiles(n)));
+    b.totals = c.take<uint32_t>((size_t)segs * 256);
+    b.base = c.take<uint32_t>((size_t)segs * 256);
+    return b;
+}
+
+static RouteState route_layout(Carve &c, uint32_t n, size_t answer_bytes) {
+    return {c.take<uint32_t>(n), c.take<uint32_t>(n), c.take<unsigned char>((size_t)n * answer_bytes), n};
+}
+
+// What adb_join_build reserves for nb build rows and np probe rows of this context: the build, the
+// routed rows, the owner's probe of about as many received keys and the finish.  The owner picks
+// its probe form from what is left, so adb_peer_exchange_reserve reserves exactly this.
+static size_t join_arena_bytes(uint32_t nb, uint32_t np) {
+    Carve c;
+    join_build_layout(c, nb);
+    route_layout(c, np, sizeof(uint2));
+    probe_layout(c, np, true, kOwnerProbe);
+    probe_layout(c, INT32_MAX, false, kOwnerProbe);   // the direct probe's sums stop growing at 8 CTAs per SM
+    probe_layout(c, np, true, kFinishProbe);
+    return c.used;
+}
+
+// P1-P3 of the partitioned probe (hash_join.cu): a segmented pass on the top 8 hash bits over the
+// windows, then the probe slice by slice, the results gathered back into key order in gc_by_j.
+static int probe_partitioned(const uint32_t *keys, uint32_t n, const ProbeBufs &b, uint32_t *hist, uint32_t *totals,
+                             uint32_t *base, uint2 *gc_by_j, StageTrace *tr) {
+    const uint32_t want_tiles = probe_window_tiles(n);
+    int k_ = adb::launch_radix_pass_segmented(keys, nullptr, b.pk, b.rows, n, adb::RadixPass{24, 8, 1}, want_tiles,
+                                              hist, totals, base, g.sm_count, g.stream);
+    if (tr) tr->lap("probe rows by window and table slice");
+    return k_ + adb::launch_hj_probe_partitioned(b.pk, b.rows, base, hist, adb::radix_segments(n, want_tiles),
+                                                 adb::radix_seg_tiles(n, want_tiles), n, b.pg, g.join.build.toff,
+                                                 g.join.part_bits, g.hj_table, b.res, gc_by_j, b.warp_base,
+                                                 b.chunk_sums, b.tot, g.stream);
+}
+
+static adb_status join_build(const int32_t *bv, const int32_t *bp, uint32_t nb, int *launches, StageTrace &tr) {
     const uint32_t part_bits = join_part_bits(nb);
     const uint32_t num_parts = 1u << part_bits;
-    if (adb_status s = arena_reserve(join_arena_bytes(nb, np, part_scratch, owner_scratch))) return s;
     auto &j = g.join;
     j.part_bits = part_bits;
     j.n_build = nb;
-    uint32_t *off1 = ARENA_TAKE(uint32_t, num_parts + 1);
-    unsigned long long *toff = ARENA_TAKE(unsigned long long, num_parts + 1);
-    j.toff = toff;
+    const JoinBuildBufs &b = j.build;
     if (nb == 0) {                             // an owner without build rows: every partition is empty
-        CU(cudaMemsetAsync(toff, 0, (size_t)(num_parts + 1) * 8, g.stream));
+        CU(cudaMemsetAsync(b.toff, 0, (size_t)(num_parts + 1) * 8, g.stream));
         j.build_pos_sorted = nullptr;
         return ADB_OK;
     }
@@ -2174,21 +2224,20 @@ static adb_status join_build(const int32_t *bv, const int32_t *bp, uint32_t nb, 
     //    passes is the build position itself, so nothing is gathered afterwards
     const adb::RadixPass sort4[4] = {{0, 8, 1}, {8, 8, 1}, {16, 8, 1}, {24, 8, 1}};
     uint32_t *bk = nullptr, *bi = nullptr;
-    if (adb_status s = radix_run(reinterpret_cast<const uint32_t *>(bv), nb, sort4, 4, nullptr, nullptr, &bk, &bi,
-                                 launches, reinterpret_cast<const uint32_t *>(bp))) return s;
+    if (adb_status s = radix_run(reinterpret_cast<const uint32_t *>(bv), nb, sort4, 4, b.radix, nullptr, nullptr, &bk,
+                                 &bi, launches, reinterpret_cast<const uint32_t *>(bp))) return s;
     j.build_pos_sorted = reinterpret_cast<int32_t *>(bi);
     tr.lap("build sort");
     // 2. partition boundaries -> table geometry: partition p gets a power-of-two slot range
     //    holding its rows at <= 80 % load (<= 4096 slots: built in shared memory)
-    *launches += adb::launch_hj_bounds(bk, nb, part_bits, num_parts, off1, g.stream);
-    *launches += adb::launch_hj_geometry(off1, num_parts, toff, ARENA_TAKE(unsigned long long, num_parts / 1024 + 2),
-                                         g.stream);
+    *launches += adb::launch_hj_bounds(bk, nb, part_bits, num_parts, b.off1, g.stream);
+    *launches += adb::launch_hj_geometry(b.off1, num_parts, b.toff, b.chunk_sums, g.stream);
     unsigned long long slots = 0;
-    if (adb_status s = read_back(&slots, toff + num_parts, sizeof slots)) return s;
+    if (adb_status s = read_back(&slots, b.toff + num_parts, sizeof slots)) return s;
     if (adb_status s = grow(g.hj_table, slots * 16, "join tables")) return s;
     tr.lap("partition boundaries");
     // 3. one table per partition
-    *launches += adb::launch_hj_table_build(bk, j.build_pos_sorted, off1, toff, num_parts, part_bits,
+    *launches += adb::launch_hj_table_build(bk, j.build_pos_sorted, b.off1, b.toff, num_parts, part_bits,
                                             g.hj_table, g.stream);
     tr.lap("per-partition tables");
     return ADB_OK;
@@ -2215,41 +2264,23 @@ static adb_status join_count(const int32_t *bv, const int32_t *bp, int64_t nb64,
     const bool partitioned = join_probe_partitioned(nb >= (6u << 20) && np >= (4u << 20));
     if (partitioned)
         if (adb_status s = ensure_radix_scratch(np > nb ? np : nb)) return s;
-    if (adb_status s = join_build(bv, bp, nb, np, &launches, tr, partitioned)) return s;
+    if (adb_status s = arena_take([&](Carve &c) {
+            g.join.build = join_build_layout(c, nb);
+            g.join.probe = probe_layout(c, np, partitioned, kJoinProbe);
+        }, "adb_join", true)) return s;
+    if (adb_status s = join_build(bv, bp, nb, &launches, tr)) return s;
     auto &j = g.join;
     j.swapped = swapped;
     j.n_probe = np;
     j.probe_pos = pp;
-    unsigned long long *tot = ARENA_TAKE(unsigned long long, 2);
     // 4. probe in row order; every warp leaves the matches of its piece, their scan = the
     //    first output slot of every piece (the expansion computes the slots inside a piece)
-    j.pg = partitioned ? adb::hj_probe_geom_partitioned(np) : adb::hj_probe_geom(np, g.sm_count);
-    j.gc_by_j = ARENA_TAKE(uint2, np);
-    j.warp_base = ARENA_TAKE(unsigned long long, j.pg.warps);
-    if (partitioned) {
-        // <= 256 windows of whole 4096-row tiles, each partitioned on the top 8 hash bits
-        const uint32_t tiles = (np + adb::kRadixTile - 1) / adb::kRadixTile;
-        const uint32_t want_tiles = (tiles + 255) / 256;
-        const uint32_t segs = adb::radix_segments(np, want_tiles);
-        const uint32_t seg_tiles = adb::radix_seg_tiles(np, want_tiles);
-        uint32_t *pk = ARENA_TAKE(uint32_t, np), *rows = ARENA_TAKE(uint32_t, np);
-        uint2 *res = ARENA_TAKE(uint2, np);
-        unsigned long long *chunk_sums = ARENA_TAKE(unsigned long long, j.pg.warps / 1024 + 2);
-        launches += adb::launch_radix_pass_segmented(reinterpret_cast<const uint32_t *>(pv), nullptr, pk, rows, np,
-                                                     adb::RadixPass{24, 8, 1}, want_tiles, g.rx_hist, g.rx_totals,
-                                                     g.rx_base, g.sm_count, g.stream);
-        tr.lap("probe rows by window and table slice");
-        // (the pass' scanned histogram stays in g.rx_hist: where each 4096-row tile's entries
-        // sit inside the cells)
-        launches += adb::launch_hj_probe_partitioned(pk, rows, g.rx_base, g.rx_hist, segs, seg_tiles, np, j.pg,
-                                                     j.toff, j.part_bits, g.hj_table,
-                                                     res, j.gc_by_j, j.warp_base, chunk_sums, tot, g.stream);
-    } else {
-        launches += adb::launch_hj_probe(reinterpret_cast<const uint32_t *>(pv), np, j.pg, j.toff, j.part_bits,
-                                         g.hj_table, j.gc_by_j, j.warp_base, tot,
-                                         g.stream);
-    }
-    if (adb_status s = read_back(&j.matches, tot, sizeof(int64_t))) return s;
+    const ProbeBufs &pb = j.probe;
+    const uint32_t *pkeys = reinterpret_cast<const uint32_t *>(pv);
+    launches += partitioned ? probe_partitioned(pkeys, np, pb, g.rx_hist, g.rx_totals, g.rx_base, pb.gc_by_j, &tr)
+                            : adb::launch_hj_probe(pkeys, np, pb.pg, j.build.toff, j.part_bits, g.hj_table, pb.gc_by_j,
+                                                   pb.warp_base, pb.tot, g.stream);
+    if (adb_status s = read_back(&j.matches, pb.tot, sizeof(int64_t))) return s;
     tr.lap(partitioned ? "probe slice by slice + back to row order" : "probe + piece offsets");
     if (adb_status s = after_launch("join_count", launches)) return s;
     if (j.matches >= (int64_t)1 << 31) {
@@ -2277,7 +2308,10 @@ adb_status adb_join_build(const int32_t *d_v, const int32_t *d_p, int64_t n, int
     int launches = 0;
     StageTrace tr;
     if (adb_status s = ensure_radix_scratch((uint32_t)(n ? n : 1))) return s;
-    if (adb_status s = join_build(d_v, d_p, (uint32_t)n, (uint32_t)probe_rows_hint, &launches, tr, true, true)) return s;
+    if (adb_status s = arena_reserve(join_arena_bytes((uint32_t)n, (uint32_t)probe_rows_hint))) return s;
+    if (adb_status s = arena_take([&](Carve &c) { g.join.build = join_build_layout(c, (uint32_t)n); }, "adb_join_build"))
+        return s;
+    if (adb_status s = join_build(d_v, d_p, (uint32_t)n, &launches, tr)) return s;
     if (adb_status s = after_launch("join_build", launches)) return s;
     CU(cudaStreamSynchronize(g.stream));               // the other contexts' probes read these tables
     g.join.built = true;
@@ -2303,13 +2337,7 @@ static adb_status route_partition(const char *what, int32_t world, const int32_t
     rt.n = n;
     if (n == 0) return ADB_OK;
     if (adb_status s = ensure_radix_scratch(n)) return s;
-    if (reserve)
-        if (adb_status s = arena_reserve(2 * arena_round((size_t)n * 4) + arena_round((size_t)n * answer_bytes) + 4096))
-            return s;
-    rt.items = ARENA_TAKE(uint32_t, n);
-    rt.rows = ARENA_TAKE(uint32_t, n);
-    rt.answers = arena_take_bytes((size_t)n * answer_bytes);
-    if (g.arena_used > g.arena.cap) return fail(ADB_ERR_NOMEM, "%s: scratch arena too small", what);
+    if (adb_status s = arena_take([&](Carve &c) { rt = route_layout(c, n, answer_bytes); }, what, reserve)) return s;
     const int k_ = adb::launch_radix_pass_segmented(reinterpret_cast<const uint32_t *>(d_in), nullptr, rt.items,
                                                     rt.rows, n, pass, 0, g.rx_hist, g.rx_totals, g.rx_base,
                                                     g.sm_count, g.stream);
@@ -2368,50 +2396,21 @@ adb_status adb_join_probe_received(int64_t n_recv) {
     if (n_recv == 0) return ADB_OK;
     const uint32_t n = (uint32_t)n_recv;
     StageTrace tr;
-    int k_ = 0;
-    // A table well beyond L2 (two or four GPUs: >= 24 M build rows here) is probed slice by slice
-    // like the one-GPU join's (hash_join.cu P1-P3), the answers gathered back into the order the
-    // keys arrived in.  The pass needs a histogram of its own: g.rx_hist / g.rx_base still hold
-    // this context's ROUTING pass, which adb_join_finish_routed reads.  No room in the arena (a
-    // skewed key set sent most of the probe side here): the direct probe.
-    bool partitioned = join_probe_partitioned(n >= (4u << 20) && j.n_build >= (24u << 20));
-    if (partitioned) {
-        const uint32_t tiles = (n + adb::kRadixTile - 1) / adb::kRadixTile;
-        const uint32_t want_tiles = (tiles + 255) / 256;
-        const uint32_t segs = adb::radix_segments(n, want_tiles);
-        const uint32_t seg_tiles = adb::radix_seg_tiles(n, want_tiles);
-        const adb::HjProbeGeom pg = adb::hj_probe_geom_partitioned(n);
-        const size_t hist_elems = adb::radix_hist_elems(n, want_tiles);
-        const size_t need = 2 * arena_round((size_t)n * 4) + arena_round((size_t)n * 8) +
-                            arena_round(hist_elems * 4) + 2 * arena_round((size_t)segs * 256 * 4) +
-                            arena_round((size_t)pg.warps * 8) + arena_round(((size_t)pg.warps / 1024 + 2) * 8) + 4096;
-        // (what adb_join_finish_routed still takes for this context's own probe rows stays free)
-        const size_t finish = arena_round((size_t)j.route.n * 8) + arena_round(((size_t)j.route.n / 512 + 8) * 8) +
-                              (1 << 20);
-        if (g.arena_used + need + finish <= g.arena.cap) {
-            uint32_t *pk = ARENA_TAKE(uint32_t, n), *rows = ARENA_TAKE(uint32_t, n);
-            uint2 *res = ARENA_TAKE(uint2, n);
-            uint32_t *hist = ARENA_TAKE(uint32_t, hist_elems);
-            uint32_t *totals = ARENA_TAKE(uint32_t, (size_t)segs * 256), *base = ARENA_TAKE(uint32_t, (size_t)segs * 256);
-            unsigned long long *sums = ARENA_TAKE(unsigned long long, pg.warps);
-            unsigned long long *chunk_sums = ARENA_TAKE(unsigned long long, pg.warps / 1024 + 2);
-            unsigned long long *tot = ARENA_TAKE(unsigned long long, 2);
-            k_ += adb::launch_radix_pass_segmented(g.rt_recv_keys, nullptr, pk, rows, n, adb::RadixPass{24, 8, 1},
-                                                   want_tiles, hist, totals, base, g.sm_count, g.stream);
-            k_ += adb::launch_hj_probe_partitioned(pk, rows, base, hist, segs, seg_tiles, n, pg, j.toff, j.part_bits,
-                                                   g.hj_table, res, g.rt_recv_res, sums,
-                                                   chunk_sums, tot, g.stream);
-        } else {
-            partitioned = false;
-        }
-    }
-    if (!partitioned) {
-        const adb::HjProbeGeom pg = adb::hj_probe_geom(n, g.sm_count);
-        unsigned long long *sums = ARENA_TAKE(unsigned long long, pg.warps);
-        if (g.arena_used > g.arena.cap) return fail(ADB_ERR_NOMEM, "adb_join_probe_received: scratch arena too small");
-        k_ += adb::launch_hj_probe_plain(g.rt_recv_keys, n, j.toff, j.part_bits, g.hj_table,
-                                         g.rt_recv_res, sums, g.sm_count, g.stream);
-    }
+    // A table well beyond L2 (two or four GPUs: >= 24 M build rows here) is probed slice by slice like
+    // the one-GPU join's.  No room for that next to what adb_join_finish_routed still takes for this
+    // context's own probe rows (a skewed key set sent most of the probe side here): the direct probe.
+    Carve need;
+    probe_layout(need, n, true, kOwnerProbe);
+    probe_layout(need, j.route.n, true, kFinishProbe);
+    const bool partitioned = join_probe_partitioned(n >= (4u << 20) && j.n_build >= (24u << 20)) &&
+                             g.arena_used + need.used <= g.arena.cap;
+    ProbeBufs b;
+    if (adb_status s = arena_take([&](Carve &c) { b = probe_layout(c, n, partitioned, kOwnerProbe); },
+                                  "adb_join_probe_received")) return s;
+    const int k_ = partitioned
+        ? probe_partitioned(g.rt_recv_keys, n, b, b.hist, b.totals, b.base, g.rt_recv_res, nullptr)
+        : adb::launch_hj_probe_plain(g.rt_recv_keys, n, j.build.toff, j.part_bits, g.hj_table, g.rt_recv_res,
+                                     b.warp_base, g.sm_count, g.stream);
     if (adb_status s = after_launch("join_probe_received", k_)) return s;
     CU(cudaStreamSynchronize(g.stream));               // the rows' homes pull the answers next
     tr.lap("received keys in + probe");
@@ -2448,17 +2447,14 @@ adb_status adb_join_finish_routed(int32_t world, const int32_t *d_pv, const int3
         if (h_matches) *h_matches = 0;
         return ADB_OK;
     }
-    unsigned long long *tot = ARENA_TAKE(unsigned long long, 2);
-    j.pg = adb::hj_probe_geom_partitioned(np);
-    j.gc_by_j = ARENA_TAKE(uint2, np);
-    j.warp_base = ARENA_TAKE(unsigned long long, j.pg.warps);
-    unsigned long long *chunk_sums = ARENA_TAKE(unsigned long long, j.pg.warps / 1024 + 2);
-    if (g.arena_used > g.arena.cap) return fail(ADB_ERR_NOMEM, "adb_join_finish_routed: scratch arena too small");
+    if (adb_status s = arena_take([&](Carve &c) { j.probe = probe_layout(c, np, true, kFinishProbe); },
+                                  "adb_join_finish_routed")) return s;
+    const ProbeBufs &b = j.probe;
     StageTrace tr;
     int launches = adb::launch_hj_unpartition_routed(j.route.rows, static_cast<const uint2 *>(j.route.answers),
-                                                     g.rx_base, g.rx_hist, np, (uint32_t)world, j.pg, j.gc_by_j,
-                                                     j.warp_base, chunk_sums, tot, g.stream);
-    if (adb_status s = read_back(&j.matches, tot, sizeof(int64_t))) return s;
+                                                     g.rx_base, g.rx_hist, np, (uint32_t)world, b.pg, b.gc_by_j,
+                                                     b.warp_base, b.chunk_sums, b.tot, g.stream);
+    if (adb_status s = read_back(&j.matches, b.tot, sizeof(int64_t))) return s;
     tr.lap("answers back to row order + piece offsets");
     if (adb_status s = after_launch("join_finish_routed", launches)) return s;
     if (j.matches >= (int64_t)1 << 31)
@@ -2517,7 +2513,7 @@ adb_status adb_peer_exchange_reserve(int64_t send_pairs, int64_t build_pairs, in
     if ((uint32_t)probe_rows > big) big = (uint32_t)probe_rows;            // the routed probe's partition pass
     if (adb_status s = ensure_radix_scratch(big ? big : 1)) return s;
     const uint32_t nb = (uint32_t)build_pairs, np = (uint32_t)probe_rows;
-    if (adb_status s = arena_reserve(join_arena_bytes(nb, np, true, true))) return s;
+    if (adb_status s = arena_reserve(join_arena_bytes(nb, np))) return s;
     const uint32_t num_parts = 1u << join_part_bits(nb);
     // tables: <= 2.5 slots per build row (power-of-two capacity at <= 80 % load) + 16 per partition
     const unsigned long long slots = (unsigned long long)nb * 5 / 2 + 16ull * num_parts + 4096;
@@ -2544,10 +2540,10 @@ adb_status adb_join_emit(int32_t *d_out1, int32_t *d_out2) {
         if (!d_out1 || !d_out2) return fail(ADB_ERR_INVALID, "adb_join_emit: NULL output");
         int32_t *ob = j.swapped ? d_out2 : d_out1, *op = j.swapped ? d_out1 : d_out2;
         const int k_ = j.sharded
-            ? adb::launch_hj_expand_sharded(j.gc_by_j, j.warp_base, j.pg, j.n_probe, j.probe_keys, j.owners,
+            ? adb::launch_hj_expand_sharded(j.probe.gc_by_j, j.probe.warp_base, j.probe.pg, j.n_probe, j.probe_keys, j.owners,
                                             j.probe_pos, ob, op, g.stream)
-            : adb::launch_hj_expand(j.gc_by_j, j.warp_base, j.pg, j.n_probe, j.build_pos_sorted, j.probe_pos, ob, op,
-                                    g.stream);
+            : adb::launch_hj_expand(j.probe.gc_by_j, j.probe.warp_base, j.probe.pg, j.n_probe, j.build_pos_sorted,
+                                    j.probe_pos, ob, op, g.stream);
         rc = after_launch("join_expand", k_);
     }
     if (j.sharded) {
@@ -2700,10 +2696,12 @@ adb_status adb_delete_rows_plan(int64_t n_rows, const int32_t *d_pos, int64_t n_
     if (!h_rows_left || (n_pos > 0 && !d_pos)) return fail(ADB_ERR_INVALID, "adb_delete_rows_plan: NULL pointer");
     if (n_rows == 0) { *h_rows_left = 0; g.del_rows = 0; return ADB_OK; }
     if (adb_status s = ensure_radix_scratch(1)) return s;
-    if (adb_status s = arena_reserve(2 * arena_round((size_t)n_rows * 4) + 4096)) return s;
-    g.del_dead = ARENA_TAKE(uint32_t, n_rows);
-    g.del_before = ARENA_TAKE(uint32_t, n_rows);
-    int64_t *tot = ARENA_TAKE(int64_t, 2);
+    int64_t *tot = nullptr;
+    if (adb_status s = arena_take([&](Carve &c) {
+            g.del_dead = c.take<uint32_t>(n_rows);
+            g.del_before = c.take<uint32_t>(n_rows);
+            tot = c.take<int64_t>(2);
+        }, "adb_delete_rows_plan", true)) return s;
     CU(cudaMemsetAsync(g.del_dead, 0, (size_t)n_rows * 4, g.stream));
     int k_ = adb::launch_mark_rows(g.del_dead, n_rows, d_pos, n_pos, base_pos, g.sm_count, g.stream);
     k_ += adb::launch_exclusive_scan(g.del_dead, 1, g.del_before, (uint32_t)n_rows, g.sc_sums, tot, g.sm_count, g.stream);
