@@ -409,7 +409,6 @@ __device__ __forceinline__ void mbox_publish(volatile unsigned long long *pub, u
     __threadfence_system();
     pub[kMboxWords] = seq;
 }
-int launch_select(const SelectArgs &a, cudaStream_t s);
 // two-phase form: mask + per-chunk counts (+ total into a.d_count), then expand into a.out
 int launch_select_mask(const SelectArgs &a, bool with_total, cudaStream_t s);
 int launch_select_expand(const SelectArgs &a, cudaStream_t s);

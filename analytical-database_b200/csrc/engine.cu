@@ -70,7 +70,7 @@ struct Engine {
     int64_t idx_pending_n = -1;         // >= 0 between adb_select_index_count and _emit
     adb::SelectArgs sel_pending{};      // valid between adb_select_*_count and adb_select_emit
     bool sel_ready = false;
-    uint64_t sel_generation = 0;        // bumped by every select_prepare (adb_select_generation)
+    uint64_t sel_generation = 0;        // bumped by every drop_pending (adb_select_generation)
     // small results travel to the host through a mapped pinned mailbox (read_back)
     unsigned long long *mbox = nullptr;  // kMboxWords payload words, then the flag word
     unsigned long long *mbox_dev = nullptr;
@@ -290,6 +290,14 @@ static adb_status mbox_wait(unsigned long long seq, void *h_dst, size_t bytes) {
 #endif
     }
     memcpy(h_dst, g.mbox, bytes);
+    return ADB_OK;
+}
+
+// An aggregate a kernel published itself: {sum, count, min | max << 32} (mbox_publish).
+static adb_status mbox_wait_agg(unsigned long long seq, adb_agg *h) {
+    unsigned long long w[3];
+    if (adb_status s = mbox_wait(seq, w, sizeof w)) return s;
+    *h = adb_agg{(int64_t)w[0], (int64_t)w[1], (int32_t)(uint32_t)w[2], (int32_t)(uint32_t)(w[2] >> 32)};
     return ADB_OK;
 }
 
@@ -908,20 +916,30 @@ static adb_status finish_count(int64_t *d_count, int64_t *h_count) {
     return read_back(h_count, d_count, sizeof(int64_t));
 }
 
+// The pending select (adb_select_count*) is dropped, and adb_select_generation() bumped, when a
+// select is about to overwrite its bitmap and when an emit consumes it.  So whether a refused call
+// drops it depends on what was refused: a select that refuses an output pointer (adb_select_scan,
+// adb_chain_select_*) leaves it as it was, one that refuses its length or input column has
+// dropped it; the deferred emit (adb_select_emit_fetch_agg*) leaves it on any refusal;
+// adb_select_emit has taken it before it checks its output.
+static void drop_pending() { g.sel_ready = false; ++g.sel_generation; }
+
+// The setup every select runs, in this order: NEED_UP, the entry point's own output-pointer rule
+// (null_out), drop_pending, then the length, the input column, the bounds, the bitmap and the
+// SelectArgs.
 // stable_val: d_val is a base column -- no operator ever writes it, so the predicate pass may
 // request its first tile while the previous kernel on the stream is still draining (any other
 // input may be that kernel's output and must wait for it: ADVICE r1, select_scan.cu).
-static adb_status select_prepare(const char *what, const int32_t *d_val, const int32_t *d_pos,
-                                 int64_t n_max, const int64_t *d_n, const int32_t *lo,
-                                 const int32_t *hi, int64_t *d_count, adb::SelectArgs *a,
-                                 bool stable_val = false) {
+static adb_status select_prepare(const char *what, bool null_out, const int32_t *d_val, int64_t n_max,
+                                 const int64_t *d_n, const int32_t *lo, const int32_t *hi,
+                                 int64_t *d_count, adb::SelectArgs *a, bool stable_val = false) {
     NEED_UP();
-    g.sel_ready = false;
-    ++g.sel_generation;
+    if (null_out) return fail(ADB_ERR_INVALID, "%s: NULL device pointer", what);
+    drop_pending();
     if (adb_status s = check_len(n_max, what)) return s;
     if (n_max > 0 && !d_val) return fail(ADB_ERR_INVALID, "%s: NULL device pointer", what);
     *a = adb::SelectArgs{};
-    a->val = d_val; a->pos_in = d_pos; a->d_n = d_n; a->n = (uint32_t)n_max;
+    a->val = d_val; a->d_n = d_n; a->n = (uint32_t)n_max;
     a->stable_val = stable_val;
     fold_range(lo, hi, &a->range);
     a->d_count = d_count ? d_count : g.scratch_count;
@@ -929,6 +947,7 @@ static adb_status select_prepare(const char *what, const int32_t *d_val, const i
     if (adb_status s = grow(g.sel_mask, sizeof(uint32_t) * adb::select_mask_words(a->n, g.sm_count), "select bitmap"))
         return s;
     a->mask = g.sel_mask; a->counts = g.sel_counts; a->sm_count = g.sm_count;
+    a->agg_scratch = g.agg_scratch; a->agg_ticket = g.agg_ticket;
     return ADB_OK;
 }
 
@@ -936,27 +955,12 @@ adb_status adb_select_scan(const int32_t *d_col, int64_t n, const int32_t *lo, c
                            int32_t base_pos, int32_t *d_pos_out, int64_t *d_count,
                            int64_t *h_count) {
     adb::SelectArgs a;
-    if (!d_count || (n > 0 && !d_pos_out)) {
-        NEED_UP();
-        return fail(ADB_ERR_INVALID, "adb_select_scan: NULL device pointer");
-    }
-    if (adb_status s = select_prepare("adb_select_scan", d_col, nullptr, n, nullptr, lo, hi, d_count, &a, true)) return s;
+    if (adb_status s = select_prepare("adb_select_scan", !d_count || (n > 0 && !d_pos_out), d_col, n, nullptr,
+                                      lo, hi, d_count, &a, true))
+        return s;
     a.base_pos = base_pos; a.out = d_pos_out;
-    if (adb_status s = after_launch("select_scan", adb::launch_select(a, g.stream))) return s;
-    return finish_count(d_count, h_count);
-}
-
-adb_status adb_select_pairs(const int32_t *d_val, const int32_t *d_pos, int64_t n_max,
-                            const int64_t *d_n, const int32_t *lo, const int32_t *hi,
-                            int32_t *d_pos_out, int64_t *d_count, int64_t *h_count) {
-    adb::SelectArgs a;
-    if (!d_count || (n_max > 0 && (!d_pos || !d_pos_out))) {
-        NEED_UP();
-        return fail(ADB_ERR_INVALID, "adb_select_pairs: NULL device pointer");
-    }
-    if (adb_status s = select_prepare("adb_select_pairs", d_val, d_pos, n_max, d_n, lo, hi, d_count, &a)) return s;
-    a.base_pos = 0; a.out = d_pos_out;
-    if (adb_status s = after_launch("select_pairs", adb::launch_select(a, g.stream))) return s;
+    const int k_ = adb::launch_select_mask(a, false, g.stream);
+    if (adb_status s = after_launch("select_scan", k_ + adb::launch_select_expand(a, g.stream))) return s;
     return finish_count(d_count, h_count);
 }
 
@@ -967,7 +971,7 @@ adb_status adb_select_count(const int32_t *d_val, int64_t n_max, const int64_t *
                             const int32_t *lo, const int32_t *hi, int64_t *d_count,
                             int64_t *h_count) {
     adb::SelectArgs a;
-    if (adb_status s = select_prepare("adb_select_count", d_val, nullptr, n_max, d_n, lo, hi, d_count, &a)) return s;
+    if (adb_status s = select_prepare("adb_select_count", false, d_val, n_max, d_n, lo, hi, d_count, &a)) return s;
     if (adb_status s = after_launch("select_count", adb::launch_select_mask(a, true, g.stream))) return s;
     g.sel_pending = a;
     g.sel_ready = true;
@@ -981,7 +985,8 @@ adb_status adb_select_count(const int32_t *d_val, int64_t n_max, const int64_t *
 adb_status adb_select_count_base(const int32_t *d_col, int64_t n, const int32_t *lo, const int32_t *hi,
                                  int32_t base_pos, int64_t *d_count, int64_t *h_count) {
     adb::SelectArgs a;
-    if (adb_status s = select_prepare("adb_select_count_base", d_col, nullptr, n, nullptr, lo, hi, d_count, &a, true)) return s;
+    if (adb_status s = select_prepare("adb_select_count_base", false, d_col, n, nullptr, lo, hi, d_count, &a, true))
+        return s;
     // the host wants the count: the kernel that totals it also hands it over (no publish launch)
     const bool fused_pub = h_count && g.mbox && a.n > 0;
     if (fused_pub) { a.pub = g.mbox_dev; a.pub_seq = ++g.mbox_seq; }
@@ -999,8 +1004,7 @@ adb_status adb_select_count_base(const int32_t *d_col, int64_t n, const int32_t 
 adb_status adb_select_emit(const int32_t *d_pos_in, int32_t base_pos, int32_t *d_pos_out) {
     NEED_UP();
     if (!g.sel_ready) return fail(ADB_ERR_INVALID, "adb_select_emit: no pending adb_select_count");
-    g.sel_ready = false;
-    ++g.sel_generation;                             // the pending count is consumed
+    drop_pending();                                 // the pending count is consumed
     adb::SelectArgs a = g.sel_pending;
     if (a.n == 0) return ADB_OK;
     if (!d_pos_out) return fail(ADB_ERR_INVALID, "adb_select_emit: NULL output");
@@ -1011,67 +1015,78 @@ adb_status adb_select_emit(const int32_t *d_pos_in, int32_t base_pos, int32_t *d
 
 uint64_t adb_select_generation(void) { return g.sel_generation; }
 
-// Deferred emit of a select whose consumers turned out to be fetch + aggregate: the fused
-// second kernel of the chain, after the host has read the count (SURVEY.md 8f rank 3).
-static adb_status emit_fetch_agg_impl(const int32_t *d_fetch_col, int32_t *d_pos_out, int32_t *d_val_out,
-                                      adb_agg *d_agg, adb_agg *h_agg, const adb::PeerExchange *px) {
-    NEED_UP();
-    if (!g.sel_ready) return fail(ADB_ERR_INVALID, "adb_select_emit_fetch_agg: no pending adb_select_count");
-    if (g.sel_pending.pos_in || g.sel_pending.d_n)
-        return fail(ADB_ERR_INVALID, "adb_select_emit_fetch_agg: the pending select is not over a base column");
-    // both outputs NULL: aggregate only -- nothing is materialised and the pending select stays
-    // pending (the bitmap is only read), so a later emit can still write the handles
-    const bool nostore = !d_pos_out && !d_val_out;
-    if (!d_agg || (g.sel_pending.n > 0 && (!d_fetch_col || (!nostore && (!d_pos_out || !d_val_out)))))
-        return fail(ADB_ERR_INVALID, "adb_select_emit_fetch_agg: NULL device pointer");
-    if (!nostore) {
-        g.sel_ready = false;
-        ++g.sel_generation;                         // the pending count is consumed
-    }
-    adb::SelectArgs a = g.sel_pending;
-    int64_t *d_count = a.d_count;                   // written by the count phase
-    a.out = d_pos_out;                              // base_pos: what the count phase recorded
-    a.d_count = g.scratch_count;                    // the expansion rewrites the same total
-    a.fetch_col = d_fetch_col; a.val_out = d_val_out;
-    a.agg_out = d_agg; a.agg_scratch = g.agg_scratch; a.agg_ticket = g.agg_ticket;
+// The second kernel of the materialised chain and of the deferred emit: positions, gather and
+// aggregate (with px, the exchange too) in one launch.  Where that kernel cannot run -- an empty
+// column, or a grid larger than the fold scratch -- the three-operator form runs instead and reads
+// the hit count from d_count; the aggregate-only form (a.out == a.val_out == NULL) has no such
+// fallback for a non-empty select.  h_agg (optional) receives the aggregate, straight from the
+// kernel when it can publish it itself.
+static adb_status fused_finish(const char *what, adb::SelectArgs &a, const int64_t *d_count,
+                               const adb::PeerExchange *px, adb_agg *h_agg) {
     if (px) a.px = *px;
+    const bool nostore = !a.out && !a.val_out;
     const bool fused_pub = nostore && h_agg && g.mbox && a.n > 0;
     if (fused_pub) { a.pub = g.mbox_dev; a.pub_seq = ++g.mbox_seq; }
     const int f_ = adb::launch_select_expand_fetch_agg(a, g.stream);
     if (f_ > 0) {
-        if (adb_status s = after_launch("select_emit_fetch_agg", f_)) return s;
-        if (fused_pub) {
-            unsigned long long w[3];
-            if (adb_status s = mbox_wait(a.pub_seq, w, sizeof w)) return s;
-            h_agg->sum = (int64_t)w[0];
-            h_agg->count = (int64_t)w[1];
-            h_agg->min = (int32_t)(uint32_t)w[2];
-            h_agg->max = (int32_t)(uint32_t)(w[2] >> 32);
-            if (px && h_agg->count < 0)
-                return fail(ADB_ERR_CUDA, "aggregate exchange: a peer did not arrive within 2 s (epoch %u)", px->epoch);
-            return ADB_OK;
-        }
+        if (adb_status s = after_launch(what, f_)) return s;
     } else if (nostore && a.n > 0) {
-        return fail(ADB_ERR_INVALID, "adb_select_emit_fetch_agg: a select over %u rows cannot be aggregated unmaterialised", a.n);
+        return fail(ADB_ERR_INVALID, "%s: a select over %u rows cannot be aggregated unmaterialised", what, a.n);
     } else {
-        // empty column (or a grid larger than the fold scratch): the three-operator form
-        if (adb_status s = after_launch("select_emit_fetch_agg", adb::launch_select_expand(a, g.stream))) return s;
-        if (adb_status s = adb_fetch(d_fetch_col, d_pos_out, a.n, d_count, a.base_pos, d_val_out)) return s;
-        if (adb_status s = adb_aggregate(d_val_out, a.n, d_count, d_agg, nullptr)) return s;
+        if (adb_status s = after_launch(what, adb::launch_select_expand(a, g.stream))) return s;
+        if (adb_status s = adb_fetch(a.fetch_col, a.out, a.n, d_count, a.base_pos, a.val_out)) return s;
+        if (adb_status s = adb_aggregate(a.val_out, a.n, d_count, a.agg_out, nullptr)) return s;
         if (px)
             if (adb_status s = after_launch("chain exchange", adb::launch_agg_combine_allreduce(*px, g.stream))) return s;
     }
-    if (h_agg) {
-        if (adb_status s = read_back(h_agg, px ? px->final_out : d_agg, sizeof(adb_agg))) return s;
-        if (px && h_agg->count < 0)
-            return fail(ADB_ERR_CUDA, "aggregate exchange: a peer did not arrive within 2 s (epoch %u)", px->epoch);
-    }
+    if (!h_agg) return ADB_OK;
+    if (adb_status s = fused_pub ? mbox_wait_agg(a.pub_seq, h_agg)
+                                 : read_back(h_agg, px ? px->final_out : a.agg_out, sizeof(adb_agg)))
+        return s;
+    if (px && h_agg->count < 0)
+        return fail(ADB_ERR_CUDA, "%s: a peer did not arrive within 2 s (epoch %u)", what, px->epoch);
     return ADB_OK;
+}
+
+// Deferred emit of a select whose consumers turned out to be fetch + aggregate: the fused
+// second kernel of the chain, after the host has read the count (SURVEY.md 8f rank 3).
+static adb_status emit_fetch_agg_impl(const char *what, const int32_t *d_fetch_col, int32_t *d_pos_out,
+                                      int32_t *d_val_out, adb_agg *d_agg, adb_agg *h_agg,
+                                      const adb::PeerExchange *px) {
+    NEED_UP();
+    if (!g.sel_ready) return fail(ADB_ERR_INVALID, "%s: no pending adb_select_count", what);
+    adb::SelectArgs a = g.sel_pending;
+    if (a.d_n) return fail(ADB_ERR_INVALID, "%s: the pending select is not over a base column", what);
+    // both outputs NULL: aggregate only -- nothing is materialised and the pending select stays
+    // pending (the bitmap is only read), so a later emit can still write the handles
+    const bool nostore = !d_pos_out && !d_val_out;
+    if (!d_agg || (a.n > 0 && (!d_fetch_col || (!nostore && (!d_pos_out || !d_val_out)))))
+        return fail(ADB_ERR_INVALID, "%s: NULL device pointer", what);
+    if (!nostore) drop_pending();                   // the pending count is consumed
+    const int64_t *d_count = a.d_count;             // written by the count phase
+    a.d_count = g.scratch_count;                    // the expansion rewrites the same total
+    a.out = d_pos_out; a.fetch_col = d_fetch_col; a.val_out = d_val_out; a.agg_out = d_agg;
+    return fused_finish(what, a, d_count, px, h_agg);     // base_pos: what the count phase recorded
 }
 
 adb_status adb_select_emit_fetch_agg(const int32_t *d_fetch_col, int32_t *d_pos_out, int32_t *d_val_out,
                                      adb_agg *d_agg, adb_agg *h_agg) {
-    return emit_fetch_agg_impl(d_fetch_col, d_pos_out, d_val_out, d_agg, h_agg, nullptr);
+    return emit_fetch_agg_impl("adb_select_emit_fetch_agg", d_fetch_col, d_pos_out, d_val_out, d_agg, h_agg, nullptr);
+}
+
+// The descriptor of this context's next aggregate exchange (epoch peer_epoch + 1).  Every
+// context must take part in every exchange, so a context that advances its epoch and then fails
+// has left the group out of step.  The three callers advance it at different points:
+//   adb_agg_combine_allreduce            once its arguments are accepted;
+//   adb_select_emit_fetch_agg_exchange   once a pending select is found, before the remaining checks;
+//   adb_chain_select_fetch_agg_exchange  only when the chain was enqueued.
+// Making them agree would change what a group does after one rank fails.
+static adb_status peer_exchange(const char *what, const adb_agg *d_parts, int32_t k, adb_agg *d_out,
+                                adb::PeerExchange *px) {
+    NEED_UP();
+    if (!g.peer_connected) return fail(ADB_ERR_INVALID, "%s: adb_peer_connect first", what);
+    *px = adb::PeerExchange{g.peer_boxes_dev, g.peer_rank, g.peer_world, g.peer_epoch + 1, d_parts, k, d_out};
+    return ADB_OK;
 }
 
 // The deferred emit with the cross-context exchange riding in the same kernel: this context's
@@ -1080,15 +1095,13 @@ adb_status adb_select_emit_fetch_agg(const int32_t *d_fetch_col, int32_t *d_pos_
 adb_status adb_select_emit_fetch_agg_exchange(const int32_t *d_fetch_col, int32_t *d_pos_out,
                                               int32_t *d_val_out, adb_agg *d_part, adb_agg *d_out,
                                               adb_agg *h_out) {
-    NEED_UP();
-    if (!g.peer_connected) return fail(ADB_ERR_INVALID, "adb_select_emit_fetch_agg_exchange: adb_peer_connect first");
-    if (!d_part || !d_out) return fail(ADB_ERR_INVALID, "adb_select_emit_fetch_agg_exchange: NULL device pointer");
-    const adb::PeerExchange px{g.peer_boxes_dev, g.peer_rank, g.peer_world, g.peer_epoch + 1, d_part, 1, d_out};
-    // the epoch advances as soon as the arguments are accepted: every context must take part
-    // in every exchange, so a context that fails below has desynchronised the group anyway
-    if (!g.sel_ready) return fail(ADB_ERR_INVALID, "adb_select_emit_fetch_agg_exchange: no pending adb_select_count_base");
+    const char *what = "adb_select_emit_fetch_agg_exchange";
+    adb::PeerExchange px;
+    if (adb_status s = peer_exchange(what, d_part, 1, d_out, &px)) return s;
+    if (!d_part || !d_out) return fail(ADB_ERR_INVALID, "%s: NULL device pointer", what);
+    if (!g.sel_ready) return fail(ADB_ERR_INVALID, "%s: no pending adb_select_count_base", what);
     ++g.peer_epoch;
-    return emit_fetch_agg_impl(d_fetch_col, d_pos_out, d_val_out, d_part, h_out, &px);
+    return emit_fetch_agg_impl(what, d_fetch_col, d_pos_out, d_val_out, d_part, h_out, &px);
 }
 
 adb_status adb_fetch(const int32_t *d_col, const int32_t *d_pos, int64_t n_max,
@@ -1224,19 +1237,16 @@ adb_status adb_peer_connect(const unsigned char *handles) {
 }
 
 adb_status adb_agg_combine_allreduce(const adb_agg *d_parts, int32_t k, adb_agg *d_out, adb_agg *h_out) {
-    NEED_UP();
-    if (!g.peer_connected) return fail(ADB_ERR_INVALID, "adb_agg_combine_allreduce: adb_peer_connect first");
+    adb::PeerExchange px;
+    if (adb_status s = peer_exchange("adb_agg_combine_allreduce", d_parts, k, d_out, &px)) return s;
     if (k < 0 || !d_out || (k > 0 && !d_parts))
         return fail(ADB_ERR_INVALID, "adb_agg_combine_allreduce: bad arguments");
-    const uint32_t epoch = ++g.peer_epoch;
-    const int k_ = adb::launch_agg_combine_allreduce(
-        adb::PeerExchange{g.peer_boxes_dev, g.peer_rank, g.peer_world, epoch, d_parts, k, d_out}, g.stream);
-    if (adb_status s = after_launch("agg_combine_allreduce", k_)) return s;
-    if (h_out) {
-        if (adb_status s = read_back(h_out, d_out, sizeof(adb_agg))) return s;
-        if (h_out->count < 0)
-            return fail(ADB_ERR_CUDA, "adb_agg_combine_allreduce: a peer did not arrive within 2 s (epoch %u)", epoch);
-    }
+    ++g.peer_epoch;
+    if (adb_status s = after_launch("agg_combine_allreduce", adb::launch_agg_combine_allreduce(px, g.stream))) return s;
+    if (!h_out) return ADB_OK;
+    if (adb_status s = read_back(h_out, d_out, sizeof(adb_agg))) return s;
+    if (h_out->count < 0)
+        return fail(ADB_ERR_CUDA, "adb_agg_combine_allreduce: a peer did not arrive within 2 s (epoch %u)", px.epoch);
     return ADB_OK;
 }
 
@@ -1505,33 +1515,22 @@ static adb_status chain_impl(const int32_t *d_sel_col, const int32_t *d_fetch_co
                              int64_t n, const int32_t *lo, const int32_t *hi,
                              int32_t *d_pos_out, int32_t *d_val_out,
                              int64_t *d_count, adb_agg *d_agg, const adb::PeerExchange *px) {
+    const char *what = "adb_chain_select_fetch_agg";
     adb::SelectArgs a;
-    if (!d_count || !d_agg || (n > 0 && (!d_pos_out || !d_val_out || !d_fetch_col))) {
-        NEED_UP();
-        return fail(ADB_ERR_INVALID, "adb_chain_select_fetch_agg: NULL device pointer");
-    }
-    if (adb_status s = select_prepare("adb_chain_select_fetch_agg", d_sel_col, nullptr, n, nullptr, lo, hi, d_count, &a, true)) return s;
-    a.base_pos = 0; a.out = d_pos_out;
-    a.fetch_col = d_fetch_col; a.val_out = d_val_out;
-    a.agg_out = d_agg; a.agg_scratch = g.agg_scratch; a.agg_ticket = g.agg_ticket;
-    if (px) a.px = *px;
+    if (adb_status s = select_prepare(what, !d_count || !d_agg || (n > 0 && (!d_pos_out || !d_val_out || !d_fetch_col)),
+                                      d_sel_col, n, nullptr, lo, hi, d_count, &a, true))
+        return s;
+    a.out = d_pos_out; a.fetch_col = d_fetch_col; a.val_out = d_val_out; a.agg_out = d_agg;
     // two launches: predicate pass -> bitmap, then expansion with the gather and the
     // aggregates fused in (positions and values are still materialised)
     const int32_t mb = g.chain_mark_base;
     g.chain_mark_base = -1;
     if (mb >= 0) adb_mark(mb);
-    int k_ = adb::launch_select_mask(a, false, g.stream);
+    if (adb_status s = after_launch(what, adb::launch_select_mask(a, false, g.stream))) return s;
     if (mb >= 0) adb_mark(mb + 1);
-    const int f_ = adb::launch_select_expand_fetch_agg(a, g.stream);
+    const adb_status s = fused_finish(what, a, d_count, px, nullptr);
     if (mb >= 0) adb_mark(mb + 2);
-    if (f_ > 0) return after_launch("chain", k_ + f_);
-    // empty column (or a grid larger than the fold scratch): the three-operator form
-    k_ += adb::launch_select_expand(a, g.stream);
-    if (adb_status s = after_launch("chain", k_)) return s;
-    if (adb_status s = adb_fetch(d_fetch_col, d_pos_out, n, d_count, 0, d_val_out)) return s;
-    if (adb_status s = adb_aggregate(d_val_out, n, d_count, d_agg, nullptr)) return s;
-    if (!px) return ADB_OK;
-    return after_launch("chain exchange", adb::launch_agg_combine_allreduce(*px, g.stream));
+    return s;
 }
 
 adb_status adb_chain_select_fetch_agg(const int32_t *d_sel_col, const int32_t *d_fetch_col,
@@ -1547,13 +1546,10 @@ adb_status adb_chain_select_agg(const int32_t *d_sel_col, const int32_t *d_fetch
                                 const int32_t *lo, const int32_t *hi, int64_t *d_count, adb_agg *d_agg,
                                 adb_agg *h_agg) {
     adb::SelectArgs a;
-    if (!d_count || !d_agg || (n > 0 && !d_fetch_col)) {
-        NEED_UP();
-        return fail(ADB_ERR_INVALID, "adb_chain_select_agg: NULL device pointer");
-    }
-    if (adb_status s = select_prepare("adb_chain_select_agg", d_sel_col, nullptr, n, nullptr, lo, hi, d_count, &a, true)) return s;
-    a.fetch_col = d_fetch_col;
-    a.agg_out = d_agg; a.agg_scratch = g.agg_scratch; a.agg_ticket = g.agg_ticket;
+    if (adb_status s = select_prepare("adb_chain_select_agg", !d_count || !d_agg || (n > 0 && !d_fetch_col),
+                                      d_sel_col, n, nullptr, lo, hi, d_count, &a, true))
+        return s;
+    a.fetch_col = d_fetch_col; a.agg_out = d_agg;
     const int f_ = adb::launch_scan_gather_agg(a, g.stream);
     if (f_ > 0) {
         if (adb_status s = after_launch("chain (unmaterialised)", f_)) return s;
@@ -1570,10 +1566,9 @@ adb_status adb_chain_select_fetch_agg_exchange(const int32_t *d_sel_col, const i
                                                int64_t n, const int32_t *lo, const int32_t *hi,
                                                int32_t *d_pos_out, int32_t *d_val_out, int64_t *d_count,
                                                adb_agg *d_parts, int32_t k, adb_agg *d_out) {
-    NEED_UP();
-    if (!g.peer_connected) return fail(ADB_ERR_INVALID, "adb_chain_select_fetch_agg_exchange: adb_peer_connect first");
+    adb::PeerExchange px;
+    if (adb_status s = peer_exchange("adb_chain_select_fetch_agg_exchange", d_parts, k, d_out, &px)) return s;
     if (k < 1 || !d_parts || !d_out) return fail(ADB_ERR_INVALID, "adb_chain_select_fetch_agg_exchange: bad arguments");
-    const adb::PeerExchange px{g.peer_boxes_dev, g.peer_rank, g.peer_world, g.peer_epoch + 1, d_parts, k, d_out};
     const adb_status s = chain_impl(d_sel_col, d_fetch_col, n, lo, hi, d_pos_out, d_val_out, d_count,
                                     d_parts + (k - 1), &px);
     if (s == ADB_OK) ++g.peer_epoch;          // the exchange was enqueued: every rank advances together
@@ -1825,17 +1820,6 @@ adb_status adb_shared_select_plan(const int32_t *lows, const int32_t *highs, int
         memcpy(plan_out, hp.bytes.data(), hp.bytes.size());
     }
     return ADB_OK;
-}
-
-adb_status adb_shared_select(const int32_t *d_col, int64_t n, const int32_t *lows,
-                             const int32_t *highs, int32_t q_count, int32_t *d_pos_out,
-                             int64_t stride, int64_t *h_counts) {
-    int64_t tmp[ADB_MAX_BATCH];
-    if (adb_status s = adb_shared_select_count(d_col, n, lows, highs, q_count, h_counts ? h_counts : tmp)) return s;
-    if (!d_pos_out && n > 0) return fail(ADB_ERR_INVALID, "adb_shared_select: NULL output");
-    int32_t *ptrs[ADB_MAX_BATCH];
-    for (int32_t q = 0; q < q_count; ++q) ptrs[q] = d_pos_out + (size_t)q * stride;
-    return adb_shared_select_emit(ptrs, stride);
 }
 
 // ---- radix sort / partition helpers ---------------------------------------------------------
@@ -2650,17 +2634,6 @@ adb_status adb_select_index_emit(const adb_index *ix, int32_t *d_pos_out) {
     if (!d_pos_out) return fail(ADB_ERR_INVALID, "adb_select_index_emit: NULL output");
     return after_launch("index_emit", adb::launch_index_emit(ix->positions, ix->n, g.idx_bounds,
                                                              d_pos_out, g.sm_count, g.stream));
-}
-
-adb_status adb_select_index(const adb_index *ix, int32_t use_btree, const int32_t *lo,
-                            const int32_t *hi, int32_t *d_pos_out, int64_t *d_count,
-                            int64_t *h_count) {
-    NEED_UP();
-    if (!ix || !d_count || (ix->n > 0 && !d_pos_out))
-        return fail(ADB_ERR_INVALID, "adb_select_index: NULL pointer");
-    if (adb_status s = adb_select_index_count(ix, use_btree, lo, hi, d_count, nullptr)) return s;
-    if (adb_status s = adb_select_index_emit(ix, d_pos_out)) return s;
-    return finish_count(d_count, h_count);
 }
 
 // ColumnIndex.positions are size_t on the host (src/include/cs165_api.h:65-68) and truncated to

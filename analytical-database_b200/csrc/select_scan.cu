@@ -609,10 +609,6 @@ int launch_scan_gather_agg(const SelectArgs &a, cudaStream_t s) {
     return 1;
 }
 
-int launch_select(const SelectArgs &a, cudaStream_t s) {
-    return launch_select_mask(a, false, s) + launch_select_expand(a, s);
-}
-
 // Load this file's kernels now (CUDA loads them lazily, on first launch): a first launch that
 // has to load code while another context's kernel spin-waits for this one can stall behind it.
 void preload_select_scan() {

@@ -121,7 +121,6 @@ class Engine:
         "adb_chain_marks": (C.c_int32, [C.c_int32]),
         "adb_mark_elapsed": (C.c_int32, [C.c_int32, C.c_int32, C.POINTER(C.c_float)]),
         "adb_select_scan": (C.c_int32, [_I32P, C.c_int64, _I32P, _I32P, C.c_int32, _I32P, _I64P, _I64P]),
-        "adb_select_pairs": (C.c_int32, [_I32P, _I32P, C.c_int64, _I64P, _I32P, _I32P, _I32P, _I64P, _I64P]),
         "adb_select_count": (C.c_int32, [_I32P, C.c_int64, _I64P, _I32P, _I32P, _I64P, _I64P]),
         "adb_select_emit": (C.c_int32, [_I32P, C.c_int32, _I32P]),
         "adb_select_emit_fetch_agg": (C.c_int32, [_I32P, _I32P, _I32P, C.POINTER(_AggStruct), C.POINTER(_AggStruct)]),
@@ -154,11 +153,9 @@ class Engine:
         "adb_chain_select_fetch_agg": (C.c_int32, [_I32P, _I32P, C.c_int64, _I32P, _I32P, _I32P, _I32P, _I64P, C.POINTER(_AggStruct)]),
         "adb_shared_select_count": (C.c_int32, [_I32P, C.c_int64, _I32P, _I32P, C.c_int32, _I64P]),
         "adb_shared_select_emit": (C.c_int32, [C.POINTER(C.c_void_p), C.c_int64]),
-        "adb_shared_select": (C.c_int32, [_I32P, C.c_int64, _I32P, _I32P, C.c_int32, _I32P, C.c_int64, _I64P]),
         "adb_shared_select_plan": (C.c_int32, [_I32P, _I32P, C.c_int32, C.c_void_p, C.c_size_t, C.POINTER(C.c_uint32)]),
         "adb_index_create": (C.c_int32, [_I32P, _I32P, C.c_int64, C.c_int32, C.POINTER(C.c_void_p)]),
         "adb_index_destroy": (C.c_int32, [C.c_void_p]),
-        "adb_select_index": (C.c_int32, [C.c_void_p, C.c_int32, _I32P, _I32P, _I32P, _I64P, _I64P]),
         "adb_index_sort": (C.c_int32, [_I32P, C.c_int64, _I32P, _I32P]),
         "adb_hash_join_count": (C.c_int32, [_I32P, _I32P, C.c_int64, _I32P, _I32P, C.c_int64, _I64P]),
         "adb_nested_loop_join_count": (C.c_int32, [_I32P, _I32P, C.c_int64, _I32P, _I32P, C.c_int64, _I64P]),
@@ -358,9 +355,9 @@ class Engine:
         out, d_count = self.alloc_i32(n_max), self.alloc(8)
         (plo, _a), (phi, _b) = _bound(lo), _bound(hi)
         h = C.c_int64(-1)
-        self._ck(self.lib.adb_select_pairs(val.i32(), pos.i32(), n_max, d_n.i64() if d_n else None,
-                                           plo, phi, out.i32(), d_count.i64(),
-                                           C.byref(h) if sync else None))
+        self._ck(self.lib.adb_select_count(val.i32(), n_max, d_n.i64() if d_n else None, plo, phi,
+                                           d_count.i64(), C.byref(h) if sync else None))
+        self._ck(self.lib.adb_select_emit(pos.i32(), 0, out.i32()))
         return out, d_count, (int(h.value) if sync else None)
 
     def select_exact(self, val: DevBuf, n: int, lo=None, hi=None, pos_in: DevBuf | None = None,
@@ -459,8 +456,8 @@ class Engine:
         out, d_count = self.alloc_i32(n), self.alloc(8)
         (plo, _a), (phi, _b) = _bound(lo), _bound(hi)
         h = C.c_int64(-1)
-        self._ck(self.lib.adb_select_index(handle, int(use_btree), plo, phi, out.i32(),
-                                           d_count.i64(), C.byref(h)))
+        self._ck(self.lib.adb_select_index_count(handle, int(use_btree), plo, phi, d_count.i64(), C.byref(h)))
+        self._ck(self.lib.adb_select_index_emit(handle, out.i32()))
         d_count.free()
         return out, int(h.value)
 

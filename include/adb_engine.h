@@ -125,20 +125,14 @@ ADB_API adb_status adb_select_scan(const int32_t *d_col, int64_t n, const int32_
                            int32_t base_pos, int32_t *d_pos_out, int64_t *d_count,
                            int64_t *h_count);
 
-/* ---- range select over a (value, position) pair list -- replaces select_result,
- * src/query.c:38-86.  n_max bounds the input length; when d_n is non-NULL the actual
- * length is read from that device int64 (<= n_max). */
-ADB_API adb_status adb_select_pairs(const int32_t *d_val, const int32_t *d_pos, int64_t n_max,
-                            const int64_t *d_n, const int32_t *lo, const int32_t *hi,
-                            int32_t *d_pos_out, int64_t *d_count, int64_t *h_count);
-
 /* ---- two-phase select: size the position list exactly (the reference mallocs row_count
  * ints per select, query.c:94; 2 GB per handle on a 500 M-row shard is not an option in
  * HBM).  adb_select_count runs the predicate pass over d_val (a base column or the value
  * half of a pair list) and returns the hit count; adb_select_emit then writes the positions:
  * base_pos + row when d_pos_in is NULL (select_column_scan), d_pos_in[row] otherwise
- * (select_result).  d_count may be NULL.  Any other select between the two calls
- * invalidates the pending count. */
+ * (select_result, src/query.c:38-86).  n_max bounds the input length; when d_n is non-NULL
+ * the actual length is read from that device int64 (<= n_max).  d_count may be NULL.  Any
+ * other select between the two calls invalidates the pending count. */
 ADB_API adb_status adb_select_count(const int32_t *d_val, int64_t n_max, const int64_t *d_n,
                             const int32_t *lo, const int32_t *hi, int64_t *d_count,
                             int64_t *h_count);
@@ -332,8 +326,7 @@ ADB_API adb_status adb_chain_select_agg(const int32_t *d_sel_col, const int32_t 
  *   adb_shared_select_count  scans, classifies, returns every query's hit count;
  *   adb_shared_select_emit   writes query q's ascending positions to d_out_ptrs[q]
  *                            (a HOST array of q_count device pointers), at most `capacity`
- *                            positions each.
- * adb_shared_select is the one-shot form: query q's list lands at d_pos_out + q * stride. */
+ *                            positions each. */
 #define ADB_MAX_BATCH 150
 ADB_API adb_status adb_shared_select_count(const int32_t *d_col, int64_t n, const int32_t *lows,
                                            const int32_t *highs, int32_t q_count, int64_t *h_counts);
@@ -343,9 +336,6 @@ ADB_API adb_status adb_shared_select_emit(int32_t *const *d_out_ptrs, int64_t ca
 ADB_API adb_status adb_shared_select_count_base(const int32_t *d_col, int64_t n, int32_t base_pos,
                                                 const int32_t *lows, const int32_t *highs, int32_t q_count,
                                                 int64_t *h_counts);
-ADB_API adb_status adb_shared_select(const int32_t *d_col, int64_t n, const int32_t *lows,
-                                     const int32_t *highs, int32_t q_count, int32_t *d_pos_out,
-                                     int64_t stride, int64_t *h_counts);
 
 /* Host-only (no device, no adb_init): the lookup tables adb_shared_select_count would upload
  * for this batch, for inspection and tests.  plan_out may be NULL to size the buffer.
@@ -369,7 +359,7 @@ ADB_API adb_status adb_shared_select_plan(const int32_t *lows, const int32_t *hi
  * to int when it emits them, query.c:187).  The arrays stay owned by the caller -- upload
  * the reference's own ColumnIndex for bit-exact tie order, or build one with
  * adb_index_sort().  with_btree additionally bulk-loads a fan-out-32 implicit B+-tree.
- * adb_select_index emits d_positions[first .. first+count) in index order with exactly the
+ * adb_select_index_emit writes d_positions[first .. first+count) in index order with exactly the
  * reference's result in its defined domain (including the low == high quirk) and scan
  * semantics where the reference crashes (low/high below the minimum, NULL bounds). */
 typedef struct adb_index adb_index;
@@ -380,11 +370,8 @@ ADB_API adb_status adb_index_destroy(adb_index *ix);
  * answers positions[lb(low) .. lb(high)) of its slice; the caller applies the low == high quirk
  * of query.c:181-188 to the whole index. */
 ADB_API adb_status adb_index_set_slice(adb_index *ix, int32_t is_slice);
-ADB_API adb_status adb_select_index(const adb_index *ix, int32_t use_btree, const int32_t *lo,
-                                    const int32_t *hi, int32_t *d_pos_out, int64_t *d_count,
-                                    int64_t *h_count);
 
-/* two-phase form, as adb_select_count / adb_select_emit */
+/* two phases, as adb_select_count / adb_select_emit */
 ADB_API adb_status adb_select_index_count(const adb_index *ix, int32_t use_btree, const int32_t *lo,
                                           const int32_t *hi, int64_t *d_count, int64_t *h_count);
 ADB_API adb_status adb_select_index_emit(const adb_index *ix, int32_t *d_pos_out);

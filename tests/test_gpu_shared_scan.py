@@ -1,4 +1,4 @@
-"""GPU parity for batch_queries/batch_execute (BASELINE config 2): adb_shared_select against
+"""GPU parity for batch_queries/batch_execute (BASELINE config 2): adb_shared_select_count/_emit against
 the oracle's restatement of shared_select (query.c:450-583) and, on the value domain where
 the reference's slicing is valid (SURVEY A6), against the unmodified reference objects.
 Mirrors milestone2.py: 2 queries disjoint / partial / subsumed (:42-160), 10 queries, and

@@ -44,16 +44,17 @@ def bench_shared(eng, scale):
     out = {"rows": n, "queries": q, "hits": hits, "ms": med, "best_ms": best,
            "rows_per_s": n / (med * 1e-3), "pred_evals_per_s": n * q / (med * 1e-3),
            "alg_gbs": (4 * n + 4 * hits) / (med * 1e-3) / 1e9}
-    # the same batch into one slab (adb_shared_select: a C caller's single call, no per-result
-    # allocation): q x stride ints
+    # the same batch into one slab (no per-result allocation): query i's list at slab + i * stride
     stride = 2 * (n // 1000) + 4096
     slab = eng.alloc_i32(q * stride)
     cnts = (C.c_int64 * q)()
     lo_p = lows.ctypes.data_as(C.POINTER(C.c_int32))
     hi_p = highs.ctypes.data_as(C.POINTER(C.c_int32))
+    ptrs = (C.c_void_p * q)(*[slab.ptr + 4 * stride * i for i in range(q)])
 
     def run_slab():
-        eng._ck(eng.lib.adb_shared_select(col.i32(), n, lo_p, hi_p, q, slab.i32(), stride, cnts))
+        eng._ck(eng.lib.adb_shared_select_count(col.i32(), n, lo_p, hi_p, q, cnts))
+        eng._ck(eng.lib.adb_shared_select_emit(ptrs, stride))
     med_s, best_s = timed(eng, run_slab)
     assert sum(cnts) == hits
     out["slab_ms"] = med_s
