@@ -510,13 +510,26 @@ int launch_shared_emit(const uint32_t *hitlist, const uint32_t *chunk_hits,
 #define ADB_RADIX_TILE 4096
 #endif
 constexpr uint32_t kRadixTile = ADB_RADIX_TILE;
+// Owner of a key among `parts` owners (the multi-GPU exchange's routing): the routing hash
+// h = key * 0x85EBCA6B scaled to [0, parts), floor(h * parts / 2^32).  Every owner takes
+// floor(2^32 / parts) or that + 1 of the hash values; for parts = 2^k it is h >> (32 - k), the top
+// k bits.  The routing pass and the sharded expansion both call this, so a key is always looked
+// up on the owner it was sent to.
+__device__ __forceinline__ uint32_t route_owner(uint32_t key, uint32_t parts) {
+    return __umulhi(key * 0x85EBCA6Bu, parts);
+}
+
 // Stable radix partition passes + generic exclusive scan (radix.cu).
 struct RadixPass {
     int shift, bits;           // digit = (f(key) >> shift) & ((1 << bits) - 1), bits <= 8
-    int hash;                  // f = key ^ 0x80000000 (0: signed order), key * 0x9E3779B1 (1: join
-                               // hash) or key * 0x85EBCA6B (2: routing hash, multi-GPU exchange);
+    int hash;                  // f = key ^ 0x80000000 (0: signed order) or key * 0x9E3779B1 (1: join
+                               // hash); 2: digit = route_owner(key, parts) (multi-GPU exchange;
+                               // shift unused, bits = ceil(log2 parts) so the histograms hold it);
                                // 3: digit = key / div (the shard a row number lives on; shift unused)
-    uint32_t div = 1;
+    union {
+        uint32_t div = 1;      // hash 3
+        uint32_t parts;        // hash 2: the owner count, 1 .. 256
+    };
 };
 struct RadixGeom {
     uint32_t rows_per_cta, ctas;
@@ -625,14 +638,14 @@ int launch_hj_expand(const uint2 *gc_by_j, const unsigned long long *warp_base, 
                      int32_t *out_build, int32_t *out_probe, cudaStream_t s);
 
 // The join sharded over several contexts (SURVEY.md 8e): the build side is hash-partitioned
-// over the owners (adb_peer_exchange_pairs' routing hash), every owner builds the tables of its
+// over the owners (adb_peer_exchange_pairs' route_owner), every owner builds the tables of its
 // share, and every context's probe rows -- in their original order -- are answered by the owner
 // of each key (the routed probe above).  Output pairs then come out probe-major per context, and
 // the contexts' outputs concatenated in shard order are the reference's list.  The expansion
 // reads a multi-row group's build positions from its owner over NVLink peer memory.
 struct JoinOwners {
     const int32_t *bpos[kMaxPeers];                  // build positions sorted by hash (multi-row groups)
-    uint32_t route_bits;                             // owner = (key * 0x85EBCA6B) >> (32 - route_bits)
+    uint32_t count;                                  // owner of a key = route_owner(key, count)
 };
 int launch_hj_expand_sharded(const uint2 *gc_by_j, const unsigned long long *warp_base, const HjProbeGeom &pg,
                              uint32_t n_probe, const uint32_t *pkeys, const JoinOwners &owners,

@@ -1285,6 +1285,16 @@ adb_status adb_peer_join_connect(const unsigned char *handles) {
     return jx_table_upload();
 }
 
+// The multi-GPU exchange's pass: digit = route_owner(key, parts), for any parts in [1, 256].  Its
+// histograms, bases and scatter cover 2^ceil(log2 parts) buckets as any pass' do; those from parts
+// up stay empty.
+static adb::RadixPass routing_pass(int parts) {
+    adb::RadixPass p{0, 0, 2};
+    while ((1 << p.bits) < parts) ++p.bits;
+    p.parts = (uint32_t)parts;
+    return p;
+}
+
 adb_status adb_peer_exchange_pairs(int32_t side, const int32_t *d_val, const int32_t *d_pos, int64_t n,
                                    int64_t *h_recv_count, const int32_t **d_recv_val,
                                    const int32_t **d_recv_pos) {
@@ -1294,11 +1304,8 @@ adb_status adb_peer_exchange_pairs(int32_t side, const int32_t *d_val, const int
     if (side < 0 || side > 1 || !h_recv_count || !d_recv_val || !d_recv_pos || (n > 0 && (!d_val || !d_pos)))
         return fail(ADB_ERR_INVALID, "adb_peer_exchange_pairs: bad arguments");
     const int world = g.peer_world;
-    if (world & (world - 1)) return fail(ADB_ERR_INVALID, "adb_peer_exchange_pairs: world size %d is not a power of two", world);
-    int bits = 0;
-    while ((1 << bits) < world) ++bits;
     if (adb_status s = ensure_radix_scratch((uint32_t)(n ? n : 1))) return s;
-    const adb::RadixPass pass{32 - bits, bits, 2};            // the routing hash of adb_route_pairs
+    const adb::RadixPass pass = routing_pass(world);          // the owners of adb_route_pairs
     const adb::PairExchange x{g.peer_boxes_dev, g.peer_rank, world, ++g.jx_epoch, g.jx_cap};
     const unsigned long long key_off = (unsigned long long)(2 * side) * g.jx_cap;
     const unsigned long long pay_off = (unsigned long long)(2 * side + 1) * g.jx_cap;
@@ -1881,14 +1888,14 @@ adb_status adb_index_sort(const int32_t *d_col, int64_t n, int32_t *d_values_out
 }
 
 // Multi-GPU join exchange, send side: stable partition of a (value, position) pair list by
-// destination rank = top log2(parts) bits of the routing hash (independent of the join's own
+// destination rank = route_owner of the value (its routing hash is independent of the join's own
 // partition hash, so the receiving rank's local partitions stay balanced).
 adb_status adb_route_pairs(const int32_t *d_val, const int32_t *d_pos, int64_t n, int32_t parts,
                            int32_t *d_val_out, int32_t *d_pos_out, int64_t *h_counts) {
     NEED_UP();
     if (adb_status s = check_len(n, "adb_route_pairs")) return s;
-    if (parts < 1 || parts > 256 || (parts & (parts - 1)) || !h_counts)
-        return fail(ADB_ERR_INVALID, "adb_route_pairs: parts must be a power of two in [1, 256]");
+    if (parts < 1 || parts > 256 || !h_counts)
+        return fail(ADB_ERR_INVALID, "adb_route_pairs: parts must be in [1, 256]");
     if (n > 0 && (!d_val || !d_pos || !d_val_out || !d_pos_out))
         return fail(ADB_ERR_INVALID, "adb_route_pairs: NULL device pointer");
     for (int32_t r = 0; r < parts; ++r) h_counts[r] = 0;
@@ -1900,13 +1907,11 @@ adb_status adb_route_pairs(const int32_t *d_val, const int32_t *d_pos, int64_t n
         return ADB_OK;
     }
     if (adb_status s = ensure_radix_scratch((uint32_t)n)) return s;
-    int bits = 0;
-    while ((1 << bits) < parts) ++bits;
     const int k_ = adb::launch_radix_pass(reinterpret_cast<const uint32_t *>(d_val),
                                           reinterpret_cast<const uint32_t *>(d_pos),
                                           reinterpret_cast<uint32_t *>(d_val_out),
                                           reinterpret_cast<uint32_t *>(d_pos_out), (uint32_t)n,
-                                          adb::RadixPass{32 - bits, bits, 2}, g.rx_hist, g.rx_totals,
+                                          routing_pass(parts), g.rx_hist, g.rx_totals,
                                           g.rx_base, g.sm_count, g.stream);
     if (adb_status s = after_launch("route_pairs", k_)) return s;
     uint32_t totals[256];
@@ -2335,7 +2340,7 @@ static adb_status route_partition(const char *what, int32_t world, const int32_t
     return ADB_OK;
 }
 
-// The sharded join's probe routes the keys by the top bits of the routing hash; the owner probes
+// The sharded join's probe routes the keys to their route_owner; the owner probes
 // them against its own tables and the rows' home puts the 8-byte answers back in row order (the
 // same gather as the one-GPU partitioned probe; cells = owners).  Probing in place and reading
 // each remote key's slot over NVLink instead costs one 32-byte response per 16 useful bytes, 8.8 G
@@ -2347,12 +2352,10 @@ adb_status adb_join_route_probe(int32_t world, const int32_t *d_pv, int64_t np64
     NEED_UP();
     auto &j = g.join;
     if (!j.built) return fail(ADB_ERR_INVALID, "adb_join_route_probe: no preceding adb_join_build on this context");
-    if (world < 2 || world > ADB_MAX_PEERS || (world & (world - 1)))
-        return fail(ADB_ERR_INVALID, "adb_join_route_probe: world %d must be a power of two in [2, %d]", world, ADB_MAX_PEERS);
+    if (world < 2 || world > ADB_MAX_PEERS)
+        return fail(ADB_ERR_INVALID, "adb_join_route_probe: world %d must be in [2, %d]", world, ADB_MAX_PEERS);
     if (np64 > (int64_t)j.n_probe) return fail(ADB_ERR_INVALID, "adb_join_route_probe: more probe rows than adb_join_build reserved for");
-    int bits = 0;
-    while ((1 << bits) < world) ++bits;
-    if (adb_status s = route_partition("adb_join_route_probe", world, d_pv, np64, adb::RadixPass{32 - bits, bits, 2},
+    if (adb_status s = route_partition("adb_join_route_probe", world, d_pv, np64, routing_pass(world),
                                        sizeof(uint2), false, j.route, h_counts, d_routed_keys, d_answers))
         return s;
     j.routed = true;
@@ -2406,8 +2409,8 @@ adb_status adb_join_finish_routed(int32_t world, const int32_t *d_pv, const int3
     NEED_UP();
     auto &j = g.join;
     if (!j.built || !j.routed) return fail(ADB_ERR_INVALID, "adb_join_finish_routed: no preceding adb_join_route_probe");
-    if (world < 2 || world > ADB_MAX_PEERS || (world & (world - 1)))
-        return fail(ADB_ERR_INVALID, "adb_join_finish_routed: world %d must be a power of two in [2, %d]", world, ADB_MAX_PEERS);
+    if (world < 2 || world > ADB_MAX_PEERS)
+        return fail(ADB_ERR_INVALID, "adb_join_finish_routed: world %d must be in [2, %d]", world, ADB_MAX_PEERS);
     if ((uint32_t)np64 != j.route.n) return fail(ADB_ERR_INVALID, "adb_join_finish_routed: row count differs from adb_join_route_probe");
     if (np64 > 0 && (!d_pv || !d_pp)) return fail(ADB_ERR_INVALID, "adb_join_finish_routed: NULL device pointer");
     const uint32_t np = (uint32_t)np64;
@@ -2417,7 +2420,7 @@ adb_status adb_join_finish_routed(int32_t world, const int32_t *d_pv, const int3
         if (!E.up || !E.join.built) return fail(ADB_ERR_INVALID, "adb_join_finish_routed: context %d has built no tables", r);
         o.bpos[r] = E.join.build_pos_sorted;
     }
-    while ((1 << o.route_bits) < world) ++o.route_bits;
+    o.count = (uint32_t)world;
     j.owners = o;
     j.sharded = true;
     j.swapped = swapped != 0;

@@ -685,18 +685,14 @@ __device__ __forceinline__ void hj_load_owners(const JoinOwners &o, HjOwnersShar
         for (int k = 0; k < kMaxPeers; ++k) s.bpos[k] = o.bpos[k];
     __syncthreads();
 }
-__device__ __forceinline__ uint32_t hj_owner(uint32_t key, uint32_t route_bits) {
-    return route_bits ? (key * 0x85EBCA6Bu) >> (32 - route_bits) : 0u;
-}
-
 struct HjOwnerLists {
     const HjOwnersShared *so;
     __device__ __forceinline__ const int32_t *list(uint32_t w) const { return so->bpos[w]; }
 };
 struct HjOwnerOfRow {                                   // whose sorted build list holds row j's group
     const uint32_t *__restrict__ pkeys;
-    uint32_t route_bits;
-    __device__ __forceinline__ uint32_t operator()(uint32_t j) const { return hj_owner(pkeys[j], route_bits); }
+    uint32_t owners;
+    __device__ __forceinline__ uint32_t operator()(uint32_t j) const { return route_owner(pkeys[j], owners); }
 };
 
 __global__ void __launch_bounds__(HJ_THREADS)
@@ -707,7 +703,7 @@ hj_expand_sharded_kernel(const uint2 *__restrict__ gc_by_j, const unsigned long 
     __shared__ HjOwnersShared so;
     hj_load_owners(owners, so);
     hj_expand_body(gc_by_j, warp_base, rows_per_warp, n_probe, HjOwnerLists{&so},
-                   HjOwnerOfRow{pkeys, owners.route_bits}, probe_pos, out_build, out_probe);
+                   HjOwnerOfRow{pkeys, owners.count}, probe_pos, out_build, out_probe);
 }
 
 // ---- launchers --------------------------------------------------------------------------------------

@@ -8,7 +8,8 @@
 //   * hash join    (hash_join.cu): one or two passes on the top bits of a multiplicative
 //     hash split both inputs into partitions small enough for a shared-memory table while
 //     keeping the original row order inside every partition (stability is what makes the
-//     join's output order reproducible).
+//     join's output order reproducible); across GPUs, one pass groups keys by owner
+//     (route_owner, any owner count).
 //
 // One pass = histogram (per-CTA, per-bucket counts) -> row scan of the [bucket][cta] matrix
 // -> bucket bases -> stable scatter.  Inside the scatter a step covers 256 consecutive rows:
@@ -33,9 +34,15 @@ struct RxDigit {
           flip(HASH == 0 ? ((0x80000000u >> p.shift) & ((1u << p.bits) - 1u)) : 0u) {}
     __device__ __forceinline__ uint32_t operator()(uint32_t key) const {
         if (HASH == 1) return ((key * 0x9E3779B1u) >> shift) & mask;
-        if (HASH == 2) return ((key * 0x85EBCA6Bu) >> shift) & mask;
         return ((key >> shift) & mask) ^ flip;
     }
+};
+// digit = the key's owner among p.parts (any count, not only powers of two)
+template <>
+struct RxDigit<2> {
+    uint32_t parts;
+    __host__ __device__ explicit RxDigit(const RadixPass &p) : parts(p.parts) {}
+    __device__ __forceinline__ uint32_t operator()(uint32_t key) const { return route_owner(key, parts); }
 };
 // digit = key / div, at most mask: floor(2^32 / div) as the multiplier is never more than one
 // below the quotient

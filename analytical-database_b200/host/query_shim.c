@@ -2764,9 +2764,9 @@ Result *sub(Result *column_one, Result *column_two, Status *ret_status) {
 /* src/query.c:585-696.  results[0] lists side-one positions, results[1] side-two positions;
  * hash join is probe-major over side two, nested-loop outer-major over side one.  The
  * caller frees the two-element array (src/server.c:432).
- * A GPU count that is not a power of two (the exchange's routing takes hash bits): the four
- * operands are brought to context 0 over peer copies and joined there. */
-/* G = 2, 4, 8, 16: the join itself is sharded.  The build side is hash-partitioned over the GPUs
+ * One GPU, or an empty side: the single-context join on context 0. */
+/* G > 1: the join itself is sharded.  A key's owner is its routing hash scaled to [0, G), so every
+ * GPU count splits the keys near evenly.  The build side is hash-partitioned over the GPUs
  * through peer memory (adb_peer_exchange_pairs), every GPU builds the tables of its keys, and
  * every GPU's slice of the probe side, in its original order, is routed to the keys' owners,
  * probed there, and the answers come home in bulk.  The slices' outputs concatenated in shard
@@ -2893,7 +2893,7 @@ static Result **join(Result *v1, Result *p1, Result *v2, Result *p2, int nested,
     t_err[0] = '\0';
     const char *what = nested ? "nested_loop_join" : "hash_join";
     if (ensure_up()) return op_fail(st, what);
-    if (S.G > 1 && (S.G & (S.G - 1)) == 0 && v1 && p1 && v2 && p2 && v1->num_tuples && v2->num_tuples &&
+    if (S.G > 1 && v1 && p1 && v2 && p2 && v1->num_tuples && v2->num_tuples &&
         p1->num_tuples >= v1->num_tuples && p2->num_tuples >= v2->num_tuples)
         return join_sharded(v1, p1, v2, p2, nested, st);
     ShardList a, b, c, d, o1, o2;

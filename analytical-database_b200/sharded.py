@@ -172,6 +172,9 @@ class EngineOps:
         return out
 
     def route_pairs(self, val, pos, parts):
+        """adb_route_pairs: the pairs grouped by destination rank, stable, and the per-rank
+        counts.  A value's rank is its routing hash scaled to [0, parts); parts = the world size,
+        any count in [1, 256]."""
         vo, po = self.empty(val.numel()), self.empty(val.numel())
         counts = (C.c_int64 * parts)()
         self.eng._ck(self.lib.adb_route_pairs(self._p(val), self._p(pos), val.numel(), parts,

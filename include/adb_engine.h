@@ -272,7 +272,7 @@ ADB_API adb_status adb_chain_select_fetch_agg_exchange(const int32_t *d_sel_col,
  * source rank and in source order inside a piece -- the layout of an all-to-all-v.  On
  * return (*h_recv_count pairs at *d_recv_val / *d_recv_pos, valid until the next exchange
  * of the same side) every source's pairs have landed.  side is 0 or 1, so both inputs of a
- * join can be resident at once.  Collective; world must be a power of two.
+ * join can be resident at once.  Collective; any world size.
  * ADB_ERR_NOMEM when some rank would receive more than cap_pairs (no rank writes anything). */
 ADB_API adb_status adb_peer_join_create(int64_t cap_pairs, unsigned char *handle_out);
 ADB_API adb_status adb_peer_join_connect(const unsigned char *handles);
@@ -448,7 +448,7 @@ ADB_API adb_status adb_join_emit(int32_t *d_out1, int32_t *d_out2);
  * Steps 1 and 2 end synchronised, so with a host barrier after each the _ready copies are safe. */
 /* The join sharded over the contexts of ONE process (SURVEY.md 8e "hash join: hash-partition both
  * (key, pos) lists by key to G GPUs"), keeping the reference's output order.  world = number of
- * contexts, a power of two >= 2; swapped as in adb_nested_loop_join_count.  Every step on every
+ * contexts, 2 .. ADB_MAX_PEERS; swapped as in adb_nested_loop_join_count.  Every step on every
  * context, a host barrier after each:
  *   1. every context routes its slice of the BUILD side to the keys' owners
  *      (adb_peer_exchange_pairs, side 0: pieces land in source-rank order = insertion order);
@@ -490,11 +490,13 @@ ADB_API adb_status adb_route_rows(int32_t world, int64_t shard_rows, const int32
 ADB_API adb_status adb_route_finish32(int32_t world, int32_t *d_out, int64_t n);
 
 /* ---- multi-GPU join exchange, send side (no reference equivalent: SURVEY.md 8e) ----------
- * Stable partition of a (value, position) pair list by destination rank = the top
- * log2(parts) bits of a routing hash of the value; parts is a power of two <= 256 (the
- * world size).  Pairs bound for rank r land contiguously, in their original order, at
- * offset sum(h_counts[0..r)) of the outputs -- exactly the send buffer and split sizes of an
- * all-to-all-v.  Equal keys always meet on the same rank. */
+ * Stable partition of a (value, position) pair list by destination rank = the routing hash
+ * h = value * 0x85EBCA6B (mod 2^32) scaled to the ranks, floor(h * parts / 2^32); parts (the
+ * world size) is in [1, 256].  Every rank owns floor(2^32 / parts) or that + 1 hash values; for
+ * a power of two parts = 2^k the rank is the top k bits of h.  Pairs bound for rank r land
+ * contiguously, in their original order, at offset sum(h_counts[0..r)) of the outputs --
+ * exactly the send buffer and split sizes of an all-to-all-v.  Equal keys always meet on the
+ * same rank. */
 ADB_API adb_status adb_route_pairs(const int32_t *d_val, const int32_t *d_pos, int64_t n, int32_t parts,
                                    int32_t *d_val_out, int32_t *d_pos_out, int64_t *h_counts);
 
