@@ -365,6 +365,7 @@ void preload_format_text();
 void preload_gather_agg();
 void preload_hash_join();
 void preload_index_lookup();
+void preload_index_ties();
 void preload_peer_agg();
 void preload_peer_exchange();
 void preload_radix();
@@ -561,6 +562,44 @@ uint32_t scan_ctas(uint32_t n, int sm_count);
 // in_stride: distance (in uint32) between consecutive inputs (2 reads the .y of a uint2 array)
 int launch_exclusive_scan(const uint32_t *in, uint32_t in_stride, uint32_t *out, uint32_t n,
                           unsigned long long *sums, int64_t *total, int sm_count, cudaStream_t s);
+
+// The reference quicksort's tie order (index_ties.cu).  A big segment [lo, hi] of one level
+// owns tiles tbase .. tbase + ceil((hi - lo + 1) / kTiesTile); small ones (<= kTiesSmall rows)
+// are sorted by one CTA each.  `big` of TiesCounters = segments << 32 | tiles.
+constexpr uint32_t kTiesTile = 4096;
+constexpr uint32_t kTiesSmall = 4096;
+struct TiesBig {
+    uint32_t lo, hi, tbase, pad;
+};
+struct TiesCounters {
+    unsigned long long big;
+    uint32_t small, pad;
+};
+struct TiesLevel {
+    const int32_t *keys;           // K: the sorted keys
+    const uint32_t *dex;           // dex[k] = #{i < k : K[i + 1] == K[i]}
+    const int32_t *cv;             // this level's (values, positions)
+    const uint32_t *cp;
+    int32_t *nv;                   // the next level's
+    uint32_t *np;
+    uint32_t *ev;                  // partition events, at the segment's own rows
+    uint32_t *pos_out;             // final positions
+    const TiesBig *big;
+    uint32_t nbig, ntiles;
+    const uint2 *small;
+    uint32_t nsmall;
+    uint4 *tile_cnt;               // per tile: L rows, descents, first push
+    uint32_t *tile_pre;            // per tile: L rows of the segment's earlier tiles
+    uint4 *info;                   // per big segment: mode, nL, lead, rotations
+    TiesBig *big_next;
+    uint2 *small_next;
+    TiesCounters *ctr_next;        // zeroed before the level
+};
+int launch_ties_dups(const int32_t *keys, uint32_t n, uint32_t *flags, unsigned long long *count, int sm_count,
+                     cudaStream_t s);
+int launch_ties_init(const int32_t *col, uint32_t n, int32_t *cv, uint32_t *cp, TiesBig *big, uint2 *small,
+                     int sm_count, cudaStream_t s);
+int launch_ties_level(const TiesLevel &a, cudaStream_t s);
 
 // Bulk CSV load (csv_load.cu).
 uint32_t csv_blocks(size_t bytes);

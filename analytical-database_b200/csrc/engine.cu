@@ -654,7 +654,7 @@ static adb_status init_current(int device_ordinal) {
     CU(cudaMemset(g.agg_ticket.p, 0, sizeof(unsigned int) * 2));
     // every kernel of the engine is loaded here, per device: see preload_* (adb_common.cuh)
     adb::preload_csv_load(); adb::preload_format_text(); adb::preload_gather_agg(); adb::preload_hash_join();
-    adb::preload_index_lookup(); adb::preload_peer_agg(); adb::preload_peer_exchange(); adb::preload_radix();
+    adb::preload_index_lookup(); adb::preload_index_ties(); adb::preload_peer_agg(); adb::preload_peer_exchange(); adb::preload_radix();
     adb::preload_select_scan(); adb::preload_shared_scan();
     { cudaFuncAttributes attr; cudaFuncGetAttributes(&attr, publish_kernel); cudaGetLastError(); }
     g.launches = 0;
@@ -1885,6 +1885,110 @@ adb_status adb_index_sort(const int32_t *d_col, int64_t n, int32_t *d_values_out
                                  reinterpret_cast<uint32_t *>(d_values_out),
                                  reinterpret_cast<uint32_t *>(d_positions_out), &k, &v, &launches)) return s;
     return after_launch("index_sort", launches);
+}
+
+// Scratch of adb_index_sort_ref_ties: the radix sort's buffers (afterwards the two (values,
+// positions) pairs the levels alternate between), event slots, the dup prefix, per-tile and
+// per-segment tables.  A big segment has more than kTiesSmall rows, so a level holds at most
+// n / (kTiesSmall + 1) + 1 of them and hands out at most twice that many small ones.
+struct TiesBufs {
+    RadixBufs rx;
+    uint32_t *ev, *dex;
+    uint4 *tile_cnt, *info;
+    uint32_t *tile_pre;
+    adb::TiesBig *big[2];
+    uint2 *small[2];
+    adb::TiesCounters *ctr;
+    unsigned long long *dups;
+    int64_t *dex_total;
+};
+static TiesBufs ties_layout(Carve &c, uint32_t n) {
+    const size_t m = n ? n : 1;
+    const size_t max_big = n / (adb::kTiesSmall + 1) + 1;
+    const size_t max_tiles = n / adb::kTiesTile + 1 + max_big;
+    TiesBufs b;
+    b.rx = radix_layout(c, n);
+    b.ev = c.take<uint32_t>(m);
+    b.dex = c.take<uint32_t>(m);
+    b.tile_cnt = c.take<uint4>(max_tiles);
+    b.tile_pre = c.take<uint32_t>(max_tiles);
+    b.info = c.take<uint4>(max_big);
+    for (int k = 0; k < 2; ++k) {
+        b.big[k] = c.take<adb::TiesBig>(max_big);
+        b.small[k] = c.take<uint2>(2 * max_big + 1);
+    }
+    b.ctr = c.take<adb::TiesCounters>(1);
+    b.dups = c.take<unsigned long long>(1);
+    b.dex_total = c.take<int64_t>(1);
+    return b;
+}
+
+adb_status adb_index_sort_ref_ties(const int32_t *d_col, int64_t n, int32_t *d_values_out,
+                                   int32_t *d_positions_out) {
+    NEED_UP();
+    if (adb_status s = check_len(n, "adb_index_sort_ref_ties")) return s;
+    if (n == 0) return ADB_OK;
+    if (!d_col || !d_values_out || !d_positions_out)
+        return fail(ADB_ERR_INVALID, "adb_index_sort_ref_ties: NULL pointer");
+    const uint32_t un = (uint32_t)n;
+    TiesBufs b;
+    if (adb_status s = arena_take([&](Carve &c) { b = ties_layout(c, un); }, "adb_index_sort_ref_ties", true)) return s;
+    // the values are the radix sort's; so are the positions when no key repeats
+    const adb::RadixPass passes[4] = {{0, 8, 0}, {8, 8, 0}, {16, 8, 0}, {24, 8, 0}};
+    uint32_t *k = nullptr, *v = nullptr;
+    int launches = 0;
+    uint32_t *pos_out = reinterpret_cast<uint32_t *>(d_positions_out);
+    if (adb_status s = radix_run(reinterpret_cast<const uint32_t *>(d_col), un, passes, 4, b.rx,
+                                 reinterpret_cast<uint32_t *>(d_values_out), pos_out, &k, &v, &launches)) return s;
+    launches += adb::launch_ties_dups(d_values_out, un, nullptr, b.dups, g.sm_count, g.stream);
+    if (adb_status s = after_launch("index_sort_ref_ties", launches)) return s;
+    unsigned long long dups = 0;
+    if (adb_status s = read_back(&dups, b.dups, sizeof dups)) return s;
+    if (dups == 0) return ADB_OK;
+
+    launches = adb::launch_ties_dups(d_values_out, un, b.ev, b.dups, g.sm_count, g.stream);
+    launches += adb::launch_exclusive_scan(b.ev, 1, b.dex, un, g.sc_sums, b.dex_total, g.sm_count, g.stream);
+    int32_t *vals[2] = {reinterpret_cast<int32_t *>(b.rx.k[0]), reinterpret_cast<int32_t *>(b.rx.k[1])};
+    uint32_t *poss[2] = {b.rx.v[0], b.rx.v[1]};
+    launches += adb::launch_ties_init(d_col, un, vals[0], poss[0], b.big[0], b.small[0], g.sm_count, g.stream);
+    adb::TiesLevel a{};
+    a.keys = d_values_out;
+    a.dex = b.dex;
+    a.ev = b.ev;
+    a.pos_out = pos_out;
+    a.tile_cnt = b.tile_cnt;
+    a.tile_pre = b.tile_pre;
+    a.info = b.info;
+    a.ctr_next = b.ctr;
+    const bool first_big = un > adb::kTiesSmall;
+    uint32_t nbig = first_big, ntiles = first_big ? (un + adb::kTiesTile - 1) / adb::kTiesTile : 0;
+    uint32_t nsmall = !first_big;
+    int levels = 0;
+    for (int cur = 0; nbig || nsmall; cur ^= 1, ++levels) {
+        a.cv = vals[cur];
+        a.cp = poss[cur];
+        a.nv = vals[cur ^ 1];
+        a.np = poss[cur ^ 1];
+        a.big = b.big[cur];
+        a.small = b.small[cur];
+        a.big_next = b.big[cur ^ 1];
+        a.small_next = b.small[cur ^ 1];
+        a.nbig = nbig;
+        a.ntiles = ntiles;
+        a.nsmall = nsmall;
+        CU(cudaMemsetAsync(b.ctr, 0, sizeof *b.ctr, g.stream));
+        launches += adb::launch_ties_level(a, g.stream);
+        if (adb_status s = after_launch("index_sort_ref_ties level", launches)) return s;
+        launches = 0;
+        adb::TiesCounters c;
+        if (adb_status s = read_back(&c, b.ctr, sizeof c)) return s;
+        nbig = (uint32_t)(c.big >> 32);
+        ntiles = (uint32_t)c.big;
+        nsmall = c.small;
+    }
+    // ADB_TRACE=1: how deep the quicksort's recursion went (one readback per level)
+    if (getenv("ADB_TRACE")) fprintf(stderr, "index_sort_ref_ties: %d levels\n", levels);
+    return ADB_OK;
 }
 
 // Multi-GPU join exchange, send side: stable partition of a (value, position) pair list by

@@ -157,6 +157,7 @@ class Engine:
         "adb_index_create": (C.c_int32, [_I32P, _I32P, C.c_int64, C.c_int32, C.POINTER(C.c_void_p)]),
         "adb_index_destroy": (C.c_int32, [C.c_void_p]),
         "adb_index_sort": (C.c_int32, [_I32P, C.c_int64, _I32P, _I32P]),
+        "adb_index_sort_ref_ties": (C.c_int32, [_I32P, C.c_int64, _I32P, _I32P]),
         "adb_hash_join_count": (C.c_int32, [_I32P, _I32P, C.c_int64, _I32P, _I32P, C.c_int64, _I64P]),
         "adb_nested_loop_join_count": (C.c_int32, [_I32P, _I32P, C.c_int64, _I32P, _I32P, C.c_int64, _I64P]),
         "adb_join_emit": (C.c_int32, [_I32P, _I32P]),
@@ -430,6 +431,12 @@ class Engine:
         """build_unclustered_index's sort (index.c:140): (values DevBuf, positions DevBuf)."""
         values, positions = self.alloc_i32(n), self.alloc_i32(n)
         self._ck(self.lib.adb_index_sort(col.i32(), n, values.i32(), positions.i32()))
+        return values, positions
+
+    def index_sort_ref_ties(self, col: DevBuf, n: int):
+        """index_sort with the reference quicksort's order of equal keys (index.c:25-46)."""
+        values, positions = self.alloc_i32(n), self.alloc_i32(n)
+        self._ck(self.lib.adb_index_sort_ref_ties(col.i32(), n, values.i32(), positions.i32()))
         return values, positions
 
     def join(self, v1: DevBuf, p1: DevBuf, n1: int, v2: DevBuf, p2: DevBuf, n2: int,

@@ -10,6 +10,9 @@
  *
  * Tie order: the engine's sort is stable (ties in ascending row order), the reference's
  * quicksort is not (SURVEY.md A3); the two agree whenever the indexed keys are unique.
+ * ADB_INDEX_TIES=reference keeps the build on the GPU with the quicksort's own tie order
+ * (adb_index_sort_ref_ties, chosen in adb_host_index_build), so the clustered siblings'
+ * layout and every select on them equal the reference's too.
  * ADB_INDEX_BUILD=reference hands the build to the reference's own, unmodified index.c
  * (compiled into the drop-in under the name reference_build_index, oracle/Makefile) for hosts
  * that need its exact tie order; the shim then uploads what it built, as in round 1.

@@ -126,6 +126,7 @@ static struct {
     int register_uploads;       /* page-lock host columns that are uploaded repeatedly (ADB_SHIM_NO_REGISTER=1: never) */
     size_t shard_min_rows;
     size_t rebalance_min;       /* index-ordered lists at least this long are re-cut evenly (ADB_REBALANCE_MIN) */
+    int ref_ties;               /* index builds keep the reference quicksort's tie order (ADB_INDEX_TIES=reference) */
     DevColumn *cols;
     int ncols, capcols;
     DevResult *slots;           /* open addressing on payload address */
@@ -665,6 +666,8 @@ static int host_init(int first_device, int gpus) {
     S.register_uploads = !(nr && nr[0] && nr[0] != '0');
     const char *rb = getenv("ADB_REBALANCE_MIN");
     S.rebalance_min = rb ? (size_t)atol(rb) : ((size_t)1 << 20);   /* shorter lists: the re-cut costs more than it saves */
+    const char *ties = getenv("ADB_INDEX_TIES");
+    S.ref_ties = ties && strcmp(ties, "reference") == 0;          /* default: stable */
     if (workers_start()) return -1;
     S.up = 1;
     S.failed = 0;
@@ -987,7 +990,10 @@ static int dev_index(DevColumn *c, Column *column) {
  * indexed column's own data and its index->positions (identity) left untouched (SURVEY.md A2).
  * Here the sort is the engine's stable LSD radix sort (adb_index_sort): ties come out in
  * ascending row order where the reference's unstable quicksort leaves another order
- * (SURVEY.md A3) -- identical whenever the keys are unique.  The host arrays the catalog owns
+ * (SURVEY.md A3) -- identical whenever the keys are unique.  With ADB_INDEX_TIES=reference the
+ * sort is adb_index_sort_ref_ties instead: the quicksort's own tie order, so the index, the
+ * clustered siblings' layout and every rebuild after an update or delete equal the reference's.
+ * Equal keys never straddle two slices, so either order survives the cut by index order.  The host arrays the catalog owns
  * (ColumnIndex.values / .positions, the siblings' data) are filled from the device, because the
  * unchanged plumbing persists them at shutdown (src/db_manager.c:396-397); the device-side
  * index slices are installed directly, so the first select re-uploads nothing.
@@ -1108,7 +1114,7 @@ int adb_host_index_build(Column **cols, int n_cols, int which) {
         vals = p;
         poss = q;
     }
-    if (adb_index_sort(all, (int64_t)n, vals, poss) != ADB_OK) goto dev_fail;
+    if ((S.ref_ties ? adb_index_sort_ref_ties : adb_index_sort)(all, (int64_t)n, vals, poss) != ADB_OK) goto dev_fail;
     /* the catalog's host copy (plain malloc: release_index frees it, db_manager.c:614-626) */
     ix = malloc(sizeof *ix);
     if (ix) {

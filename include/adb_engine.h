@@ -383,6 +383,14 @@ ADB_API adb_status adb_select_index_emit(const adb_index *ix, int32_t *d_pos_out
  * permutes the sibling columns with adb_fetch(sibling, positions) (index.c:105-135). */
 ADB_API adb_status adb_index_sort(const int32_t *d_col, int64_t n, int32_t *d_values_out,
                                   int32_t *d_positions_out);
+/* The same (values, positions) with equal keys in exactly the order the reference's quicksort
+ * leaves them (init_column_index + quicksort, src/index.c:25-46,89-101), positions narrowed to
+ * int32.  Same arguments and refusals as adb_index_sort; the values always equal its values,
+ * the positions differ only inside runs of equal keys.  When no key repeats it costs the radix
+ * sort plus one pass over the sorted keys; otherwise the quicksort's levels run on the GPU, all
+ * segments of a level at once. */
+ADB_API adb_status adb_index_sort_ref_ties(const int32_t *d_col, int64_t n, int32_t *d_values_out,
+                                           int32_t *d_positions_out);
 /* ColumnIndex.positions are size_t on the host (src/include/cs165_api.h:65-68) and truncated
  * to int when emitted (src/query.c:187): d_dst[i] = (int32_t) d_src_u64[i]. */
 ADB_API adb_status adb_narrow_u64_to_i32(const void *d_src_u64, int64_t n, int32_t *d_dst);
