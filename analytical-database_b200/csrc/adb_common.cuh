@@ -527,11 +527,18 @@ struct RadixPass {
                                // hash); 2: digit = route_owner(key, parts) (multi-GPU exchange;
                                // shift unused, bits = ceil(log2 parts) so the histograms hold it);
                                // 3: digit = key / div (the shard a row number lives on; shift unused)
+                               // 4: digit = #{splitters < key}, signed (the index slice a key
+                               // belongs to): 15 nondecreasing int32 splitters in device memory,
+                               // padded with INT32_MAX; their address is carried in shift (low
+                               // half) and split_hi, so the struct keeps the size every other
+                               // pass' kernels take as a parameter
     union {
         uint32_t div = 1;      // hash 3
         uint32_t parts;        // hash 2: the owner count, 1 .. 256
+        uint32_t split_hi;     // hash 4
     };
 };
+constexpr int kRangeSplitters = 15;          // hash 4: slices 0 .. 15 = up to kMaxPeers destinations
 struct RadixGeom {
     uint32_t rows_per_cta, ctas;
 };
@@ -558,6 +565,11 @@ int launch_radix_scatter_remote(const uint32_t *keys_in, const uint32_t *pay_in,
                                 const uint32_t *hist, const uint32_t *base, uint32_t *const *peer_base,
                                 unsigned long long key_off, unsigned long long pay_off,
                                 const uint32_t *abort_flag, int sm_count, cudaStream_t s);
+// One round of the multi-target radix select: hist[i * 256 + digit] += keys whose sign-flipped
+// value f = key ^ 0x80000000 has top 8 * round bits equal to prefixes[i] and next 8 bits = digit
+// (round 0..3; n_prefixes <= kMaxPeers distinct prefixes; hist zeroed by the caller).
+int launch_rank_hist(const int32_t *keys, uint32_t n, const uint32_t *prefixes, uint32_t n_prefixes, uint32_t round,
+                     uint32_t *hist, int sm_count, cudaStream_t s);
 uint32_t scan_ctas(uint32_t n, int sm_count);
 // in_stride: distance (in uint32) between consecutive inputs (2 reads the .y of a uint2 array)
 int launch_exclusive_scan(const uint32_t *in, uint32_t in_stride, uint32_t *out, uint32_t n,

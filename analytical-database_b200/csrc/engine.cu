@@ -1991,6 +1991,93 @@ adb_status adb_index_sort_ref_ties(const int32_t *d_col, int64_t n, int32_t *d_v
     return ADB_OK;
 }
 
+// ---- index build over several contexts: exact splitters, range routing, pairs sort -------------
+adb_status adb_rank_hist(const int32_t *d_col, int64_t n, const uint32_t *h_prefixes, int32_t n_prefixes,
+                         int32_t round, uint32_t *h_hist) {
+    NEED_UP();
+    if (adb_status s = check_len(n, "adb_rank_hist")) return s;
+    if (round < 0 || round > 3 || n_prefixes < 1 || n_prefixes > ADB_MAX_PEERS || !h_prefixes || !h_hist)
+        return fail(ADB_ERR_INVALID, "adb_rank_hist: round %d must be in [0, 3], prefixes %d in [1, %d]", round,
+                    n_prefixes, ADB_MAX_PEERS);
+    for (int32_t i = 0; i < n_prefixes; ++i)
+        if (((uint64_t)h_prefixes[i] >> (8 * round)) || (i && h_prefixes[i] <= h_prefixes[i - 1]))
+            return fail(ADB_ERR_INVALID, "adb_rank_hist: prefixes must be ascending and below 2^%d", 8 * round);
+    if (n > 0 && !d_col) return fail(ADB_ERR_INVALID, "adb_rank_hist: NULL pointer");
+    uint32_t *pre = nullptr, *hist = nullptr;
+    if (adb_status s = arena_take([&](Carve &c) {
+            pre = c.take<uint32_t>(ADB_MAX_PEERS);
+            hist = c.take<uint32_t>((size_t)ADB_MAX_PEERS * 256);
+        }, "adb_rank_hist", true)) return s;
+    const size_t hist_bytes = sizeof(uint32_t) * 256 * (size_t)n_prefixes;
+    if (adb_status s = upload_blob(pre, h_prefixes, sizeof(uint32_t) * (size_t)n_prefixes)) return s;
+    CU(cudaMemsetAsync(hist, 0, hist_bytes, g.stream));
+    const int k_ = adb::launch_rank_hist(d_col, (uint32_t)n, pre, (uint32_t)n_prefixes, (uint32_t)round, hist,
+                                         g.sm_count, g.stream);
+    if (adb_status s = after_launch("rank_hist", k_)) return s;
+    return read_back(h_hist, hist, hist_bytes);
+}
+
+adb_status adb_route_range(const int32_t *d_keys, int64_t n, int64_t row_base, const int32_t *h_splitters,
+                           int32_t parts, int32_t *d_keys_out, int32_t *d_rows_out, int64_t *h_counts) {
+    NEED_UP();
+    if (adb_status s = check_len(n, "adb_route_range")) return s;
+    if (parts < 1 || parts > ADB_MAX_PEERS || !h_counts || (parts > 1 && !h_splitters))
+        return fail(ADB_ERR_INVALID, "adb_route_range: parts must be in [1, %d]", ADB_MAX_PEERS);
+    if (row_base < 0 || row_base + n > ((int64_t)1 << 31))
+        return fail(ADB_ERR_INVALID, "adb_route_range: rows %lld + %lld past 2^31", (long long)row_base, (long long)n);
+    for (int32_t i = 1; i + 1 < parts; ++i)
+        if (h_splitters[i] < h_splitters[i - 1])
+            return fail(ADB_ERR_INVALID, "adb_route_range: splitters must not decrease");
+    if (n > 0 && (!d_keys || !d_keys_out || !d_rows_out))
+        return fail(ADB_ERR_INVALID, "adb_route_range: NULL device pointer");
+    for (int32_t r = 0; r < parts; ++r) h_counts[r] = 0;
+    if (n == 0) return ADB_OK;
+    int32_t split[adb::kRangeSplitters + 1];
+    for (int i = 0; i <= adb::kRangeSplitters; ++i) split[i] = i + 1 < parts ? h_splitters[i] : INT32_MAX;
+    int32_t *d_split = nullptr;
+    uint32_t *rows = nullptr;
+    if (adb_status s = arena_take([&](Carve &c) {
+            d_split = c.take<int32_t>(adb::kRangeSplitters + 1);
+            rows = c.take<uint32_t>((size_t)n);
+        }, "adb_route_range", true)) return s;
+    if (adb_status s = ensure_radix_scratch((uint32_t)n)) return s;
+    if (adb_status s = upload_blob(d_split, split, sizeof split)) return s;
+    const uint64_t at = reinterpret_cast<uintptr_t>(d_split);
+    adb::RadixPass pass{(int)(uint32_t)at, 0, 4};
+    pass.split_hi = (uint32_t)(at >> 32);
+    while ((1 << pass.bits) < parts) ++pass.bits;
+    int k_ = adb::launch_iota(reinterpret_cast<int32_t *>(rows), n, (int32_t)row_base, g.sm_count, g.stream);
+    k_ += adb::launch_radix_pass(reinterpret_cast<const uint32_t *>(d_keys), rows,
+                                 reinterpret_cast<uint32_t *>(d_keys_out), reinterpret_cast<uint32_t *>(d_rows_out),
+                                 (uint32_t)n, pass, g.rx_hist, g.rx_totals, g.rx_base, g.sm_count, g.stream);
+    if (adb_status s = after_launch("route_range", k_)) return s;
+    uint32_t totals[ADB_MAX_PEERS];
+    CU(cudaMemcpyAsync(totals, g.rx_totals, sizeof(uint32_t) * parts, cudaMemcpyDeviceToHost, g.stream));
+    CU(cudaStreamSynchronize(g.stream));
+    for (int32_t r = 0; r < parts; ++r) h_counts[r] = totals[r];
+    return ADB_OK;
+}
+
+adb_status adb_index_sort_pairs(const int32_t *d_keys, const int32_t *d_payload, int64_t n, int32_t *d_values_out,
+                                int32_t *d_payload_out) {
+    NEED_UP();
+    if (adb_status s = check_len(n, "adb_index_sort_pairs")) return s;
+    if (n == 0) return ADB_OK;
+    if (!d_keys || !d_payload || !d_values_out || !d_payload_out)
+        return fail(ADB_ERR_INVALID, "adb_index_sort_pairs: NULL pointer");
+    const adb::RadixPass passes[4] = {{0, 8, 0}, {8, 8, 0}, {16, 8, 0}, {24, 8, 0}};
+    RadixBufs b;
+    if (adb_status s = arena_take([&](Carve &c) { b = radix_layout(c, (uint32_t)n); }, "adb_index_sort_pairs", true))
+        return s;
+    uint32_t *k = nullptr, *v = nullptr;
+    int launches = 0;
+    if (adb_status s = radix_run(reinterpret_cast<const uint32_t *>(d_keys), (uint32_t)n, passes, 4, b,
+                                 reinterpret_cast<uint32_t *>(d_values_out),
+                                 reinterpret_cast<uint32_t *>(d_payload_out), &k, &v, &launches,
+                                 reinterpret_cast<const uint32_t *>(d_payload))) return s;
+    return after_launch("index_sort_pairs", launches);
+}
+
 // Multi-GPU join exchange, send side: stable partition of a (value, position) pair list by
 // destination rank = route_owner of the value (its routing hash is independent of the join's own
 // partition hash, so the receiving rank's local partitions stay balanced).

@@ -9,7 +9,10 @@
 //     hash split both inputs into partitions small enough for a shared-memory table while
 //     keeping the original row order inside every partition (stability is what makes the
 //     join's output order reproducible); across GPUs, one pass groups keys by owner
-//     (route_owner, any owner count).
+//     (route_owner, any owner count);
+//   * index build over several GPUs: one pass groups a shard's keys by the index slice that will
+//     hold them (digit = number of splitters below the key), and rank_hist_kernel finds those
+//     splitters exactly (a multi-target radix select).
 //
 // One pass = histogram (per-CTA, per-bucket counts) -> row scan of the [bucket][cta] matrix
 // -> bucket bases -> stable scatter.  Inside the scatter a step covers 256 consecutive rows:
@@ -57,6 +60,23 @@ struct RxDigit<3> {
         uint32_t q = __umulhi(key, magic);
         if ((unsigned long long)(q + 1) * div <= key) ++q;
         return min(q, mask);
+    }
+};
+
+// digit = the index slice of the key: how many of the 15 sorted splitters lie below it (signed),
+// a branchless binary search over L1-cached device memory
+template <>
+struct RxDigit<4> {
+    const int32_t *split;
+    __host__ __device__ explicit RxDigit(const RadixPass &p)
+        : split(reinterpret_cast<const int32_t *>(((uint64_t)p.split_hi << 32) | (uint32_t)p.shift)) {}
+    __device__ __forceinline__ uint32_t operator()(uint32_t key) const {
+        static_assert(kRangeSplitters == 15, "the search below covers 8 + 4 + 2 + 1 splitters");
+        uint32_t d = 0;
+#pragma unroll
+        for (uint32_t step = 8; step; step >>= 1)
+            if (__ldg(split + d + step - 1) < (int32_t)key) d += step;
+        return d;
     }
 };
 
@@ -389,6 +409,7 @@ static void rx_set_attributes() {
     allow(&rx_scatter_kernel<2, 0, false>);
     allow(&rx_scatter_kernel<2, 0, true>);
     allow(&rx_scatter_kernel<3, 0, false>);
+    allow(&rx_scatter_kernel<4, 0, false>);
     done[dev & 63] = true;
 }
 
@@ -404,6 +425,7 @@ static void rx_launch_scatter(uint32_t ctas, const uint32_t *keys_in, const uint
     else if (p.hash == 0) RX_LAUNCH(0, 0);
     else if (p.hash == 1) RX_LAUNCH(1, 0);
     else if (p.hash == 3) RX_LAUNCH(3, 0);
+    else if (p.hash == 4) RX_LAUNCH(4, 0);
     else RX_LAUNCH(2, 0);
 #undef RX_LAUNCH
 }
@@ -413,6 +435,7 @@ static void launch_hist(const uint32_t *keys_in, uint32_t n, const RadixGeom &g,
     if (p.hash == 1) rx_hist_kernel<1><<<g.ctas, RX_THREADS, 0, s>>>(keys_in, n, g.rows_per_cta, p, seg_tiles, hist);
     else if (p.hash == 2) rx_hist_kernel<2><<<g.ctas, RX_THREADS, 0, s>>>(keys_in, n, g.rows_per_cta, p, seg_tiles, hist);
     else if (p.hash == 3) rx_hist_kernel<3><<<g.ctas, RX_THREADS, 0, s>>>(keys_in, n, g.rows_per_cta, p, seg_tiles, hist);
+    else if (p.hash == 4) rx_hist_kernel<4><<<g.ctas, RX_THREADS, 0, s>>>(keys_in, n, g.rows_per_cta, p, seg_tiles, hist);
     else rx_hist_kernel<0><<<g.ctas, RX_THREADS, 0, s>>>(keys_in, n, g.rows_per_cta, p, seg_tiles, hist);
 }
 
@@ -483,6 +506,59 @@ int launch_radix_scatter_remote(const uint32_t *keys_in, const uint32_t *pay_in,
     const RadixGeom g = radix_geom(n, sm_count);
     rx_scatter_kernel<2, 0, true><<<g.ctas, RX_ST, sizeof(RxShared), s>>>(
         keys_in, pay_in, n, p, g.ctas, hist, base, nullptr, nullptr, peer_base, key_off, pay_off, abort_flag);
+    return 1;
+}
+
+// ---- multi-target radix select -----------------------------------------------------------------
+// Round r of four: every key whose sign-flipped top 8r bits equal one of the (distinct) prefixes
+// counts its next 8 bits in that prefix's histogram.  The host sums the contexts' histograms and
+// narrows every target's prefix and remaining rank, so four streaming passes give exact order
+// statistics.  The prefixes sit in shared memory (an indexed kernel-parameter array would be
+// copied to local memory by every thread, DESIGN §3).
+constexpr int RS_THREADS = 256;
+__global__ void __launch_bounds__(RS_THREADS)
+rank_hist_kernel(const int32_t *__restrict__ keys, uint32_t n, const uint32_t *__restrict__ prefixes, uint32_t n_pre,
+                 uint32_t round, uint32_t *__restrict__ hist) {
+    __shared__ uint32_t s_h[kMaxPeers * 256];
+    __shared__ uint32_t s_pre[kMaxPeers];
+    for (uint32_t i = threadIdx.x; i < n_pre * 256; i += RS_THREADS) s_h[i] = 0;
+    if (threadIdx.x < n_pre) s_pre[threadIdx.x] = prefixes[threadIdx.x];
+    __syncthreads();
+    const uint32_t dshift = 24 - 8 * round;
+    auto count = [&](int32_t key) {
+        const uint32_t f = (uint32_t)key ^ 0x80000000u;
+        const uint32_t top = round ? f >> (32 - 8 * round) : 0u;
+        for (uint32_t i = 0; i < n_pre; ++i)
+            if (s_pre[i] == top) {
+                atomicAdd(&s_h[i * 256 + ((f >> dshift) & 255u)], 1u);
+                break;
+            }
+    };
+    // the unaligned head and the tail one key at a time, the rest 16 bytes at a time
+    const uint32_t stride = gridDim.x * RS_THREADS;
+    const uint32_t lead = min((uint32_t)((16 - (reinterpret_cast<uintptr_t>(keys) & 15)) & 15) / 4, n);
+    const uint32_t n4 = (n - lead) / 4, tail = lead + 4 * n4;
+    const int4 *k4 = reinterpret_cast<const int4 *>(keys + lead);
+    for (uint32_t i = blockIdx.x * RS_THREADS + threadIdx.x; i < n4; i += stride) {
+        const int4 k = ld_stream(k4 + i);
+        count(k.x);
+        count(k.y);
+        count(k.z);
+        count(k.w);
+    }
+    for (uint32_t i = blockIdx.x * RS_THREADS + threadIdx.x; i < lead + (n - tail); i += stride)
+        count(keys[i < lead ? i : tail + (i - lead)]);
+    __syncthreads();
+    for (uint32_t i = threadIdx.x; i < n_pre * 256; i += RS_THREADS)
+        if (s_h[i]) atomicAdd(&hist[i], s_h[i]);
+}
+
+int launch_rank_hist(const int32_t *keys, uint32_t n, const uint32_t *prefixes, uint32_t n_prefixes, uint32_t round,
+                     uint32_t *hist, int sm_count, cudaStream_t s) {
+    if (n == 0) return 0;
+    uint32_t ctas = (n + RS_THREADS * 16 - 1) / (RS_THREADS * 16);
+    if (ctas > (uint32_t)sm_count * 4) ctas = (uint32_t)sm_count * 4;
+    rank_hist_kernel<<<ctas, RS_THREADS, 0, s>>>(keys, n, prefixes, n_prefixes, round, hist);
     return 1;
 }
 
@@ -568,6 +644,7 @@ void preload_radix() {
     { auto *fp = &rx_hist_kernel<1>; preload_one(reinterpret_cast<const void *>(fp)); }
     { auto *fp = &rx_hist_kernel<2>; preload_one(reinterpret_cast<const void *>(fp)); }
     { auto *fp = &rx_hist_kernel<3>; preload_one(reinterpret_cast<const void *>(fp)); }
+    { auto *fp = &rx_hist_kernel<4>; preload_one(reinterpret_cast<const void *>(fp)); }
     preload_one(reinterpret_cast<const void *>(&rx_row_scan_kernel));
     preload_one(reinterpret_cast<const void *>(&rx_row_scan_warp_kernel));
     preload_one(reinterpret_cast<const void *>(&rx_bucket_base_kernel));
@@ -578,6 +655,8 @@ void preload_radix() {
     { auto *fp = &rx_scatter_kernel<2, 0, false>; preload_one(reinterpret_cast<const void *>(fp)); }
     { auto *fp = &rx_scatter_kernel<2, 0, true>; preload_one(reinterpret_cast<const void *>(fp)); }
     { auto *fp = &rx_scatter_kernel<3, 0, false>; preload_one(reinterpret_cast<const void *>(fp)); }
+    { auto *fp = &rx_scatter_kernel<4, 0, false>; preload_one(reinterpret_cast<const void *>(fp)); }
+    preload_one(reinterpret_cast<const void *>(&rank_hist_kernel));
     preload_one(reinterpret_cast<const void *>(&sc_chunk_scan_kernel));
     preload_one(reinterpret_cast<const void *>(&sc_chunk_sum_kernel));
     rx_set_attributes();

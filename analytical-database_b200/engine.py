@@ -202,6 +202,10 @@ class Engine:
                                              C.POINTER(_AggStruct)]),
         "adb_synth_affine": (C.c_int32, [_I32P, C.c_int64, C.c_uint64, C.c_uint64, C.c_uint64, C.c_uint64]),
         "adb_histogram_i32": (C.c_int32, [_I32P, C.c_int64, C.c_int32, C.c_int32, C.POINTER(C.c_uint64)]),
+        "adb_rank_hist": (C.c_int32, [_I32P, C.c_int64, C.POINTER(C.c_uint32), C.c_int32, C.c_int32,
+                                      C.POINTER(C.c_uint32)]),
+        "adb_route_range": (C.c_int32, [_I32P, C.c_int64, C.c_int64, _I32P, C.c_int32, _I32P, _I32P, _I64P]),
+        "adb_index_sort_pairs": (C.c_int32, [_I32P, _I32P, C.c_int64, _I32P, _I32P]),
     }
 
     def __init__(self, device: int = 0):
@@ -438,6 +442,29 @@ class Engine:
         values, positions = self.alloc_i32(n), self.alloc_i32(n)
         self._ck(self.lib.adb_index_sort_ref_ties(col.i32(), n, values.i32(), positions.i32()))
         return values, positions
+
+    def rank_hist(self, col: DevBuf, n: int, prefixes, rnd: int) -> np.ndarray:
+        """One multi-target radix-select round: a (len(prefixes), 256) uint32 histogram."""
+        pre = np.ascontiguousarray(prefixes, dtype=np.uint32)
+        hist = np.zeros((pre.size, 256), dtype=np.uint32)
+        self._ck(self.lib.adb_rank_hist(col.i32(), n, pre.ctypes.data_as(C.POINTER(C.c_uint32)), pre.size, rnd,
+                                        hist.ctypes.data_as(C.POINTER(C.c_uint32))))
+        return hist
+
+    def route_range(self, keys: DevBuf, n: int, row_base: int, splitters, parts: int):
+        """Stable partition by index slice: (keys DevBuf, rows DevBuf, counts per slice)."""
+        split = np.ascontiguousarray(splitters, dtype=np.int32)
+        counts = (C.c_int64 * max(parts, 1))()
+        keys_out, rows_out = self.alloc_i32(n), self.alloc_i32(n)
+        self._ck(self.lib.adb_route_range(keys.i32(), n, row_base, split.ctypes.data_as(_I32P), parts,
+                                          keys_out.i32(), rows_out.i32(), counts))
+        return keys_out, rows_out, [int(counts[i]) for i in range(parts)]
+
+    def index_sort_pairs(self, keys: DevBuf, payload: DevBuf, n: int):
+        """index_sort carrying the given payload: (values DevBuf, payload DevBuf)."""
+        values, pay = self.alloc_i32(n), self.alloc_i32(n)
+        self._ck(self.lib.adb_index_sort_pairs(keys.i32(), payload.i32(), n, values.i32(), pay.i32()))
+        return values, pay
 
     def join(self, v1: DevBuf, p1: DevBuf, n1: int, v2: DevBuf, p2: DevBuf, n2: int,
              nested_loop: bool = False):

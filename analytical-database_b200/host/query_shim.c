@@ -186,11 +186,15 @@ static void op_ok(Status *st) {
 #include <time.h>
 enum { PF_SELECT, PF_SELECT_JOB, PF_FETCH, PF_FETCH_JOB, PF_AGG, PF_AGG_JOB, PF_NEWRESULT, PF_RELEASE,
        PF_FREE_JOB, PF_LOAD_UPLOAD, PF_LOAD_PARSE, PF_LOAD_FILL, PF_LOAD_RECUT, PF_LOAD_AGG, PF_LOAD_DOWNLOAD,
-       PF_COUNT };
+       PF_IX_SPLIT, PF_IX_ROUTE, PF_IX_RESERVE, PF_IX_PULL, PF_IX_SORT, PF_IX_CATALOG, PF_IX_GLOBAL, PF_IX_SIBLINGS,
+       PF_IX_SLICES, PF_COUNT };
 static const char *const pf_names[PF_COUNT] = {"select_column", "  its shard job", "fetch_column", "  its shard job",
                                                "aggregate", "  its shard job", "new_dev_result", "payload release",
                                                "  free job", "load: upload", "load: index+parse", "load: fill",
-                                               "load: re-cut", "load: aggregate", "load: download"};
+                                               "load: re-cut", "load: aggregate", "load: download",
+                                               "index: splitters", "index: route", "index: reserve", "index: pulls",
+                                               "index: sort", "index: catalog", "index: sort on GPU 0",
+                                               "index: siblings", "index: slices"};
 static struct { int on; double t[PF_COUNT]; long n[PF_COUNT]; } PF;
 static inline double pf_now(void) {
     struct timespec ts;
@@ -999,9 +1003,11 @@ static int dev_index(DevColumn *c, Column *column) {
  * index slices are installed directly, so the first select re-uploads nothing.
  *
  * cols[0 .. n_cols) are the table's columns in declaration order, `which` the indexed one
- * (its sorted / clustered flags say what to build).  The sort itself runs on context 0 (a
- * global sort; SURVEY.md 8e: "clustered index build: does not shard"); the sibling permutation
- * is one peer gather per GPU. */
+ * (its sorted / clustered flags say what to build).  With one GPU, or with ADB_INDEX_TIES=reference
+ * (the quicksort's tie order depends on the whole array), the sort runs on context 0 and the slices
+ * are copied out to the contexts that hold them.  With G > 1 and the stable order every context
+ * sorts its own slice (sharded_build_sort below): the keys are routed to the slice that will hold
+ * them first.  The sibling permutation is one peer gather per GPU either way. */
 static int slice_bounds(DevColumn *c, const int *v, size_t n) {
     const size_t per = (n + (size_t)S.G - 1) / (size_t)S.G;
     c->ix_begin[0] = 0;
@@ -1030,7 +1036,8 @@ static int slice_bounds(DevColumn *c, const int *v, size_t n) {
 typedef struct PermuteJob {
     ShardErr err;
     DevColumn *sib;
-    const int32_t *order0;      /* sorted positions, on context 0 */
+    int32_t *const *order;      /* entries [begin[d], begin[d+1]) of the sorted positions, on context d */
+    const size_t *begin;
     int *host_out;
     int32_t *fresh[MAXG];
 } PermuteJob;
@@ -1043,7 +1050,15 @@ static void permute_shard(int g, void *arg) {
     a->fresh[g] = out;
     if (!n) return;
     SCK(adb_alloc(&ord, 4 * n));
-    if (adb_copy_from_ctx(ord, 0, a->order0 + (size_t)g * c->shard_rows, 4 * n) != ADB_OK ||
+    /* rows [lo, hi) of index order, from every slice that covers them */
+    const size_t lo = (size_t)g * c->shard_rows, hi = lo + n;
+    adb_status st = ADB_OK;
+    for (int d = 0; d < S.G && st == ADB_OK; ++d) {
+        const size_t a0 = lo > a->begin[d] ? lo : a->begin[d], a1 = hi < a->begin[d + 1] ? hi : a->begin[d + 1];
+        if (a0 < a1)
+            st = adb_copy_from_ctx((int32_t *)ord + (a0 - lo), d, a->order[d] + (a0 - a->begin[d]), 4 * (a1 - a0));
+    }
+    if (st != ADB_OK ||
         (S.G == 1 ? adb_fetch(c->d_data[0], ord, (int64_t)n, NULL, 0, out)
                   : adb_fetch_sharded((const int32_t *const *)c->d_data, S.G, (int64_t)c->shard_rows, ord,
                                       (int64_t)n, NULL, out)) != ADB_OK ||
@@ -1075,6 +1090,203 @@ static void slice_shard(int g, void *arg) {
     SCK(adb_sync());                    /* the sort buffers on context 0 are released next */
 }
 
+/* ---- index build on every context (G > 1, stable tie order) ------------------------------------
+ * slice_bounds ends slice g after #{keys <= t_g}, t_g = the key of rank g*per - 1 in sorted order
+ * (+inf when g*per >= n): a plain cut at g*per and a cut moved to the end of a run of equal keys
+ * both land there, and t_g never decreases, so its clamp never fires.  A key k therefore belongs
+ * to slice #{g : t_g < k}.  With the exact t_g (a radix select summed over the contexts) every
+ * context routes its own rows to the slice that will hold them and each slice is sorted where it
+ * lives: the same slices, entry for entry.  Each slice receives its pieces in source order, i.e.
+ * in ascending row order, so the stable sort leaves equal keys in row order, as adb_index_sort of
+ * the whole column does. */
+typedef struct ShardedBuild {
+    ShardErr err;
+    int phase;
+    DevColumn *c;
+    ColumnIndex *ix;
+    int clustered, with_btree;
+    size_t begin[MAXG + 1];             /* slice d = entries [begin[d], begin[d+1]) */
+    /* phase SB_SELECT: one radix-select round over every context's keys */
+    uint32_t prefixes[MAXG];
+    int n_prefixes, round;
+    uint32_t hist[MAXG][MAXG * 256];    /* [context][prefix * 256 + digit] */
+    /* phase SB_ROUTE: context g's keys and row numbers grouped by slice; sent[g][d] of them for d */
+    int32_t split[MAXG];                /* t_1 .. t_{G-1} */
+    int32_t *rk[MAXG], *rr[MAXG];
+    int64_t sent[MAXG][MAXG];
+    /* slice d: what it received (keys, then row numbers; afterwards the catalog staging), then its
+     * sorted values and positions, which become the device index slice */
+    int32_t *recv[MAXG], *vals[MAXG], *poss[MAXG];
+    adb_index *handle[MAXG];
+} ShardedBuild;
+enum { SB_SELECT, SB_ROUTE, SB_RESERVE, SB_PULL, SB_SORT, SB_CATALOG, SB_FINISH };
+
+static void sharded_build_shard(int g, void *arg) {
+    ShardedBuild *a = arg;
+    const size_t b = a->begin[g], m = a->begin[g + 1] - b;
+    switch (a->phase) {
+    case SB_SELECT: {
+        const DevColumn *c = a->c;
+        SCK(adb_rank_hist(c->d_data[g], (int64_t)shard_len(c->rows, c->shard_rows, g), a->prefixes, a->n_prefixes,
+                          a->round, a->hist[g]));
+        break;
+    }
+    case SB_ROUTE: {
+        const DevColumn *c = a->c;
+        const size_t len = shard_len(c->rows, c->shard_rows, g);
+        void *k = NULL, *r = NULL;
+        SCK(adb_alloc(&k, 4 * len));
+        a->rk[g] = k;
+        SCK(adb_alloc(&r, 4 * len));
+        a->rr[g] = r;
+        SCK(adb_route_range(c->d_data[g], (int64_t)len, (int64_t)g * (int64_t)c->shard_rows, a->split, S.G, a->rk[g],
+                            a->rr[g], a->sent[g]));
+        break;
+    }
+    case SB_RESERVE: {                  /* everything this slice needs, before any pull starts */
+        void *p = NULL;
+        SCK(adb_alloc(&p, 8 * m));
+        a->recv[g] = p;
+        SCK(adb_alloc(&p, 4 * m));
+        a->vals[g] = p;
+        SCK(adb_alloc(&p, 4 * m));
+        a->poss[g] = p;
+        break;
+    }
+    case SB_PULL:                       /* source order; starting at its own piece, as route_pull */
+        for (int k = 0; k < S.G; ++k) {
+            const int src = (g + k) % S.G;
+            size_t at = 0, from = 0;
+            for (int t = 0; t < src; ++t) at += (size_t)a->sent[t][g];
+            for (int o = 0; o < g; ++o) from += (size_t)a->sent[src][o];
+            const size_t cnt = (size_t)a->sent[src][g];
+            if (!cnt) continue;
+            SCK(adb_copy_from_ctx_ready(a->recv[g] + at, src, a->rk[src] + from, 4 * cnt));
+            SCK(adb_copy_from_ctx_ready(a->recv[g] + m + at, src, a->rr[src] + from, 4 * cnt));
+        }
+        SCK(adb_sync());
+        break;
+    case SB_SORT:                       /* every pull has finished: the routed pieces can go */
+        adb_free(a->rk[g]);
+        adb_free(a->rr[g]);
+        a->rk[g] = a->rr[g] = NULL;
+        SCK(adb_index_sort_pairs(a->recv[g], a->recv[g] + m, (int64_t)m, a->vals[g], a->poss[g]));
+        SCK(adb_sync());
+        break;
+    case SB_CATALOG:                    /* over every context's own host link at once */
+        if (m) SCK(adb_download(a->ix->values + b, a->vals[g], 4 * m));
+        if (m && !a->clustered) {
+            SCK(adb_widen_i32_to_u64(a->poss[g], (int64_t)m, a->recv[g]));
+            SCK(adb_download(a->ix->positions + b, a->recv[g], 8 * m));
+        }
+        SCK(adb_sync());
+        break;
+    case SB_FINISH:                     /* a clustered index's positions are the identity */
+        if (a->clustered) {
+            SCK(adb_iota_i32(a->poss[g], (int64_t)m, (int32_t)b));
+            if (m) {
+                SCK(adb_widen_i32_to_u64(a->poss[g], (int64_t)m, a->recv[g]));
+                SCK(adb_download(a->ix->positions + b, a->recv[g], 8 * m));
+            }
+        }
+        SCK(adb_index_create(a->vals[g], a->poss[g], (int64_t)m, a->with_btree, &a->handle[g]));
+        SCK(adb_index_set_slice(a->handle[g], 1));
+        adb_free(a->recv[g]);
+        a->recv[g] = NULL;
+        break;
+    }
+}
+
+static int sharded_build_run(ShardedBuild *a, int phase) {
+    static const int pf[] = {PF_IX_SPLIT, PF_IX_ROUTE, PF_IX_RESERVE, PF_IX_PULL, PF_IX_SORT, PF_IX_CATALOG, PF_IX_SLICES};
+    const double t0 = PF.on ? pf_now() : 0.0;
+    a->phase = phase;
+    run_shards(sharded_build_shard, a);
+    if (PF.on) {
+        PF.t[pf[phase]] += pf_now() - t0;
+        ++PF.n[pf[phase]];
+    }
+    return shard_errs(&a->err);
+}
+
+/* what a failed build leaves behind */
+static void sharded_build_free(ShardedBuild *a) {
+    for (int g = 0; g < S.G; ++g) {
+        on_ctx(g);
+        if (a->handle[g]) adb_index_destroy(a->handle[g]);
+        int32_t *bufs[5] = {a->rk[g], a->rr[g], a->recv[g], a->vals[g], a->poss[g]};
+        for (int i = 0; i < 5; ++i)
+            if (bufs[i]) adb_free(bufs[i]);
+    }
+    on_ctx(0);
+}
+
+/* t_1 .. t_{G-1} (INT32_MAX past the end) and the smallest key by a radix select of their ranks
+ * over all contexts: four rounds of 8 bits of the sign-flipped key, histograms summed here. */
+static int sharded_build_splitters(ShardedBuild *a, size_t n, int *min_key) {
+    const size_t per = (n + (size_t)S.G - 1) / (size_t)S.G;
+    size_t rank[MAXG];                  /* target 0: rank 0 (the minimum); target i: t_slice[i] */
+    int slice[MAXG], nt = 0;
+    if (n) {
+        rank[nt] = 0;
+        slice[nt++] = 0;
+    }
+    for (int g = 1; g < S.G; ++g) {
+        a->split[g - 1] = INT32_MAX;
+        if ((size_t)g * per < n) {
+            rank[nt] = (size_t)g * per - 1;
+            slice[nt++] = g;
+        }
+    }
+    uint32_t prefix[MAXG] = {0};        /* the targets' high bits found so far, in increasing order */
+    for (int round = 0; round < 4 && nt; ++round) {
+        int which[MAXG];                /* target -> its prefix's row of the histogram */
+        a->n_prefixes = 0;
+        for (int t = 0; t < nt; ++t) {
+            if (!a->n_prefixes || a->prefixes[a->n_prefixes - 1] != prefix[t]) a->prefixes[a->n_prefixes++] = prefix[t];
+            which[t] = a->n_prefixes - 1;
+        }
+        a->round = round;
+        if (sharded_build_run(a, SB_SELECT)) return -1;
+        for (int t = 0; t < nt; ++t) {
+            size_t left = rank[t];
+            int d = 0;
+            for (;; ++d) {
+                size_t cnt = 0;
+                for (int g = 0; g < S.G; ++g) cnt += a->hist[g][which[t] * 256 + d];
+                if (left < cnt || d == 255) break;
+                left -= cnt;
+            }
+            rank[t] = left;
+            prefix[t] = prefix[t] << 8 | (uint32_t)d;
+        }
+    }
+    for (int t = 0; t < nt; ++t) {
+        const int32_t key = (int32_t)(prefix[t] ^ 0x80000000u);
+        if (slice[t]) a->split[slice[t] - 1] = key;
+        else *min_key = key;
+    }
+    return 0;
+}
+
+/* Sorts the column into its slices on the contexts that hold them and fills the catalog's arrays;
+ * a clustered index's positions are filled by SB_FINISH, after the siblings have been permuted. */
+static int sharded_build_sort(ShardedBuild *a, size_t n, int *min_key) {
+    *min_key = 0;
+    if (sharded_build_splitters(a, n, min_key) || sharded_build_run(a, SB_ROUTE)) return -1;
+    a->begin[0] = 0;
+    for (int d = 0; d < S.G; ++d) {
+        a->begin[d + 1] = a->begin[d];
+        for (int src = 0; src < S.G; ++src) a->begin[d + 1] += (size_t)a->sent[src][d];
+    }
+    if (a->begin[S.G] != n) {
+        set_err("index build: the slices hold %zu of %zu rows", a->begin[S.G], n);
+        return -1;
+    }
+    return sharded_build_run(a, SB_RESERVE) || sharded_build_run(a, SB_PULL) || sharded_build_run(a, SB_SORT) ||
+                   sharded_build_run(a, SB_CATALOG) ? -1 : 0;
+}
+
 int adb_host_index_build(Column **cols, int n_cols, int which) {
     t_err[0] = '\0';
     if (ensure_up()) return -1;
@@ -1090,31 +1302,11 @@ int adb_host_index_build(Column **cols, int n_cols, int which) {
     int32_t *all = NULL, *vals = NULL, *poss = NULL;
     void *wide = NULL;
     ColumnIndex *ix = NULL;
-    int own_all = 0;
-    /* the whole column on context 0 */
-    if (S.G == 1) {
-        all = c->d_data[0];
-    } else {
-        void *p = NULL;
-        if (adb_alloc(&p, 4 * n) != ADB_OK) goto dev_fail;
-        all = p;
-        own_all = 1;
-        for (int g = 0; g < S.G; ++g) {
-            const size_t len = shard_len(c->rows, c->shard_rows, g);
-            if (len && adb_copy_from_ctx(all + (size_t)g * c->shard_rows, g, c->d_data[g], 4 * len) != ADB_OK)
-                goto dev_fail;
-        }
-    }
-    {
-        void *p = NULL, *q = NULL;
-        if (adb_alloc(&p, 4 * n) != ADB_OK || adb_alloc(&q, 4 * n) != ADB_OK) {
-            if (p) adb_free(p);
-            goto dev_fail;
-        }
-        vals = p;
-        poss = q;
-    }
-    if ((S.ref_ties ? adb_index_sort_ref_ties : adb_index_sort)(all, (int64_t)n, vals, poss) != ADB_OK) goto dev_fail;
+    ShardedBuild *sb = NULL;
+    int own_all = 0, min_key = 0;
+    /* where the sorted positions are: slice d of them on context d */
+    int32_t *order[MAXG] = {0};
+    size_t order_begin[MAXG + 1];
     /* the catalog's host copy (plain malloc: release_index frees it, db_manager.c:614-626) */
     ix = malloc(sizeof *ix);
     if (ix) {
@@ -1125,15 +1317,60 @@ int adb_host_index_build(Column **cols, int n_cols, int which) {
         set_err("out of host memory for the index of %zu rows", n);
         goto fail;
     }
-    if (n) {
-        if (adb_alloc(&wide, 8 * n) != ADB_OK) goto dev_fail;
-        if (adb_download(ix->values, vals, 4 * n) != ADB_OK ||
-            adb_widen_i32_to_u64(column->clustered ? NULL : poss, (int64_t)n, wide) != ADB_OK ||
-            adb_download(ix->positions, wide, 8 * n) != ADB_OK)
-            goto dev_fail;
-        adb_free(wide);
-        wide = NULL;
+    if (S.G > 1 && !S.ref_ties) {
+        sb = calloc(1, sizeof *sb);
+        if (!sb) {
+            set_err("out of host memory for the index build");
+            goto fail;
+        }
+        sb->c = c;
+        sb->ix = ix;
+        sb->clustered = column->clustered;
+        sb->with_btree = !column->sorted;
+        if (sharded_build_sort(sb, n, &min_key)) goto fail;
+        for (int d = 0; d < S.G; ++d) order[d] = sb->poss[d];
+        memcpy(order_begin, sb->begin, sizeof order_begin);
+    } else {
+        PF_BEGIN(PF_IX_GLOBAL);
+        /* the whole column on context 0 */
+        if (S.G == 1) {
+            all = c->d_data[0];
+        } else {
+            void *p = NULL;
+            if (adb_alloc(&p, 4 * n) != ADB_OK) goto dev_fail;
+            all = p;
+            own_all = 1;
+            for (int g = 0; g < S.G; ++g) {
+                const size_t len = shard_len(c->rows, c->shard_rows, g);
+                if (len && adb_copy_from_ctx(all + (size_t)g * c->shard_rows, g, c->d_data[g], 4 * len) != ADB_OK)
+                    goto dev_fail;
+            }
+        }
+        {
+            void *p = NULL, *q = NULL;
+            if (adb_alloc(&p, 4 * n) != ADB_OK || adb_alloc(&q, 4 * n) != ADB_OK) {
+                if (p) adb_free(p);
+                goto dev_fail;
+            }
+            vals = p;
+            poss = q;
+        }
+        if ((S.ref_ties ? adb_index_sort_ref_ties : adb_index_sort)(all, (int64_t)n, vals, poss) != ADB_OK) goto dev_fail;
+        if (n) {
+            if (adb_alloc(&wide, 8 * n) != ADB_OK) goto dev_fail;
+            if (adb_download(ix->values, vals, 4 * n) != ADB_OK ||
+                adb_widen_i32_to_u64(column->clustered ? NULL : poss, (int64_t)n, wide) != ADB_OK ||
+                adb_download(ix->positions, wide, 8 * n) != ADB_OK)
+                goto dev_fail;
+            adb_free(wide);
+            wide = NULL;
+        }
+        PF_END(PF_IX_GLOBAL);
+        order[0] = poss;
+        order_begin[0] = 0;
+        for (int g = 1; g <= S.G; ++g) order_begin[g] = n;
     }
+    PF_BEGIN(PF_IX_SIBLINGS);
     if (column->clustered) {
         /* every OTHER column (by name, index.c:128-133) moves into index order */
         for (int j = 0; j < n_cols; ++j) {
@@ -1154,7 +1391,8 @@ int adb_host_index_build(Column **cols, int n_cols, int which) {
             PermuteJob job;
             memset(&job, 0, sizeof job);
             job.sib = dc;
-            job.order0 = poss;
+            job.order = order;
+            job.begin = order_begin;
             job.host_out = sib->data;               /* in place: the mmap is the catalog's truth */
             run_shards(permute_shard, &job);
             if (shard_errs(&job.err)) {
@@ -1169,10 +1407,24 @@ int adb_host_index_build(Column **cols, int n_cols, int which) {
             }
         }
     }
+    PF_END(PF_IX_SIBLINGS);
     /* device-side index slices, cut by index order */
-    dev_index_drop(c);
-    slice_bounds(c, ix->values, n);
-    {
+    if (sb) {
+        if (sharded_build_run(sb, SB_FINISH)) goto fail;
+        dev_index_drop(c);
+        memcpy(c->ix_begin, sb->begin, sizeof c->ix_begin);
+        c->ix_min = min_key;
+        for (int d = 0; d < S.G; ++d) {
+            c->d_ix_values[d] = sb->vals[d];
+            c->d_ix_positions[d] = sb->poss[d];
+            c->ix[d] = sb->handle[d];
+            sb->vals[d] = sb->poss[d] = NULL;
+            sb->handle[d] = NULL;
+        }
+    } else {
+        PF_BEGIN(PF_IX_SLICES);
+        dev_index_drop(c);
+        slice_bounds(c, ix->values, n);
         SliceJob job;
         memset(&job, 0, sizeof job);
         job.c = c;
@@ -1180,6 +1432,7 @@ int adb_host_index_build(Column **cols, int n_cols, int which) {
         job.poss0 = column->clustered ? NULL : poss;
         job.with_btree = !column->sorted;
         run_shards(slice_shard, &job);
+        PF_END(PF_IX_SLICES);
         if (shard_errs(&job.err)) {
             dev_index_drop(c);
             goto fail;
@@ -1200,6 +1453,10 @@ fail:
         free(ix);
     }
 done:
+    if (sb) {
+        sharded_build_free(sb);
+        free(sb);
+    }
     if (wide) adb_free(wide);
     if (vals) adb_free(vals);
     if (poss) adb_free(poss);

@@ -391,6 +391,28 @@ ADB_API adb_status adb_index_sort(const int32_t *d_col, int64_t n, int32_t *d_va
  * segments of a level at once. */
 ADB_API adb_status adb_index_sort_ref_ties(const int32_t *d_col, int64_t n, int32_t *d_values_out,
                                            int32_t *d_positions_out);
+/* The index build over several contexts (range-partitioned slices, see adb_index_set_slice):
+ *   adb_rank_hist        one round of a multi-target radix select over this context's keys.  With
+ *                        f = key ^ 0x80000000 (signed order), h_hist[i * 256 + d] = keys whose top
+ *                        8 * round bits of f equal h_prefixes[i] and whose next 8 bits are d.  round
+ *                        in [0, 3]; 1 .. ADB_MAX_PEERS prefixes, ascending, each below 2^(8 * round)
+ *                        (round 0: the one prefix 0).  Summed over the contexts, four rounds narrow
+ *                        any number of ranks to their exact keys.
+ *   adb_route_range      stable partition of this context's keys by the slice that holds them:
+ *                        slice(k) = #{i < parts - 1 : h_splitters[i] < k} (signed), the splitters
+ *                        nondecreasing, parts in [1, ADB_MAX_PEERS].  Rows bound for slice s land
+ *                        contiguously, in row order, at offset sum(h_counts[0..s)) of d_keys_out,
+ *                        their row numbers row_base + local row at the same offsets of d_rows_out
+ *                        (row_base + n <= 2^31).  Synchronises.
+ *   adb_index_sort_pairs adb_index_sort of d_keys carrying the given payload instead of the input
+ *                        index: the same four stable 8-bit LSD passes, equal keys keep their input
+ *                        order.  The outputs must not overlap the inputs. */
+ADB_API adb_status adb_rank_hist(const int32_t *d_col, int64_t n, const uint32_t *h_prefixes, int32_t n_prefixes,
+                                 int32_t round, uint32_t *h_hist);
+ADB_API adb_status adb_route_range(const int32_t *d_keys, int64_t n, int64_t row_base, const int32_t *h_splitters,
+                                   int32_t parts, int32_t *d_keys_out, int32_t *d_rows_out, int64_t *h_counts);
+ADB_API adb_status adb_index_sort_pairs(const int32_t *d_keys, const int32_t *d_payload, int64_t n,
+                                        int32_t *d_values_out, int32_t *d_payload_out);
 /* ColumnIndex.positions are size_t on the host (src/include/cs165_api.h:65-68) and truncated
  * to int when emitted (src/query.c:187): d_dst[i] = (int32_t) d_src_u64[i]. */
 ADB_API adb_status adb_narrow_u64_to_i32(const void *d_src_u64, int64_t n, int32_t *d_dst);
