@@ -1323,6 +1323,14 @@ adb_status adb_peer_exchange_pairs(int32_t side, const int32_t *d_val, const int
                                      g.rx_totals, g.sm_count, g.stream);
     }
     k_ += adb::launch_jx_counts(x, g.rx_totals, g.rx_base, g.jx_total, g.jx_status, g.stream);
+    // Nothing of this context may wait in a hardware queue behind its spinning jx_counts_kernel.
+    // The contexts' streams share the device's few hardware work queues, and when a peer's stream
+    // lands in the same queue, a launch that depends on the spinning kernel (the scatter) blocks
+    // that queue's head: the peer's own jx_counts_kernel behind it cannot start, and both give up
+    // after 2 s.  Which streams share a queue depends on how many were created before, so this
+    // struck some first joins on freshly started contexts only.  The scatter is enqueued once
+    // every count row has arrived.
+    CU(cudaStreamSynchronize(g.stream));
     if (world == 1) {
         if (n) {
             CU(cudaMemcpyAsync(g.jx_recv + key_off, d_val, (size_t)n * 4, cudaMemcpyDeviceToDevice, g.stream));

@@ -3039,6 +3039,7 @@ typedef struct JoinJob {
     ShardList *bv, *bp, *pv, *pp;
     int swapped, phase, overflow;
     size_t cap;                                     /* pairs a GPU can receive */
+    size_t pairs[MAXG];                             /* each context's share of the output (phase 3) */
     ShardList o1, o2;
     Route route;                                    /* routed probe (phases 1-3): items = probe keys */
 } JoinJob;
@@ -3078,10 +3079,15 @@ static void join_shard(int g, void *arg) {
         SCK(adb_join_probe_received(n_recv));
         return;
     }
-    /* phase 3, 3c: the owners' answers come home, back to row order, expand */
-    SCK(route_return(g, r, 8));
-    int64_t m = 0;
-    SCK(adb_join_finish_routed(S.G, a->pv->d[g], a->pp->d[g], (int64_t)a->pv->n[g], a->swapped, &m));
+    if (a->phase == 3) {                            /* 3c: the owners' answers come home, back to row order */
+        SCK(route_return(g, r, 8));
+        int64_t m = 0;
+        SCK(adb_join_finish_routed(S.G, a->pv->d[g], a->pp->d[g], (int64_t)a->pv->n[g], a->swapped, &m));
+        a->pairs[g] = (size_t)m;
+        return;
+    }
+    /* phase 4: expand into this context's share of the output */
+    const size_t m = a->pairs[g];
     void *x = NULL, *y = NULL;
     SCK(adb_alloc(&x, 4 * (size_t)m));
     a->o1.d[g] = x;
@@ -3143,6 +3149,20 @@ static Result **join_sharded(Result *v1, Result *p1, Result *v2, Result *p2, int
         }
     }
     if (run_routed(join_shard, &job, &job.phase, &job.err)) goto fail;
+    {
+        /* the one-context join's bound (join_count, engine.cu) on the whole result, before any
+         * output is allocated: every context's share can stay below 2^31 while their sum does not */
+        size_t total = 0;
+        for (int g = 0; g < S.G; ++g) total += job.pairs[g];
+        if (total >= ((size_t)1 << 31)) {
+            set_err("%s: join produces %zu pairs; the reference indexes its output with an int "
+                    "(query.c:657) so the result must stay below 2^31", what, total);
+            goto fail;
+        }
+    }
+    job.phase = 4;
+    run_shards(join_shard, &job);
+    if (shard_errs(&job.err)) goto fail;
     list_release(&a); list_release(&b); list_release(&c); list_release(&d);
     return hand_out_pair(&job.o1, &job.o2, st, what);
 fail:
